@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- agent-updates/s of the Double-DQN learn step (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3] [--dump-outputs DIR]
 
 A "step" is one learn sweep: every agent of the workload runs one ``learn()`` (sample B
 transitions from its ring, target + online forward, backward, Adam, target sync).
@@ -13,6 +13,8 @@ every rank holds the per-GPU workload.  The same JSON line carries, under "block
 BASELINE.json names: cfg3 strong-scaled (256 agents in total over the ranks), cfg4 (512 agents per GPU, batch 512)
 and cfg5 (one shared network, hidden 512, global batch 1024, gradient reduction over the ranks); "act" is measured
 on a working set larger than the L2.  One JSON line on stdout (rank 0).
+--dump-outputs DIR writes what the last timed learn sweep left to its caller as DIR/<name>.npy (learn_outputs); every
+input is seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -175,6 +177,33 @@ def synth_fill(grp, seed):
     grp.done_ring.copy_((torch.rand((n, c), device=grp.device, generator=gen) < 1 / 240).to(torch.uint8))
     grp.n_written.fill_(c + 777)
     grp.n_written_host[:] = c + 777
+
+
+DUMP_SAMPLE, DUMP_SEED, DUMP_LIMIT = 1 << 20, 0, 64 << 20
+
+
+def learn_outputs(grp, metrics):
+    """What a caller of AgentGroup.learn holds after the call: the metrics it returns ([G, 8] float32: loss, q mean, q std,
+    action histogram, learned flag) and the network state it updated (online and target weights, Adam moments).  Those
+    four are sampled at DUMP_SAMPLE positions drawn with DUMP_SEED from every network's parameters in AgentGroup.unpack's
+    (Keras) order, layout padding left out: the same positions for the same workload, whatever the parameter layout."""
+    logical = torch.cat([t.reshape(-1) for t in grp.unpack(torch.arange(grp.layout.stride, dtype=torch.float64))]).long()
+    per_net = logical.numel()
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(grp.n_nets * per_net, min(grp.n_nets * per_net, DUMP_SAMPLE), replace=False))
+    net, j = np.divmod(pick, per_net)
+    flat = (torch.as_tensor(net) * grp.layout.stride + logical[torch.as_tensor(j)]).to(grp.device)
+    out = {"metrics": metrics.cpu().numpy()}
+    for name, t in (("theta", grp.theta), ("theta_target", grp.theta_tgt), ("adam_m", grp.adam_m), ("adam_v", grp.adam_v)):
+        out[f"{name}_sample"] = t.reshape(-1)[flat].cpu().numpy()
+    return out
+
+
+def dump_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def _events(n):
@@ -568,11 +597,13 @@ def run_ours(args):
     e0, e1 = _events(2)
     e0.record(stream)
     for i in range(K):
-        grp.learn(draws[W + i])
+        metrics = grp.learn(draws[W + i])
     e1.record(stream)
     _barrier(world)
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:                        # before anything below moves the weights on
+        dump_outputs(args.dump_outputs, learn_outputs(grp, metrics))
 
     # ---- per-kernel durations: same sweep, one stage per call, events in between ----------
     stage_ms = stage_times(grp, draws[W:], K)
@@ -766,7 +797,13 @@ def main():
     ap.add_argument("--blocks", default="all", help="all | none | comma list of act,cfg2,strong_cfg3,cfg4,cfg5")
     ap.add_argument("--block-steps", type=int, default=30)
     ap.add_argument("--cpu-budget", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed learn sweep (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -3,6 +3,8 @@ declares, and its argument validation / layout helpers work without a GPU."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -50,9 +52,11 @@ def test_bad_dims_are_rejected_with_a_message(lib, field, value):
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from dmdqn_b200.group import AgentGroup
-    with pytest.raises(N.NativeError, match="no CPU fallback"):
-        AgentGroup(2, {"nn_layers": [64, 64]})
+    """Without a CUDA device AgentGroup refuses to start.  A child process with every device hidden makes the check
+    the same on a machine with a GPU."""
+    code = ("from dmdqn_b200 import _native as N\nfrom dmdqn_b200.group import AgentGroup\n"
+            "try:\n    AgentGroup(2, {'nn_layers': [64, 64]})\nexcept N.NativeError as exc:\n    print(exc)\n")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT, timeout=600,
+                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 0, out.stderr[-500:]
+    assert "no CPU fallback" in out.stdout, out.stdout
