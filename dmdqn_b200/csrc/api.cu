@@ -165,6 +165,25 @@ static int check_learn_args(const dmdqn_hparams* hp, const dmdqn_replay* replay,
     return DMDQN_OK;
 }
 
+// Validation, the sample kernel (when `stages` has it) and the learn kernels of one step.  grads != NULL: K4b stores
+// dL/dtheta there instead of applying Adam, with the loss mean over global_batch.
+static int run_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay, const dmdqn_nets* nets,
+                     const void* draws, const uint8_t* learn_mask, float* metrics_out, void* workspace,
+                     size_t workspace_bytes, int32_t stages, float* grads, int32_t global_batch, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    rc = check_learn_args(hp, replay, nets, draws);
+    if (rc) return rc;
+    if (grads) DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    if (stages & DMDQN_STAGE_SAMPLE) {
+        rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, (cudaStream_t)stream);
+        if (rc) return rc;
+    }
+    return launch_learn(*dims, *hp, *replay, *nets, metrics_out, (char*)workspace, w, stages, grads, global_batch,
+                        (cudaStream_t)stream);
+}
+
 int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                  const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t advance_step,
                  void* workspace, size_t workspace_bytes, void* stream) {
@@ -192,24 +211,15 @@ int dmdqn_gather(const dmdqn_dims* dims, const dmdqn_replay* replay, const void*
 int dmdqn_learn_stages(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                        const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, float* metrics_out,
                        void* workspace, size_t workspace_bytes, int32_t stages, void* stream) {
-    Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
-    if (rc) return rc;
-    rc = check_learn_args(hp, replay, nets, draws);
-    if (rc) return rc;
-    if (stages & DMDQN_STAGE_SAMPLE) {
-        rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return launch_learn(*dims, *hp, *replay, *nets, metrics_out, (char*)workspace, w, stages, nullptr, 0, nullptr,
-                        (cudaStream_t)stream);
+    return run_learn(dims, hp, replay, nets, draws, learn_mask, metrics_out, workspace, workspace_bytes, stages, nullptr, 0,
+                     stream);
 }
 
 int dmdqn_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                 const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, float* metrics_out,
                 void* workspace, size_t workspace_bytes, void* stream) {
-    return dmdqn_learn_stages(dims, hp, replay, nets, draws, learn_mask, metrics_out, workspace, workspace_bytes,
-                              DMDQN_STAGE_SAMPLE | DMDQN_STAGE_TARGET | DMDQN_STAGE_ONLINE | DMDQN_STAGE_WGRAD, stream);
+    return run_learn(dims, hp, replay, nets, draws, learn_mask, metrics_out, workspace, workspace_bytes, kAllStages, nullptr,
+                     0, stream);
 }
 
 int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
@@ -237,18 +247,9 @@ int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn
 int dmdqn_learn_grads(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                       const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
                       float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream) {
-    Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
-    if (rc) return rc;
-    rc = check_learn_args(hp, replay, nets, draws);
-    if (rc) return rc;
     DMDQN_CHECK_ARG(grads_out != nullptr, "grads_out is NULL");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
-    rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, (cudaStream_t)stream);
-    if (rc) return rc;
-    return launch_learn(*dims, *hp, *replay, *nets, metrics_out, (char*)workspace, w,
-                        DMDQN_STAGE_SAMPLE | DMDQN_STAGE_TARGET | DMDQN_STAGE_ONLINE | DMDQN_STAGE_WGRAD, grads_out, global_batch, nullptr,
-                        (cudaStream_t)stream);
+    return run_learn(dims, hp, replay, nets, draws, learn_mask, metrics_out, workspace, workspace_bytes, kAllStages,
+                     grads_out, global_batch, stream);
 }
 
 int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const float* grads,
@@ -258,8 +259,7 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     if (rc) return rc;
     DMDQN_CHECK_ARG(hp && nets && nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && grads,
                     "adam_apply: NULL argument");
-    dmdqn_replay none = {};
-    return launch_learn(*dims, *hp, none, *nets, nullptr, (char*)workspace, w, 0, nullptr, 0, grads, (cudaStream_t)stream);
+    return launch_adam_apply(*dims, *hp, *nets, grads, (char*)workspace, w, (cudaStream_t)stream);
 }
 
 int dmdqn_allreduce_adam(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_peers* peers,

@@ -59,13 +59,14 @@ inline int row_tiles(int batch, int bm) { return (batch + bm - 1) / bm; }
 
 // Workspace carve-up (device scratch of sample/learn), offsets in bytes, 256-aligned.
 struct Workspace {
-    size_t rows, r_hat, act_b, done_b, active, step_t, y, gcoef, q_all, q_next, tq_all;
+    size_t rows, r_hat, act_b, done_b, active, y, q_all, q_next, tq_all;
     size_t h1, dh1, dh2;              // [n_nets][B][H] floats each ([H][B] per network on the tcgen05 path)
-    size_t tc_error;                  // int: set by a tcgen05 kernel whose mbarrier wait timed out
+    size_t tc_error;                  // int: set by a tcgen05 kernel whose mbarrier wait timed out, or by K5 on a peer timeout
     size_t mask2;                     // tcgen05 path: relu'(h2) bits, uint32 [n_nets][B][H/32]
     size_t ga;                        // tcgen05 path: float2 [n_nets][B] {dL/dq of the taken action, action bits}
     size_t w3_copy;                   // tcgen05 path: W3 as K4a saw it, [n_nets][H][4] (K4b rebuilds dh2 while W3 is being updated)
-    size_t adam_sc;                   // [n_nets] float4 {alpha_t, eps_eff, sync mode bits, -}: written by the sample kernel
+    size_t adam_sc;                   // [n_nets] float4 {alpha_t, eps_eff, sync mode bits, -}: the step's Adam scalars, written
+                                      // by the sample kernel for the active networks, read by every Adam kernel (adam_step)
     size_t part_loss;                 // [n_nets][T][8]
     size_t part_b3;                   // [n_nets][T][4]
     size_t part_w3;                   // [n_nets][T][H][4]
@@ -73,7 +74,8 @@ struct Workspace {
     size_t sync;                      // tcgen05 path, int32: [0] K4b work counter, [1..3] spare, [4 ..] k4a_done[n_nets], then
                                       // k3_done[n_nets][T]; zeroed by the sample kernel (dataflow flags between the learn kernels)
     size_t total;
-    int tiles;
+    int tiles;                        // T: row tiles per network of the FFMA kernels (Tile<H>::BM rows); the tcgen05 path's
+                                      // 128-row tiles are fewer, so its partials fit the same arrays
 };
 inline int tile_bm(int h) { return h >= 512 ? 32 : 64; }
 inline Workspace make_workspace(const dmdqn_dims& d) {
@@ -88,9 +90,7 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
     w.act_b = take(nb * 4);
     w.done_b = take(nb * 4);
     w.active = take((size_t)d.n_nets * 4);
-    w.step_t = take((size_t)d.n_nets * 4);
     w.y = take(nb * 4);
-    w.gcoef = take(nb * 4);
     w.q_all = take(nb * 16);
     w.q_next = take(nb * 16);
     w.tq_all = take(nb * 16);
@@ -113,6 +113,75 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
 }
 
 int validate_dims(const dmdqn_dims* d);
+
+constexpr int kAllStages = DMDQN_STAGE_SAMPLE | DMDQN_STAGE_TARGET | DMDQN_STAGE_ONLINE | DMDQN_STAGE_WGRAD;   // dmdqn_learn
+
+// Arguments of every learn kernel of both paths (learn.cu, learn_tc.cu) and of the Adam kernels that finish a
+// shared-parameter step; make_learn_args resolves the workspace pointers.  The tcgen05 launcher adds its own part:
+// tc_tiles, chain and the k4a_done / k3_done flag pointers.
+struct LearnArgs {
+    dmdqn_dims d;
+    Layout L;
+    dmdqn_replay rp;
+    dmdqn_nets nets;
+    float gamma;
+    int loss, double_dqn;
+    int loss_batch;                   // batch the loss mean runs over (== batch, or the global batch when ranks split it)
+    float one_m_b1, one_m_b2, tau;    // Adam constants of the call; the per-step scalars are in adam_sc
+    int ws_tiles;                     // Workspace::tiles: row tiles of the FFMA kernels, the per-network stride of k3_done
+    int tc_tiles;                     // tcgen05 path: 128-row tiles per network (its K3 / K4a items and part_* slots)
+    const int32_t *rows, *act_b, *active;
+    const float *r_hat, *done_b;
+    const float4* adam_sc;
+    float *y, *q_all, *q_next, *tq_all, *h1, *dh1, *dh2;
+    float *part_loss, *part_b3, *part_w3, *part_b2, *part_b1;
+    uint32_t* mask2;                  // relu'(h2) bits [n_nets][B][H/32]: the eight words of a batch row are adjacent
+    float2* ga;                       // [n_nets][B] {dL/dq of the taken action, action as int bits}: what K4b needs per row
+    float* w3_copy;                   // [n_nets][H][4]
+    int* error;                       // Workspace::tc_error
+    float* metrics;
+    float* grads;                     // non-NULL: K4b stores dL/dtheta here instead of applying Adam (shared parameters)
+    // Dataflow between the tcgen05 learn kernels of one dmdqn_learn call (`chain`: the sample kernel of the same call has
+    // reset the flags): K4a / K4b are programmatic dependent launches whose CTAs start on SMs the previous kernel has left
+    // and wait per (network, tile) / per network instead of for the whole previous grid.
+    int chain;
+    int *sched, *k4a_done, *k3_done;  // Workspace::sync: K4b work counter | K4a items finished per network | K3 items finished
+                                      // per (network, tile)
+};
+LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                          char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch);
+
+// Adam scalars of one network's step.  alpha_t, eps_eff and the sync mode are evaluated once per network by the sample
+// kernel into adam_sc; every Adam kernel loads them here.
+struct AdamStep {
+    float alpha, eps, one_m_b1, one_m_b2, tau;
+    int sync;                         // 0 none, 1 hard copy, 2 Polyak
+};
+__device__ __forceinline__ AdamStep adam_step(const LearnArgs& A, int g) {
+    const float4 sc = __ldg(A.adam_sc + g);
+    return {sc.x, sc.y, A.one_m_b1, A.one_m_b2, A.tau, __float_as_int(sc.z)};
+}
+
+// Metrics row of network g (include/dmdqn_b200.h) from its `tiles` loss partials, summed in tile order in float64.
+// `ld` reads one partial: the tcgen05 K4b reads through L2 (K4a CTAs of the same chain may have written them while it ran).
+// The loop stays rolled: it runs on one thread per network, and unrolled it cost the tcgen05 K4b spill bytes.
+template <typename Load>
+__device__ __forceinline__ void finish_metrics(const LearnArgs& A, int g, int tiles, Load ld) {
+    double ls = 0, qs = 0, qq = 0, hist[4] = {0, 0, 0, 0};
+#pragma unroll 1
+    for (int r = 0; r < tiles; ++r) {
+        const float* pl = A.part_loss + ((size_t)g * tiles + r) * 8;
+        ls += ld(pl); qs += ld(pl + 1); qq += ld(pl + 2);
+        for (int a = 0; a < 4; ++a) hist[a] += ld(pl + 3 + a);
+    }
+    const double cnt = (double)A.d.batch * A.d.n_actions, mean = qs / cnt, var = fmax(qq / cnt - mean * mean, 0.0);
+    float* m = A.metrics + g * DMDQN_METRICS_STRIDE;
+    m[0] = (float)(ls / A.loss_batch);                // batch-mean loss (dqn_agent.py:352)
+    m[1] = (float)mean;
+    m[2] = (float)sqrt(var);
+    for (int a = 0; a < 4; ++a) m[3 + a] = (float)hist[a];
+    m[7] = 1.f;
+}
 
 // Per-DEVICE launch state.  The dynamic shared-memory opt-in (cudaFuncSetAttribute) and the SM count belong to a
 // device, not to the process: a host that drives several GPUs from one process (one AgentGroup per device) must
@@ -144,12 +213,11 @@ int launch_gather(const dmdqn_dims& d, const dmdqn_replay& rp, const char* ws, c
                   float* states, int32_t* actions, float* rewards, float* next_states, float* dones,
                   int32_t* active_out, cudaStream_t s);
 int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                 float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch,
-                 const float* apply_grads, cudaStream_t s);
+                 float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch, cudaStream_t s);
 bool tc_supported(const dmdqn_dims& d);
-int launch_learn_tc(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                    float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch,
-                    cudaStream_t s);
+int launch_learn_tc(const LearnArgs& A, int precision, int stages, cudaStream_t s);
+int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads, char* ws,
+                      const Workspace& w, cudaStream_t s);
 int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau,
                        cudaStream_t s);
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,

@@ -217,24 +217,6 @@ struct Smem {
     }
 };
 
-struct LearnArgs {
-    dmdqn_dims d;
-    Layout L;
-    dmdqn_replay rp;
-    dmdqn_nets nets;
-    float gamma;
-    int loss, double_dqn, adam_form, freq;
-    double lr, beta1, beta2, adam_eps, tau;
-    int tiles;
-    const int32_t *rows, *act_b, *active, *step_t;
-    const float *r_hat, *done_b;
-    float *y, *q_all, *q_next, *tq_all, *h1, *dh1, *dh2;
-    float *part_loss, *part_b3, *part_w3, *part_b2, *part_b1;
-    float* metrics;
-    float* grads;       // non-NULL: K4b stores dL/dtheta here instead of applying Adam (shared parameters, N>1 ranks)
-    int loss_batch;     // batch the loss mean runs over (== batch, or the global batch when ranks split it)
-};
-
 // ------------------------------------------------------------------------------------------
 // K3: TD targets.
 // ------------------------------------------------------------------------------------------
@@ -242,7 +224,7 @@ template <int H>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs A) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
-    const int g = blockIdx.x / A.tiles, rt = blockIdx.x % A.tiles;
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
     if (!A.active[g]) return;
     const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM;
     Smem<H> S(smem, Dp);
@@ -290,7 +272,7 @@ template <int H>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs A) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
-    const int g = blockIdx.x / A.tiles, rt = blockIdx.x % A.tiles;
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
     if (!A.active[g]) return;
     const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM;
     Smem<H> S(smem, Dp);
@@ -332,7 +314,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
         terms[i] = term;
     }
     __syncthreads();
-    const size_t pt = (size_t)g * A.tiles + rt;      // partial slot of this (network, row tile)
+    const size_t pt = (size_t)g * A.ws_tiles + rt;   // partial slot of this (network, row tile)
     if (threadIdx.x == 0) {                          // per-tile loss / metric / db3 partials, rows in order
         float ls = 0.f, qsum = 0.f, qsq = 0.f, hist[4] = {0.f, 0.f, 0.f, 0.f}, db3[4] = {0.f, 0.f, 0.f, 0.f};
         for (int i = 0; i < T::BM && r0 + i < B; ++i) {
@@ -406,28 +388,9 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
 // ------------------------------------------------------------------------------------------
 // K4b: weight gradients with Adam + target sync in the epilogue.
 // ------------------------------------------------------------------------------------------
-struct AdamCoef {
-    float alpha, eps, one_m_b1, one_m_b2, tau;
-    int sync;  // 0 none, 1 hard copy, 2 Polyak
-};
-
-__device__ __forceinline__ AdamCoef adam_coef(const LearnArgs& A, int t) {
-    AdamCoef k;
-    // alpha_t = lr * sqrt(1 - b2^t) / (1 - b1^t), float64 then rounded (oracle/dqn.py adam_scalars)
-    const double bc1 = 1.0 - pow(A.beta1, (double)t);
-    const double bc2 = 1.0 - pow(A.beta2, (double)t);
-    k.alpha = (float)(A.lr * sqrt(bc2) / bc1);
-    k.eps = (float)(A.adam_form == DMDQN_ADAM_KERAS ? A.adam_eps : A.adam_eps * sqrt(bc2));
-    k.one_m_b1 = (float)(1.0 - A.beta1);
-    k.one_m_b2 = (float)(1.0 - A.beta2);
-    k.tau = (float)A.tau;
-    k.sync = A.tau >= 0.0 ? 2 : (t % A.freq == 0 ? 1 : 0);   // counter already incremented (:359,376)
-    return k;
-}
-
 // keras 3.9.2 Adam.update_step op order: m += (g-m)(1-b1); v += (g*g-v)(1-b2);
 // theta -= (m*alpha)/(sqrt(v)+eps); then theta_tgt per the sync mode.
-__device__ __forceinline__ void adam_elem(const AdamCoef& k, float g, float& th, float& m, float& v, float& tg) {
+__device__ __forceinline__ void adam_elem(const AdamStep& k, float g, float& th, float& m, float& v, float& tg) {
     m = m + (g - m) * k.one_m_b1;
     v = v + (g * g - v) * k.one_m_b2;
     th = th - (m * k.alpha) / (sqrtf(v) + k.eps);
@@ -435,7 +398,7 @@ __device__ __forceinline__ void adam_elem(const AdamCoef& k, float g, float& th,
     else if (k.sync == 2) tg = k.tau * th + (1.0f - k.tau) * tg;
 }
 
-__device__ __forceinline__ void adam_vec4(const AdamCoef& k, const float* g, float* th, float* m, float* v,
+__device__ __forceinline__ void adam_vec4(const AdamStep& k, const float* g, float* th, float* m, float* v,
                                           float* tg) {
     float4 t4 = *reinterpret_cast<float4*>(th), m4 = *reinterpret_cast<float4*>(m);
     float4 v4 = *reinterpret_cast<float4*>(v);
@@ -474,22 +437,22 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
             if (threadIdx.x < DMDQN_METRICS_STRIDE && A.metrics) A.metrics[g * DMDQN_METRICS_STRIDE + threadIdx.x] = 0.f;
             return;
         }
-        const AdamCoef k = adam_coef(A, A.step_t[g]);
-        const size_t p0 = (size_t)g * A.tiles;
+        const AdamStep k = adam_step(A, g);
+        const size_t p0 = (size_t)g * A.ws_tiles;
         for (int e = threadIdx.x; e < 6 * H + 4; e += T::NT) {
             float gsum = 0.f;
             int64_t off;
             if (e < H) {                                   // b1
-                for (int r = 0; r < A.tiles; ++r) gsum += A.part_b1[(p0 + r) * H + e];
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b1[(p0 + r) * H + e];
                 off = A.L.b1 + e;
             } else if (e < 2 * H) {                        // b2
-                for (int r = 0; r < A.tiles; ++r) gsum += A.part_b2[(p0 + r) * H + (e - H)];
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b2[(p0 + r) * H + (e - H)];
                 off = A.L.b2 + (e - H);
             } else if (e < 6 * H) {                        // W3[j][a]
-                for (int r = 0; r < A.tiles; ++r) gsum += A.part_w3[(p0 + r) * H * 4 + (e - 2 * H)];
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_w3[(p0 + r) * H * 4 + (e - 2 * H)];
                 off = A.L.w3 + (e - 2 * H);
             } else {                                       // b3
-                for (int r = 0; r < A.tiles; ++r) gsum += A.part_b3[(p0 + r) * 4 + (e - 6 * H)];
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b3[(p0 + r) * 4 + (e - 6 * H)];
                 off = A.L.b3 + (e - 6 * H);
             }
             if (A.grads) {
@@ -500,22 +463,7 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
             adam_elem(k, gsum, th[off], am[off], av[off], tgv);
             if (k.sync) tg[off] = tgv;
         }
-        if (threadIdx.x == 0 && A.metrics) {
-            double ls = 0, qs = 0, qq = 0, hist[4] = {0, 0, 0, 0};
-            for (int r = 0; r < A.tiles; ++r) {
-                const float* pl = A.part_loss + (p0 + r) * 8;
-                ls += pl[0]; qs += pl[1]; qq += pl[2];
-                for (int a = 0; a < 4; ++a) hist[a] += pl[3 + a];
-            }
-            const double cnt = (double)B * A.d.n_actions;
-            const double mean = qs / cnt, var = fmax(qq / cnt - mean * mean, 0.0);
-            float* m = A.metrics + g * DMDQN_METRICS_STRIDE;
-            m[0] = (float)(ls / A.loss_batch);             // batch-mean loss (:352)
-            m[1] = (float)mean;
-            m[2] = (float)sqrt(var);
-            for (int a = 0; a < 4; ++a) m[3 + a] = (float)hist[a];
-            m[7] = 1.f;
-        }
+        if (threadIdx.x == 0 && A.metrics) finish_metrics(A, g, A.ws_tiles, [](const float* p) { return *p; });
         return;
     }
     if (!A.active[g]) return;
@@ -582,7 +530,7 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
         buf ^= 1;
     }
 
-    const AdamCoef k = adam_coef(A, A.step_t[g]);
+    const AdamStep k = adam_step(A, g);
     const int64_t wbase = is_w2 ? A.L.w2 : A.L.w1;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -624,7 +572,7 @@ __global__ void sync_target_kernel(int64_t stride, const float* __restrict__ the
 __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ grads) {
     const int g = blockIdx.y;
     if (!A.active[g]) return;
-    const AdamCoef k = adam_coef(A, A.step_t[g]);
+    const AdamStep k = adam_step(A, g);
     const size_t base = (size_t)g * A.L.stride;
     const int64_t n4 = (A.L.b3 + 4) / 4;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
@@ -649,7 +597,7 @@ __device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p) {
 }
 __global__ void __launch_bounds__(256)
 peer_reduce_adam_kernel(const LearnArgs A, const dmdqn_peers P, const float* __restrict__ my_loss_src,
-                        float* __restrict__ loss_out, int* __restrict__ error) {
+                        float* __restrict__ loss_out) {
     __shared__ int timed_out;
     const int b = blockIdx.x, tid = threadIdx.x;
     if (tid == 0) timed_out = 0;
@@ -671,11 +619,11 @@ peer_reduce_adam_kernel(const LearnArgs A, const dmdqn_peers P, const float* __r
     }
     __syncthreads();
     if (timed_out) {
-        if (tid == 0) atomicExch(error, DMDQN_PEER_TIMEOUT);
+        if (tid == 0) atomicExch(A.error, DMDQN_PEER_TIMEOUT);
         return;
     }
     if (!A.active[0]) return;                       // (the learn decision is collective: every rank or none)
-    const AdamCoef k = adam_coef(A, A.step_t[0]);
+    const AdamStep k = adam_step(A, 0);
     const int64_t n4 = (A.L.b3 + 4) / 4;
     for (int64_t i = b * (int64_t)blockDim.x + tid; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         float4 v[DMDQN_MAX_PEERS];
@@ -705,7 +653,7 @@ int launch_learn_h(const LearnArgs& A, int stages, cudaStream_t s) {
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(target_kernel<H>), smem, cfg_t)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(online_kernel<H>), smem, cfg_o)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(wgrad_adam_kernel<H>), smem_w, cfg_w)) return rc;
-    const int grid = A.d.n_nets * A.tiles;
+    const int grid = A.d.n_nets * A.ws_tiles;
     if (stages & DMDQN_STAGE_TARGET) {
         target_kernel<H><<<grid, T::NT, smem, s>>>(A);
         DMDQN_CUDA(cudaGetLastError());
@@ -724,18 +672,9 @@ int launch_learn_h(const LearnArgs& A, int stages, cudaStream_t s) {
 
 }  // namespace
 
-int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                 float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch,
-                 const float* apply_grads, cudaStream_t s) {
-    if (hp.precision != DMDQN_PRECISION_FP32 && !apply_grads) {
-        if (!tc_supported(d)) {
-            set_error("precision=%d (tcgen05) needs hidden=256 and obs_stride in {32,64,96}; got hidden=%d obs_stride=%d",
-                      hp.precision, d.hidden, d.obs_stride);
-            return DMDQN_ERR_ARG;
-        }
-        return launch_learn_tc(d, hp, rp, nets, metrics, ws, w, stages, grads, loss_batch, s);
-    }
-    LearnArgs A;
+LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                          char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch) {
+    LearnArgs A = {};
     A.d = d;
     A.L = make_layout(d.obs_stride, d.hidden);
     A.rp = rp;
@@ -743,16 +682,17 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
     A.gamma = (float)hp.gamma;
     A.loss = hp.loss;
     A.double_dqn = hp.double_dqn;
-    A.adam_form = hp.adam_form;
-    A.freq = hp.target_update_frequency > 0 ? hp.target_update_frequency : 1;
-    A.lr = hp.learning_rate; A.beta1 = hp.beta1; A.beta2 = hp.beta2; A.adam_eps = hp.adam_eps; A.tau = hp.tau;
-    A.tiles = w.tiles;
+    A.loss_batch = loss_batch > 0 ? loss_batch : d.batch;
+    A.one_m_b1 = (float)(1.0 - hp.beta1);
+    A.one_m_b2 = (float)(1.0 - hp.beta2);
+    A.tau = (float)hp.tau;
+    A.ws_tiles = w.tiles;
     A.rows = reinterpret_cast<const int32_t*>(ws + w.rows);
     A.act_b = reinterpret_cast<const int32_t*>(ws + w.act_b);
     A.active = reinterpret_cast<const int32_t*>(ws + w.active);
-    A.step_t = reinterpret_cast<const int32_t*>(ws + w.step_t);
     A.r_hat = reinterpret_cast<const float*>(ws + w.r_hat);
     A.done_b = reinterpret_cast<const float*>(ws + w.done_b);
+    A.adam_sc = reinterpret_cast<const float4*>(ws + w.adam_sc);
     A.y = reinterpret_cast<float*>(ws + w.y);
     A.q_all = reinterpret_cast<float*>(ws + w.q_all);
     A.q_next = reinterpret_cast<float*>(ws + w.q_next);
@@ -765,14 +705,26 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
     A.part_w3 = reinterpret_cast<float*>(ws + w.part_w3);
     A.part_b2 = reinterpret_cast<float*>(ws + w.part_b2);
     A.part_b1 = reinterpret_cast<float*>(ws + w.part_b1);
+    A.mask2 = reinterpret_cast<uint32_t*>(ws + w.mask2);
+    A.ga = reinterpret_cast<float2*>(ws + w.ga);
+    A.w3_copy = reinterpret_cast<float*>(ws + w.w3_copy);
+    A.error = reinterpret_cast<int*>(ws + w.tc_error);
+    A.sched = reinterpret_cast<int*>(ws + w.sync);
     A.metrics = metrics;
     A.grads = grads;
-    A.loss_batch = loss_batch > 0 ? loss_batch : d.batch;
-    if (apply_grads) {
-        dim3 grid(64, d.n_nets);
-        adam_apply_kernel<<<grid, 256, 0, s>>>(A, apply_grads);
-        DMDQN_CUDA(cudaGetLastError());
-        return DMDQN_OK;
+    return A;
+}
+
+int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                 float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch, cudaStream_t s) {
+    const LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    if (hp.precision != DMDQN_PRECISION_FP32) {
+        if (!tc_supported(d)) {
+            set_error("precision=%d (tcgen05) needs hidden=256 and obs_stride in {32,64,96}; got hidden=%d obs_stride=%d",
+                      hp.precision, d.hidden, d.obs_stride);
+            return DMDQN_ERR_ARG;
+        }
+        return launch_learn_tc(A, hp.precision, stages, s);
     }
     switch (d.hidden) {
         case 64: return launch_learn_h<64>(A, stages, s);
@@ -784,19 +736,18 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
     return DMDQN_ERR_ARG;
 }
 
+int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads, char* ws,
+                      const Workspace& w, cudaStream_t s) {
+    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,
                      const float* my_loss_src, float* loss_out, char* ws, const Workspace& w, cudaStream_t s) {
-    LearnArgs A = {};
-    A.d = d;
-    A.L = make_layout(d.obs_stride, d.hidden);
-    A.nets = nets;
-    A.adam_form = hp.adam_form;
-    A.freq = hp.target_update_frequency > 0 ? hp.target_update_frequency : 1;
-    A.lr = hp.learning_rate; A.beta1 = hp.beta1; A.beta2 = hp.beta2; A.adam_eps = hp.adam_eps; A.tau = hp.tau;
-    A.active = reinterpret_cast<const int32_t*>(ws + w.active);
-    A.step_t = reinterpret_cast<const int32_t*>(ws + w.step_t);
-    peer_reduce_adam_kernel<<<DMDQN_PEER_BLOCKS, 256, 0, s>>>(A, peers, my_loss_src, loss_out,
-                                                              reinterpret_cast<int*>(ws + w.tc_error));
+    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    peer_reduce_adam_kernel<<<DMDQN_PEER_BLOCKS, 256, 0, s>>>(A, peers, my_loss_src, loss_out);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

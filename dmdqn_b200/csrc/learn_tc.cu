@@ -190,29 +190,6 @@ __device__ __forceinline__ uint32_t off_mn(int mn_total, int k, int mn) {
                       ((((mn & 31) >> 3) ^ (k & 3)) << 5) + ((mn & 7) << 2));
 }
 
-struct TcArgs {
-    dmdqn_dims d;
-    Layout L;
-    dmdqn_replay rp;
-    dmdqn_nets nets;
-    float gamma;
-    int loss, double_dqn, adam_form, freq, loss_batch, tiles;
-    double lr, beta1, beta2, adam_eps, tau;
-    const int32_t *rows, *act_b, *active, *step_t;
-    const float *r_hat, *done_b;
-    const float4* adam_sc;
-    uint32_t* mask2;              // relu'(h2) bits [n_nets][B][H/32]: the eight words of a batch row are adjacent
-    float2* ga;                   // [n_nets][B] {dL/dq of the taken action, action as int bits}: what K4b needs per row
-    float* w3_copy;               // [n_nets][H][4]
-    float *y, *gcoef, *q_all, *q_next, *tq_all, *h1, *dh1, *dh2, *part_loss, *part_b3, *part_w3, *part_b2, *metrics, *grads;
-    int* error;
-    // Dataflow between the learn kernels of one dmdqn_learn call (`chain`: the sample kernel of the same call has reset the
-    // flags): K4a / K4b are programmatic dependent launches whose CTAs start on SMs the previous kernel has left and wait
-    // per (network, tile) / per network instead of for the whole previous grid.
-    int chain, tiles_ws;
-    int *sched, *k4a_done, *k3_done;      // K4b work counter | K4a items finished per network | K3 items finished per (network, tile)
-};
-
 // Release / acquire on a global flag (gpu scope).  The producer calls flag_release after a CTA-wide barrier that follows
 // its last global store of the item; the consumer's bounded spin ends in an error flag, never in a hung GPU.
 __device__ __forceinline__ void flag_release_add(int* f) {
@@ -649,20 +626,20 @@ __device__ __forceinline__ void tc_epilogue(uint32_t tmem) {
 // 148 SMs); K4a combines them into the TD target of its rows (reference :342-347).  A CTA walks the items
 // blockIdx.x, + gridDim.x, ... of active networks; every role runs the same walk.
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ int k3_next(const TcArgs& A, int q, int n_items) {
-    while (q < n_items && !A.active[(q >> 1) / A.tiles]) q += gridDim.x;
+__device__ __forceinline__ int k3_next(const LearnArgs& A, int q, int n_items) {
+    while (q < n_items && !A.active[(q >> 1) / A.tc_tiles]) q += gridDim.x;
     return q;
 }
 
 template <int PASSES>
-__global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, const __grid_constant__ CUtensorMap tm_w1,
+__global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, const __grid_constant__ CUtensorMap tm_w1,
                                                             const __grid_constant__ CUtensorMap tm_w2,
                                                             const __grid_constant__ CUtensorMap tm_w1t,
                                                             const __grid_constant__ CUtensorMap tm_w2t) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const int B = A.d.batch, Dp = A.d.obs_stride;
-    const int n_items = 2 * A.d.n_nets * A.tiles;
+    const int n_items = 2 * A.d.n_nets * A.tc_tiles;
     const int warp = threadIdx.x >> 5;
     KT_BEGIN;
     const uint32_t tmem = tc_prologue(sbase);
@@ -682,7 +659,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
             int prev = -1;
             for (int q = k3_next(A, blockIdx.x, n_items); q < n_items; q = k3_next(A, q + gridDim.x, n_items)) {
                 ok = mma_gemm<PASSES, false>(sbase, tmem, sbase + Fwd::R, sbase + Fwd::XLO, 0, Dp, ring, ok);
-                if (prev >= 0) flag_release_add(A.k3_done + (size_t)((prev >> 1) / A.tiles) * A.tiles_ws + (prev >> 1) % A.tiles);
+                if (prev >= 0) flag_release_add(A.k3_done + (size_t)((prev >> 1) / A.tc_tiles) * A.ws_tiles + (prev >> 1) % A.tc_tiles);
                 prev = q;
                 ok = mma_gemm<PASSES, false>(sbase, tmem, sbase + Fwd::R, 0, tmem + 256u, H, ring, ok);
             }
@@ -692,10 +669,10 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
       } else if (warp == W_TMA) {
         if ((threadIdx.x & 31) == 0) {
             for (int q = k3_next(A, blockIdx.x, n_items); q < n_items;) {
-                const int g = (q >> 1) / A.tiles;
+                const int g = (q >> 1) / A.tc_tiles;
                 const float* P = ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride;
                 const int qn = k3_next(A, q + gridDim.x, n_items);
-                const float* Pn = qn < n_items ? ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)((qn >> 1) / A.tiles) * A.L.stride + A.L.w1 : nullptr;
+                const float* Pn = qn < n_items ? ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)((qn >> 1) / A.tc_tiles) * A.L.stride + A.L.w1 : nullptr;
                 ok = tma_fwd(sbase, (q & 1) ? &tm_w1t : &tm_w1, g, P + A.L.w1, Dp, ring, ok, P + A.L.w2);
                 ok = tma_fwd(sbase, (q & 1) ? &tm_w2t : &tm_w2, g, P + A.L.w2, H, ring, ok, Pn);
                 q = qn;
@@ -717,13 +694,13 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
         XGather<PASSES> xg;
         int q = k3_next(A, blockIdx.x, n_items);
         if (q < n_items) {
-            const int g = (q >> 1) / A.tiles, rt = (q >> 1) % A.tiles;
+            const int g = (q >> 1) / A.tc_tiles, rt = (q >> 1) % A.tc_tiles;
             xg.begin(A.rp.next_obs, A.rows + (size_t)g * B, rt * BM, B, Dp, ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride, A.L);
         }
         int q_last = -1;                                       // the last item is published here, the others by the MMA lane
         while (q < n_items) {
             const int item = q >> 1, pass = q & 1;            // 0: online(s')  1: target(s')
-            const int g = item / A.tiles, rt = item % A.tiles, r0 = rt * BM;
+            const int g = item / A.tc_tiles, rt = item % A.tc_tiles, r0 = rt * BM;
             const float* P = (pass == 0 ? A.nets.theta : A.nets.theta_tgt) + (size_t)g * A.L.stride;
             TS_DECL;
             TS();
@@ -740,7 +717,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
             TS();
             const int qn = k3_next(A, q + gridDim.x, n_items);
             if (qn < n_items) {                                // the next tile's rows travel while layer 2 runs
-                const int gn = (qn >> 1) / A.tiles, rtn = (qn >> 1) % A.tiles;
+                const int gn = (qn >> 1) / A.tc_tiles, rtn = (qn >> 1) % A.tc_tiles;
                 xg.begin(A.rp.next_obs, A.rows + (size_t)gn * B, rtn * BM, B, Dp,
                          ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)gn * A.L.stride, A.L);
             }
@@ -759,7 +736,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
             q = qn;
         }
         epi_sync();
-        if (q_last >= 0 && threadIdx.x == 0) flag_release_add(A.k3_done + (size_t)((q_last >> 1) / A.tiles) * A.tiles_ws + (q_last >> 1) % A.tiles);
+        if (q_last >= 0 && threadIdx.x == 0) flag_release_add(A.k3_done + (size_t)((q_last >> 1) / A.tc_tiles) * A.ws_tiles + (q_last >> 1) % A.tc_tiles);
         if (!ok && threadIdx.x == 0) atomicExch(A.error, 3);
         KT_END("K3");
     }
@@ -769,20 +746,20 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const TcArgs A, cons
 // ------------------------------------------------------------------------------------------
 // K4a: item = (network, 128-row tile).
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ int k4_next(const TcArgs& A, int q, int n_items) {
-    while (q < n_items && !A.active[q / A.tiles]) q += gridDim.x;
+__device__ __forceinline__ int k4_next(const LearnArgs& A, int q, int n_items) {
+    while (q < n_items && !A.active[q / A.tc_tiles]) q += gridDim.x;
     return q;
 }
 
 template <int PASSES>
-__global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, const __grid_constant__ CUtensorMap tmap_w2,
+__global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, const __grid_constant__ CUtensorMap tmap_w2,
                                                             const __grid_constant__ CUtensorMap tm_w1,
                                                             const __grid_constant__ CUtensorMap tm_w2) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
     float* sf = reinterpret_cast<float*>(__cvta_shared_to_generic((size_t)sbase));
     const int B = A.d.batch, Dp = A.d.obs_stride;
-    const int n_items = A.d.n_nets * A.tiles;
+    const int n_items = A.d.n_nets * A.tc_tiles;
     const int warp = threadIdx.x >> 5;
     KT_BEGIN;
     const uint32_t tmem = tc_prologue(sbase);
@@ -799,7 +776,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
                 ok = mma_gemm<PASSES, false>(sbase, tmem, sbase + Fwd::R, 0, tmem + 256u, H, ring, ok);
                 // (the epilogue issues the second half of an item's dh1^T stores after it has published the NEXT item's layer-1
                 // operand, so the previous item is complete only once this item's LAYER-2 operand has been published)
-                if (prev >= 0) flag_release_add(A.k4a_done + prev / A.tiles);
+                if (prev >= 0) flag_release_add(A.k4a_done + prev / A.tc_tiles);
                 prev = q;
                 ok = mma_gemm<PASSES, true>(sbase, tmem, sbase + Fwd::R, 0, tmem + 256u, H, ring, ok);
             }
@@ -809,12 +786,12 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
       } else if (warp == W_TMA) {
         if ((threadIdx.x & 31) == 0) {
             for (int q = k4_next(A, blockIdx.x, n_items); q < n_items; q = k4_next(A, q + gridDim.x, n_items)) {
-                const int g = q / A.tiles;
+                const int g = q / A.tc_tiles;
                 // K3 may still be running on other SMs: both halves of this tile's TD-target inputs must have been published
-                if (A.chain && ok) ok = flag_acquire_ge(A.k3_done + (size_t)g * A.tiles_ws + q % A.tiles, 2);
+                if (A.chain && ok) ok = flag_acquire_ge(A.k3_done + (size_t)g * A.ws_tiles + q % A.tc_tiles, 2);
                 const float* P = A.nets.theta + (size_t)g * A.L.stride;
                 const int qn = k4_next(A, q + gridDim.x, n_items);
-                const float* Pn = qn < n_items ? A.nets.theta + (size_t)(qn / A.tiles) * A.L.stride + A.L.w1 : nullptr;
+                const float* Pn = qn < n_items ? A.nets.theta + (size_t)(qn / A.tc_tiles) * A.L.stride + A.L.w1 : nullptr;
                 // one ring for all three GEMMs: a stage is reused as soon as its MMAs have retired, whatever GEMM they belong to
                 ok = tma_fwd(sbase, &tm_w1, g, P + A.L.w1, Dp, ring, ok, P + A.L.w2);
                 ok = tma_fwd(sbase, &tm_w2, g, P + A.L.w2, H, ring, ok, Pn);
@@ -837,10 +814,10 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
         const Epi e;
         XGather<PASSES> xg;
         int q = k4_next(A, blockIdx.x, n_items);
-        if (q < n_items) xg.begin(A.rp.obs, A.rows + (size_t)(q / A.tiles) * B, (q % A.tiles) * BM, B, Dp, A.nets.theta + (size_t)(q / A.tiles) * A.L.stride, A.L);
+        if (q < n_items) xg.begin(A.rp.obs, A.rows + (size_t)(q / A.tc_tiles) * B, (q % A.tc_tiles) * BM, B, Dp, A.nets.theta + (size_t)(q / A.tc_tiles) * A.L.stride, A.L);
         int q_last = -1;                                       // the last item is published here, the others by the MMA lane
         while (q < n_items) {
-            const int g = q / A.tiles, rt = q % A.tiles, r0 = rt * BM;
+            const int g = q / A.tc_tiles, rt = q % A.tc_tiles, r0 = rt * BM;
             const size_t sb = (size_t)g * B;
             const float* P = A.nets.theta + (size_t)g * A.L.stride;
             const int gr = r0 + e.row;
@@ -904,7 +881,6 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
                     gi = fminf(fmaxf(err, -1.0f), 1.0f) / (float)A.loss_batch;
                 }
                 if (e.part == 0) {
-                    A.gcoef[sb + gr] = gi;
                     A.ga[sb + gr] = make_float2(gi, __int_as_float(ai));
                     *reinterpret_cast<float4*>(A.q_all + (sb + gr) * 4) = make_float4(qv[0], qv[1], qv[2], qv[3]);
                 }
@@ -939,7 +915,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
             if (threadIdx.x < 11) {
                 const float* wp = rowf + 7 * BM + threadIdx.x;
                 const float tot = ((wp[0] + wp[11]) + wp[22]) + wp[33];
-                const size_t pt = (size_t)g * A.tiles + rt;
+                const size_t pt = (size_t)g * A.tc_tiles + rt;
                 if (threadIdx.x < 7) A.part_loss[pt * 8 + threadIdx.x] = tot;      // loss, q sum, q^2 sum, action histogram
                 else A.part_b3[pt * 4 + (threadIdx.x - 7)] = tot;
             }
@@ -995,7 +971,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
                 }
                 epi_sync();
                 if (rh == 0 && rg == 0) {
-                    const size_t pt = (size_t)g * A.tiles + rt;
+                    const size_t pt = (size_t)g * A.tc_tiles + rt;
                     float sb2[4];
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
@@ -1039,7 +1015,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
             TS();
             const int qn = k4_next(A, q + gridDim.x, n_items);
             if (qn < n_items)                                     // the next tile's rows travel while the backward GEMM runs
-                xg.begin(A.rp.obs, A.rows + (size_t)(qn / A.tiles) * B, (qn % A.tiles) * BM, B, Dp, A.nets.theta + (size_t)(qn / A.tiles) * A.L.stride, A.L);
+                xg.begin(A.rp.obs, A.rows + (size_t)(qn / A.tc_tiles) * B, (qn % A.tc_tiles) * BM, B, Dp, A.nets.theta + (size_t)(qn / A.tc_tiles) * A.L.stride, A.L);
             // dh1 = (dh2 W2^T) * relu'(h1)
             ok = wait_gemm(sbase, ring, ok);
             TS();
@@ -1072,7 +1048,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
             q = qn;
         }
         epi_sync();
-        if (q_last >= 0 && threadIdx.x == 0) flag_release_add(A.k4a_done + q_last / A.tiles);
+        if (q_last >= 0 && threadIdx.x == 0) flag_release_add(A.k4a_done + q_last / A.tc_tiles);
         if (!ok && threadIdx.x == 0) atomicExch(A.error, 4);
         KT_END("K4a");
     }
@@ -1082,24 +1058,9 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const TcArgs A, cons
 // ------------------------------------------------------------------------------------------
 // K4b
 // ------------------------------------------------------------------------------------------
-struct AdamK {
-    float alpha, eps, omb1, omb2, tau;
-    int sync;
-};
-__device__ __forceinline__ AdamK adam_k(const TcArgs& A, int g) {   // scalars prepared by the sample kernel
-    AdamK k;
-    const float4 sc = __ldg(A.adam_sc + g);
-    k.alpha = sc.x;
-    k.eps = sc.y;
-    k.sync = __float_as_int(sc.z);
-    k.omb1 = (float)(1.0 - A.beta1);
-    k.omb2 = (float)(1.0 - A.beta2);
-    k.tau = (float)A.tau;
-    return k;
-}
-__device__ __forceinline__ void adam1(const AdamK& k, float g, float& th, float& m, float& v, float& tg) {
-    m = m + (g - m) * k.omb1;
-    v = v + (g * g - v) * k.omb2;
+__device__ __forceinline__ void adam1(const AdamStep& k, float g, float& th, float& m, float& v, float& tg) {
+    m = m + (g - m) * k.one_m_b1;
+    v = v + (g * g - v) * k.one_m_b2;
     // MUFU square root and reciprocal (each within ~2 ulp): the quotient is a step of at most ~lr, so a few
     // ulp of it are far below one ulp of the weight it is subtracted from; the IEEE sequences cost ~60
     // dependent instructions per element and made the epilogue issue-bound
@@ -1111,9 +1072,9 @@ __device__ __forceinline__ void adam1(const AdamK& k, float g, float& th, float&
 }
 
 // Adam on one element without the target sync (the caller applies it per 16-byte group)
-__device__ __forceinline__ void adam_fast(const AdamK& k, float g, float& th, float& m, float& v) {
-    m = m + (g - m) * k.omb1;
-    v = v + (g * g - v) * k.omb2;
+__device__ __forceinline__ void adam_fast(const AdamStep& k, float g, float& th, float& m, float& v) {
+    m = m + (g - m) * k.one_m_b1;
+    v = v + (g * g - v) * k.one_m_b2;
     float sq;
     asm("sqrt.approx.f32 %0, %1;" : "=f"(sq) : "f"(v));
     th = th - __fdividef(m * k.alpha, sq + k.eps);
@@ -1198,7 +1159,7 @@ __device__ __forceinline__ float ldcg_f(const float* p) {        // L2 loads: da
 // against 768 cycles of tensor time).  The epilogue is pure HBM traffic (24 bytes per parameter) and the GEMM needs
 // almost none, so running them concurrently on every SM keeps HBM busy for the whole kernel.
 template <int PASSES>
-__global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const TcArgs A, const __grid_constant__ CUtensorMap tmap_h1,
+__global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const LearnArgs A, const __grid_constant__ CUtensorMap tmap_h1,
                                                               const __grid_constant__ CUtensorMap tmap_dh1) {
     extern __shared__ uint8_t smem_raw[];
     const int B = A.d.batch, Dp = A.d.obs_stride, G = A.d.n_nets;
@@ -1314,7 +1275,7 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const TcArgs A, co
                     // the tensor-map / bulk reads below are async-proxy reads of data written through the generic proxy
                     int fine = 1;
                     if (lane == 0) {
-                        fine = flag_acquire_ge(A.k4a_done + g, A.tiles) ? 1 : 0;
+                        fine = flag_acquire_ge(A.k4a_done + g, A.tc_tiles) ? 1 : 0;
                         asm volatile("fence.proxy.async;" ::: "memory");
                     }
                     ok = __shfl_sync(0xffffffffu, fine, 0) != 0;
@@ -1499,7 +1460,7 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const TcArgs A, co
             float* tg = A.nets.theta_tgt + pb;
             float* am = A.nets.adam_m + pb;
             float* av = A.nets.adam_v + pb;
-            const AdamK k = adam_k(A, g);
+            const AdamStep k = adam_step(A, g);
             const bool is_w2 = t < 2;
             const int m0 = is_w2 ? t * BM : 0;
             if (t == 2 && poisoned) {
@@ -1512,9 +1473,9 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const TcArgs A, co
                     adam1(k, grad, th[off], am[off], av[off], tgv);
                     if (k.sync) tg[off] = tgv;
                 };
-                const size_t p0 = (size_t)g * A.tiles;
+                const size_t p0 = (size_t)g * A.tc_tiles;
                 float s2 = 0.f, w[4] = {0.f, 0.f, 0.f, 0.f};
-                for (int r = 0; r < A.tiles; ++r) {
+                for (int r = 0; r < A.tc_tiles; ++r) {
                     s2 += ldcg_f(A.part_b2 + (p0 + r) * H + et);
                     const float4 pw = ldg_plain(A.part_w3 + ((p0 + r) * H + et) * 4);
                     w[0] += pw.x; w[1] += pw.y; w[2] += pw.z; w[3] += pw.w;
@@ -1523,22 +1484,10 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const TcArgs A, co
                 for (int a = 0; a < 4; ++a) upd(A.L.w3 + (int64_t)et * 4 + a, w[a]);
                 if (et < 4) {
                     float s3 = 0.f;
-                    for (int r = 0; r < A.tiles; ++r) s3 += ldcg_f(A.part_b3 + (p0 + r) * 4 + et);
+                    for (int r = 0; r < A.tc_tiles; ++r) s3 += ldcg_f(A.part_b3 + (p0 + r) * 4 + et);
                     upd(A.L.b3 + et, s3);
                 }
-                if (et == 0 && A.metrics) {
-                    double ls = 0, qs = 0, qq = 0, hist[4] = {0, 0, 0, 0};
-                    for (int r = 0; r < A.tiles; ++r) {
-                        const float* pl = A.part_loss + (p0 + r) * 8;
-                        ls += ldcg_f(pl); qs += ldcg_f(pl + 1); qq += ldcg_f(pl + 2);
-                        for (int a = 0; a < 4; ++a) hist[a] += ldcg_f(pl + 3 + a);
-                    }
-                    const double cnt = (double)B * A.d.n_actions, mean = qs / cnt, var = fmax(qq / cnt - mean * mean, 0.0);
-                    float* m = A.metrics + g * DMDQN_METRICS_STRIDE;
-                    m[0] = (float)(ls / A.loss_batch); m[1] = (float)mean; m[2] = (float)sqrt(var);
-                    for (int a = 0; a < 4; ++a) m[3 + a] = (float)hist[a];
-                    m[7] = 1.f;
-                }
+                if (et == 0 && A.metrics) finish_metrics(A, g, A.tc_tiles, [](const float* p) { return ldcg_f(p); });
             }
             const uint32_t acc_buf = (uint32_t)(n & 1);
             WG_TS();
@@ -1691,25 +1640,25 @@ int encode_map3(CUtensorMap* out, const float* base, cuuint64_t d0, cuuint64_t d
 }
 // x.W chunks in the UMMA MN-major layout straight from TMA (tma_fwd): the [K][256] matrix at float offset `woff` of every
 // network's parameter block as {32 columns, 4 k-rows, 8 column blocks, K / 4 k-groups, network}.
-int make_fwd_tensor_map(const TcArgs& A, const float* theta, int64_t woff, int K, CUtensorMap* out) {
+int make_fwd_tensor_map(const LearnArgs& A, const float* theta, int64_t woff, int K, CUtensorMap* out) {
     const cuuint64_t dims[5] = {32, 4, (cuuint64_t)(H / 32), (cuuint64_t)(K / 4), (cuuint64_t)A.d.n_nets};
     const cuuint64_t strides[4] = {(cuuint64_t)H * 4, 128, (cuuint64_t)H * 16, (cuuint64_t)A.L.stride * 4};
     const cuuint32_t box[5] = {32, 4, (cuuint32_t)(H / 32), 2, 1};
     return encode_tiled(out, theta + woff, 5, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
 }
-int make_w2_tensor_map(const TcArgs& A, CUtensorMap* out) {
+int make_w2_tensor_map(const LearnArgs& A, CUtensorMap* out) {
     return encode_map3(out, A.nets.theta + A.L.w2, H, H, A.d.n_nets, (cuuint64_t)H * sizeof(float),
                        (cuuint64_t)A.L.stride * sizeof(float), 8, H, CU_TENSOR_MAP_SWIZZLE_32B);
 }
 // K4b's K-major operands: the transposed scratch [n_nets][H features][B batch] as {B, H, n_nets}, box = {16 batch columns,
 // `rows` features}, landing with the 64-byte swizzle of the UMMA K-major SW64 layout (16-byte piece ^= (row / 2) % 4).
-int make_scratch_tensor_map(const TcArgs& A, const float* scratch, int rows, CUtensorMap* out) {
+int make_scratch_tensor_map(const LearnArgs& A, const float* scratch, int rows, CUtensorMap* out) {
     return encode_map3(out, scratch, A.d.batch, H, A.d.n_nets, (cuuint64_t)A.d.batch * sizeof(float),
                        (cuuint64_t)A.d.batch * H * sizeof(float), KC, (cuuint32_t)rows, CU_TENSOR_MAP_SWIZZLE_64B);
 }
 
 template <int PASSES>
-int launch_tc(const TcArgs& A, int stages, cudaStream_t s) {
+int launch_tc(const LearnArgs& A, int stages, cudaStream_t s) {
     const size_t smem_f = Fwd::TOTAL + 1024, smem_w = Wg::TOTAL + 1024;
     int n_sm = 0;
     if (int rc = device_sm_count(&n_sm)) return rc;
@@ -1717,7 +1666,7 @@ int launch_tc(const TcArgs& A, int stages, cudaStream_t s) {
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_target_kernel<PASSES>), smem_f, cfg_t)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_online_kernel<PASSES>), smem_f, cfg_o)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_wgrad_kernel<PASSES>), smem_w, cfg_w)) return rc;
-    const int items = A.d.n_nets * A.tiles;                       // persistent: one CTA per SM walks its items
+    const int items = A.d.n_nets * A.tc_tiles;                    // persistent: one CTA per SM walks its items
     // In a chain (sample + K3 + K4a + K4b issued by one call) K4a and K4b are programmatic dependent launches: their CTAs
     // are scheduled as soon as every CTA of the previous kernel is resident, take over SMs as that kernel's CTAs leave, and
     // order themselves behind the data they need with the per-tile / per-network flags.  Every CTA of the producer is
@@ -1773,54 +1722,13 @@ bool tc_supported(const dmdqn_dims& d) {
     return d.hidden == H && d.obs_stride % 32 == 0 && d.obs_stride <= 96 && d.batch % 4 == 0 && d.batch <= 4096;
 }
 
-int launch_learn_tc(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                    float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch,
-                    cudaStream_t s) {
-    TcArgs A;
-    A.d = d;
-    A.L = make_layout(d.obs_stride, d.hidden);
-    A.rp = rp;
-    A.nets = nets;
-    A.gamma = (float)hp.gamma;
-    A.loss = hp.loss;
-    A.double_dqn = hp.double_dqn;
-    A.adam_form = hp.adam_form;
-    A.freq = hp.target_update_frequency > 0 ? hp.target_update_frequency : 1;
-    A.loss_batch = loss_batch > 0 ? loss_batch : d.batch;
-    A.tiles = (d.batch + BM - 1) / BM;
-    A.lr = hp.learning_rate; A.beta1 = hp.beta1; A.beta2 = hp.beta2; A.adam_eps = hp.adam_eps; A.tau = hp.tau;
-    A.rows = reinterpret_cast<const int32_t*>(ws + w.rows);
-    A.act_b = reinterpret_cast<const int32_t*>(ws + w.act_b);
-    A.active = reinterpret_cast<const int32_t*>(ws + w.active);
-    A.step_t = reinterpret_cast<const int32_t*>(ws + w.step_t);
-    A.adam_sc = reinterpret_cast<const float4*>(ws + w.adam_sc);
-    A.mask2 = reinterpret_cast<uint32_t*>(ws + w.mask2);
-    A.ga = reinterpret_cast<float2*>(ws + w.ga);
-    A.w3_copy = reinterpret_cast<float*>(ws + w.w3_copy);
-    A.r_hat = reinterpret_cast<const float*>(ws + w.r_hat);
-    A.done_b = reinterpret_cast<const float*>(ws + w.done_b);
-    A.y = reinterpret_cast<float*>(ws + w.y);
-    A.gcoef = reinterpret_cast<float*>(ws + w.gcoef);
-    A.q_all = reinterpret_cast<float*>(ws + w.q_all);
-    A.q_next = reinterpret_cast<float*>(ws + w.q_next);
-    A.tq_all = reinterpret_cast<float*>(ws + w.tq_all);
-    A.h1 = reinterpret_cast<float*>(ws + w.h1);
-    A.dh1 = reinterpret_cast<float*>(ws + w.dh1);
-    A.dh2 = reinterpret_cast<float*>(ws + w.dh2);
-    A.part_loss = reinterpret_cast<float*>(ws + w.part_loss);
-    A.part_b3 = reinterpret_cast<float*>(ws + w.part_b3);
-    A.part_w3 = reinterpret_cast<float*>(ws + w.part_w3);
-    A.part_b2 = reinterpret_cast<float*>(ws + w.part_b2);
-    A.metrics = metrics;
-    A.grads = grads;
-    A.error = reinterpret_cast<int*>(ws + w.tc_error);
-    const int all = DMDQN_STAGE_SAMPLE | DMDQN_STAGE_TARGET | DMDQN_STAGE_ONLINE | DMDQN_STAGE_WGRAD;
-    A.chain = (stages & all) == all ? 1 : 0;      // the sample kernel of this call has just reset the flags
-    A.tiles_ws = w.tiles;
-    A.sched = reinterpret_cast<int*>(ws + w.sync);
+int launch_learn_tc(const LearnArgs& args, int precision, int stages, cudaStream_t s) {
+    LearnArgs A = args;
+    A.tc_tiles = (A.d.batch + BM - 1) / BM;
+    A.chain = (stages & kAllStages) == kAllStages ? 1 : 0;      // the sample kernel of this call has just reset the flags
     A.k4a_done = A.sched + 4;
-    A.k3_done = A.k4a_done + d.n_nets;
-    return hp.precision == DMDQN_PRECISION_TF32 ? launch_tc<1>(A, stages, s) : launch_tc<3>(A, stages, s);
+    A.k3_done = A.k4a_done + A.d.n_nets;
+    return precision == DMDQN_PRECISION_TF32 ? launch_tc<1>(A, stages, s) : launch_tc<3>(A, stages, s);
 }
 
 }  // namespace dmdqn

@@ -66,8 +66,8 @@ __global__ void __launch_bounds__(kSampleThreads)
 sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restrict__ learn_step,
               const uint32_t* __restrict__ draws, const uint8_t* __restrict__ learn_mask, int advance,
               int32_t* __restrict__ rows, float* __restrict__ r_hat, int32_t* __restrict__ act_b,
-              float* __restrict__ done_b, int32_t* __restrict__ active, int32_t* __restrict__ step_t,
-              float4* __restrict__ adam_sc, int32_t* __restrict__ sync, int tiles) {
+              float* __restrict__ done_b, int32_t* __restrict__ active, float4* __restrict__ adam_sc,
+              int32_t* __restrict__ sync, int tiles) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int B = d.batch, Bp = (B + 1) & ~1;
     int* js = reinterpret_cast<int*>(smem_raw);
@@ -97,14 +97,13 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
         active[g] = on ? 1 : 0;
         int t = learn_step[g];
         if (on && advance) learn_step[g] = ++t;    // dqn_agent.py:359
-        step_t[g] = t;
         t_step = t;
     }
     if (!on) return;
-    // Adam scalars of this step, once per network instead of once per thread of K4b: alpha_t = lr * sqrt(1 - b2^t) / (1 - b1^t)
-    // in float64, then rounded (oracle/dqn.py adam_scalars).  Two double-precision pow() calls (~2 us) by ONE thread: thread 0
-    // runs them while the other warps are still in their index scan (warp 0's is the shortest), not in front of a barrier
-    // every thread waits at.
+    // Adam scalars of this step, the only place they are evaluated (every Adam kernel loads them with adam_step, common.cuh):
+    // alpha_t = lr * sqrt(1 - b2^t) / (1 - b1^t) in float64, then rounded (oracle/dqn.py adam_scalars).  Two double-precision
+    // pow() calls (~2 us) by ONE thread: thread 0 runs them while the other warps are still in their index scan (warp 0's is
+    // the shortest), not in front of a barrier every thread waits at.
     auto adam_scalars = [&]() {
         const int t = t_step;
         const double bc1 = 1.0 - pow(hp.beta1, (double)t), bc2 = 1.0 - pow(hp.beta2, (double)t);
@@ -257,8 +256,8 @@ int launch_sample(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repl
         d, hp, rp, nets.learn_step, static_cast<const uint32_t*>(draws), learn_mask, advance,
         reinterpret_cast<int32_t*>(ws + w.rows), reinterpret_cast<float*>(ws + w.r_hat),
         reinterpret_cast<int32_t*>(ws + w.act_b), reinterpret_cast<float*>(ws + w.done_b),
-        reinterpret_cast<int32_t*>(ws + w.active), reinterpret_cast<int32_t*>(ws + w.step_t),
-        reinterpret_cast<float4*>(ws + w.adam_sc), reinterpret_cast<int32_t*>(ws + w.sync), w.tiles);
+        reinterpret_cast<int32_t*>(ws + w.active), reinterpret_cast<float4*>(ws + w.adam_sc),
+        reinterpret_cast<int32_t*>(ws + w.sync), w.tiles);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

@@ -266,7 +266,8 @@ int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn
  * the same step but K4b stores dL/dtheta into grads_out[n_nets][layout.stride] instead of
  * applying Adam, with the loss mean taken over global_batch (= batch * ranks), so that the
  * caller can sum the blocks over ranks (ncclAllReduce) and finish with dmdqn_adam_apply,
- * which reads the step counters dmdqn_learn_grads left in the workspace. */
+ * which takes the step's learn flags and Adam scalars (alpha_t, eps, target-sync mode) from the
+ * workspace of the preceding dmdqn_learn_grads: pass it the same hparams. */
 int dmdqn_learn_grads(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                       const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
                       int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
@@ -285,6 +286,7 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
  * writing step t+1 while this rank still reads step t); flags[p] is uint32[DMDQN_MAX_PEERS][DMDQN_PEER_BLOCKS],
  * zero-initialised once; epoch = 1, 2, 3, ... identical on every rank.  my_loss_src is this rank's share of the loss
  * (metrics_out[0] of dmdqn_learn_grads), published to loss[rank] by the kernel; loss_out receives the sum.
+ * Like dmdqn_adam_apply it takes the step's learn flag and Adam scalars from the workspace of dmdqn_learn_grads.
  * A peer that never arrives ends in DMDQN_PEER_TIMEOUT in the workspace error flag (no update applied), not in a hang. */
 #define DMDQN_MAX_PEERS 8
 #define DMDQN_PEER_TIMEOUT 77     /* value of the workspace error flag after a peer never arrived */
