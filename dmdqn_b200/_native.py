@@ -10,7 +10,8 @@ LIB_PATH = os.path.join(HERE, "libdmdqn_b200.so")
 
 OK, ERR_ARG, ERR_CUDA, ERR_WORKSPACE = 0, -1, -2, -3
 LOSS = {"mse": 0, "huber": 1}
-SAMPLE = {"indices": 0, "fisher_yates": 1, "replacement": 2}
+SAMPLE = {"indices": 0, "fisher_yates": 1, "replacement": 2, "prioritized": 3}
+PER_MAX_CAPACITY = 8192 * 128
 ADAM = {"keras": 0, "torch": 1}
 PRECISION = {"fp32": 0, "tf32": 1, "tf32x3": 2}
 METRICS_STRIDE = 8
@@ -26,7 +27,7 @@ class Layout(C.Structure):
 
 
 class Replay(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("obs", "next_obs", "act", "rew", "done", "n_written")]
+    _fields_ = [(n, C.c_void_p) for n in ("obs", "next_obs", "act", "rew", "done", "n_written", "priority", "priority_max")]
 
 
 class Nets(C.Structure):
@@ -36,11 +37,12 @@ class Nets(C.Structure):
 class HParams(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("gamma", "learning_rate", "beta1", "beta2", "adam_eps", "tau")] + \
                [(n, C.c_int32) for n in ("target_update_frequency", "loss", "normalize_rewards", "double_dqn",
-                                         "adam_form", "sample_mode", "precision")]
+                                         "adam_form", "sample_mode", "precision")] + \
+               [(n, C.c_double) for n in ("per_alpha", "per_beta0", "per_eps")] + [("per_beta_steps", C.c_int32)]
 
 
 class DebugViews(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("y", "q_all", "q_next", "tq_all", "rows", "r_hat", "active", "tc_error", "dh1", "dh2", "relu2_bits")]
+    _fields_ = [(n, C.c_void_p) for n in ("y", "q_all", "q_next", "tq_all", "rows", "r_hat", "active", "tc_error", "dh1", "dh2", "relu2_bits", "is_w")]
 
 
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
@@ -112,7 +114,7 @@ def lib() -> C.CDLL:
         for name, (res, args) in SIGNATURES.items():
             fn = getattr(handle, name)  # AttributeError if the .so does not export it
             fn.restype, fn.argtypes = res, args
-        if handle.dmdqn_abi_version() != 2:      # 2: + dmdqn_allreduce_adam, dmdqn_ipc_* (round 2)
+        if handle.dmdqn_abi_version() != 3:      # 3: + prioritized replay fields at the end of the replay / hparams / debug structs
             raise NativeError("libdmdqn_b200.so ABI version mismatch: rebuild")
         _lib = handle
     return _lib

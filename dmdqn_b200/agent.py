@@ -8,7 +8,9 @@ src/experimental/agent.py:148-152 (src/scripts/test.py:88 calls it).  Each objec
 1-agent view (offset pointers) onto an :class:`AgentGroup`; the arithmetic runs in
 libdmdqn_b200.so.  Host-side randomness follows the reference exactly -- ``np.random`` for
 the explore draw (:263-265) and ``random.sample`` for the replay indices (:63) -- so a
-seeded reference run and a seeded facade run pick the same actions and transitions.
+seeded reference run and a seeded facade run pick the same actions and transitions.  With
+``sample_mode: prioritized`` ``learn()`` draws its batch on the device from the ring's priorities
+instead (the reference has no prioritized replay, so there is no index stream to follow).
 """
 from __future__ import annotations
 
@@ -152,8 +154,11 @@ class DQNAgent:
         size = len(self.replay_buffer)
         if size < self.batch_size:
             return None
-        idx = np.asarray(random.sample(range(size), self.batch_size), np.int32)[None]   # :63
-        metrics = self._g.learn(idx, sample_mode="indices")
+        if self._g.prioritized:     # proportional prioritized replay: the kernel draws from device words
+            metrics = self._g.learn()
+        else:
+            idx = np.asarray(random.sample(range(size), self.batch_size), np.int32)[None]   # :63
+            metrics = self._g.learn(idx, sample_mode="indices")
         self.learn_step_counter += 1                                        # :359
         self.last_metrics = metrics[0]
         return metrics[0, 0].clone()

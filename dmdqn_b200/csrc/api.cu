@@ -146,19 +146,27 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
     if (rc) return rc;
     DMDQN_CHECK_ARG(replay && replay->obs && replay->next_obs && replay->act && replay->rew && replay->done &&
                         replay->n_written, "push: NULL replay pointer");
+    DMDQN_CHECK_ARG(!replay->priority || replay->priority_max, "push: priority is set but priority_max is NULL");
     DMDQN_CHECK_ARG(obs && act && rew && next_obs && done, "push: NULL transition pointer");
     DMDQN_CHECK_ARG(in_stride >= dims->obs_dim, "in_stride=%d < obs_dim=%d", in_stride, dims->obs_dim);
     return launch_push(*dims, *replay, obs, act, rew, next_obs, done, in_stride, mask, (cudaStream_t)stream);
 }
 
-static int check_learn_args(const dmdqn_hparams* hp, const dmdqn_replay* replay, const dmdqn_nets* nets,
-                            const void* draws) {
+static int check_learn_args(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
+                            const dmdqn_nets* nets, const void* draws) {
     DMDQN_CHECK_ARG(hp && replay && nets && draws, "NULL argument");
     DMDQN_CHECK_ARG(replay->obs && replay->next_obs && replay->act && replay->rew && replay->done &&
                         replay->n_written, "NULL replay pointer");
     DMDQN_CHECK_ARG(nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && nets->learn_step,
                     "NULL network pointer");
-    DMDQN_CHECK_ARG(hp->sample_mode >= 0 && hp->sample_mode <= 2, "sample_mode=%d", hp->sample_mode);
+    DMDQN_CHECK_ARG(hp->sample_mode >= 0 && hp->sample_mode <= DMDQN_SAMPLE_PRIORITIZED, "sample_mode=%d", hp->sample_mode);
+    if (hp->sample_mode == DMDQN_SAMPLE_PRIORITIZED) {
+        DMDQN_CHECK_ARG(replay->priority && replay->priority_max,
+                        "sample_mode=prioritized needs the replay's priority and priority_max arrays (NULL priority pointer)");
+        DMDQN_CHECK_ARG(!(dims->n_nets == 1 && dims->n_agents > 1),
+                        "sample_mode=prioritized serves independent networks only (n_nets=%d, n_agents=%d share parameters)",
+                        dims->n_nets, dims->n_agents);
+    }
     DMDQN_CHECK_ARG(hp->loss == DMDQN_LOSS_MSE || hp->loss == DMDQN_LOSS_HUBER, "loss=%d", hp->loss);
     DMDQN_CHECK_ARG(hp->precision >= DMDQN_PRECISION_FP32 && hp->precision <= DMDQN_PRECISION_TF32X3, "precision=%d",
                     hp->precision);
@@ -173,7 +181,7 @@ static int run_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     Workspace w;
     int rc = check_workspace(dims, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    rc = check_learn_args(hp, replay, nets, draws);
+    rc = check_learn_args(dims, hp, replay, nets, draws);
     if (rc) return rc;
     if (grads) DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     if (stages & DMDQN_STAGE_SAMPLE) {
@@ -190,7 +198,7 @@ int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_re
     Workspace w;
     int rc = check_workspace(dims, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    rc = check_learn_args(hp, replay, nets, draws);
+    rc = check_learn_args(dims, hp, replay, nets, draws);
     if (rc) return rc;
     return launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, advance_step, (char*)workspace, w,
                          (cudaStream_t)stream);
@@ -343,6 +351,7 @@ int dmdqn_debug(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes,
     out->dh1 = (const float*)(ws + w.dh1);
     out->dh2 = (const float*)(ws + w.dh2);
     out->relu2_bits = (const uint32_t*)(ws + w.mask2);
+    out->is_w = (const float*)(ws + w.is_w);
     return DMDQN_OK;
 }
 

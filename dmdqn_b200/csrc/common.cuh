@@ -71,6 +71,8 @@ struct Workspace {
     size_t part_b3;                   // [n_nets][T][4]
     size_t part_w3;                   // [n_nets][T][H][4]
     size_t part_b2, part_b1;          // [n_nets][T][H]
+    size_t is_w;                      // [n_nets][B] float: importance weights of a prioritized sample (written by the sample
+                                      // kernel, read by K4a)
     size_t sync;                      // tcgen05 path, int32: [0] K4b work counter, [1..3] spare, [4 ..] k4a_done[n_nets], then
                                       // k3_done[n_nets][T]; zeroed by the sample kernel (dataflow flags between the learn kernels)
     size_t total;
@@ -107,6 +109,7 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
     w.part_w3 = take(nt * d.hidden * 4 * 4);
     w.part_b2 = take(nt * d.hidden * 4);
     w.part_b1 = take(nt * d.hidden * 4);
+    w.is_w = take(nb * 4);
     w.sync = take((4 + (size_t)d.n_nets + nt) * 4);
     w.total = off;
     return w;
@@ -145,11 +148,25 @@ struct LearnArgs {
     // reset the flags): K4a / K4b are programmatic dependent launches whose CTAs start on SMs the previous kernel has left
     // and wait per (network, tile) / per network instead of for the whole previous grid.
     int chain;
-    int *sched, *k4a_done, *k3_done;  // Workspace::sync: K4b work counter | K4a items finished per network | K3 items finished
+    int *sched, *k4a_done, *k3_done;
+    // Prioritized replay (per = 1 only in DMDQN_SAMPLE_PRIORITIZED): K4a weights each row by is_w and writes its priority
+    int per;
+    const float* is_w;                // Workspace::is_w
+    double per_alpha, per_eps;  // Workspace::sync: K4b work counter | K4a items finished per network | K3 items finished
                                       // per (network, tile)
 };
 LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                           char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch);
+
+// Prioritized replay, K4a of both paths: the priority of the transition behind row `row` (agent * C + slot) from its TD
+// error, (float)pow(|delta| + eps, alpha) in float64, and the agent's running maximum (positive floats order like their
+// int bits, so atomicMax gives the same result in any order).  A non-finite priority is not stored.
+__device__ __forceinline__ void per_store_priority(const LearnArgs& A, int row, float delta) {
+    const float p = (float)pow(fabs((double)delta) + A.per_eps, A.per_alpha);
+    if (!isfinite(p)) return;
+    A.rp.priority[row] = p;
+    atomicMax(reinterpret_cast<int*>(A.rp.priority_max) + row / A.d.capacity, __float_as_int(p));
+}
 
 // Adam scalars of one network's step.  alpha_t, eps_eff and the sync mode are evaluated once per network by the sample
 // kernel into adam_sc; every Adam kernel loads them here.

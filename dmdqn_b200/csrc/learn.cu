@@ -307,6 +307,12 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
                 term = ae <= 1.0f ? 0.5f * e * e : ae - 0.5f;
                 gi = fminf(fmaxf(e, -1.0f), 1.0f) / (float)A.loss_batch;
             }
+            if (A.per) {                             // prioritized replay: importance weight, then the new priority
+                const float wi = A.is_w[sb + gr];
+                term = wi * term;
+                gi = wi * gi;
+                per_store_priority(A, rows[gr], e);
+            }
             for (int k = 0; k < 4; ++k) A.q_all[(sb + gr) * 4 + k] = S.qs0[i * 4 + k];
         }
         S.gs[i] = gi;
@@ -712,6 +718,10 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
     A.sched = reinterpret_cast<int*>(ws + w.sync);
     A.metrics = metrics;
     A.grads = grads;
+    A.per = hp.sample_mode == DMDQN_SAMPLE_PRIORITIZED && rp.priority != nullptr;
+    A.is_w = reinterpret_cast<const float*>(ws + w.is_w);
+    A.per_alpha = hp.per_alpha;
+    A.per_eps = hp.per_eps;
     return A;
 }
 

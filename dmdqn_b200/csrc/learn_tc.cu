@@ -880,6 +880,12 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, c
                     term = ae <= 1.0f ? 0.5f * err * err : ae - 0.5f;
                     gi = fminf(fmaxf(err, -1.0f), 1.0f) / (float)A.loss_batch;
                 }
+                if (A.per) {                                  // prioritized replay: importance weight, then the new priority
+                    const float wi = A.is_w[sb + gr];
+                    term = wi * term;
+                    gi = wi * gi;
+                    if (e.part == 0 && ok) per_store_priority(A, A.rows[sb + gr], err);
+                }
                 if (e.part == 0) {
                     A.ga[sb + gr] = make_float2(gi, __int_as_float(ai));
                     *reinterpret_cast<float4*>(A.q_all + (sb + gr) * 4) = make_float4(qv[0], qv[1], qv[2], qv[3]);

@@ -33,11 +33,14 @@ push_kernel(dmdqn_dims d, dmdqn_replay rp, const float* __restrict__ obs, const 
         rp.rew[row] = rew[a];
         rp.done[row] = done[a] ? 1 : 0;
         rp.n_written[a] = nw + 1;
+        if (rp.priority) rp.priority[row] = rp.priority_max[a];   // a new transition gets the ring's largest priority
     }
 }
 
 // ---------------------------------------------------------------- sample ----------------
 constexpr int kSampleThreads = 256;
+constexpr int kPerChunk = 128;                 // prioritized replay: slots per chunk of the canonical priority sum
+constexpr int kPerScan = 8;                    // chunks a warp loads before it adds (32 loads in flight per lane)
 
 // Canonical float64 tree sum over a batch held in shared memory: lane l adds elements
 // l, l+32, ... in order, then an xor butterfly (16,8,4,2,1).  oracle/replay.py
@@ -62,12 +65,14 @@ __device__ __forceinline__ double tree_sum(int n, int lane, F elem) {
 // pj / pt come from a B x B compare (thread i scans k < i; every read is a shared-memory broadcast) and
 // the W chains (almost always of length 0 or 1) are chased read-only.  Same integers as the sequential
 // loop for every input (oracle/replay.py fisher_yates_indices replays the loop itself).
+// PER: DMDQN_SAMPLE_PRIORITIZED (its own instantiation, so the uniform modes compile to the same code as without it).
+template <bool PER>
 __global__ void __launch_bounds__(kSampleThreads)
 sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restrict__ learn_step,
               const uint32_t* __restrict__ draws, const uint8_t* __restrict__ learn_mask, int advance,
               int32_t* __restrict__ rows, float* __restrict__ r_hat, int32_t* __restrict__ act_b,
               float* __restrict__ done_b, int32_t* __restrict__ active, float4* __restrict__ adam_sc,
-              int32_t* __restrict__ sync, int tiles) {
+              int32_t* __restrict__ sync, int tiles, float* __restrict__ is_w) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int B = d.batch, Bp = (B + 1) & ~1;
     int* js = reinterpret_cast<int*>(smem_raw);
@@ -75,7 +80,10 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
     int* words = pt + Bp;
     double* rs = reinterpret_cast<double*>(words + Bp);
     __shared__ double stat[2];
+    __shared__ int per_last, per_pmin;         // prioritized replay: last slot with a non-zero priority, min drawn priority (bits)
+    __shared__ double per_beta;
     const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const bool per = hp.sample_mode == DMDQN_SAMPLE_PRIORITIZED;
     const bool shared_net = d.n_nets == 1 && d.n_agents > 1;
     // dataflow flags of the tcgen05 learn kernels (learn_tc.cu): this launch is ordered after every kernel of the previous
     // step, so it is the one place where they can be reset without a race
@@ -114,7 +122,82 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
                                  __int_as_float(sync_mode), 0.f);
     };
 
-    if (hp.sample_mode == DMDQN_SAMPLE_FISHER_YATES) {
+    if constexpr (PER) {
+        // Proportional prioritized replay (include/dmdqn_b200.h; tests/per_oracle.py restates every step): words[i] is
+        // the drawn PHYSICAL slot here, not a logical index.
+        const int C = d.capacity, nch = (C + kPerChunk - 1) / kPerChunk, warp = tid >> 5;
+        const float* __restrict__ pr = rp.priority + (size_t)g * C;
+        double* prefix = rs + Bp;                       // [nch + 1]: chunk totals, then their exclusive prefixes
+        if (tid == 0) { per_last = -1; per_pmin = 0x7f800000; }
+        int last = -1;
+        for (int c0 = warp * kPerScan; c0 < nch; c0 += (kSampleThreads / 32) * kPerScan) {
+            float v[kPerScan][4];
+#pragma unroll
+            for (int u = 0; u < kPerScan; ++u)          // every load of the group is issued before the first add
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const int sl = (c0 + u) * kPerChunk + 32 * k + lane;
+                    v[u][k] = sl < C ? __ldg(pr + sl) : 0.f;
+                }
+#pragma unroll
+            for (int u = 0; u < kPerScan; ++u) {        // chunk total: lane l adds slots l, l+32, l+64, l+96, then the butterfly
+                double acc = 0.0;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    acc = __dadd_rn(acc, (double)v[u][k]);
+                    if (v[u][k] > 0.f) last = (c0 + u) * kPerChunk + 32 * k + lane;
+                }
+                for (int off = 16; off; off >>= 1) acc = __dadd_rn(acc, __shfl_xor_sync(0xffffffffu, acc, off));
+                if (lane == 0 && c0 + u < nch) prefix[c0 + u + 1] = acc;
+            }
+        }
+        last = __reduce_max_sync(0xffffffffu, last);
+        __syncthreads();                                // per_last / per_pmin initialised, chunk totals in place
+        if (lane == 0 && last >= 0) atomicMax(&per_last, last);
+        if (tid == 32) {                                // chunk totals -> exclusive prefixes, in chunk order
+            double run = 0.0;
+            prefix[0] = 0.0;
+            for (int c = 1; c <= nch; ++c) {
+                run = __dadd_rn(run, prefix[c]);
+                prefix[c] = run;
+            }
+        }
+        if (tid == 0) {
+            adam_scalars();
+            double beta = hp.per_beta0;                 // beta_t of this step, t = learn_step after the increment
+            if (hp.per_beta_steps > 0)
+                beta = fmin(1.0, __dadd_rn(hp.per_beta0, __ddiv_rn(__dmul_rn(__dsub_rn(1.0, hp.per_beta0), (double)t_step),
+                                                                   (double)hp.per_beta_steps)));
+            per_beta = beta;
+        }
+        __syncthreads();
+        const double S = prefix[nch];
+        for (int i = tid; i < B; i += kSampleThreads) {
+            const double w = (double)draws[(size_t)g * B + i];
+            const double u = __ddiv_rn(__dmul_rn(__dadd_rn((double)i, __dmul_rn(w, 0x1p-32)), S), (double)B);
+            int lo = 0, hi = nch - 1;                   // the last chunk whose exclusive prefix is <= u
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (prefix[mid] <= u) lo = mid; else hi = mid - 1;
+            }
+            const int base = lo * kPerChunk;
+            double run = prefix[lo];
+            int slot = -1;
+            for (int s0 = 0; s0 < kPerChunk && slot < 0; s0 += 32) {   // walk the chunk in slot order, 32 loads ahead of the adds
+                float v[32];
+#pragma unroll
+                for (int k = 0; k < 32; ++k) v[k] = base + s0 + k < C ? __ldg(pr + base + s0 + k) : 0.f;
+#pragma unroll
+                for (int k = 0; k < 32; ++k) {
+                    run = __dadd_rn(run, (double)v[k]);
+                    if (slot < 0 && run > u) slot = base + s0 + k;
+                }
+            }
+            if (slot < 0) slot = per_last >= 0 ? per_last : 0;         // rounding carried the walk past the chunk
+            words[i] = slot;
+            atomicMin(&per_pmin, __float_as_int(__ldg(pr + slot)));
+        }
+    } else if (hp.sample_mode == DMDQN_SAMPLE_FISHER_YATES) {
         const int n = (int)pop;
         for (int i = tid; i < B; i += kSampleThreads)
             js[i] = (int)__umulhi(draws[(size_t)g * B + i], (unsigned)(n - i));
@@ -162,8 +245,12 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
         const int lj = shared_net ? logical % size0 : logical;
         const long long nw = shared_net ? rp.n_written[agent] : nw0;
         const long long sz = nw < d.capacity ? nw : d.capacity;
-        const int slot = (int)((nw - sz + lj) % d.capacity);
+        const int slot = per ? words[i] : (int)((nw - sz + lj) % d.capacity);
         const int row = agent * d.capacity + slot;
+        if constexpr (PER) {                            // importance weight (p_min / p_i)^beta_t in float64
+            const float p = rp.priority[row];
+            is_w[(size_t)g * B + i] = p > 0.f ? (float)pow(__ddiv_rn((double)__int_as_float(per_pmin), (double)p), per_beta) : 1.f;
+        }
         rows[(size_t)g * B + i] = row;
         // (an L2 prefetch of the two sampled rows was measured here: +6 us in this kernel, nothing gained in K3 / K4a)
         act_b[(size_t)g * B + i] = rp.act[row];
@@ -249,15 +336,21 @@ int launch_sample(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repl
                   const void* draws, const uint8_t* learn_mask, int advance, char* ws, const Workspace& w,
                   cudaStream_t s) {
     DMDQN_CHECK_ARG(d.batch <= 4096, "batch %d: the sample kernel serves batches up to 4096", d.batch);
-    const size_t smem = (size_t)((d.batch + 1) & ~1) * (3 * 4 + 8);
-    static size_t configured[kMaxDevices] = {};
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(sample_kernel), smem, configured)) return rc;
-    sample_kernel<<<d.n_nets, kSampleThreads, smem, s>>>(
+    const bool per = hp.sample_mode == DMDQN_SAMPLE_PRIORITIZED;
+    // prioritized replay keeps the chunk prefixes of the ring in shared memory (8 bytes per 128 slots)
+    DMDQN_CHECK_ARG(!per || d.capacity <= DMDQN_PER_MAX_CAPACITY,
+                    "capacity=%d: prioritized replay serves rings of up to %d slots", d.capacity, DMDQN_PER_MAX_CAPACITY);
+    const size_t smem = (size_t)((d.batch + 1) & ~1) * (3 * 4 + 8) +
+                        (per ? (size_t)((d.capacity + kPerChunk - 1) / kPerChunk + 1) * 8 : 0);
+    static size_t configured[2][kMaxDevices] = {};
+    const auto kernel = per ? sample_kernel<true> : sample_kernel<false>;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kernel), smem, configured[per])) return rc;
+    kernel<<<d.n_nets, kSampleThreads, smem, s>>>(
         d, hp, rp, nets.learn_step, static_cast<const uint32_t*>(draws), learn_mask, advance,
         reinterpret_cast<int32_t*>(ws + w.rows), reinterpret_cast<float*>(ws + w.r_hat),
         reinterpret_cast<int32_t*>(ws + w.act_b), reinterpret_cast<float*>(ws + w.done_b),
         reinterpret_cast<int32_t*>(ws + w.active), reinterpret_cast<float4*>(ws + w.adam_sc),
-        reinterpret_cast<int32_t*>(ws + w.sync), w.tiles);
+        reinterpret_cast<int32_t*>(ws + w.sync), w.tiles, reinterpret_cast<float*>(ws + w.is_w));
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

@@ -33,6 +33,9 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # new keys (SURVEY.md section 5 "Config / flags"); defaults = reference behaviour
     "tau": None, "loss": "mse", "normalize_rewards": True, "double_dqn": True, "adam_form": "keras",
     "share_parameters": False, "precision": "auto", "sample_mode": "fisher_yates",
+    # prioritized replay (sample_mode "prioritized"): priority exponent, initial importance exponent (annealed to 1 over
+    # per_beta_steps learn steps), priority offset
+    "per_alpha": 0.6, "per_beta": 0.4, "per_beta_steps": 100000, "per_eps": 1e-6,
 }
 
 
@@ -80,6 +83,10 @@ class AgentGroup:
             raise ValueError(f"nn_layers={layers}: the CUDA path supports two equal hidden layers [H, H]")
         self.n_agents = int(n_agents)
         self.shared = bool(cfg["share_parameters"])
+        self.prioritized = cfg["sample_mode"] == "prioritized"
+        if self.prioritized and self.shared:
+            raise ValueError("sample_mode='prioritized' serves independent networks only: it cannot be combined with "
+                             "share_parameters=true")
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -106,7 +113,8 @@ class AgentGroup:
             -1.0 if cfg["tau"] is None else float(cfg["tau"]),
             int(cfg["target_update_frequency"]), N.LOSS[cfg["loss"]], int(bool(cfg["normalize_rewards"])),
             int(bool(cfg["double_dqn"])), N.ADAM[cfg["adam_form"]], N.SAMPLE[cfg["sample_mode"]],
-            N.PRECISION[cfg["precision"]])
+            N.PRECISION[cfg["precision"]], float(cfg["per_alpha"]), float(cfg["per_beta"]), float(cfg["per_eps"]),
+            int(cfg["per_beta_steps"]))
 
         dev, n, c, dp, g = self.device, self.n_agents, self.capacity, self.obs_stride, self.n_nets
         if _parent is None:
@@ -121,6 +129,9 @@ class AgentGroup:
             self.adam_m = torch.zeros_like(self.theta)
             self.adam_v = torch.zeros_like(self.theta)
             self.learn_step = torch.zeros((g,), dtype=torch.int32, device=dev)
+            # prioritized replay: p^alpha per physical slot (0 = never written) and each ring's largest priority
+            self.priority = torch.zeros((n, c), dtype=torch.float32, device=dev) if self.prioritized else None
+            self.priority_max = torch.ones((n,), dtype=torch.float32, device=dev) if self.prioritized else None
             self.n_written_host = np.zeros((n,), np.int64)       # host mirrors: no device sync
             self.learn_step_host = np.zeros((g,), np.int64)
         else:
@@ -129,13 +140,15 @@ class AgentGroup:
             self.obs, self.next_obs = p.obs[i:i + 1], p.next_obs[i:i + 1]
             self.act_ring, self.rew_ring, self.done_ring = p.act_ring[i:i + 1], p.rew_ring[i:i + 1], p.done_ring[i:i + 1]
             self.n_written = p.n_written[i:i + 1]
+            self.priority = None if p.priority is None else p.priority[i:i + 1]
+            self.priority_max = None if p.priority_max is None else p.priority_max[i:i + 1]
             self.theta, self.theta_tgt = p.theta[j:j + 1], p.theta_tgt[j:j + 1]
             self.adam_m, self.adam_v = p.adam_m[j:j + 1], p.adam_v[j:j + 1]
             self.learn_step = p.learn_step[j:j + 1]
             self.n_written_host = p.n_written_host[i:i + 1]
             self.learn_step_host = p.learn_step_host[j:j + 1]
         self.replay = N.Replay(_ptr(self.obs), _ptr(self.next_obs), _ptr(self.act_ring), _ptr(self.rew_ring),
-                               _ptr(self.done_ring), _ptr(self.n_written))
+                               _ptr(self.done_ring), _ptr(self.n_written), _ptr(self.priority), _ptr(self.priority_max))
         self.nets = N.Nets(_ptr(self.theta), _ptr(self.theta_tgt), _ptr(self.adam_m), _ptr(self.adam_v),
                            _ptr(self.learn_step))
         nbytes = C.c_size_t()
@@ -505,7 +518,8 @@ class AgentGroup:
         out = {"y": view(v.y, torch.float32, (g, b)), "q_all": view(v.q_all, torch.float32, (g, b, 4)),
                "q_next": view(v.q_next, torch.float32, (g, b, 4)), "tq_all": view(v.tq_all, torch.float32, (g, b, 4)),
                "rows": view(v.rows, torch.int32, (g, b)), "r_hat": view(v.r_hat, torch.float32, (g, b)),
-               "active": view(v.active, torch.int32, (g,)), "tc_error": view(v.tc_error, torch.int32, (1,))}
+               "active": view(v.active, torch.int32, (g,)), "tc_error": view(v.tc_error, torch.int32, (1,)),
+               "is_weights": view(v.is_w, torch.float32, (g, b))}
         if self.hp.precision != 0:
             # the tcgen05 path keeps its activation scratch transposed ([feature][batch]) and never
             # materialises dh2: "dh2" is relu'(h2) as 0/1 here (its non-zero pattern is what the tests use)

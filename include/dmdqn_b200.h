@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define DMDQN_ABI_VERSION 2
+#define DMDQN_ABI_VERSION 3
 
 #define DMDQN_OK            0
 #define DMDQN_ERR_ARG      -1   /* bad dims / null pointer / unsupported size          */
@@ -56,6 +56,7 @@ extern "C" {
 #define DMDQN_SAMPLE_INDICES     0  /* host supplies logical indices (e.g. CPython random.sample) */
 #define DMDQN_SAMPLE_FISHER_YATES 1 /* uint32 draws, without replacement (partial Fisher-Yates)   */
 #define DMDQN_SAMPLE_REPLACEMENT 2  /* uint32 draws, with replacement (deviation, flagged)        */
+#define DMDQN_SAMPLE_PRIORITIZED 3  /* uint32 draws, proportional prioritized replay (see below)   */
 
 #define DMDQN_ADAM_KERAS 0      /* eps = adam_eps                       (keras 3.9.2)      */
 #define DMDQN_ADAM_TORCH 1      /* eps = adam_eps * sqrt(1 - beta2^t)   (torch.optim.Adam) */
@@ -92,6 +93,13 @@ typedef struct dmdqn_replay {   /* all device pointers */
     double*  rew;
     uint8_t* done;
     int64_t* n_written;
+    /* Prioritized replay (DMDQN_SAMPLE_PRIORITIZED; NULL = none, every other mode ignores them):
+     *   priority     float[n_agents][capacity]  p^alpha of each PHYSICAL slot; 0 = never written (never drawn)
+     *   priority_max float[n_agents]            largest priority seen by the agent's ring; the host starts it at 1.0
+     * dmdqn_push writes priority_max[a] into the slot it fills; the learn step writes the new priority of every
+     * sampled row (see dmdqn_learn). */
+    float*   priority;
+    float*   priority_max;
 } dmdqn_replay;
 
 typedef struct dmdqn_nets {     /* all device pointers */
@@ -116,6 +124,11 @@ typedef struct dmdqn_hparams {
     int32_t adam_form;                /* DMDQN_ADAM_*                                      */
     int32_t sample_mode;              /* DMDQN_SAMPLE_*                                    */
     int32_t precision;                /* DMDQN_PRECISION_*                                 */
+    /* prioritized replay (read in DMDQN_SAMPLE_PRIORITIZED only): priority = (|delta| + per_eps)^per_alpha,
+     * importance exponent beta_t = min(1, per_beta0 + (1 - per_beta0) * t / per_beta_steps) with t the network's
+     * learn_step after the increment (per_beta_steps <= 0: beta_t = per_beta0) */
+    double  per_alpha, per_beta0, per_eps;
+    int32_t per_beta_steps;
 } dmdqn_hparams;
 
 /* Per-network learn outputs, 8 floats each: loss, q_mean, q_std (population, over the
@@ -204,7 +217,21 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
  *          and its ring(s) hold >= batch transitions (dqn_agent.py:61-62,333-335).
  *   advance_step: 1 when called as the first stage of a learn step (bumps learn_step of
  *          active networks, dqn_agent.py:359); 0 for a stand-alone sample().
- * Results stay in the workspace (rows, r_hat, actions, dones, active flags). */
+ * Results stay in the workspace (rows, r_hat, actions, dones, active flags).
+ *
+ * DMDQN_SAMPLE_PRIORITIZED (proportional prioritized replay, Schaul et al. 2016; independent networks only, and
+ * replay->priority must be set; capacity <= DMDQN_PER_MAX_CAPACITY).  Network g draws from agent g's ring:
+ *   1. S = sum of priority[g][0..C) in float64: chunks of 128 consecutive slots, each summed as lane l (0..31) adding
+ *      slots l, l+32, l+64, l+96 in order, then an xor butterfly (16,8,4,2,1); chunk totals prefix-summed in chunk order.
+ *   2. u_k = ((k + w_k * 2^-32) * S) / B in float64, left to right (stratified: one draw per 1/B of the mass).
+ *   3. the chunk c is the last one whose exclusive prefix is <= u_k (binary search); inside it the slots are walked in
+ *      order adding to a running sum that starts at the prefix, and the first slot whose running sum exceeds u_k is
+ *      drawn.  If rounding carries the walk past the chunk, the last slot of the ring with a non-zero priority is drawn
+ *      (a ring whose priorities are all zero draws slot 0).  Zero-priority slots are never drawn.
+ *   4. importance weights w_i = (p_min / p_i)^beta_t in float64, rounded to float (p_min: the smallest priority drawn
+ *      in this batch; 1 for a slot of priority 0), kept in the workspace (dmdqn_debug_views.is_w).  The oracle (tests/per_oracle.py) restates
+ *      this order, so the drawn rows are bit-exact. */
+#define DMDQN_PER_MAX_CAPACITY (8192 * 128)
 int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                  const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
                  int32_t advance_step, void* workspace, size_t workspace_bytes, void* stream);
@@ -223,6 +250,11 @@ int dmdqn_gather(const dmdqn_dims* dims, const dmdqn_replay* replay, const void*
  * sample, target-net forward + online argmax + TD target, online forward, MSE/Huber,
  * backward, Adam, hard/Polyak target sync.
  *   metrics_out device float[n_nets][DMDQN_METRICS_STRIDE].
+ * With DMDQN_SAMPLE_PRIORITIZED the online kernel (K4a) multiplies each row's loss term and dL/dq by the row's
+ * importance weight (metrics[0] is the weighted batch-mean loss; weight 1 gives the uniform path's bits) and stores
+ * priority[row] = (float)pow(|q(s_i)[a_i] - y_i| + per_eps, per_alpha) (float64), raising priority_max[agent] to it
+ * (atomicMax on the bits: order-independent).  A row whose priority is not finite writes nothing; nor does a row of a
+ * tcgen05 K4a whose bounded waits expired.  A transition drawn twice has one delta, so both rows store the same value.
  * On the tcgen05 path the four kernels of one call form a dataflow chain (programmatic dependent launches:
  * K3 starts under the sample kernel's tail, K4a / K4b take over SMs while the previous kernel is still running
  * and wait on per-tile / per-network flags in the workspace, which the sample kernel resets).  Results are
@@ -318,6 +350,7 @@ typedef struct dmdqn_debug_views {
     /* tcgen05 path: dh2 is never materialised; relu'(h2) as bits, uint32 [n_nets][B][H/32]
      * (bit j of word w of row i = column 32 w + j), dh2 = bit ? g_i * W3[col][a_i] : 0 */
     const uint32_t* relu2_bits;
+    const float* is_w;         /* [n_nets][B] importance-sampling weights of the last prioritized sample */
 } dmdqn_debug_views;
 int dmdqn_debug(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_debug_views* out);
 
