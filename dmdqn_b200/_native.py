@@ -12,6 +12,7 @@ OK, ERR_ARG, ERR_CUDA, ERR_WORKSPACE = 0, -1, -2, -3
 LOSS = {"mse": 0, "huber": 1}
 SAMPLE = {"indices": 0, "fisher_yates": 1, "replacement": 2, "prioritized": 3}
 PER_MAX_CAPACITY = 8192 * 128
+MAX_NSTEP = 16
 ADAM = {"keras": 0, "torch": 1}
 PRECISION = {"fp32": 0, "tf32": 1, "tf32x3": 2}
 METRICS_STRIDE = 8
@@ -38,11 +39,16 @@ class HParams(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("gamma", "learning_rate", "beta1", "beta2", "adam_eps", "tau")] + \
                [(n, C.c_int32) for n in ("target_update_frequency", "loss", "normalize_rewards", "double_dqn",
                                          "adam_form", "sample_mode", "precision")] + \
-               [(n, C.c_double) for n in ("per_alpha", "per_beta0", "per_eps")] + [("per_beta_steps", C.c_int32)]
+               [(n, C.c_double) for n in ("per_alpha", "per_beta0", "per_eps")] + [("per_beta_steps", C.c_int32)] + \
+               [("n_step", C.c_int32)]      # in what was tail padding: sizeof stays 112
 
 
 class DebugViews(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("y", "q_all", "q_next", "tq_all", "rows", "r_hat", "active", "tc_error", "dh1", "dh2", "relu2_bits", "is_w")]
+
+
+class NStepViews(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("next_rows", "discount")]
 
 
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
@@ -88,6 +94,7 @@ SIGNATURES = {
     "dmdqn_ipc_open": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_void_p)]),
     "dmdqn_ipc_close": (C.c_int, [_P, C.c_uint64]),
     "dmdqn_debug": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(DebugViews)]),
+    "dmdqn_debug_nstep": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(NStepViews)]),
     "dmdqn_sync_target": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_double, _P]),
 }
 

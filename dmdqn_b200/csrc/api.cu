@@ -152,9 +152,16 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
     return launch_push(*dims, *replay, obs, act, rew, next_obs, done, in_stride, mask, (cudaStream_t)stream);
 }
 
+static int check_n_step(const dmdqn_hparams* hp) {
+    DMDQN_CHECK_ARG(hp->n_step >= 0 && hp->n_step <= DMDQN_MAX_NSTEP, "n_step=%d must be in [0, %d] (0 and 1: one-step targets)",
+                    hp->n_step, DMDQN_MAX_NSTEP);
+    return DMDQN_OK;
+}
+
 static int check_learn_args(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                             const dmdqn_nets* nets, const void* draws) {
     DMDQN_CHECK_ARG(hp && replay && nets && draws, "NULL argument");
+    if (int rc = check_n_step(hp)) return rc;
     DMDQN_CHECK_ARG(replay->obs && replay->next_obs && replay->act && replay->rew && replay->done &&
                         replay->n_written, "NULL replay pointer");
     DMDQN_CHECK_ARG(nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && nets->learn_step,
@@ -235,7 +242,9 @@ int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn
                     float* metrics_dev, float* metrics_host, void* workspace, size_t workspace_bytes, void* stream) {
     int rc = validate_dims(dims);
     if (rc) return rc;
-    DMDQN_CHECK_ARG(blk && host_block && device_block && metrics_dev && metrics_host, "step_host: NULL argument");
+    DMDQN_CHECK_ARG(hp && blk && host_block && device_block && metrics_dev && metrics_host, "step_host: NULL argument");
+    rc = check_n_step(hp);            // before the copy and the push: a refused step changes nothing
+    if (rc) return rc;
     const size_t offs[6] = {blk->obs_off, blk->next_obs_off, blk->act_off, blk->rew_off, blk->done_off, blk->draws_off};
     for (size_t o : offs) DMDQN_CHECK_ARG(o % 16 == 0 && o < blk->bytes, "step_host: offset %zu is not a multiple of 16 inside the block", o);
     cudaStream_t s = (cudaStream_t)stream;
@@ -352,6 +361,16 @@ int dmdqn_debug(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes,
     out->dh2 = (const float*)(ws + w.dh2);
     out->relu2_bits = (const uint32_t*)(ws + w.mask2);
     out->is_w = (const float*)(ws + w.is_w);
+    return DMDQN_OK;
+}
+
+int dmdqn_debug_nstep(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_nstep_views* out) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    out->next_rows = (const int32_t*)((char*)workspace + w.nrows);
+    out->discount = (const float*)((char*)workspace + w.disc_b);
     return DMDQN_OK;
 }
 

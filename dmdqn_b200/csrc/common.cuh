@@ -75,6 +75,8 @@ struct Workspace {
                                       // kernel, read by K4a)
     size_t sync;                      // tcgen05 path, int32: [0] K4b work counter, [1..3] spare, [4 ..] k4a_done[n_nets], then
                                       // k3_done[n_nets][T]; zeroed by the sample kernel (dataflow flags between the learn kernels)
+    size_t nrows, disc_b;             // [n_nets][B] int32 bootstrap row (agent*C + slot) and float discount of each row's TD
+                                      // target (the drawn row and gamma * (1 - done) for one-step targets; see dmdqn_sample)
     size_t total;
     int tiles;                        // T: row tiles per network of the FFMA kernels (Tile<H>::BM rows); the tcgen05 path's
                                       // 128-row tiles are fewer, so its partials fit the same arrays
@@ -111,6 +113,8 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
     w.part_b1 = take(nt * d.hidden * 4);
     w.is_w = take(nb * 4);
     w.sync = take((4 + (size_t)d.n_nets + nt) * 4);
+    w.nrows = take(nb * 4);
+    w.disc_b = take(nb * 4);
     w.total = off;
     return w;
 }
@@ -127,14 +131,13 @@ struct LearnArgs {
     Layout L;
     dmdqn_replay rp;
     dmdqn_nets nets;
-    float gamma;
     int loss, double_dqn;
     int loss_batch;                   // batch the loss mean runs over (== batch, or the global batch when ranks split it)
     float one_m_b1, one_m_b2, tau;    // Adam constants of the call; the per-step scalars are in adam_sc
     int ws_tiles;                     // Workspace::tiles: row tiles of the FFMA kernels, the per-network stride of k3_done
     int tc_tiles;                     // tcgen05 path: 128-row tiles per network (its K3 / K4a items and part_* slots)
-    const int32_t *rows, *act_b, *active;
-    const float *r_hat, *done_b;
+    const int32_t *rows, *nrows, *act_b, *active;     // nrows: bootstrap rows, whose next_obs K3 reads as s'
+    const float *r_hat, *disc_b;                       // TD target y = r_hat + disc_b * Q_tgt(s')
     const float4* adam_sc;
     float *y, *q_all, *q_next, *tq_all, *h1, *dh1, *dh2;
     float *part_loss, *part_b3, *part_w3, *part_b2, *part_b1;

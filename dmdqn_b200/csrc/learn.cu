@@ -229,8 +229,8 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs 
     const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM;
     Smem<H> S(smem, Dp);
     const Coord<H> c;
-    const int32_t* rows = A.rows + (size_t)g * B;
-    gather_tile<H>(S.Xs, S.ldx, A.rp.next_obs, rows, r0, B, Dp);
+    const int32_t* nrows = A.nrows + (size_t)g * B;
+    gather_tile<H>(S.Xs, S.ldx, A.rp.next_obs, nrows, r0, B, Dp);
 
     float acc[8][8];
 #pragma unroll 1
@@ -256,8 +256,8 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs 
         }
         const float tq = A.double_dqn ? qt[best] : tmax;
         const size_t o = (size_t)g * B + gr;
-        // targets = r + gamma * (1 - done) * target_q, left to right (:347)
-        A.y[o] = A.r_hat[o] + (A.gamma * (1.0f - A.done_b[o])) * tq;
+        // targets = r + gamma * (1 - done) * target_q, left to right (:347); the sample kernel formed the discount
+        A.y[o] = A.r_hat[o] + A.disc_b[o] * tq;
         for (int k = 0; k < 4; ++k) {
             A.q_next[o * 4 + k] = qo[k];
             A.tq_all[o * 4 + k] = qt[k];
@@ -685,7 +685,6 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
     A.L = make_layout(d.obs_stride, d.hidden);
     A.rp = rp;
     A.nets = nets;
-    A.gamma = (float)hp.gamma;
     A.loss = hp.loss;
     A.double_dqn = hp.double_dqn;
     A.loss_batch = loss_batch > 0 ? loss_batch : d.batch;
@@ -694,10 +693,11 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
     A.tau = (float)hp.tau;
     A.ws_tiles = w.tiles;
     A.rows = reinterpret_cast<const int32_t*>(ws + w.rows);
+    A.nrows = reinterpret_cast<const int32_t*>(ws + w.nrows);
     A.act_b = reinterpret_cast<const int32_t*>(ws + w.act_b);
     A.active = reinterpret_cast<const int32_t*>(ws + w.active);
     A.r_hat = reinterpret_cast<const float*>(ws + w.r_hat);
-    A.done_b = reinterpret_cast<const float*>(ws + w.done_b);
+    A.disc_b = reinterpret_cast<const float*>(ws + w.disc_b);
     A.adam_sc = reinterpret_cast<const float4*>(ws + w.adam_sc);
     A.y = reinterpret_cast<float*>(ws + w.y);
     A.q_all = reinterpret_cast<float*>(ws + w.q_all);

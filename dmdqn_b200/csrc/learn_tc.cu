@@ -695,7 +695,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, c
         int q = k3_next(A, blockIdx.x, n_items);
         if (q < n_items) {
             const int g = (q >> 1) / A.tc_tiles, rt = (q >> 1) % A.tc_tiles;
-            xg.begin(A.rp.next_obs, A.rows + (size_t)g * B, rt * BM, B, Dp, ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride, A.L);
+            xg.begin(A.rp.next_obs, A.nrows + (size_t)g * B, rt * BM, B, Dp, ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride, A.L);
         }
         int q_last = -1;                                       // the last item is published here, the others by the MMA lane
         while (q < n_items) {
@@ -718,7 +718,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, c
             const int qn = k3_next(A, q + gridDim.x, n_items);
             if (qn < n_items) {                                // the next tile's rows travel while layer 2 runs
                 const int gn = (qn >> 1) / A.tc_tiles, rtn = (qn >> 1) % A.tc_tiles;
-                xg.begin(A.rp.next_obs, A.rows + (size_t)gn * B, rtn * BM, B, Dp,
+                xg.begin(A.rp.next_obs, A.nrows + (size_t)gn * B, rtn * BM, B, Dp,
                          ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)gn * A.L.stride, A.L);
             }
             ok = wait_gemm(sbase, ring, ok);
@@ -855,7 +855,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, c
                     }
                 }
                 tq = A.double_dqn ? tq : tmax;
-                yi = A.r_hat[sb + gr] + (A.gamma * (1.0f - A.done_b[sb + gr])) * tq;
+                yi = A.r_hat[sb + gr] + A.disc_b[sb + gr] * tq;
                 if (e.part == 0) A.y[sb + gr] = yi;
             }
             const int ai_pre = valid ? A.act_b[sb + gr] : 0;

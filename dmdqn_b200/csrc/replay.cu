@@ -53,6 +53,29 @@ __device__ __forceinline__ double tree_sum(int n, int lane, F elem) {
     return acc;
 }
 
+// n-step return of a row whose first-step term is z0: the later rewards of rows j+1 .. j+m-1 (ring row `row` = row j)
+// are read again here, L1/L2-hot since the lookahead read their done flags; every load is issued before the sum.
+// R = z0; g = 1; for k = 1..m-1: g = g * gamma; R = R + g * z_k, float64 with separate multiply and add.
+__device__ __forceinline__ double nstep_return(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, int row,
+                                               int m, double z0, double mean, double denom, bool normalize) {
+    if (m <= 1) return z0;
+    const int C = d.capacity, agent = row / C, slot = row - agent * C;
+    const double* rw = rp.rew + (size_t)agent * C;
+    double r[DMDQN_MAX_NSTEP - 1];
+#pragma unroll
+    for (int k = 1; k < DMDQN_MAX_NSTEP; ++k) r[k - 1] = k < m ? rw[slot + k < C ? slot + k : slot + k - C] : 0.0;
+    double ret = z0, gk = 1.0;
+#pragma unroll
+    for (int k = 1; k < DMDQN_MAX_NSTEP; ++k) {
+        if (k < m) {
+            gk = __dmul_rn(gk, hp.gamma);
+            const double z = normalize ? __ddiv_rn(__dsub_rn(r[k - 1], mean), denom) : r[k - 1];
+            ret = __dadd_rn(ret, __dmul_rn(gk, z));
+        }
+    }
+    return ret;
+}
+
 // One CTA per network.  smem: js[B] (draws in, then j_i), pt[B], words[B] (logical indices out), rs[B].
 //
 // Draw without replacement = CPython random.sample's pool path with randbelow(m) := (w*m) >> 32
@@ -66,13 +89,16 @@ __device__ __forceinline__ double tree_sum(int n, int lane, F elem) {
 // the W chains (almost always of length 0 or 1) are chased read-only.  Same integers as the sequential
 // loop for every input (oracle/replay.py fisher_yates_indices replays the loop itself).
 // PER: DMDQN_SAMPLE_PRIORITIZED (its own instantiation, so the uniform modes compile to the same code as without it).
-template <bool PER>
+// NSTEP: hp.n_step > 1, n-step returns (include/dmdqn_b200.h dmdqn_sample; tests/nstep_oracle.py restates every step).  The
+// one-step instantiation writes the drawn row as the bootstrap row and gamma * (1 - done) as the discount.
+template <bool PER, bool NSTEP>
 __global__ void __launch_bounds__(kSampleThreads)
 sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restrict__ learn_step,
               const uint32_t* __restrict__ draws, const uint8_t* __restrict__ learn_mask, int advance,
               int32_t* __restrict__ rows, float* __restrict__ r_hat, int32_t* __restrict__ act_b,
               float* __restrict__ done_b, int32_t* __restrict__ active, float4* __restrict__ adam_sc,
-              int32_t* __restrict__ sync, int tiles, float* __restrict__ is_w) {
+              int32_t* __restrict__ sync, int tiles, float* __restrict__ is_w, int32_t* __restrict__ nrows,
+              float* __restrict__ disc_b) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int B = d.batch, Bp = (B + 1) & ~1;
     int* js = reinterpret_cast<int*>(smem_raw);
@@ -254,10 +280,41 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
         rows[(size_t)g * B + i] = row;
         // (an L2 prefetch of the two sampled rows was measured here: +6 us in this kernel, nothing gained in K3 / K4a)
         act_b[(size_t)g * B + i] = rp.act[row];
-        done_b[(size_t)g * B + i] = rp.done[row] ? 1.f : 0.f;
+        if constexpr (!NSTEP) {
+            const bool dn = rp.done[row];
+            done_b[(size_t)g * B + i] = dn ? 1.f : 0.f;
+            js[i] = row;                                // the draw's scratch is free now: row and done for the pass below
+            pt[i] = dn;
+        }
         rs[i] = rp.rew[row];
+        if constexpr (NSTEP) {
+            // the return covers rows j .. j+m-1 of this agent's ring: up to n_step, the first done, the newest row
+            const int C = d.capacity;
+            const int j = per ? (int)(((long long)slot - (nw - sz) % C + C) % C) : lj;
+            const int lim = min(hp.n_step, (int)sz - j);
+            const uint8_t* dn = rp.done + (size_t)agent * C;
+            unsigned bits = 0;                          // bit k: row j+k is done; every load is issued before the scan
+#pragma unroll
+            for (int k = 0; k < DMDQN_MAX_NSTEP; ++k)
+                if (k < lim && dn[slot + k < C ? slot + k : slot + k - C]) bits |= 1u << k;
+            const int m = bits ? __ffs(bits) : lim;
+            double gm = hp.gamma;                       // gamma^m, float64, left to right
+            for (int k = 1; k < m; ++k) gm = __dmul_rn(gm, hp.gamma);
+            const int last = slot + m - 1;
+            nrows[(size_t)g * B + i] = agent * C + (last < C ? last : last - C);
+            done_b[(size_t)g * B + i] = bits ? 1.f : 0.f;      // the return ends on its first done, if any
+            disc_b[(size_t)g * B + i] = bits ? 0.f : (float)gm;
+            js[i] = row;                                // the draw's scratch is free now: row and m for the reward pass
+            pt[i] = m;
+        }
     }
     __syncthreads();
+    if constexpr (!NSTEP) {     // one-step targets bootstrap from the drawn row: warps 1.. write them while warp 0 sums
+        for (int i = tid - 32; tid >= 32 && i < B; i += kSampleThreads - 32) {
+            nrows[(size_t)g * B + i] = js[i];
+            disc_b[(size_t)g * B + i] = (float)hp.gamma * (1.0f - (pt[i] ? 1.f : 0.f));
+        }
+    }
     if (hp.normalize_rewards) {                         // dqn_agent.py:66-69, float64; warp 0 keeps the canonical tree
         if (tid < 32) {
             const double mean = __ddiv_rn(tree_sum(B, lane, [&](int i) { return rs[i]; }), (double)B);
@@ -269,10 +326,13 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
         }
         __syncthreads();
         const double mean = stat[0], denom = stat[1];
-        for (int i = tid; i < B; i += kSampleThreads)
-            r_hat[(size_t)g * B + i] = (float)__ddiv_rn(__dsub_rn(rs[i], mean), denom);
+        for (int i = tid; i < B; i += kSampleThreads) {
+            const double z = __ddiv_rn(__dsub_rn(rs[i], mean), denom);
+            r_hat[(size_t)g * B + i] = (float)(NSTEP ? nstep_return(d, hp, rp, js[i], pt[i], z, mean, denom, true) : z);
+        }
     } else {
-        for (int i = tid; i < B; i += kSampleThreads) r_hat[(size_t)g * B + i] = (float)rs[i];
+        for (int i = tid; i < B; i += kSampleThreads)
+            r_hat[(size_t)g * B + i] = (float)(NSTEP ? nstep_return(d, hp, rp, js[i], pt[i], rs[i], 0.0, 1.0, false) : rs[i]);
     }
 }
 
@@ -283,7 +343,8 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
 // the pieces are exchanged through shuffles so that lane l writes columns l, l + 32, l + 64 (consecutive lanes ->
 // consecutive addresses, whole 128-byte segments).
 __global__ void __launch_bounds__(128)
-gather_kernel(dmdqn_dims d, dmdqn_replay rp, const int32_t* __restrict__ rows, const float* __restrict__ r_hat,
+gather_kernel(dmdqn_dims d, dmdqn_replay rp, const int32_t* __restrict__ rows, const int32_t* __restrict__ nrows,
+              const float* __restrict__ r_hat,
               const int32_t* __restrict__ act_b, const float* __restrict__ done_b,
               const int32_t* __restrict__ active, float* __restrict__ states, int32_t* __restrict__ actions,
               float* __restrict__ rewards, float* __restrict__ next_states, float* __restrict__ dones,
@@ -295,12 +356,13 @@ gather_kernel(dmdqn_dims d, dmdqn_replay rp, const int32_t* __restrict__ rows, c
     const int g = (int)(r / d.batch);
     if (active_out && (r % d.batch) == 0 && lane == 0) active_out[g] = active[g];
     if (!active[g]) return;
-    const size_t src = (size_t)rows[r] * d.obs_stride;
+    const size_t src = (size_t)rows[r] * d.obs_stride;             // s of the drawn row
+    const size_t nsrc = (size_t)nrows[r] * d.obs_stride;           // s' of its bootstrap row (n-step returns)
     const int q = d.obs_stride >> 2;                               // 16-byte pieces per row (<= 32: obs_stride <= 128)
     float4 s4 = make_float4(0.f, 0.f, 0.f, 0.f), n4 = s4;
     if (lane < q) {
         s4 = __ldg(reinterpret_cast<const float4*>(rp.obs + src) + lane);
-        n4 = __ldg(reinterpret_cast<const float4*>(rp.next_obs + src) + lane);
+        n4 = __ldg(reinterpret_cast<const float4*>(rp.next_obs + nsrc) + lane);
     }
 #pragma unroll
     for (int k = 0; k < 4; ++k) {                                   // column c = 32 k + lane lives in piece c / 4 = 8 k + lane / 4, component lane % 4
@@ -342,15 +404,18 @@ int launch_sample(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repl
                     "capacity=%d: prioritized replay serves rings of up to %d slots", d.capacity, DMDQN_PER_MAX_CAPACITY);
     const size_t smem = (size_t)((d.batch + 1) & ~1) * (3 * 4 + 8) +
                         (per ? (size_t)((d.capacity + kPerChunk - 1) / kPerChunk + 1) * 8 : 0);
-    static size_t configured[2][kMaxDevices] = {};
-    const auto kernel = per ? sample_kernel<true> : sample_kernel<false>;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kernel), smem, configured[per])) return rc;
+    const bool nstep = hp.n_step > 1;
+    static size_t configured[4][kMaxDevices] = {};
+    const auto kernel = per ? (nstep ? sample_kernel<true, true> : sample_kernel<true, false>)
+                            : (nstep ? sample_kernel<false, true> : sample_kernel<false, false>);
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kernel), smem, configured[2 * per + nstep])) return rc;
     kernel<<<d.n_nets, kSampleThreads, smem, s>>>(
         d, hp, rp, nets.learn_step, static_cast<const uint32_t*>(draws), learn_mask, advance,
         reinterpret_cast<int32_t*>(ws + w.rows), reinterpret_cast<float*>(ws + w.r_hat),
         reinterpret_cast<int32_t*>(ws + w.act_b), reinterpret_cast<float*>(ws + w.done_b),
         reinterpret_cast<int32_t*>(ws + w.active), reinterpret_cast<float4*>(ws + w.adam_sc),
-        reinterpret_cast<int32_t*>(ws + w.sync), w.tiles, reinterpret_cast<float*>(ws + w.is_w));
+        reinterpret_cast<int32_t*>(ws + w.sync), w.tiles, reinterpret_cast<float*>(ws + w.is_w),
+        reinterpret_cast<int32_t*>(ws + w.nrows), reinterpret_cast<float*>(ws + w.disc_b));
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
@@ -360,7 +425,8 @@ int launch_gather(const dmdqn_dims& d, const dmdqn_replay& rp, const char* ws, c
                   int32_t* active_out, cudaStream_t s) {
     const long long total = (long long)d.n_nets * d.batch;
     gather_kernel<<<(unsigned)((total + 3) / 4), 128, 0, s>>>(
-        d, rp, reinterpret_cast<const int32_t*>(ws + w.rows), reinterpret_cast<const float*>(ws + w.r_hat),
+        d, rp, reinterpret_cast<const int32_t*>(ws + w.rows), reinterpret_cast<const int32_t*>(ws + w.nrows),
+        reinterpret_cast<const float*>(ws + w.r_hat),
         reinterpret_cast<const int32_t*>(ws + w.act_b), reinterpret_cast<const float*>(ws + w.done_b),
         reinterpret_cast<const int32_t*>(ws + w.active), states, actions, rewards, next_states, dones,
         active_out);

@@ -36,6 +36,8 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # prioritized replay (sample_mode "prioritized"): priority exponent, initial importance exponent (annealed to 1 over
     # per_beta_steps learn steps), priority offset
     "per_alpha": 0.6, "per_beta": 0.4, "per_beta_steps": 100000, "per_eps": 1e-6,
+    # n-step returns: transitions per TD target (1 = the reference's one-step target), at most N.MAX_NSTEP
+    "n_step": 1,
 }
 
 
@@ -87,6 +89,9 @@ class AgentGroup:
         if self.prioritized and self.shared:
             raise ValueError("sample_mode='prioritized' serves independent networks only: it cannot be combined with "
                              "share_parameters=true")
+        self.n_step = int(cfg["n_step"])
+        if not 1 <= self.n_step <= N.MAX_NSTEP:
+            raise ValueError(f"n_step={cfg['n_step']}: must be in [1, {N.MAX_NSTEP}] (1 = one-step TD targets)")
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -114,7 +119,7 @@ class AgentGroup:
             int(cfg["target_update_frequency"]), N.LOSS[cfg["loss"]], int(bool(cfg["normalize_rewards"])),
             int(bool(cfg["double_dqn"])), N.ADAM[cfg["adam_form"]], N.SAMPLE[cfg["sample_mode"]],
             N.PRECISION[cfg["precision"]], float(cfg["per_alpha"]), float(cfg["per_beta"]), float(cfg["per_eps"]),
-            int(cfg["per_beta_steps"]))
+            int(cfg["per_beta_steps"]), self.n_step)
 
         dev, n, c, dp, g = self.device, self.n_agents, self.capacity, self.obs_stride, self.n_nets
         if _parent is None:
@@ -515,11 +520,14 @@ class AgentGroup:
             off = ptr - base
             nbytes = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
             return self.workspace[off:off + nbytes].view(dtype).view(*shape)
+        nv = N.NStepViews()
+        N.check(self.lib.dmdqn_debug_nstep(C.byref(self.dims), _ptr(self.workspace), self.workspace.numel(), C.byref(nv)))
         out = {"y": view(v.y, torch.float32, (g, b)), "q_all": view(v.q_all, torch.float32, (g, b, 4)),
                "q_next": view(v.q_next, torch.float32, (g, b, 4)), "tq_all": view(v.tq_all, torch.float32, (g, b, 4)),
                "rows": view(v.rows, torch.int32, (g, b)), "r_hat": view(v.r_hat, torch.float32, (g, b)),
                "active": view(v.active, torch.int32, (g,)), "tc_error": view(v.tc_error, torch.int32, (1,)),
-               "is_weights": view(v.is_w, torch.float32, (g, b))}
+               "is_weights": view(v.is_w, torch.float32, (g, b)),
+               "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
         if self.hp.precision != 0:
             # the tcgen05 path keeps its activation scratch transposed ([feature][batch]) and never
             # materialises dh2: "dh2" is relu'(h2) as 0/1 here (its non-zero pattern is what the tests use)

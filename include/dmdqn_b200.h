@@ -129,7 +129,11 @@ typedef struct dmdqn_hparams {
      * learn_step after the increment (per_beta_steps <= 0: beta_t = per_beta0) */
     double  per_alpha, per_beta0, per_eps;
     int32_t per_beta_steps;
+    /* n-step returns (every sample mode; see dmdqn_sample): transitions per TD target, 0 or 1 = one-step,
+     * at most DMDQN_MAX_NSTEP.  Placed in what was the struct's tail padding: offset 108, sizeof stays 112. */
+    int32_t n_step;
 } dmdqn_hparams;
+#define DMDQN_MAX_NSTEP 16
 
 /* Per-network learn outputs, 8 floats each: loss, q_mean, q_std (population, over the
  * [B,A] online Q of the sampled states), action histogram[4], learned flag (0/1)
@@ -230,7 +234,20 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
  *      (a ring whose priorities are all zero draws slot 0).  Zero-priority slots are never drawn.
  *   4. importance weights w_i = (p_min / p_i)^beta_t in float64, rounded to float (p_min: the smallest priority drawn
  *      in this batch; 1 for a slot of priority 0), kept in the workspace (dmdqn_debug_views.is_w).  The oracle (tests/per_oracle.py) restates
- *      this order, so the drawn rows are bit-exact. */
+ *      this order, so the drawn rows are bit-exact.
+ *
+ * n-step returns (hp->n_step = n > 1, any sample mode).  They assume that successive pushes of one agent are successive
+ * steps in time, which is what a train loop that pushes every agent once per environment step does.  For a drawn row at
+ * logical index j of agent a's ring (size sz; in prioritized mode j = (slot - (n_written - sz)) mod C; with shared
+ * parameters the lookahead stays in the row's own agent's ring):
+ *   m    = min(n, steps up to and including the first done at or after j, sz - j)   (the newest rows get shorter returns)
+ *   z_k  = (rew[j+k] - mu) / sigma with the batch statistics of the first-step rewards (normalize_rewards), else rew[j+k]
+ *   R    = z_0; g = 1; for k = 1..m-1: g = g * gamma; R = R + g * z_k   (float64, no FMA; rounded to float)
+ *   the bootstrap row is j + m - 1 (its next_obs is s'), the terminal flag is its done, and the discount is 0 if it
+ *   is done, else (float)(gamma^m) with gamma^m the float64 product formed left to right.
+ * The workspace keeps R as r_hat, the terminal flag as the batch's dones, and the bootstrap rows and discounts
+ * (dmdqn_debug_nstep).  n = 0 or 1 is the one-step target: R = r_hat, discount = (float)gamma * (1 - done), and the
+ * bootstrap row is the drawn row.  n < 0 or n > DMDQN_MAX_NSTEP is refused. */
 #define DMDQN_PER_MAX_CAPACITY (8192 * 128)
 int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                  const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
@@ -240,7 +257,9 @@ int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_re
  * dqn_agent.py:80-85) from the workspace of the last dmdqn_sample.
  *   states, next_states device float[n_nets][batch][obs_dim] (dense, no padding)
  *   actions int32, rewards float (z-scored), dones float: device [n_nets][batch]
- *   active_out device int32[n_nets] or NULL. */
+ *   active_out device int32[n_nets] or NULL.
+ * With n-step returns (hp->n_step > 1 in dmdqn_sample) next_states are those of each row's bootstrap row, rewards are
+ * the returns R and dones the terminal flags of the returns; states and actions stay those of the drawn rows. */
 int dmdqn_gather(const dmdqn_dims* dims, const dmdqn_replay* replay, const void* workspace,
                  size_t workspace_bytes, float* states, int32_t* actions, float* rewards,
                  float* next_states, float* dones, int32_t* active_out, void* stream);
@@ -250,6 +269,8 @@ int dmdqn_gather(const dmdqn_dims* dims, const dmdqn_replay* replay, const void*
  * sample, target-net forward + online argmax + TD target, online forward, MSE/Huber,
  * backward, Adam, hard/Polyak target sync.
  *   metrics_out device float[n_nets][DMDQN_METRICS_STRIDE].
+ * The TD target of row i is y_i = R_i + discount_i * Q_tgt(s'_i), with s' the next_obs of the row's bootstrap row
+ * (dmdqn_sample: the drawn row itself, gamma * (1 - done) and the one-step reward unless hp->n_step > 1).
  * With DMDQN_SAMPLE_PRIORITIZED the online kernel (K4a) multiplies each row's loss term and dL/dq by the row's
  * importance weight (metrics[0] is the weighted batch-mean loss; weight 1 gives the uniform path's bits) and stores
  * priority[row] = (float)pow(|q(s_i)[a_i] - y_i| + per_eps, per_alpha) (float64), raising priority_max[agent] to it
@@ -353,6 +374,12 @@ typedef struct dmdqn_debug_views {
     const float* is_w;         /* [n_nets][B] importance-sampling weights of the last prioritized sample */
 } dmdqn_debug_views;
 int dmdqn_debug(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_debug_views* out);
+/* n-step views of the last sample (its own struct: dmdqn_debug_views keeps its size for existing callers):
+ * next_rows int32[n_nets][B] (agent*C + slot of each row's bootstrap row), discount float[n_nets][B]. */
+typedef struct dmdqn_nstep_views {
+    const int32_t* next_rows; const float* discount;
+} dmdqn_nstep_views;
+int dmdqn_debug_nstep(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_nstep_views* out);
 
 /* theta_tgt <- theta for the networks whose mask is set (NULL = all).
  * Replaces DQNAgent.update_target_network (dqn_agent.py:382-384) when called explicitly. */
