@@ -89,8 +89,9 @@ __device__ __forceinline__ double nstep_return(const dmdqn_dims& d, const dmdqn_
 // the W chains (almost always of length 0 or 1) are chased read-only.  Same integers as the sequential
 // loop for every input (oracle/replay.py fisher_yates_indices replays the loop itself).
 // PER: DMDQN_SAMPLE_PRIORITIZED (its own instantiation, so the uniform modes compile to the same code as without it).
-// NSTEP: hp.n_step > 1, n-step returns (include/dmdqn_b200.h dmdqn_sample; tests/nstep_oracle.py restates every step).  The
+// NSTEP: hp.n_step > 1, n-step returns (include/dmdqn_b200.h dmdqn_sample; tests/replay_oracle.py restates every step).  The
 // one-step instantiation writes the drawn row as the bootstrap row and gamma * (1 - done) as the discount.
+// (Running n_step 1 through the n-step path instead was measured slower at n_step 1: DESIGN.md section 8.)
 template <bool PER, bool NSTEP>
 __global__ void __launch_bounds__(kSampleThreads)
 sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restrict__ learn_step,
@@ -149,7 +150,7 @@ sample_kernel(dmdqn_dims d, dmdqn_hparams hp, dmdqn_replay rp, int32_t* __restri
     };
 
     if constexpr (PER) {
-        // Proportional prioritized replay (include/dmdqn_b200.h; tests/per_oracle.py restates every step): words[i] is
+        // Proportional prioritized replay (include/dmdqn_b200.h; tests/replay_oracle.py restates every step): words[i] is
         // the drawn PHYSICAL slot here, not a logical index.
         const int C = d.capacity, nch = (C + kPerChunk - 1) / kPerChunk, warp = tid >> 5;
         const float* __restrict__ pr = rp.priority + (size_t)g * C;

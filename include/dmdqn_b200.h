@@ -233,8 +233,8 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
  *      drawn.  If rounding carries the walk past the chunk, the last slot of the ring with a non-zero priority is drawn
  *      (a ring whose priorities are all zero draws slot 0).  Zero-priority slots are never drawn.
  *   4. importance weights w_i = (p_min / p_i)^beta_t in float64, rounded to float (p_min: the smallest priority drawn
- *      in this batch; 1 for a slot of priority 0), kept in the workspace (dmdqn_debug_views.is_w).  The oracle (tests/per_oracle.py) restates
- *      this order, so the drawn rows are bit-exact.
+ *      in this batch; 1 for a slot of priority 0), kept in the workspace (dmdqn_debug_views.is_w).  The oracle
+ *      (tests/replay_oracle.py) restates this order, so the drawn rows are bit-exact.
  *
  * n-step returns (hp->n_step = n > 1, any sample mode).  They assume that successive pushes of one agent are successive
  * steps in time, which is what a train loop that pushes every agent once per environment step does.  For a drawn row at

@@ -74,38 +74,45 @@ def zscore(rewards: np.ndarray) -> np.ndarray:
     return (r - np.mean(r)) / (np.std(r) + 1e-8)
 
 
-def zscore_canonical(rewards: np.ndarray) -> np.ndarray:
-    """Same statistic with the FIXED summation tree the CUDA kernel uses, so the
-    device result can be compared bit-for-bit (float64 ops are IEEE on both sides):
+def _tree_sum(x: np.ndarray) -> np.ndarray:
+    """Canonical float64 sum over the last axis: lane l (0..31) adds x[l], x[l+32], ... in
+    order, then the lanes are combined with an xor butterfly (offsets 16,8,4,2,1)."""
+    pad = (-x.shape[-1]) % 32
+    if pad:
+        x = np.concatenate([x, np.zeros(x.shape[:-1] + (pad,), np.float64)], axis=-1)
+    x = x.reshape(x.shape[:-1] + (-1, 32))
+    acc = np.zeros(x.shape[:-2] + (32,), np.float64)
+    for row in range(x.shape[-2]):
+        acc = acc + x[..., row, :]
+    lanes = np.arange(32)
+    for off in (16, 8, 4, 2, 1):
+        acc = acc + acc[..., lanes ^ off]
+    return acc[..., 0]
 
-      lane l (0..31) sums r[l], r[l+32], ... sequentially; lanes are combined with an
-      xor butterfly (offsets 16,8,4,2,1); mean = total / B; the squared deviations
-      ``(r-mean)*(r-mean)`` (multiply rounded, then added: no FMA) go through the same
-      tree; std = sqrt(total / B); out = (r - mean) / (std + 1e-8).
+
+def zscore_stats(rewards: np.ndarray) -> tuple[np.ndarray, np.ndarray]:
+    """``(mean, std + 1e-8)`` of ``[..., B]`` float64 rewards with the CUDA kernel's fixed
+    summation tree (:func:`_tree_sum`): mean = total / B; the squared deviations
+    ``(r-mean)*(r-mean)`` (multiply rounded, then added: no FMA) go through the same tree;
+    std = sqrt(total / B).  The n-step returns normalise every reward with these."""
+    r = np.asarray(rewards, dtype=np.float64)
+    b = r.shape[-1]
+    mean = _tree_sum(r) / b
+    dev = r - mean[..., None]
+    var = _tree_sum(dev * dev) / b
+    return mean, np.sqrt(var) + 1e-8
+
+
+def zscore_canonical(rewards: np.ndarray) -> np.ndarray:
+    """Same statistic as :func:`zscore` with the FIXED summation tree the CUDA kernel uses
+    (:func:`zscore_stats`), so the device result can be compared bit-for-bit (float64 ops
+    are IEEE on both sides): out = (r - mean) / (std + 1e-8).
 
     ``rewards`` is ``[..., B]`` float64; leading dims are independent batches.
     """
     r = np.asarray(rewards, dtype=np.float64)
-    b = r.shape[-1]
-
-    def tree_sum(x: np.ndarray) -> np.ndarray:
-        pad = (-b) % 32
-        if pad:
-            x = np.concatenate([x, np.zeros(x.shape[:-1] + (pad,), np.float64)], axis=-1)
-        x = x.reshape(x.shape[:-1] + (-1, 32))
-        acc = np.zeros(x.shape[:-2] + (32,), np.float64)
-        for row in range(x.shape[-2]):
-            acc = acc + x[..., row, :]
-        lanes = np.arange(32)
-        for off in (16, 8, 4, 2, 1):
-            acc = acc + acc[..., lanes ^ off]
-        return acc[..., 0]
-
-    mean = tree_sum(r) / b
-    dev = r - mean[..., None]
-    var = tree_sum(dev * dev) / b
-    std = np.sqrt(var)
-    return dev / (std[..., None] + 1e-8)
+    mean, denom = zscore_stats(r)
+    return (r - mean[..., None]) / denom[..., None]
 
 
 # ----------------------------------------------------------------------------

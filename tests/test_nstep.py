@@ -5,8 +5,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
-import nstep_oracle as NS
-from oracle.replay import RingReplay, zscore_canonical
+import replay_oracle as NS
+from oracle.replay import RingReplay, zscore_canonical, zscore_stats
 
 
 def _ring(capacity, n_written, done_logical, seed=0):
@@ -57,7 +57,7 @@ def test_oracle_matches_a_naive_walk_over_the_deque(cap, nw, dones, n, normalize
     logical = np.arange(size)
     slots = ring.logical_to_slot(0, logical)
     out = NS.nstep_batch(ring, np.zeros(size, np.int64), slots, n, gamma, normalize)
-    mean, denom = NS.batch_stats(ring.rew[0, slots]) if normalize else (0.0, 1.0)
+    mean, denom = zscore_stats(ring.rew[0, slots]) if normalize else (0.0, 1.0)
     for j in range(size):
         ret, disc, last, term = _naive(ring, j, n, gamma, mean, denom)
         assert out["next_slot"][j] == ring.logical_to_slot(0, np.array([last]))[0], f"row {j}: bootstrap row"
@@ -92,19 +92,19 @@ def test_one_step_is_ring_gather_bit_for_bit(n, normalize):
 
 def test_batch_stats_are_the_canonical_zscore():
     r = -np.random.default_rng(2).integers(0, 5000, 300) * 0.7
-    mean, denom = NS.batch_stats(r)
+    mean, denom = zscore_stats(r)
     assert np.array_equal((r - mean) / denom, zscore_canonical(r))
 
 
 def test_per_row_discounts_of_gamma_times_one_minus_done_give_the_one_step_learn_step():
-    from per_oracle import WeightedStackedOracle
+    from oracle.dqn import StackedOracle
     rng = np.random.default_rng(3)
     n, b = 2, 16
     s, s2 = rng.integers(-1, 20, (n, b, 89)).astype(np.float32), rng.integers(-1, 20, (n, b, 89)).astype(np.float32)
     a, r = rng.integers(0, 4, (n, b)).astype(np.int32), rng.standard_normal((n, b)).astype(np.float32)
     d = (rng.random((n, b)) < 0.2).astype(np.float32)
     kw = dict(gamma=0.99, learning_rate=5e-4, loss="mse", target_update_frequency=3, seed0=11)
-    ns, ws = NS.NStepStackedOracle(n, 89, [32, 32], 4, **kw), WeightedStackedOracle(n, 89, [32, 32], 4, **kw)
+    ns, ws = NS.ReplayStackedOracle(n, 89, [32, 32], 4, **kw), StackedOracle(n, 89, [32, 32], 4, **kw)
     disc = np.float32(0.99) * (np.float32(1.0) - d)
     for _ in range(2):
         x, y = ns.learn_on_batch(s, a, r, s2, d, discounts=disc), ws.learn_on_batch(s, a, r, s2, d)

@@ -7,7 +7,7 @@ import pytest
 import torch
 from scipy import stats
 
-import per_oracle as P
+import replay_oracle as P
 
 
 def _searchsorted_draw(priority, u):
@@ -91,7 +91,7 @@ def _oracle_batch(seed, n=2, b=16, h=32, loss="mse"):
     r = rng.standard_normal((n, b)).astype(np.float32)
     d = (rng.random((n, b)) < 0.1).astype(np.float32)
     kw = dict(gamma=0.99, learning_rate=5e-4, loss=loss, target_update_frequency=3, seed0=11)
-    return (s, a, r, s2, d), P.WeightedStackedOracle(n, 89, [h, h], 4, **kw), P.StackedOracle(n, 89, [h, h], 4, **kw)
+    return (s, a, r, s2, d), P.ReplayStackedOracle(n, 89, [h, h], 4, **kw), P.StackedOracle(n, 89, [h, h], 4, **kw)
 
 
 @pytest.mark.parametrize("loss", ["mse", "huber"])
