@@ -88,7 +88,9 @@ SIGNATURES = {
     "dmdqn_learn_grads": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Replay), C.POINTER(Nets), _P, _P,
                                     C.c_int32, _P, _P, _P, C.c_size_t, _P]),
     "dmdqn_adam_apply": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), _P, _P, C.c_size_t, _P]),
-    "dmdqn_allreduce_adam": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.POINTER(Peers), _P, _P, _P,
+    "dmdqn_clip_adam_apply": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), _P, C.c_double, _P, _P,
+                                        C.c_size_t, _P]),
+    "dmdqn_allreduce_adam":(C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.POINTER(Peers), _P, _P, _P,
                                        C.c_size_t, _P]),
     "dmdqn_ipc_export": (C.c_int, [_P, _P, C.POINTER(C.c_uint64)]),
     "dmdqn_ipc_open": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_void_p)]),

@@ -279,6 +279,19 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     return launch_adam_apply(*dims, *hp, *nets, grads, (char*)workspace, w, (cudaStream_t)stream);
 }
 
+int dmdqn_clip_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const float* grads,
+                          double global_clipnorm, float* norms_out, void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(hp && nets && nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && grads,
+                    "clip_adam_apply: NULL argument");
+    DMDQN_CHECK_ARG(global_clipnorm > 0.0 && isfinite(global_clipnorm),
+                    "global_clipnorm=%g must be a positive finite number", global_clipnorm);
+    return launch_clip_adam_apply(*dims, *hp, *nets, grads, global_clipnorm, norms_out, (char*)workspace, w,
+                                  (cudaStream_t)stream);
+}
+
 int dmdqn_allreduce_adam(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_peers* peers,
                          const float* my_loss_src, float* loss_out, void* workspace, size_t workspace_bytes, void* stream) {
     Workspace w;

@@ -238,6 +238,8 @@ bool tc_supported(const dmdqn_dims& d);
 int launch_learn_tc(const LearnArgs& A, int precision, int stages, cudaStream_t s);
 int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads, char* ws,
                       const Workspace& w, cudaStream_t s);
+int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads,
+                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
 int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau,
                        cudaStream_t s);
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,

@@ -589,6 +589,120 @@ __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ g
     }
 }
 
+// Global-norm clipping in front of the same Adam + target sync (dmdqn_clip_adam_apply, include/dmdqn_b200.h): one
+// cluster of kClipCtas CTAs per network.  CTA r of the cluster owns float4s [r * per, (r + 1) * per) of the block
+// [0, b3 + 4): it brings them into shared memory with one bulk copy, forms their float64 sum of squares in a fixed
+// order, and after a cluster barrier every CTA adds the kClipCtas partials over DSMEM in rank order, so all of them
+// hold the same norm n.  The gradient is then read from shared memory, scaled by s = c / max(n, c) and applied by
+// adam_vec4 exactly as adam_apply_kernel applies it; the block is read from HBM once.
+constexpr int kClipCtas = 8;            // the portable cluster size
+constexpr int kClipThreads = 256;
+
+inline int64_t clip_per_cta(const Layout& L) { return ((L.b3 + 4) / 4 + kClipCtas - 1) / kClipCtas; }   // float4s
+
+__device__ __forceinline__ void clip_mbar_wait(uint32_t bar, bool& ok) {
+    unsigned long long t0, t1;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
+    for (;;) {
+        uint32_t done;
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
+                     : "=r"(done) : "r"(bar) : "memory");
+        if (done) return;
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
+        if (t1 - t0 > 2000000000ull) { ok = false; return; }     // ~2 s: a copy that never lands is an error, not a hang
+    }
+}
+
+__global__ void __cluster_dims__(kClipCtas, 1, 1) __launch_bounds__(kClipThreads)
+clip_adam_apply_kernel(const LearnArgs A, const float* __restrict__ grads, int64_t per, double clipnorm,
+                       float* __restrict__ norms_out) {
+    extern __shared__ __align__(16) float4 gsm[];       // this CTA's slice of the gradient block
+    __shared__ __align__(8) uint64_t bar;
+    __shared__ double warp_sum[kClipThreads / 32];
+    __shared__ double part;                             // this CTA's sum of squares: read by every CTA of the cluster
+    __shared__ int part_ok;                             // 0: the copy timed out or the step was poisoned
+    __shared__ float scale_sh;
+    __shared__ int apply_sh;
+    const int g = blockIdx.y, tid = threadIdx.x;
+    const uint32_t rank = blockIdx.x;                   // == %cluster_ctarank: the cluster spans gridDim.x
+    if (!A.active[g]) {                                 // the same for every CTA of the cluster: no barrier is pending
+        if (rank == 0 && tid == 0 && norms_out) norms_out[g] = 0.f;
+        return;
+    }
+    const int64_t n4 = (A.L.b3 + 4) / 4, i0 = (int64_t)rank * per;
+    const int cnt = (int)max((int64_t)0, min(per, n4 - i0));
+    const size_t base = (size_t)g * A.L.stride + (size_t)i0 * 4;
+    const uint32_t sbar = (uint32_t)__cvta_generic_to_shared(&bar);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(sbar) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        if (cnt > 0) {
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(sbar), "r"((uint32_t)cnt * 16u) : "memory");
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                         ::"r"((uint32_t)__cvta_generic_to_shared(gsm)), "l"(grads + base), "r"((uint32_t)cnt * 16u), "r"(sbar)
+                         : "memory");
+        }
+    }
+    __syncthreads();
+    bool ok = true;
+    if (cnt > 0) clip_mbar_wait(sbar, ok);
+    double ss = 0.0;                                    // float squares are exact in float64
+    for (int i = tid; i < cnt; i += kClipThreads) {
+        const float4 v = gsm[i];
+        ss = fma((double)v.x, (double)v.x, ss); ss = fma((double)v.y, (double)v.y, ss);
+        ss = fma((double)v.z, (double)v.z, ss); ss = fma((double)v.w, (double)v.w, ss);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
+    const int any_bad = __syncthreads_or(!ok);
+    if ((tid & 31) == 0) warp_sum[tid >> 5] = ss;
+    __syncthreads();
+    if (tid == 0) {
+        double s = 0.0;
+        for (int w = 0; w < kClipThreads / 32; ++w) s += warp_sum[w];
+        part = s;
+        // a tcgen05 K4b whose bounded waits expired wrote no gradient for this step and set the error flag
+        part_ok = !any_bad && *reinterpret_cast<volatile int*>(A.error) == 0;
+    }
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+    if (tid == 0) {
+        double total = 0.0;
+        int all_ok = 1;
+        const uint32_t mine = (uint32_t)__cvta_generic_to_shared(&part), mine_ok = (uint32_t)__cvta_generic_to_shared(&part_ok);
+        for (uint32_t r = 0; r < kClipCtas; ++r) {       // rank order on every CTA: one n per cluster
+            uint32_t pa, po;
+            double p;
+            int o;
+            asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(pa) : "r"(mine), "r"(r));
+            asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(po) : "r"(mine_ok), "r"(r));
+            asm volatile("ld.shared::cluster.f64 %0, [%1];" : "=d"(p) : "r"(pa) : "memory");
+            asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(o) : "r"(po) : "memory");
+            total += p;
+            all_ok &= o;
+        }
+        const double n = sqrt(total);
+        scale_sh = isfinite(n) ? (float)(clipnorm / fmax(n, clipnorm)) : 1.f;
+        apply_sh = all_ok;
+        if (rank == 0 && norms_out) norms_out[g] = all_ok ? (float)n : 0.f;
+    }
+    __syncthreads();
+    const float s = scale_sh;
+    const bool scaled = s != 1.f;                       // s == 1: the unscaled gradient, as dmdqn_adam_apply reads it
+    if (apply_sh) {                                     // adam_apply_kernel's loop, the gradient from shared memory
+        const AdamStep k = adam_step(A, g);
+#pragma unroll 4
+        for (int i = tid; i < cnt; i += kClipThreads) {
+            float4 g4 = gsm[i];
+            if (scaled) { g4.x *= s; g4.y *= s; g4.z *= s; g4.w *= s; }
+            const float gv[4] = {g4.x, g4.y, g4.z, g4.w};
+            adam_vec4(k, gv, A.nets.theta + base + i * 4, A.nets.adam_m + base + i * 4, A.nets.adam_v + base + i * 4,
+                      A.nets.theta_tgt + base + i * 4);
+        }
+    }
+    // no CTA may leave while a peer can still read its partial
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
 // K5: all-reduce of the shared network's gradient block over NVLink peer memory fused with Adam + target sync
 // (include/dmdqn_b200.h dmdqn_allreduce_adam).  Block b of every rank exchanges its own flag with block b of every
 // peer, so there is no grid-wide dependency inside a GPU and no co-residency requirement; the gradient blocks were
@@ -750,6 +864,18 @@ int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_
                       const Workspace& w, cudaStream_t s) {
     const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
     adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads,
+                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
+    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    const int64_t per = clip_per_cta(A.L);
+    const size_t smem = (size_t)per * 16;
+    static size_t cfg[kMaxDevices] = {};
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, cfg)) return rc;
+    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

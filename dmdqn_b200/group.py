@@ -20,6 +20,7 @@ from __future__ import annotations
 import ctypes as C
 import functools
 import math
+import numbers
 
 import numpy as np
 import torch
@@ -38,6 +39,8 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     "per_alpha": 0.6, "per_beta": 0.4, "per_beta_steps": 100000, "per_eps": 1e-6,
     # n-step returns: transitions per TD target (1 = the reference's one-step target), at most N.MAX_NSTEP
     "n_step": 1,
+    # global-norm gradient clipping (Keras global_clipnorm): None, or c > 0 to scale each network's gradient to a norm <= c
+    "global_clipnorm": None,
 }
 
 
@@ -92,6 +95,11 @@ class AgentGroup:
         self.n_step = int(cfg["n_step"])
         if not 1 <= self.n_step <= N.MAX_NSTEP:
             raise ValueError(f"n_step={cfg['n_step']}: must be in [1, {N.MAX_NSTEP}] (1 = one-step TD targets)")
+        clip = cfg["global_clipnorm"]
+        if clip is not None and (isinstance(clip, bool) or not isinstance(clip, numbers.Real) or not math.isfinite(clip)
+                                 or clip <= 0):
+            raise ValueError(f"global_clipnorm={clip!r}: must be None (no clipping) or a positive finite number")
+        self.global_clipnorm = None if clip is None else float(clip)
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -137,6 +145,9 @@ class AgentGroup:
             # prioritized replay: p^alpha per physical slot (0 = never written) and each ring's largest priority
             self.priority = torch.zeros((n, c), dtype=torch.float32, device=dev) if self.prioritized else None
             self.priority_max = torch.ones((n,), dtype=torch.float32, device=dev) if self.prioritized else None
+            # gradient clipping: the raw gradient blocks of a step and each network's norm before clipping (last step)
+            self.grads = torch.zeros_like(self.theta) if self.global_clipnorm is not None else None
+            self.grad_norms = torch.zeros((g,), dtype=torch.float32, device=dev) if self.global_clipnorm is not None else None
             self.n_written_host = np.zeros((n,), np.int64)       # host mirrors: no device sync
             self.learn_step_host = np.zeros((g,), np.int64)
         else:
@@ -150,6 +161,8 @@ class AgentGroup:
             self.theta, self.theta_tgt = p.theta[j:j + 1], p.theta_tgt[j:j + 1]
             self.adam_m, self.adam_v = p.adam_m[j:j + 1], p.adam_v[j:j + 1]
             self.learn_step = p.learn_step[j:j + 1]
+            self.grads = None if p.grads is None else p.grads[j:j + 1]
+            self.grad_norms = None if p.grad_norms is None else p.grad_norms[j:j + 1]
             self.n_written_host = p.n_written_host[i:i + 1]
             self.learn_step_host = p.learn_step_host[j:j + 1]
         self.replay = N.Replay(_ptr(self.obs), _ptr(self.next_obs), _ptr(self.act_ring), _ptr(self.rew_ring),
@@ -388,6 +401,20 @@ class AgentGroup:
         return states, actions, rewards, next_states, dones, active
 
     # ------------------------------------------------------------------ K1b+K3+K4 -------
+    def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
+        """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
+        (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``)."""
+        ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.global_clipnorm is None:
+            N.check(self.lib.dmdqn_learn(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
+                                         draws_ptr, mask_ptr, _ptr(self.metrics), ws, nws, stream_ptr))
+            return
+        N.check(self.lib.dmdqn_learn_grads(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
+                                           draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), _ptr(self.metrics), ws, nws,
+                                           stream_ptr))
+        N.check(self.lib.dmdqn_clip_adam_apply(C.byref(self.dims), C.byref(hp), C.byref(self.nets), _ptr(self.grads),
+                                               self.global_clipnorm, _ptr(self.grad_norms), ws, nws, stream_ptr))
+
     @_on_device
     def learn(self, draws=None, mask=None, sample_mode: str | None = None) -> torch.Tensor:
         """One Double-DQN step for every network whose ring holds >= batch transitions
@@ -396,9 +423,7 @@ class AgentGroup:
         hp = self._hp_for(sample_mode)
         d = self._draws(draws, hp.sample_mode)
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
-        N.check(self.lib.dmdqn_learn(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                     _ptr(d), _ptr(mask_t), _ptr(self.metrics), _ptr(self.workspace),
-                                     self.workspace.numel(), self._stream))
+        self._learn_call(hp, _ptr(d), _ptr(mask_t), self._stream)
         self.learn_step_host += self.active_host(mask).astype(np.int64)
         return self.metrics
 
@@ -415,9 +440,7 @@ class AgentGroup:
         side.wait_stream(torch.cuda.current_stream(self.device))
 
         def launch(stream_ptr, advance_host):
-            N.check(self.lib.dmdqn_learn(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                         _ptr(draws), None, _ptr(self.metrics), _ptr(self.workspace),
-                                         self.workspace.numel(), stream_ptr))
+            self._learn_call(hp, _ptr(draws), None, stream_ptr)
             if advance_host:
                 self.learn_step_host += self.active_host().astype(np.int64)
         with torch.cuda.stream(side):           # warm-up outside the capture: per-device launch attributes are set here
@@ -456,15 +479,29 @@ class AgentGroup:
                 "host": {k: view(host, k) for k in offs}, "dev": {k: view(dev, k) for k in offs},
                 "metrics_host": torch.zeros((g, N.METRICS_STRIDE), dtype=torch.float32).pin_memory()}
 
+    def _step_host_call(self, hp, sb, stream_ptr) -> None:
+        """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
+        one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy."""
+        if self.global_clipnorm is None:
+            N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
+                                             C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
+                                             _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
+                                             self.workspace.numel(), stream_ptr))
+            return
+        desc, dev = sb["desc"], sb["dev_block"].data_ptr()
+        sb["dev_block"].copy_(sb["host_block"], non_blocking=True)
+        N.check(self.lib.dmdqn_push(C.byref(self.dims), C.byref(self.replay), dev + desc.obs_off, dev + desc.act_off,
+                                    dev + desc.rew_off, dev + desc.next_obs_off, dev + desc.done_off, desc.in_stride, None,
+                                    stream_ptr))
+        self._learn_call(hp, dev + desc.draws_off, None, stream_ptr)
+        sb["metrics_host"].copy_(self.metrics, non_blocking=True)
+
     @_on_device
     def step_host(self, sb) -> torch.Tensor:
         """remember + replay for every agent from the HOST block ``sb`` (``make_step_block``): one H2D copy, push, learn,
         metrics back to ``sb["metrics_host"]`` -- all queued on the current stream by ONE library call
         (train.py:274-292).  Synchronise the stream before reading the returned pinned tensor."""
-        N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(self._hp_for(None)), C.byref(self.replay), C.byref(self.nets),
-                                         C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
-                                         _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
-                                         self.workspace.numel(), self._stream))
+        self._step_host_call(self._hp_for(None), sb, self._stream)
         self.n_written_host += 1
         self.learn_step_host += self.active_host().astype(np.int64)
         return sb["metrics_host"]
@@ -479,10 +516,7 @@ class AgentGroup:
         side.wait_stream(torch.cuda.current_stream(self.device))
 
         def launch(stream_ptr):
-            N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                             C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
-                                             _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
-                                             self.workspace.numel(), stream_ptr))
+            self._step_host_call(hp, sb, stream_ptr)
         with torch.cuda.stream(side):           # warm-up outside the capture (per-device launch attributes): one real step
             launch(side.cuda_stream)
             self.n_written_host += 1

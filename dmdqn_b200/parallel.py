@@ -201,14 +201,20 @@ class SharedParameterStep:
     def for_group(cls, grp, group=None, fused: bool | None = None, exchange: "PeerExchange | None" = None) -> "SharedParameterStep":
         """Bind to an AgentGroup built with ``share_parameters=True``.  ``fused`` (default: whenever there is more
         than one rank) runs the all-reduce and Adam as one peer-memory kernel; ``fused=False`` is the NCCL
-        all-reduce + ``dmdqn_adam_apply`` baseline.  ``exchange``: a PeerExchange already connected (tests)."""
+        all-reduce + ``dmdqn_adam_apply`` baseline.  A group with ``global_clipnorm`` takes the NCCL path and finishes with
+        ``dmdqn_clip_adam_apply`` on the all-reduced block; ``fused=True`` is refused there.  ``exchange``: a PeerExchange
+        already connected (tests)."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
             raise ValueError("SharedParameterStep needs share_parameters=True")
         world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+        clip = grp.global_clipnorm
+        if clip is not None and fused:
+            raise ValueError("global_clipnorm is set: the fused peer-memory kernel (dmdqn_allreduce_adam) does not clip; "
+                             "use fused=False (the NCCL all-reduce + dmdqn_clip_adam_apply path)")
         if fused is None:
-            fused = world > 1 or exchange is not None
+            fused = clip is None and (world > 1 or exchange is not None)
         if fused and exchange is None:
             rank = dist.get_rank(group) if world > 1 else 0
             exchange = PeerExchange(grp, rank, world).connect(group)
@@ -249,6 +255,11 @@ class SharedParameterStep:
 
         def apply(g: torch.Tensor):
             with torch.cuda.device(grp.device):
+                if clip is not None:            # the norm of the all-reduced block: the same scale on every replica
+                    N.check(grp.lib.dmdqn_clip_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g), clip,
+                                                          _ptr(grp.grad_norms), _ptr(grp.workspace), grp.workspace.numel(),
+                                                          grp._stream))
+                    return
                 N.check(grp.lib.dmdqn_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g),
                                                  _ptr(grp.workspace), grp.workspace.numel(), grp._stream))
         step = cls(local_grads, apply, grp.batch_size, group, local_ready=local_ready, flag_device=grp.device,

@@ -328,6 +328,27 @@ int dmdqn_learn_grads(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmd
 int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets,
                      const float* grads, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Global-norm gradient clipping (Keras `global_clipnorm`, tf.clip_by_global_norm, torch clip_grad_norm_): dmdqn_adam_apply
+ * with every network's gradient scaled to a global norm of at most c = global_clipnorm first.  A clipped learn step is
+ * dmdqn_learn_grads(..., global_batch = batch, grads, ...) followed by this call (with shared parameters across ranks: on
+ * the all-reduced block, so every replica scales by the same n).  For every network g that learned this step:
+ *   1. G = grads[g][0 .. layout.b3 + 4), the range dmdqn_adam_apply updates;
+ *   2. n = sqrt(sum G_i^2) in float64 (the squares are exact); the summation order is fixed by the kernel (8 contiguous
+ *      slices, each summed by its CTA in a fixed thread order, the 8 partials added in slice order) and does not depend
+ *      on the other networks or on how many networks the call covers;
+ *   3. s = (float)(c / max(n, c)), the clipped gradient is G_i * s in fp32.  n <= c gives s == 1 and the update of
+ *      dmdqn_adam_apply bit for bit; a non-finite n applies no scaling;
+ *   4. Adam and the target sync as in dmdqn_adam_apply (the same workspace Adam scalars and the same per-element
+ *      arithmetic);
+ *   5. norms_out[g] (device float[n_nets], or NULL) = (float)n, the norm before clipping; 0 for a network that did not
+ *      learn this step (its metrics row is 0 too).
+ * A network whose step was poisoned (the workspace error flag is set: a tcgen05 kernel's bounded wait expired, so
+ * metrics[g][7] < 0 and K4b wrote no gradient) gets no update and norm 0.  global_clipnorm <= 0, NaN or infinite is
+ * refused with DMDQN_ERR_ARG before anything is launched. */
+int dmdqn_clip_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets,
+                          const float* grads, double global_clipnorm, float* norms_out, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* K5, shared-parameter mode over NVLink peer memory (BASELINE.json cfg5; SURVEY.md section 8 row B2/E2): ONE kernel per
  * rank that (1) announces its gradient block of this step to every peer (release store of `epoch` into the peers'
  * flag arrays), (2) waits for the peers' announcements, (3) reads every rank's block through peer pointers, sums
