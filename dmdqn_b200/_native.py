@@ -27,6 +27,10 @@ class Layout(C.Structure):
     _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "w2", "b2", "w3", "b3", "stride")]
 
 
+class DuelingLayout(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "w2", "b2", "w3", "b3", "wv", "bv", "stride")]
+
+
 class Replay(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("obs", "next_obs", "act", "rew", "done", "n_written", "priority", "priority_max")]
 
@@ -39,8 +43,22 @@ class HParams(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("gamma", "learning_rate", "beta1", "beta2", "adam_eps", "tau")] + \
                [(n, C.c_int32) for n in ("target_update_frequency", "loss", "normalize_rewards", "double_dqn",
                                          "adam_form", "sample_mode", "precision")] + \
+               [("dueling", C.c_int32)] + \
                [(n, C.c_double) for n in ("per_alpha", "per_beta0", "per_eps")] + [("per_beta_steps", C.c_int32)] + \
                [("n_step", C.c_int32)]      # in what was tail padding: sizeof stays 112
+    # dueling sits at offset 76 (interior padding), between precision and per_alpha.  It is keyword-only, so positional
+    # constructions keep the order of every field before it; later fields are keyword-only as well.
+    _ARGS = ("gamma", "learning_rate", "beta1", "beta2", "adam_eps", "tau", "target_update_frequency", "loss",
+             "normalize_rewards", "double_dqn", "adam_form", "sample_mode", "precision", "per_alpha", "per_beta0", "per_eps",
+             "per_beta_steps", "n_step")
+
+    def __init__(self, *args, **kwargs):
+        if len(args) > len(self._ARGS):
+            raise TypeError(f"HParams takes at most {len(self._ARGS)} positional arguments; dueling is keyword-only")
+        super().__init__(**dict(zip(self._ARGS, args)), **kwargs)
+
+
+assert C.sizeof(HParams) == 112 and HParams.dueling.offset == 76, "dmdqn_hparams layout (include/dmdqn_b200.h)"
 
 
 class DebugViews(C.Structure):
@@ -49,6 +67,10 @@ class DebugViews(C.Structure):
 
 class NStepViews(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("next_rows", "discount")]
+
+
+class DuelingViews(C.Structure):
+    _fields_ = [("head", C.c_void_p)]
 
 
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
@@ -70,11 +92,13 @@ SIGNATURES = {
     "dmdqn_last_error": (C.c_char_p, []),
     "dmdqn_abi_version": (C.c_int, []),
     "dmdqn_param_layout": (C.c_int, [C.POINTER(Dims), C.POINTER(Layout)]),
+    "dmdqn_param_layout_dueling": (C.c_int, [C.POINTER(Dims), C.POINTER(DuelingLayout)]),
     "dmdqn_workspace_bytes": (C.c_int, [C.POINTER(Dims), C.POINTER(C.c_size_t)]),
     "dmdqn_featurize": (C.c_int, [C.c_int32, _P, _P, _P, _P, C.c_double, _P, _P, _P, _P, C.c_double,
                                   C.c_double, _P, _P, C.c_int32, _P, _P, _P, _P]),
     "dmdqn_featurize_alt": (C.c_int, [C.c_int32, _P, _P, _P, _P, C.c_double, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "dmdqn_act": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    "dmdqn_act_dueling": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "dmdqn_push": (C.c_int, [C.POINTER(Dims), C.POINTER(Replay), _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "dmdqn_sample": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Replay), C.POINTER(Nets), _P, _P,
                                C.c_int32, _P, C.c_size_t, _P]),
@@ -97,7 +121,9 @@ SIGNATURES = {
     "dmdqn_ipc_close": (C.c_int, [_P, C.c_uint64]),
     "dmdqn_debug": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(DebugViews)]),
     "dmdqn_debug_nstep": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(NStepViews)]),
+    "dmdqn_debug_dueling": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(DuelingViews)]),
     "dmdqn_sync_target": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_double, _P]),
+    "dmdqn_sync_target_dueling": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_double, _P]),
 }
 
 _lib = None

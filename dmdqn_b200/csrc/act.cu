@@ -102,7 +102,9 @@ __device__ __forceinline__ void gemv_slice_loop(cg::cluster_group& cluster, cons
     cluster.sync();
 }
 
-template <int H_>
+// DUELING: the block is in the dueling layout and the head is folded (include/dmdqn_b200.h) in registers: every CTA folds
+// its W3 rows with their wv weights, rank 0 folds the bias.
+template <int H_, bool DUELING>
 __global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads, 4)
 act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float* __restrict__ obs, int stride,
            const double* __restrict__ eps, const uint32_t* __restrict__ w_explore,
@@ -166,7 +168,12 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
     float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
     if (threadIdx.x < Hs) {
         const int j = rank * Hs + threadIdx.x;
-        const float4 w = __ldg(reinterpret_cast<const float4*>(P + L.w3) + j);
+        float4 w = __ldg(reinterpret_cast<const float4*>(P + L.w3) + j);
+        if constexpr (DUELING) {
+            float x[4] = {w.x, w.y, w.z, w.w};
+            head_fold(x, __ldg(P + layout_wv(L) + j), d.n_actions);
+            w = make_float4(x[0], x[1], x[2], x[3]);
+        }
         const float hv = h2[j];
         p = make_float4(hv * w.x, hv * w.y, hv * w.z, hv * w.w);
     }
@@ -188,6 +195,7 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
     cluster.sync();
     if (threadIdx.x == 0 && rank == 0) {
         float q[4] = {P[L.b3 + 0], P[L.b3 + 1], P[L.b3 + 2], P[L.b3 + 3]};
+        if constexpr (DUELING) head_fold(q, P[layout_bv(L, H)], d.n_actions);
         for (int r = 0; r < kActCluster; ++r) {
             const float4 t = reinterpret_cast<const float4*>(part)[16 + r];
             q[0] += t.x; q[1] += t.y; q[2] += t.z; q[3] += t.w;
@@ -204,16 +212,21 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
 }  // namespace
 
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
-               const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
+               const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,
                cudaStream_t s) {
-    const Layout L = make_layout(d.obs_stride, d.hidden);
+    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
     const size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4) * sizeof(float);
     const dim3 grid(d.n_agents * kActCluster);
-    switch (d.hidden) {
-        case 64: act_kernel<64><<<grid, kActThreads, smem, s>>>(d, L, nets.theta, obs, stride, eps, w1, w2, actions, q_out); break;
-        case 128: act_kernel<128><<<grid, kActThreads, smem, s>>>(d, L, nets.theta, obs, stride, eps, w1, w2, actions, q_out); break;
-        case 256: act_kernel<256><<<grid, kActThreads, smem, s>>>(d, L, nets.theta, obs, stride, eps, w1, w2, actions, q_out); break;
-        case 512: act_kernel<512><<<grid, kActThreads, smem, s>>>(d, L, nets.theta, obs, stride, eps, w1, w2, actions, q_out); break;
+    auto run = [&](auto kernel) { kernel<<<grid, kActThreads, smem, s>>>(d, L, nets.theta, obs, stride, eps, w1, w2, actions, q_out); };
+    switch (d.hidden * 2 + (dueling ? 1 : 0)) {
+        case 128: run(act_kernel<64, false>); break;
+        case 129: run(act_kernel<64, true>); break;
+        case 256: run(act_kernel<128, false>); break;
+        case 257: run(act_kernel<128, true>); break;
+        case 512: run(act_kernel<256, false>); break;
+        case 513: run(act_kernel<256, true>); break;
+        case 1024: run(act_kernel<512, false>); break;
+        case 1025: run(act_kernel<512, true>); break;
         default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
     }
     DMDQN_CUDA(cudaGetLastError());

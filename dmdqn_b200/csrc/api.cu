@@ -93,6 +93,17 @@ int dmdqn_param_layout(const dmdqn_dims* dims, dmdqn_layout* out) {
     return DMDQN_OK;
 }
 
+int dmdqn_param_layout_dueling(const dmdqn_dims* dims, dmdqn_dueling_layout* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const Layout l = make_layout(dims->obs_stride, dims->hidden, true);
+    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
+    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
+    out->wv = layout_wv(l); out->bv = layout_bv(l, dims->hidden);
+    return DMDQN_OK;
+}
+
 int dmdqn_workspace_bytes(const dmdqn_dims* dims, size_t* out_bytes) {
     int rc = validate_dims(dims);
     if (rc) return rc;
@@ -128,15 +139,27 @@ int dmdqn_featurize_alt(int32_t n, const int32_t* halting, const int32_t* phase,
                                 obs_out, obs_out_stride, reward_out, (cudaStream_t)stream);
 }
 
-int dmdqn_act(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
-              const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out,
-              float* q_out, void* stream) {
+static int run_act(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
+                   const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out,
+                   float* q_out, bool dueling, void* stream) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(nets && nets->theta && obs && eps && w_explore && w_action && actions_out, "act: NULL argument");
     DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
-    return launch_act(*dims, *nets, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out,
+    return launch_act(*dims, *nets, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out, dueling,
                       (cudaStream_t)stream);
+}
+
+int dmdqn_act(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
+              const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out,
+              float* q_out, void* stream) {
+    return run_act(dims, nets, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out, false, stream);
+}
+
+int dmdqn_act_dueling(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
+                      const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out,
+                      float* q_out, void* stream) {
+    return run_act(dims, nets, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out, true, stream);
 }
 
 int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* obs, const int32_t* act,
@@ -158,10 +181,19 @@ static int check_n_step(const dmdqn_hparams* hp) {
     return DMDQN_OK;
 }
 
+static_assert(offsetof(dmdqn_hparams, dueling) == 76 && sizeof(dmdqn_hparams) == 112,
+              "dueling sits in the former interior padding of dmdqn_hparams: no other field moves");
+
+static int check_dueling(const dmdqn_hparams* hp) {
+    DMDQN_CHECK_ARG(hp->dueling == 0 || hp->dueling == 1, "dueling=%d must be 0 (plain head) or 1 (dueling heads)", hp->dueling);
+    return DMDQN_OK;
+}
+
 static int check_learn_args(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                             const dmdqn_nets* nets, const void* draws) {
     DMDQN_CHECK_ARG(hp && replay && nets && draws, "NULL argument");
     if (int rc = check_n_step(hp)) return rc;
+    if (int rc = check_dueling(hp)) return rc;
     DMDQN_CHECK_ARG(replay->obs && replay->next_obs && replay->act && replay->rew && replay->done &&
                         replay->n_written, "NULL replay pointer");
     DMDQN_CHECK_ARG(nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && nets->learn_step,
@@ -192,6 +224,10 @@ static int run_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     if (rc) return rc;
     if (grads) DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     if (stages & DMDQN_STAGE_SAMPLE) {
+        if (hp->dueling) {            // W3e | b3e of this step's weights, complete before the sample -> K3 -> K4a -> K4b chain
+            rc = launch_fold(*dims, *nets, (char*)workspace, w, (cudaStream_t)stream);
+            if (rc) return rc;
+        }
         rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, (cudaStream_t)stream);
         if (rc) return rc;
     }
@@ -245,6 +281,8 @@ int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn
     DMDQN_CHECK_ARG(hp && blk && host_block && device_block && metrics_dev && metrics_host, "step_host: NULL argument");
     rc = check_n_step(hp);            // before the copy and the push: a refused step changes nothing
     if (rc) return rc;
+    rc = check_dueling(hp);
+    if (rc) return rc;
     const size_t offs[6] = {blk->obs_off, blk->next_obs_off, blk->act_off, blk->rew_off, blk->done_off, blk->draws_off};
     for (size_t o : offs) DMDQN_CHECK_ARG(o % 16 == 0 && o < blk->bytes, "step_host: offset %zu is not a multiple of 16 inside the block", o);
     cudaStream_t s = (cudaStream_t)stream;
@@ -276,6 +314,8 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     if (rc) return rc;
     DMDQN_CHECK_ARG(hp && nets && nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && grads,
                     "adam_apply: NULL argument");
+    rc = check_dueling(hp);
+    if (rc) return rc;
     return launch_adam_apply(*dims, *hp, *nets, grads, (char*)workspace, w, (cudaStream_t)stream);
 }
 
@@ -286,6 +326,8 @@ int dmdqn_clip_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const
     if (rc) return rc;
     DMDQN_CHECK_ARG(hp && nets && nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && grads,
                     "clip_adam_apply: NULL argument");
+    rc = check_dueling(hp);
+    if (rc) return rc;
     DMDQN_CHECK_ARG(global_clipnorm > 0.0 && isfinite(global_clipnorm),
                     "global_clipnorm=%g must be a positive finite number", global_clipnorm);
     return launch_clip_adam_apply(*dims, *hp, *nets, grads, global_clipnorm, norms_out, (char*)workspace, w,
@@ -299,6 +341,8 @@ int dmdqn_allreduce_adam(const dmdqn_dims* dims, const dmdqn_hparams* hp, const 
     if (rc) return rc;
     DMDQN_CHECK_ARG(hp && nets && nets->theta && nets->theta_tgt && nets->adam_m && nets->adam_v && peers && my_loss_src,
                     "allreduce_adam: NULL argument");
+    rc = check_dueling(hp);
+    if (rc) return rc;
     DMDQN_CHECK_ARG(dims->n_nets == 1, "allreduce_adam serves the shared network (n_nets == 1), got n_nets=%d", dims->n_nets);
     DMDQN_CHECK_ARG(peers->world >= 1 && peers->world <= DMDQN_MAX_PEERS && peers->rank >= 0 && peers->rank < peers->world,
                     "allreduce_adam: rank %d of world %d (at most %d peers)", peers->rank, peers->world, DMDQN_MAX_PEERS);
@@ -387,12 +431,31 @@ int dmdqn_debug_nstep(const dmdqn_dims* dims, void* workspace, size_t workspace_
     return DMDQN_OK;
 }
 
-int dmdqn_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau,
-                      void* stream) {
+int dmdqn_debug_dueling(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_dueling_views* out) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    out->head = (const float*)((char*)workspace + w.head);
+    return DMDQN_OK;
+}
+
+static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau, bool dueling,
+                           void* stream) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt, "sync_target: NULL network pointer");
-    return launch_sync_target(*dims, *nets, mask, tau, (cudaStream_t)stream);
+    return launch_sync_target(*dims, *nets, mask, tau, dueling, (cudaStream_t)stream);
+}
+
+int dmdqn_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau,
+                      void* stream) {
+    return run_sync_target(dims, nets, mask, tau, false, stream);
+}
+
+int dmdqn_sync_target_dueling(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau,
+                              void* stream) {
+    return run_sync_target(dims, nets, mask, tau, true, stream);
 }
 
 }  // extern "C"

@@ -26,11 +26,13 @@ void set_error(const char* fmt, ...);
         }                                                                             \
     } while (0)
 
-// Float offsets of W1|b1|W2|b2|W3|b3 inside one parameter block (include/dmdqn_b200.h).
+// Float offsets of W1|b1|W2|b2|W3|b3 inside one parameter block (include/dmdqn_b200.h).  `end` closes the range the
+// Adam kernels update: b3 + 4, or with the dueling value head wv[H] | bv | pad[3] after b3, b3 + 8 + H.
 struct Layout {
     int64_t w1, b1, w2, b2, w3, b3, stride;
+    int64_t end;
 };
-__host__ __device__ inline Layout make_layout(int dp, int h) {
+__host__ __device__ inline Layout make_layout(int dp, int h, bool dueling = false) {
     Layout l;
     l.w1 = 0;
     l.b1 = (int64_t)dp * h;
@@ -38,8 +40,36 @@ __host__ __device__ inline Layout make_layout(int dp, int h) {
     l.b2 = l.w2 + (int64_t)h * h;
     l.w3 = l.b2 + h;
     l.b3 = l.w3 + (int64_t)h * 4;
-    l.stride = (l.b3 + 4 + 31) / 32 * 32;  // blocks start on 128-byte lines
+    l.end = l.b3 + 4 + (dueling ? h + 4 : 0);
+    l.stride = (l.end + 31) / 32 * 32;  // blocks start on 128-byte lines
     return l;
+}
+// Dueling value head: wv[H] right after b3 (16-byte aligned), bv after it.
+__host__ __device__ inline int64_t layout_wv(const Layout& l) { return l.b3 + 4; }
+__host__ __device__ inline int64_t layout_bv(const Layout& l, int h) { return l.b3 + 4 + h; }
+
+// The dueling fold (include/dmdqn_b200.h): the mean over the first A of four values, summed left to right in fp32 and
+// divided by A, and the effective head value (x - mean) + v.  Shared by the fold kernel, act and both head updates.
+// (The loops are unrolled with predicated terms so that the four values stay in registers.)
+__host__ __device__ __forceinline__ float head_sum(const float (&x)[4], int A) {
+    float s = x[0];
+#pragma unroll
+    for (int b = 1; b < 4; ++b)
+        if (b < A) s += x[b];
+    return s;
+}
+// W3e / b3e of one row of four advantage values x and its value weight v (columns >= A are 0)
+__host__ __device__ __forceinline__ void head_fold(float (&x)[4], float v, int A) {
+    const float m = head_sum(x, A) / (float)A;
+#pragma unroll
+    for (int a = 0; a < 4; ++a) x[a] = a < A ? (x[a] - m) + v : 0.f;
+}
+// The projection of the folded head's gradient G onto the advantage row (in place) and the value weight (returned)
+__host__ __device__ __forceinline__ float head_project(float (&g)[4], int A) {
+    const float s = head_sum(g, A), m = s / (float)A;
+#pragma unroll
+    for (int a = 0; a < 4; ++a) g[a] = a < A ? g[a] - m : 0.f;
+    return s;
 }
 
 // Tile geometry of the fused MLP kernels for hidden width H (DESIGN.md "K3/K4 tiling").
@@ -77,6 +107,8 @@ struct Workspace {
                                       // k3_done[n_nets][T]; zeroed by the sample kernel (dataflow flags between the learn kernels)
     size_t nrows, disc_b;             // [n_nets][B] int32 bootstrap row (agent*C + slot) and float discount of each row's TD
                                       // target (the drawn row and gamma * (1 - done) for one-step targets; see dmdqn_sample)
+    size_t head;                      // dueling: float [2][n_nets][4H + 4], W3e | b3e of the online and the target network
+                                      // (the fold kernel's output, read by K3 / K4a); carved last so no other offset moves
     size_t total;
     int tiles;                        // T: row tiles per network of the FFMA kernels (Tile<H>::BM rows); the tcgen05 path's
                                       // 128-row tiles are fewer, so its partials fit the same arrays
@@ -115,6 +147,7 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
     w.sync = take((4 + (size_t)d.n_nets + nt) * 4);
     w.nrows = take(nb * 4);
     w.disc_b = take(nb * 4);
+    w.head = take(2 * (size_t)d.n_nets * (4 * (size_t)d.hidden + 4) * 4);
     w.total = off;
     return w;
 }
@@ -157,6 +190,12 @@ struct LearnArgs {
     const float* is_w;                // Workspace::is_w
     double per_alpha, per_eps;  // Workspace::sync: K4b work counter | K4a items finished per network | K3 items finished
                                       // per (network, tile)
+    // Where K3 / K4a read the head W3[H][4] | b3[4] of network g: head[0] (online) / head[1] (target) + g * head_stride.
+    // Plain: theta / theta_tgt + L.w3 with the parameter stride; dueling: the folded W3e | b3e in Workspace::head.  (The
+    // plain tcgen05 K3 / K4a instantiations read the head from the parameter block directly: learn_tc.cu head_w3.)
+    const float* head[2];
+    int64_t head_stride;
+    int dueling;                      // K4b projects the head gradient onto W3 / b3 / wv / bv
 };
 LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                           char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch);
@@ -221,7 +260,7 @@ int launch_featurize_alt(int32_t n, const int32_t* halting, const int32_t* phase
                          const uint8_t* signal_valid, double sim_time, const int32_t* nbr_idx, const double* prev_own,
                          double* own_out, float* obs_out, int32_t obs_out_stride, double* reward_out, cudaStream_t s);
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
-               const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
+               const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,
                cudaStream_t s);
 int launch_push(const dmdqn_dims& d, const dmdqn_replay& rp, const float* obs, const int32_t* act,
                 const double* rew, const float* next_obs, const uint8_t* done, int32_t in_stride,
@@ -240,8 +279,9 @@ int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_
                       const Workspace& w, cudaStream_t s);
 int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads,
                            double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
-int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau,
+int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau, bool dueling,
                        cudaStream_t s);
+int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Workspace& w, cudaStream_t s);
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,
                      const float* my_loss_src, float* loss_out, char* ws, const Workspace& w, cudaStream_t s);
 

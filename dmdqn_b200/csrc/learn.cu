@@ -217,10 +217,18 @@ struct Smem {
     }
 };
 
+// The head W3 | b3 of network g's parameter set `tgt` (P: that set's block): the plain instantiations of K3 / K4a read it
+// from P, the same code as before dueling heads existed; the dueling ones read the fold kernel's W3e | b3e.
+template <bool DUELING>
+__device__ __forceinline__ const float* head_w3(const LearnArgs& A, const float* P, int tgt, int g) {
+    if constexpr (DUELING) return (tgt ? A.head[1] : A.head[0]) + (size_t)g * A.head_stride;
+    else return P + A.L.w3;
+}
+
 // ------------------------------------------------------------------------------------------
 // K3: TD targets.
 // ------------------------------------------------------------------------------------------
-template <int H>
+template <int H, bool DUELING>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs A) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
@@ -236,12 +244,13 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs 
 #pragma unroll 1
     for (int pass = 0; pass < 2; ++pass) {          // 0: online(s')  1: target(s')
         const float* P = (pass == 0 ? A.nets.theta : A.nets.theta_tgt) + (size_t)g * A.L.stride;
+        const float* W3 = head_w3<DUELING>(A, P, pass, g);
         gemm_rowA<H, false>(acc, c, S.Xs, S.ldx, P + A.L.w1, H, Dp, S.Ws);
         store_relu<H>(acc, c, P + A.L.b1, S.Hs1, nullptr, r0, B);
         gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
         store_relu<H>(acc, c, P + A.L.b2, S.Hs2, nullptr, r0, B);
         __syncthreads();
-        layer3<H>(S.Hs2, P + A.L.w3, P + A.L.b3, pass == 0 ? S.qs0 : S.qs1, S.Ws);
+        layer3<H>(S.Hs2, W3, DUELING ? W3 + 4 * H : P + A.L.b3, pass == 0 ? S.qs0 : S.qs1, S.Ws);
     }
     for (int i = threadIdx.x; i < T::BM; i += T::NT) {
         const int gr = r0 + i;
@@ -268,7 +277,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) target_kernel(const LearnArgs 
 // ------------------------------------------------------------------------------------------
 // K4a: online forward on s, loss gradient, activation gradients.
 // ------------------------------------------------------------------------------------------
-template <int H>
+template <int H, bool DUELING>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs A) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
@@ -279,6 +288,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
     const Coord<H> c;
     const int32_t* rows = A.rows + (size_t)g * B;
     const float* P = A.nets.theta + (size_t)g * A.L.stride;
+    const float* W3 = head_w3<DUELING>(A, P, 0, g);
     const size_t sb = (size_t)g * B;                 // this network's rows in [n_nets][B][...]
     gather_tile<H>(S.Xs, S.ldx, A.rp.obs, rows, r0, B, Dp);
 
@@ -288,7 +298,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
     gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
     store_relu<H>(acc, c, P + A.L.b2, S.Hs2, nullptr, r0, B);
     __syncthreads();
-    layer3<H>(S.Hs2, P + A.L.w3, P + A.L.b3, S.qs0, S.Ws);
+    layer3<H>(S.Hs2, W3, DUELING ? W3 + 4 * H : P + A.L.b3, S.qs0, S.Ws);
 
     // loss terms and dL/dpred per row (:349-352; SURVEY App. A.8)
     float* terms = S.qs1;                            // [BM] loss terms
@@ -340,7 +350,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) online_kernel(const LearnArgs 
     }
     // dW3 partial, dh2 = (dq W3^T) * relu'(h2) in place, db2 partial: one thread per column
     for (int j = threadIdx.x; j < H; j += T::NT) {
-        const float4 w3 = __ldg(reinterpret_cast<const float4*>(P + A.L.w3) + j);
+        const float4 w3 = __ldg(reinterpret_cast<const float4*>(W3) + j);
         float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f, sb2 = 0.f;
         for (int i = 0; i < T::BM; ++i) {
             const float h = S.Hs2[i * T::LDH + j];
@@ -445,29 +455,39 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
         }
         const AdamStep k = adam_step(A, g);
         const size_t p0 = (size_t)g * A.ws_tiles;
-        for (int e = threadIdx.x; e < 6 * H + 4; e += T::NT) {
-            float gsum = 0.f;
-            int64_t off;
-            if (e < H) {                                   // b1
-                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b1[(p0 + r) * H + e];
-                off = A.L.b1 + e;
-            } else if (e < 2 * H) {                        // b2
-                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b2[(p0 + r) * H + (e - H)];
-                off = A.L.b2 + (e - H);
-            } else if (e < 6 * H) {                        // W3[j][a]
-                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_w3[(p0 + r) * H * 4 + (e - 2 * H)];
-                off = A.L.w3 + (e - 2 * H);
-            } else {                                       // b3
-                for (int r = 0; r < A.ws_tiles; ++r) gsum += A.part_b3[(p0 + r) * 4 + (e - 6 * H)];
-                off = A.L.b3 + (e - 6 * H);
-            }
+        auto upd = [&](int64_t off, float gsum) {
             if (A.grads) {
                 A.grads[(size_t)g * A.L.stride + off] = gsum;
-                continue;
+                return;
             }
             float tgv = k.sync == 2 ? tg[off] : 0.f;
             adam_elem(k, gsum, th[off], am[off], av[off], tgv);
             if (k.sync) tg[off] = tgv;
+        };
+        for (int e = threadIdx.x; e < 3 * H + 1; e += T::NT) {
+            if (e < 2 * H) {                               // b1, b2
+                const float* part = e < H ? A.part_b1 : A.part_b2;
+                const int j = e < H ? e : e - H;
+                float gsum = 0.f;
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += part[(p0 + r) * H + j];
+                upd((e < H ? A.L.b1 : A.L.b2) + j, gsum);
+                continue;
+            }
+            // one head row: W3[j][0..3] (j < H) or b3 (j == H); dueling: projected, with its value weight wv[j] / bv
+            const int j = e - 2 * H;
+            float w[4] = {0.f, 0.f, 0.f, 0.f};
+            for (int r = 0; r < A.ws_tiles; ++r) {
+                const float4 pw = j < H ? *reinterpret_cast<const float4*>(A.part_w3 + ((p0 + r) * H + j) * 4)
+                                        : *reinterpret_cast<const float4*>(A.part_b3 + (p0 + r) * 4);
+                w[0] += pw.x; w[1] += pw.y; w[2] += pw.z; w[3] += pw.w;
+            }
+            if (A.dueling) {
+                upd(j < H ? layout_wv(A.L) + j : layout_bv(A.L, H), head_project(w, A.d.n_actions));
+                if (j == H && A.grads)                     // the pad after bv is inside the Adam range: its gradient is 0
+                    for (int p = 1; p < 4; ++p) A.grads[(size_t)g * A.L.stride + layout_bv(A.L, H) + p] = 0.f;
+            }
+            const int64_t off = j < H ? A.L.w3 + (int64_t)j * 4 : A.L.b3;
+            for (int a = 0; a < 4; ++a) upd(off + a, w[a]);
         }
         if (threadIdx.x == 0 && A.metrics) finish_metrics(A, g, A.ws_tiles, [](const float* p) { return *p; });
         return;
@@ -554,6 +574,21 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
     }
 }
 
+// Dueling fold (include/dmdqn_b200.h): W3e | b3e of network blockIdx.x's online (blockIdx.y = 0) or target (1) block into
+// head[blockIdx.y][blockIdx.x], one thread per W3 row and one more for the bias.
+__global__ void __launch_bounds__(256) fold_kernel(Layout L, int H, int n_actions, const float* __restrict__ theta,
+                                                   const float* __restrict__ theta_tgt, float* __restrict__ head) {
+    const int g = blockIdx.x, n_nets = gridDim.x;
+    const float* P = (blockIdx.y ? theta_tgt : theta) + (size_t)g * L.stride;
+    float* out = head + ((size_t)blockIdx.y * n_nets + g) * (4 * H + 4);
+    for (int j = threadIdx.x; j <= H; j += blockDim.x) {
+        const float4 w = __ldg(reinterpret_cast<const float4*>(P + (j < H ? L.w3 + 4 * j : L.b3)));
+        float x[4] = {w.x, w.y, w.z, w.w};
+        head_fold(x, __ldg(P + (j < H ? layout_wv(L) + j : layout_bv(L, H))), n_actions);
+        reinterpret_cast<float4*>(out)[j] = make_float4(x[0], x[1], x[2], x[3]);
+    }
+}
+
 // theta_tgt <- theta (tau < 0) or Polyak (tau >= 0) for the masked networks.
 __global__ void sync_target_kernel(int64_t stride, const float* __restrict__ theta, float* __restrict__ tgt,
                                    const uint8_t* __restrict__ mask, float tau) {
@@ -580,7 +615,7 @@ __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ g
     if (!A.active[g]) return;
     const AdamStep k = adam_step(A, g);
     const size_t base = (size_t)g * A.L.stride;
-    const int64_t n4 = (A.L.b3 + 4) / 4;
+    const int64_t n4 = A.L.end / 4;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         const float4 g4 = *reinterpret_cast<const float4*>(grads + base + i * 4);
         const float gv[4] = {g4.x, g4.y, g4.z, g4.w};
@@ -598,7 +633,7 @@ __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ g
 constexpr int kClipCtas = 8;            // the portable cluster size
 constexpr int kClipThreads = 256;
 
-inline int64_t clip_per_cta(const Layout& L) { return ((L.b3 + 4) / 4 + kClipCtas - 1) / kClipCtas; }   // float4s
+inline int64_t clip_per_cta(const Layout& L) { return (L.end / 4 + kClipCtas - 1) / kClipCtas; }   // float4s
 
 __device__ __forceinline__ void clip_mbar_wait(uint32_t bar, bool& ok) {
     unsigned long long t0, t1;
@@ -629,7 +664,7 @@ clip_adam_apply_kernel(const LearnArgs A, const float* __restrict__ grads, int64
         if (rank == 0 && tid == 0 && norms_out) norms_out[g] = 0.f;
         return;
     }
-    const int64_t n4 = (A.L.b3 + 4) / 4, i0 = (int64_t)rank * per;
+    const int64_t n4 = A.L.end / 4, i0 = (int64_t)rank * per;
     const int cnt = (int)max((int64_t)0, min(per, n4 - i0));
     const size_t base = (size_t)g * A.L.stride + (size_t)i0 * 4;
     const uint32_t sbar = (uint32_t)__cvta_generic_to_shared(&bar);
@@ -744,7 +779,7 @@ peer_reduce_adam_kernel(const LearnArgs A, const dmdqn_peers P, const float* __r
     }
     if (!A.active[0]) return;                       // (the learn decision is collective: every rank or none)
     const AdamStep k = adam_step(A, 0);
-    const int64_t n4 = (A.L.b3 + 4) / 4;
+    const int64_t n4 = A.L.end / 4;
     for (int64_t i = b * (int64_t)blockDim.x + tid; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         float4 v[DMDQN_MAX_PEERS];
 #pragma unroll
@@ -764,22 +799,22 @@ peer_reduce_adam_kernel(const LearnArgs A, const dmdqn_peers P, const float* __r
     }
 }
 
-template <int H>
+template <int H, bool DUELING>
 int launch_learn_h(const LearnArgs& A, int stages, cudaStream_t s) {
     using T = Tile<H>;
     const size_t smem = Smem<H>::bytes(A.d.obs_stride);
     const size_t smem_w = sizeof(float) * 2 * T::KC * ((T::BM + 4) + T::LDW);
     static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};    // per device, not per process
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(target_kernel<H>), smem, cfg_t)) return rc;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(online_kernel<H>), smem, cfg_o)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(target_kernel<H, DUELING>), smem, cfg_t)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(online_kernel<H, DUELING>), smem, cfg_o)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(wgrad_adam_kernel<H>), smem_w, cfg_w)) return rc;
     const int grid = A.d.n_nets * A.ws_tiles;
     if (stages & DMDQN_STAGE_TARGET) {
-        target_kernel<H><<<grid, T::NT, smem, s>>>(A);
+        target_kernel<H, DUELING><<<grid, T::NT, smem, s>>>(A);
         DMDQN_CUDA(cudaGetLastError());
     }
     if (stages & DMDQN_STAGE_ONLINE) {
-        online_kernel<H><<<grid, T::NT, smem, s>>>(A);
+        online_kernel<H, DUELING><<<grid, T::NT, smem, s>>>(A);
         DMDQN_CUDA(cudaGetLastError());
     }
     if (stages & DMDQN_STAGE_WGRAD) {
@@ -796,7 +831,7 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
                           char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch) {
     LearnArgs A = {};
     A.d = d;
-    A.L = make_layout(d.obs_stride, d.hidden);
+    A.L = make_layout(d.obs_stride, d.hidden, hp.dueling == 1);
     A.rp = rp;
     A.nets = nets;
     A.loss = hp.loss;
@@ -836,6 +871,16 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
     A.is_w = reinterpret_cast<const float*>(ws + w.is_w);
     A.per_alpha = hp.per_alpha;
     A.per_eps = hp.per_eps;
+    A.dueling = hp.dueling == 1;
+    if (A.dueling) {
+        A.head_stride = 4 * (int64_t)d.hidden + 4;
+        A.head[0] = reinterpret_cast<const float*>(ws + w.head);
+        A.head[1] = A.head[0] + (size_t)d.n_nets * A.head_stride;
+    } else {
+        A.head_stride = A.L.stride;
+        A.head[0] = nets.theta + A.L.w3;
+        A.head[1] = nets.theta_tgt + A.L.w3;
+    }
     return A;
 }
 
@@ -851,10 +896,10 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
         return launch_learn_tc(A, hp.precision, stages, s);
     }
     switch (d.hidden) {
-        case 64: return launch_learn_h<64>(A, stages, s);
-        case 128: return launch_learn_h<128>(A, stages, s);
-        case 256: return launch_learn_h<256>(A, stages, s);
-        case 512: return launch_learn_h<512>(A, stages, s);
+        case 64: return A.dueling ? launch_learn_h<64, true>(A, stages, s) : launch_learn_h<64, false>(A, stages, s);
+        case 128: return A.dueling ? launch_learn_h<128, true>(A, stages, s) : launch_learn_h<128, false>(A, stages, s);
+        case 256: return A.dueling ? launch_learn_h<256, true>(A, stages, s) : launch_learn_h<256, false>(A, stages, s);
+        case 512: return A.dueling ? launch_learn_h<512, true>(A, stages, s) : launch_learn_h<512, false>(A, stages, s);
     }
     set_error("unsupported hidden width %d", d.hidden);
     return DMDQN_ERR_ARG;
@@ -888,9 +933,17 @@ int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_n
     return DMDQN_OK;
 }
 
-int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau,
+int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Workspace& w, cudaStream_t s) {
+    const Layout L = make_layout(d.obs_stride, d.hidden, true);
+    fold_kernel<<<dim3(d.n_nets, 2), 256, 0, s>>>(L, d.hidden, d.n_actions, nets.theta, nets.theta_tgt,
+                                                  reinterpret_cast<float*>(ws + w.head));
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau, bool dueling,
                        cudaStream_t s) {
-    const Layout L = make_layout(d.obs_stride, d.hidden);
+    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
     dim3 grid(32, d.n_nets);
     sync_target_kernel<<<grid, 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
     DMDQN_CUDA(cudaGetLastError());

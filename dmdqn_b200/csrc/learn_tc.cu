@@ -449,14 +449,15 @@ struct XGather {
     int n;
     float4 sp;                                                // this thread's share of the item's small parameters (b1 | b2 | W3)
 
-    // (P: the parameter block the item uses.  Its biases and head weights -- 6 KB that every epilogue reads from shared memory
-    // -- travel with the rows, one item ahead, instead of being fetched at the top of the item with the epilogue warps waiting.)
+    // (P: the parameter block the item uses, W3: its head (LearnArgs::head).  Its biases and head weights -- 6 KB that every
+    // epilogue reads from shared memory -- travel with the rows, one item ahead, instead of being fetched at the top of the item
+    // with the epilogue warps waiting.)
     __device__ __forceinline__ void begin(const float* __restrict__ ring, const int32_t* __restrict__ rows, int r0, int B, int Dp,
-                                          const float* __restrict__ P, const Layout& L) {
+                                          const float* __restrict__ P, const float* __restrict__ W3, const Layout& L) {
         {
             const int j = threadIdx.x;
             if (j < H) { sp.x = __ldg(P + L.b1 + j); sp.y = __ldg(P + L.b2 + j); }
-            else sp = __ldg(reinterpret_cast<const float4*>(P + L.w3) + (j - H));
+            else sp = __ldg(reinterpret_cast<const float4*>(W3) + (j - H));
         }
         const int q = Dp >> 2;                                // 16-byte pieces per row
         n = BM * q / NT;
@@ -626,12 +627,26 @@ __device__ __forceinline__ void tc_epilogue(uint32_t tmem) {
 // 148 SMs); K4a combines them into the TD target of its rows (reference :342-347).  A CTA walks the items
 // blockIdx.x, + gridDim.x, ... of active networks; every role runs the same walk.
 // ------------------------------------------------------------------------------------------
+// The head K3 / K4a read for network g's parameter set `tgt` (P: that set's block): the plain instantiation reads W3 | b3
+// from P itself, the same code as before dueling heads existed; the dueling one reads the fold kernel's W3e | b3e
+// (LearnArgs::head).  b3 follows W3 in both.
+template <bool DUELING>
+__device__ __forceinline__ const float* head_w3(const LearnArgs& A, const float* P, int tgt, int g) {
+    if constexpr (DUELING) return (tgt ? A.head[1] : A.head[0]) + (size_t)g * A.head_stride;
+    else return P + A.L.w3;
+}
+template <bool DUELING>
+__device__ __forceinline__ const float* head_b3(const LearnArgs& A, const float* P, int tgt, int g) {
+    if constexpr (DUELING) return head_w3<true>(A, P, tgt, g) + 4 * H;
+    else return P + A.L.b3;
+}
+
 __device__ __forceinline__ int k3_next(const LearnArgs& A, int q, int n_items) {
     while (q < n_items && !A.active[(q >> 1) / A.tc_tiles]) q += gridDim.x;
     return q;
 }
 
-template <int PASSES>
+template <int PASSES, bool DUELING>
 __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, const __grid_constant__ CUtensorMap tm_w1,
                                                             const __grid_constant__ CUtensorMap tm_w2,
                                                             const __grid_constant__ CUtensorMap tm_w1t,
@@ -695,7 +710,8 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, c
         int q = k3_next(A, blockIdx.x, n_items);
         if (q < n_items) {
             const int g = (q >> 1) / A.tc_tiles, rt = (q >> 1) % A.tc_tiles;
-            xg.begin(A.rp.next_obs, A.nrows + (size_t)g * B, rt * BM, B, Dp, ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride, A.L);
+            const float* P = ((q & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride;
+            xg.begin(A.rp.next_obs, A.nrows + (size_t)g * B, rt * BM, B, Dp, P, head_w3<DUELING>(A, P, q & 1, g), A.L);
         }
         int q_last = -1;                                       // the last item is published here, the others by the MMA lane
         while (q < n_items) {
@@ -718,13 +734,13 @@ __global__ void __launch_bounds__(NT_F, 1) tc_target_kernel(const LearnArgs A, c
             const int qn = k3_next(A, q + gridDim.x, n_items);
             if (qn < n_items) {                                // the next tile's rows travel while layer 2 runs
                 const int gn = (qn >> 1) / A.tc_tiles, rtn = (qn >> 1) % A.tc_tiles;
-                xg.begin(A.rp.next_obs, A.nrows + (size_t)gn * B, rtn * BM, B, Dp,
-                         ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)gn * A.L.stride, A.L);
+                const float* Pn = ((qn & 1) ? A.nets.theta_tgt : A.nets.theta) + (size_t)gn * A.L.stride;
+                xg.begin(A.rp.next_obs, A.nrows + (size_t)gn * B, rtn * BM, B, Dp, Pn, head_w3<DUELING>(A, Pn, qn & 1, gn), A.L);
             }
             ok = wait_gemm(sbase, ring, ok);
             TS();
             float qv[4];
-            epi_head(sbase, tmem, e, false, mask, qv, P + A.L.b3);
+            epi_head(sbase, tmem, e, false, mask, qv, head_b3<DUELING>(A, P, pass, g));
             TS();
             TS_PRINT("K3 store L1 epi1 L2 epi2");
             const int gr = r0 + e.row;
@@ -751,7 +767,7 @@ __device__ __forceinline__ int k4_next(const LearnArgs& A, int q, int n_items) {
     return q;
 }
 
-template <int PASSES>
+template <int PASSES, bool DUELING>
 __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, const __grid_constant__ CUtensorMap tmap_w2,
                                                             const __grid_constant__ CUtensorMap tm_w1,
                                                             const __grid_constant__ CUtensorMap tm_w2) {
@@ -814,7 +830,10 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, c
         const Epi e;
         XGather<PASSES> xg;
         int q = k4_next(A, blockIdx.x, n_items);
-        if (q < n_items) xg.begin(A.rp.obs, A.rows + (size_t)(q / A.tc_tiles) * B, (q % A.tc_tiles) * BM, B, Dp, A.nets.theta + (size_t)(q / A.tc_tiles) * A.L.stride, A.L);
+        if (q < n_items) {
+            const float* P = A.nets.theta + (size_t)(q / A.tc_tiles) * A.L.stride;
+            xg.begin(A.rp.obs, A.rows + (size_t)(q / A.tc_tiles) * B, (q % A.tc_tiles) * BM, B, Dp, P, head_w3<DUELING>(A, P, 0, q / A.tc_tiles), A.L);
+        }
         int q_last = -1;                                       // the last item is published here, the others by the MMA lane
         while (q < n_items) {
             const int g = q / A.tc_tiles, rt = q % A.tc_tiles, r0 = rt * BM;
@@ -862,7 +881,7 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, c
             ok = wait_gemm(sbase, ring, ok);
             TS();
             float qv[4];
-            epi_head(sbase, tmem, e, true, mask2, qv, P + A.L.b3);
+            epi_head(sbase, tmem, e, true, mask2, qv, head_b3<DUELING>(A, P, 0, g));
             TS();
 
             // loss term and dL/dpred of this row (reference :349-352)
@@ -1020,8 +1039,11 @@ __global__ void __launch_bounds__(NT_F, 1) tc_online_kernel(const LearnArgs A, c
             a_ready(sbase);
             TS();
             const int qn = k4_next(A, q + gridDim.x, n_items);
-            if (qn < n_items)                                     // the next tile's rows travel while the backward GEMM runs
-                xg.begin(A.rp.obs, A.rows + (size_t)(qn / A.tc_tiles) * B, (qn % A.tc_tiles) * BM, B, Dp, A.nets.theta + (size_t)(qn / A.tc_tiles) * A.L.stride, A.L);
+            if (qn < n_items) {                                   // the next tile's rows travel while the backward GEMM runs
+                const float* Pn = A.nets.theta + (size_t)(qn / A.tc_tiles) * A.L.stride;
+                xg.begin(A.rp.obs, A.rows + (size_t)(qn / A.tc_tiles) * B, (qn % A.tc_tiles) * BM, B, Dp, Pn, head_w3<DUELING>(A, Pn, 0, qn / A.tc_tiles),
+                         A.L);
+            }
             // dh1 = (dh2 W2^T) * relu'(h1)
             ok = wait_gemm(sbase, ring, ok);
             TS();
@@ -1487,8 +1509,20 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const LearnArgs A,
                     w[0] += pw.x; w[1] += pw.y; w[2] += pw.z; w[3] += pw.w;
                 }
                 upd(A.L.b2 + et, s2);
+                if (A.dueling) {          // the folded head's gradient projected onto W3[et][.] | wv[et], and b3 | bv by one thread
+                    upd(layout_wv(A.L) + et, head_project(w, A.d.n_actions));
+                    if (et == 0) {
+                        float b[4] = {0.f, 0.f, 0.f, 0.f};
+                        for (int r = 0; r < A.tc_tiles; ++r)
+                            for (int a = 0; a < 4; ++a) b[a] += ldcg_f(A.part_b3 + (p0 + r) * 4 + a);
+                        upd(layout_bv(A.L, H), head_project(b, A.d.n_actions));
+                        for (int a = 0; a < 4; ++a) upd(A.L.b3 + a, b[a]);
+                        if (A.grads)              // the pad after bv is inside the Adam range: its gradient is 0
+                            for (int p = 1; p < 4; ++p) A.grads[pb + layout_bv(A.L, H) + p] = 0.f;
+                    }
+                }
                 for (int a = 0; a < 4; ++a) upd(A.L.w3 + (int64_t)et * 4 + a, w[a]);
-                if (et < 4) {
+                if (et < 4 && !A.dueling) {
                     float s3 = 0.f;
                     for (int r = 0; r < A.tc_tiles; ++r) s3 += ldcg_f(A.part_b3 + (p0 + r) * 4 + et);
                     upd(A.L.b3 + et, s3);
@@ -1663,14 +1697,14 @@ int make_scratch_tensor_map(const LearnArgs& A, const float* scratch, int rows, 
                        (cuuint64_t)A.d.batch * H * sizeof(float), KC, (cuuint32_t)rows, CU_TENSOR_MAP_SWIZZLE_64B);
 }
 
-template <int PASSES>
+template <int PASSES, bool DUELING>
 int launch_tc(const LearnArgs& A, int stages, cudaStream_t s) {
     const size_t smem_f = Fwd::TOTAL + 1024, smem_w = Wg::TOTAL + 1024;
     int n_sm = 0;
     if (int rc = device_sm_count(&n_sm)) return rc;
     static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};    // per device, not per process
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_target_kernel<PASSES>), smem_f, cfg_t)) return rc;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_online_kernel<PASSES>), smem_f, cfg_o)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_target_kernel<PASSES, DUELING>), smem_f, cfg_t)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_online_kernel<PASSES, DUELING>), smem_f, cfg_o)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(tc_wgrad_kernel<PASSES>), smem_w, cfg_w)) return rc;
     const int items = A.d.n_nets * A.tc_tiles;                    // persistent: one CTA per SM walks its items
     // In a chain (sample + K3 + K4a + K4b issued by one call) K4a and K4b are programmatic dependent launches: their CTAs
@@ -1693,7 +1727,7 @@ int launch_tc(const LearnArgs& A, int stages, cudaStream_t s) {
         if (int rc = make_fwd_tensor_map(A, A.nets.theta, A.L.w2, H, &m2)) return rc;
         if (int rc = make_fwd_tensor_map(A, A.nets.theta_tgt, A.L.w1, A.d.obs_stride, &m1t)) return rc;
         if (int rc = make_fwd_tensor_map(A, A.nets.theta_tgt, A.L.w2, H, &m2t)) return rc;
-        DMDQN_CUDA(cudaLaunchKernelEx(&cfg, tc_target_kernel<PASSES>, A, m1, m2, m1t, m2t));
+        DMDQN_CUDA(cudaLaunchKernelEx(&cfg, tc_target_kernel<PASSES, DUELING>, A, m1, m2, m1t, m2t));
     }
     if (stages & DMDQN_STAGE_ONLINE) {
         CUtensorMap tmap;
@@ -1705,7 +1739,7 @@ int launch_tc(const LearnArgs& A, int stages, cudaStream_t s) {
         CUtensorMap m1, m2;
         if (int rc = make_fwd_tensor_map(A, A.nets.theta, A.L.w1, A.d.obs_stride, &m1)) return rc;
         if (int rc = make_fwd_tensor_map(A, A.nets.theta, A.L.w2, H, &m2)) return rc;
-        DMDQN_CUDA(cudaLaunchKernelEx(&cfg, tc_online_kernel<PASSES>, A, tmap, m1, m2));
+        DMDQN_CUDA(cudaLaunchKernelEx(&cfg, tc_online_kernel<PASSES, DUELING>, A, tmap, m1, m2));
     }
     if (stages & DMDQN_STAGE_WGRAD) {
         const int items = A.d.n_nets * 3;
@@ -1734,7 +1768,8 @@ int launch_learn_tc(const LearnArgs& args, int precision, int stages, cudaStream
     A.chain = (stages & kAllStages) == kAllStages ? 1 : 0;      // the sample kernel of this call has just reset the flags
     A.k4a_done = A.sched + 4;
     A.k3_done = A.k4a_done + A.d.n_nets;
-    return precision == DMDQN_PRECISION_TF32 ? launch_tc<1>(A, stages, s) : launch_tc<3>(A, stages, s);
+    if (A.dueling) return precision == DMDQN_PRECISION_TF32 ? launch_tc<1, true>(A, stages, s) : launch_tc<3, true>(A, stages, s);
+    return precision == DMDQN_PRECISION_TF32 ? launch_tc<1, false>(A, stages, s) : launch_tc<3, false>(A, stages, s);
 }
 
 }  // namespace dmdqn

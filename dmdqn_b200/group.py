@@ -41,6 +41,8 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     "n_step": 1,
     # global-norm gradient clipping (Keras global_clipnorm): None, or c > 0 to scale each network's gradient to a norm <= c
     "global_clipnorm": None,
+    # dueling Q-networks (Wang et al. 2016): value and advantage heads on the shared trunk, Q = V + Adv - mean(Adv)
+    "dueling": False,
 }
 
 
@@ -60,9 +62,10 @@ def _on_device(method):
     return wrapper
 
 
-def keras_init(seed: int, state_size: int, hidden: int, action_size: int) -> list[torch.Tensor]:
+def keras_init(seed: int, state_size: int, hidden: int, action_size: int, dueling: bool = False) -> list[torch.Tensor]:
     """HeNormal hidden kernels, GlorotUniform head, zero biases (dqn_agent.py:166-181), as
-    [W1,b1,W2,b2,W3,b3] in Keras ``get_weights()`` order, kernels ``[in,out]``."""
+    [W1,b1,W2,b2,W3,b3] in Keras ``get_weights()`` order, kernels ``[in,out]``.  ``dueling`` appends the value head
+    [Wv [H,1], bv [1]], Wv GlorotUniform drawn from the same generator after W3 (the other draws do not change)."""
     gen = torch.Generator().manual_seed(int(seed))
     out = []
     dims = [state_size, hidden, hidden]
@@ -73,6 +76,9 @@ def keras_init(seed: int, state_size: int, hidden: int, action_size: int) -> lis
         out += [w, torch.zeros(dims[i + 1])]
     limit = math.sqrt(6.0 / (hidden + action_size))
     out += [(torch.rand(hidden, action_size, generator=gen) * 2 - 1) * limit, torch.zeros(action_size)]
+    if dueling:
+        limit = math.sqrt(6.0 / (hidden + 1))
+        out += [(torch.rand(hidden, 1, generator=gen) * 2 - 1) * limit, torch.zeros(1)]
     return out
 
 
@@ -100,6 +106,9 @@ class AgentGroup:
                                  or clip <= 0):
             raise ValueError(f"global_clipnorm={clip!r}: must be None (no clipping) or a positive finite number")
         self.global_clipnorm = None if clip is None else float(clip)
+        if cfg["dueling"] not in (True, False):
+            raise ValueError(f"dueling={cfg['dueling']!r}: must be true or false")
+        self.dueling = bool(cfg["dueling"])
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -115,8 +124,12 @@ class AgentGroup:
 
         self.dims = N.Dims(self.n_agents, self.n_nets, self.state_size, self.obs_stride, self.hidden,
                            self.action_size, self.batch_size, self.capacity)
-        self.layout = N.Layout()
-        N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
+        if self.dueling:        # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
+            self.layout = N.DuelingLayout()
+            N.check(self.lib.dmdqn_param_layout_dueling(C.byref(self.dims), C.byref(self.layout)))
+        else:
+            self.layout = N.Layout()
+            N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
         if cfg["precision"] == "auto":   # fp32-class either way (same 1e-5 bar): tcgen05 3xTF32 where that path is built, FFMA elsewhere
             cfg["precision"] = "tf32x3" if (self.hidden == 256 and self.obs_stride in (32, 64, 96) and self.batch_size % 4 == 0
                                             and self.batch_size <= 4096) else "fp32"
@@ -127,7 +140,7 @@ class AgentGroup:
             int(cfg["target_update_frequency"]), N.LOSS[cfg["loss"]], int(bool(cfg["normalize_rewards"])),
             int(bool(cfg["double_dqn"])), N.ADAM[cfg["adam_form"]], N.SAMPLE[cfg["sample_mode"]],
             N.PRECISION[cfg["precision"]], float(cfg["per_alpha"]), float(cfg["per_beta"]), float(cfg["per_eps"]),
-            int(cfg["per_beta_steps"]), self.n_step)
+            int(cfg["per_beta_steps"]), self.n_step, dueling=int(self.dueling))
 
         dev, n, c, dp, g = self.device, self.n_agents, self.capacity, self.obs_stride, self.n_nets
         if _parent is None:
@@ -210,9 +223,12 @@ class AgentGroup:
 
     # ------------------------------------------------------------------ weights ---------
     def pack(self, weights) -> torch.Tensor:
-        """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]) -> one parameter block."""
+        """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]; dueling: + [Wv [H,1], bv [1]]) -> one parameter block."""
         L, H, A = self.layout, self.hidden, self.action_size
-        w1, b1, w2, b2, w3, b3 = [torch.as_tensor(np.asarray(w), dtype=torch.float32) for w in weights]
+        ws = [torch.as_tensor(np.asarray(w), dtype=torch.float32) for w in weights]
+        if len(ws) != (8 if self.dueling else 6):
+            raise ValueError(f"expected {8 if self.dueling else 6} weight tensors, got {len(ws)}")
+        w1, b1, w2, b2, w3, b3 = ws[:6]
         blk = torch.zeros((L.stride,), dtype=torch.float32)
         blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size] = w1
         blk[L.b1:L.b1 + H] = b1
@@ -220,20 +236,26 @@ class AgentGroup:
         blk[L.b2:L.b2 + H] = b2
         blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A] = w3
         blk[L.b3:L.b3 + A] = b3
+        if self.dueling:
+            blk[L.wv:L.wv + H] = ws[6].reshape(H)
+            blk[L.bv:L.bv + 1] = ws[7].reshape(1)
         return blk
 
     def unpack(self, blk: torch.Tensor) -> list[torch.Tensor]:
         L, H, A = self.layout, self.hidden, self.action_size
         blk = blk.detach().cpu()
-        return [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
-                blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(),
-                blk[L.b2:L.b2 + H].clone(), blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(),
-                blk[L.b3:L.b3 + A].clone()]
+        out = [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
+               blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(),
+               blk[L.b2:L.b2 + H].clone(), blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(),
+               blk[L.b3:L.b3 + A].clone()]
+        if self.dueling:
+            out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
+        return out
 
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
         (dqn_agent.py:129-137)."""
-        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, self.action_size))
+        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, self.action_size, self.dueling))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
@@ -317,8 +339,9 @@ class AgentGroup:
         q = torch.full((n, 4), float("nan"), dtype=torch.float32, device=self.device) if return_q else None
         nets = self.nets if not target else N.Nets(_ptr(self.theta_tgt), _ptr(self.theta_tgt), _ptr(self.adam_m),
                                                    _ptr(self.adam_v), _ptr(self.learn_step))
-        N.check(self.lib.dmdqn_act(C.byref(self.dims), C.byref(nets), _ptr(obs), obs.shape[1], _ptr(eps_t),
-                                   _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream))
+        act = self.lib.dmdqn_act_dueling if self.dueling else self.lib.dmdqn_act
+        N.check(act(C.byref(self.dims), C.byref(nets), _ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions),
+                    _ptr(q), self._stream))
         return (actions, q) if return_q else actions
 
     def draw_words(self, shape) -> torch.Tensor:
@@ -562,6 +585,10 @@ class AgentGroup:
                "active": view(v.active, torch.int32, (g,)), "tc_error": view(v.tc_error, torch.int32, (1,)),
                "is_weights": view(v.is_w, torch.float32, (g, b)),
                "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
+        if self.dueling:         # the folded heads W3e[H][4] | b3e[4] of the last learn step, online (0) and target (1)
+            dv = N.DuelingViews()
+            N.check(self.lib.dmdqn_debug_dueling(C.byref(self.dims), _ptr(self.workspace), self.workspace.numel(), C.byref(dv)))
+            out["head"] = view(dv.head, torch.float32, (2, g, 4 * self.hidden + 4))
         if self.hp.precision != 0:
             # the tcgen05 path keeps its activation scratch transposed ([feature][batch]) and never
             # materialises dh2: "dh2" is relu'(h2) as 0/1 here (its non-zero pattern is what the tests use)
@@ -578,5 +605,5 @@ class AgentGroup:
     def sync_target(self, mask=None, tau: float | None = None) -> None:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
-        N.check(self.lib.dmdqn_sync_target(C.byref(self.dims), C.byref(self.nets), _ptr(mask_t),
-                                           -1.0 if tau is None else float(tau), self._stream))
+        sync = self.lib.dmdqn_sync_target_dueling if self.dueling else self.lib.dmdqn_sync_target
+        N.check(sync(C.byref(self.dims), C.byref(self.nets), _ptr(mask_t), -1.0 if tau is None else float(tau), self._stream))

@@ -32,6 +32,14 @@
  *   dqn_agent.py:153-184), one contiguous block of dmdqn_layout.stride floats:
  *     W1[obs_stride][H] | b1[H] | W2[H][H] | b2[H] | W3[H][4] | b3[4] | pad
  *   theta, theta_tgt, adam_m, adam_v all use that block layout; learn_step: int32[n_nets].
+ *   dueling networks (dmdqn_hparams.dueling = 1; dmdqn_param_layout_dueling) append the value head after b3:
+ *     W1 | b1 | W2 | b2 | W3[H][4] | b3[4] | wv[H] | bv | pad[3] | pad
+ *   with the same offsets up to b3, wv at b3 + 4 (16-byte aligned), bv at b3 + 4 + H, Adam over [0, b3 + 8 + H) (the
+ *   three pad floats keep gradient 0 and stay 0) and the stride rounded up to 32 floats.  Q is
+ *     Q(s, a) = V(s) + Adv(s, a) - (1/A) sum_{b<A} Adv(s, b),  Adv = h2 . W3[:, a] + b3[a],  V = h2 . wv + bv
+ *   (Wang et al. 2016), which is the plain 4-wide head with the effective weights
+ *     W3e[k][a] = (W3[k][a] - mean_{b<A} W3[k][b]) + wv[k]  (a < A; 0 for a >= A),  b3e[a] = (b3[a] - mean_{b<A} b3[b]) + bv
+ *   each mean summed left to right in fp32 and divided by A (IEEE division).  Advantage columns >= A keep gradient 0.
  */
 #ifndef DMDQN_B200_H
 #define DMDQN_B200_H
@@ -124,6 +132,9 @@ typedef struct dmdqn_hparams {
     int32_t adam_form;                /* DMDQN_ADAM_*                                      */
     int32_t sample_mode;              /* DMDQN_SAMPLE_*                                    */
     int32_t precision;                /* DMDQN_PRECISION_*                                 */
+    int32_t dueling;                  /* 0 = plain head, 1 = dueling value + advantage heads (parameter blocks in the
+                                         dueling layout); any other value is refused.  In what was interior padding:
+                                         offset 76, sizeof stays 112 */
     /* prioritized replay (read in DMDQN_SAMPLE_PRIORITIZED only): priority = (|delta| + per_eps)^per_alpha,
      * importance exponent beta_t = min(1, per_beta0 + (1 - per_beta0) * t / per_beta_steps) with t the network's
      * learn_step after the increment (per_beta_steps <= 0: beta_t = per_beta0) */
@@ -145,6 +156,14 @@ int dmdqn_abi_version(void);
 
 /* Parameter block layout for the given dims. */
 int dmdqn_param_layout(const dmdqn_dims* dims, dmdqn_layout* out);
+
+/* Parameter block layout of a dueling network (dmdqn_hparams.dueling = 1): dmdqn_param_layout's offsets up to b3, the
+ * value head's wv[H] and bv, and the dueling stride.  Every call that takes dueling blocks and no hparams has a
+ * *_dueling sibling below; passing dueling blocks to dmdqn_act or dmdqn_sync_target is a caller error. */
+typedef struct dmdqn_dueling_layout {
+    int64_t w1, b1, w2, b2, w3, b3, wv, bv, stride;
+} dmdqn_dueling_layout;
+int dmdqn_param_layout_dueling(const dmdqn_dims* dims, dmdqn_dueling_layout* out);
 
 /* Bytes of device scratch dmdqn_sample / dmdqn_learn need for these dims. */
 int dmdqn_workspace_bytes(const dmdqn_dims* dims, size_t* out_bytes);
@@ -204,6 +223,11 @@ int dmdqn_featurize_alt(int32_t n, const int32_t* halting, const int32_t* phase,
 int dmdqn_act(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
               const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
               int32_t* actions_out, float* q_out, void* stream);
+/* The same on dueling parameter blocks: the head is folded into W3e / b3e in registers with the arithmetic above, so
+ * q_out and the actions equal dmdqn_act's on a plain block holding the folded head, bit for bit. */
+int dmdqn_act_dueling(const dmdqn_dims* dims, const dmdqn_nets* nets, const float* obs, int32_t obs_in_stride,
+                      const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
+                      int32_t* actions_out, float* q_out, void* stream);
 
 /* K1a -- append one transition per agent to its ring.
  * Replaces ReplayBuffer.add / DQNAgent.remember / store_experience
@@ -247,7 +271,8 @@ int dmdqn_push(const dmdqn_dims* dims, const dmdqn_replay* replay, const float* 
  *   is done, else (float)(gamma^m) with gamma^m the float64 product formed left to right.
  * The workspace keeps R as r_hat, the terminal flag as the batch's dones, and the bootstrap rows and discounts
  * (dmdqn_debug_nstep).  n = 0 or 1 is the one-step target: R = r_hat, discount = (float)gamma * (1 - done), and the
- * bootstrap row is the drawn row.  n < 0 or n > DMDQN_MAX_NSTEP is refused. */
+ * bootstrap row is the drawn row.  n < 0 or n > DMDQN_MAX_NSTEP is refused.
+ * hp->dueling other than 0 or 1 is refused here and by every other call that takes hparams. */
 #define DMDQN_PER_MAX_CAPACITY (8192 * 128)
 int dmdqn_sample(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                  const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
@@ -279,14 +304,23 @@ int dmdqn_gather(const dmdqn_dims* dims, const dmdqn_replay* replay, const void*
  * On the tcgen05 path the four kernels of one call form a dataflow chain (programmatic dependent launches:
  * K3 starts under the sample kernel's tail, K4a / K4b take over SMs while the previous kernel is still running
  * and wait on per-tile / per-network flags in the workspace, which the sample kernel resets).  Results are
- * bit-identical to the stage-by-stage form below; the workspace must not be shared by two calls in flight. */
+ * bit-identical to the stage-by-stage form below; the workspace must not be shared by two calls in flight.
+ * Dueling (hp->dueling = 1): before the sample kernel, a fold kernel writes W3e | b3e of the online and the target
+ * network into the workspace (dmdqn_debug_dueling); K3 / K4a read the head from there, so their Q values, TD targets,
+ * losses and trunk gradients are those of a plain network with the folded head.  The head update projects the folded
+ * head's gradient G back onto the true parameters:
+ *   dW3[k][a] = G[k][a] - (1/A) sum_{b<A} G[k][b] (a < A, else 0),  dwv[k] = sum_{b<A} G[k][b]   (likewise db3, dbv)
+ * and dmdqn_learn_grads stores these at the W3 / b3 / wv / bv offsets. */
 int dmdqn_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
                 const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
                 float* metrics_out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* The same step, one stage per call, so a caller can bracket each kernel with CUDA events
  * (bench.py roofline): stages is a bit mask of DMDQN_STAGE_*; all four in order == dmdqn_learn (same bits;
- * kernels of different calls are ordered by the stream alone, only a call with all four stages is chained). */
+ * kernels of different calls are ordered by the stream alone, only a call with all four stages is chained).
+ * Dueling (hp->dueling = 1): the fold of the heads runs with the SAMPLE stage of this call, so the TARGET and ONLINE stages
+ * need a preceding SAMPLE stage of dmdqn_learn_stages (or dmdqn_learn) on the same weights; a batch drawn by dmdqn_sample
+ * leaves the folded heads of an earlier step (or none) in the workspace. */
 #define DMDQN_STAGE_SAMPLE 1   /* K1b */
 #define DMDQN_STAGE_TARGET 2   /* K3  */
 #define DMDQN_STAGE_ONLINE 4   /* K4a */
@@ -316,7 +350,8 @@ int dmdqn_step_host(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn
                     float* metrics_dev, float* metrics_host, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Shared-parameter mode across ranks (n_nets == 1; not in the reference, BASELINE.json cfg5):
- * the same step but K4b stores dL/dtheta into grads_out[n_nets][layout.stride] instead of
+ * the same step but K4b stores dL/dtheta into grads_out[n_nets][layout.stride] (every float of the range the Adam calls
+ * update: [0, b3 + 4), or [0, b3 + 8 + H) for dueling blocks, whose three pad floats get gradient 0) instead of
  * applying Adam, with the loss mean taken over global_batch (= batch * ranks), so that the
  * caller can sum the blocks over ranks (ncclAllReduce) and finish with dmdqn_adam_apply,
  * which takes the step's learn flags and Adam scalars (alpha_t, eps, target-sync mode) from the
@@ -332,7 +367,8 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
  * with every network's gradient scaled to a global norm of at most c = global_clipnorm first.  A clipped learn step is
  * dmdqn_learn_grads(..., global_batch = batch, grads, ...) followed by this call (with shared parameters across ranks: on
  * the all-reduced block, so every replica scales by the same n).  For every network g that learned this step:
- *   1. G = grads[g][0 .. layout.b3 + 4), the range dmdqn_adam_apply updates;
+ *   1. G = grads[g][0 .. layout.b3 + 4), the range dmdqn_adam_apply updates; for dueling blocks (hp->dueling = 1)
+ *      [0 .. b3 + 8 + H): W3, b3, the value head wv, bv and its three pad floats;
  *   2. n = sqrt(sum G_i^2) in float64 (the squares are exact); the summation order is fixed by the kernel (8 contiguous
  *      slices, each summed by its CTA in a fixed thread order, the 8 partials added in slice order) and does not depend
  *      on the other networks or on how many networks the call covers;
@@ -401,11 +437,20 @@ typedef struct dmdqn_nstep_views {
     const int32_t* next_rows; const float* discount;
 } dmdqn_nstep_views;
 int dmdqn_debug_nstep(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_nstep_views* out);
+/* Dueling view of the last learn step: head float[2][n_nets][4H + 4], W3e[H][4] | b3e[4] of the online (0) and the target
+ * (1) network as the fold kernel wrote them. */
+typedef struct dmdqn_dueling_views {
+    const float* head;
+} dmdqn_dueling_views;
+int dmdqn_debug_dueling(const dmdqn_dims* dims, void* workspace, size_t workspace_bytes, dmdqn_dueling_views* out);
 
 /* theta_tgt <- theta for the networks whose mask is set (NULL = all).
  * Replaces DQNAgent.update_target_network (dqn_agent.py:382-384) when called explicitly. */
 int dmdqn_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask,
                       double tau, void* stream);
+/* The same on dueling parameter blocks: the whole dueling stride, value head included. */
+int dmdqn_sync_target_dueling(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask,
+                              double tau, void* stream);
 
 #ifdef __cplusplus
 }
