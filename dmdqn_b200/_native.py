@@ -73,6 +73,14 @@ class DuelingViews(C.Structure):
     _fields_ = [("head", C.c_void_p)]
 
 
+class Noisy(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("sigma", "sigma_tgt", "sigma_m", "sigma_v", "eff", "eff_tgt", "noise", "key")]
+
+
+class NoiseRecord(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("w1_in", "w1_out", "w2_in", "w2_out", "w3_in", "w3_out", "v_in", "v_out", "stride")]
+
+
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
 
 
@@ -124,6 +132,15 @@ SIGNATURES = {
     "dmdqn_debug_dueling": (C.c_int, [C.POINTER(Dims), _P, C.c_size_t, C.POINTER(DuelingViews)]),
     "dmdqn_sync_target": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_double, _P]),
     "dmdqn_sync_target_dueling": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), _P, C.c_double, _P]),
+    "dmdqn_noise_layout": (C.c_int, [C.POINTER(Dims), C.POINTER(NoiseRecord)]),
+    "dmdqn_noisy_fold": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.POINTER(Noisy), _P]),
+    "dmdqn_learn_grads_noisy": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Replay), C.POINTER(Nets),
+                                          C.POINTER(Noisy), _P, _P, C.c_int32, _P, _P, _P, C.c_size_t, _P]),
+    "dmdqn_noisy_adam_apply": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.POINTER(Noisy), _P, _P,
+                                         C.c_size_t, _P]),
+    "dmdqn_act_noisy": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32, _P, C.c_int32, _P, _P, _P,
+                                  _P, _P, _P]),
+    "dmdqn_sync_target_noisy": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32, _P, C.c_double, _P]),
 }
 
 _lib = None

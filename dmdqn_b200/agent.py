@@ -78,7 +78,8 @@ class _Network:
         """Q-values ``[n, A]`` for ``states [n, D]`` (one act-kernel launch per row)."""
         x = torch.as_tensor(states, dtype=torch.float32).reshape(-1, self._g.state_size)
         target = self._which == "target"
-        return torch.stack([self._g.act(row[None], return_q=True, target=target)[1][0, : self._g.action_size] for row in x])
+        return torch.stack([self._g.act(row[None], return_q=True, target=target, noisy=False)[1][0, : self._g.action_size]
+                            for row in x])
 
 
 class DQNAgent:
@@ -108,6 +109,8 @@ class DQNAgent:
         if _group is None:
             _group = AgentGroup(1, config, self.state_size, self.action_size, seed=config.get("seed", 0))
         self._g = _group.agent_view(_index)
+        if self._g.noisy:       # noisy networks explore through their learned noise: no epsilon-greedy
+            self.epsilon = self.epsilon_min = 0.0
         self.online_network = _Network(self._g, "online")
         self.target_network = _Network(self._g, "target")
         self.replay_buffer = ReplayBuffer(self.buffer_size, _group=self._g)
@@ -117,18 +120,27 @@ class DQNAgent:
 
     # -- act -----------------------------------------------------------------------------
     def update_epsilon_before_action(self) -> float:
-        """The src/agents schedule, evaluated before the explore draw (:258-261); a no-op for 'linear'."""
+        """The src/agents schedule, evaluated before the explore draw (:258-261); a no-op for 'linear'.  Always 0 for
+        noisy networks."""
+        if self._g.noisy:
+            return self.epsilon
         self.epsilon = epsilon_schedules.before_action(self.epsilon_schedule, self.epsilon, self.epsilon_min,
                                                        self.global_step_count)
         return self.epsilon
 
     def update_epsilon_after_action(self) -> float:
         """The variant's linear decay, applied after the action was chosen (experimental/agent.py:140-144)."""
+        if self._g.noisy:
+            return self.epsilon
         self.epsilon = epsilon_schedules.after_action(self.epsilon_schedule, self.epsilon, self.epsilon_min,
                                                       self.epsilon_decay_rate)
         return self.epsilon
 
     def select_action(self, state_tensor) -> int:
+        """Epsilon-greedy on the online network; with ``noisy: true`` greedy on the noisy online network (the noise of the
+        next learn step), with no epsilon draw."""
+        if self._g.noisy:
+            return int(self._g.act(torch.as_tensor(state_tensor, dtype=torch.float32).reshape(1, -1)).item())
         self.update_epsilon_before_action()
         if np.random.rand() < self.epsilon:                                 # :263-265
             action = np.random.randint(0, self.action_size)
@@ -138,7 +150,8 @@ class DQNAgent:
         return action
 
     def select_greedy_action(self, state_tensor) -> int:
-        return int(self._g.act(torch.as_tensor(state_tensor, dtype=torch.float32).reshape(1, -1)).item())
+        """Greedy on the online network; for noisy networks on the mean weights mu alone (greedy evaluation)."""
+        return int(self._g.act(torch.as_tensor(state_tensor, dtype=torch.float32).reshape(1, -1), noisy=False).item())
 
     # -- remember ------------------------------------------------------------------------
     def store_experience(self, experience) -> None:                        # :306-310

@@ -440,6 +440,101 @@ int dmdqn_debug_dueling(const dmdqn_dims* dims, void* workspace, size_t workspac
     return DMDQN_OK;
 }
 
+int dmdqn_noise_layout(const dmdqn_dims* dims, dmdqn_noise_record* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const NoiseRec r = make_noise_rec(dims->obs_stride, dims->hidden);
+    int64_t* f[8] = {&out->w1_in, &out->w1_out, &out->w2_in, &out->w2_out, &out->w3_in, &out->w3_out, &out->v_in, &out->v_out};
+    for (int v = 0; v < 8; ++v) *f[v] = r.off[v];
+    out->stride = r.stride;
+    return DMDQN_OK;
+}
+
+// Every pointer of the noisy blocks, and the 16-byte alignment the float4 kernels need.
+static int check_noisy(const dmdqn_nets* nets, const dmdqn_noisy* nz, bool adam) {
+    DMDQN_CHECK_ARG(nets && nz && nets->theta && nets->theta_tgt && nets->learn_step, "noisy: NULL network pointer");
+    DMDQN_CHECK_ARG(nz->sigma && nz->sigma_tgt && nz->eff && nz->eff_tgt && nz->noise && nz->key, "noisy: NULL noisy pointer");
+    if (adam) DMDQN_CHECK_ARG(nets->adam_m && nets->adam_v && nz->sigma_m && nz->sigma_v, "noisy: NULL Adam moment pointer");
+    const void* p[] = {nets->theta, nets->theta_tgt, nz->sigma, nz->sigma_tgt, nz->eff, nz->eff_tgt, nz->noise,
+                       adam ? nz->sigma_m : nz->sigma, adam ? nz->sigma_v : nz->sigma};
+    for (const void* q : p) DMDQN_CHECK_ARG((uintptr_t)q % 16 == 0, "noisy: pointer %p is not 16-byte aligned", q);
+    return DMDQN_OK;
+}
+
+int dmdqn_noisy_fold(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                     void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(hp != nullptr, "noisy_fold: hp is NULL");
+    if ((rc = check_dueling(hp))) return rc;
+    if ((rc = check_noisy(nets, noisy, false))) return rc;
+    return launch_noisy_fold(*dims, hp->dueling == 1, *nets, *noisy, (cudaStream_t)stream);
+}
+
+int dmdqn_learn_grads_noisy(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
+                            const dmdqn_nets* nets, const dmdqn_noisy* noisy, const void* draws, const uint8_t* learn_mask,
+                            int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
+                            size_t workspace_bytes, void* stream) {
+    Workspace w;                      // everything run_learn checks, before the fold is launched
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    if ((rc = check_noisy(nets, noisy, true))) return rc;
+    DMDQN_CHECK_ARG(grads_out != nullptr, "grads_out is NULL");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32 || tc_supported(*dims),
+                    "precision=%d (tcgen05) needs hidden=256 and obs_stride in {32,64,96}; got hidden=%d obs_stride=%d",
+                    hp->precision, dims->hidden, dims->obs_stride);
+    if ((rc = launch_noisy_fold(*dims, hp->dueling == 1, *nets, *noisy, (cudaStream_t)stream))) return rc;
+    dmdqn_nets eff = *nets;
+    eff.theta = noisy->eff;
+    eff.theta_tgt = noisy->eff_tgt;
+    return run_learn(dims, hp, replay, &eff, draws, learn_mask, metrics_out, workspace, workspace_bytes, kAllStages, grads_out,
+                     global_batch, stream);
+}
+
+int dmdqn_noisy_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                           const float* grads, void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(hp && grads, "noisy_adam_apply: NULL argument");
+    if ((rc = check_dueling(hp))) return rc;
+    if ((rc = check_noisy(nets, noisy, true))) return rc;
+    DMDQN_CHECK_ARG((uintptr_t)grads % 16 == 0, "noisy_adam_apply: grads is not 16-byte aligned");
+    return launch_noisy_adam_apply(*dims, *hp, *nets, *noisy, grads, (char*)workspace, w, (cudaStream_t)stream);
+}
+
+int dmdqn_act_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
+                    const float* obs, int32_t obs_in_stride, const double* eps, const uint32_t* w_explore,
+                    const uint32_t* w_action, int32_t* actions_out, float* q_out, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(dueling == 0 || dueling == 1, "dueling=%d must be 0 or 1", dueling);
+    DMDQN_CHECK_ARG(nets && nets->theta && nets->learn_step && noisy && noisy->sigma && noisy->key, "act_noisy: NULL network pointer");
+    DMDQN_CHECK_ARG((uintptr_t)nets->theta % 16 == 0 && (uintptr_t)noisy->sigma % 16 == 0,
+                    "act_noisy: theta and sigma must be 16-byte aligned");
+    DMDQN_CHECK_ARG(obs && eps && w_explore && w_action && actions_out, "act_noisy: NULL argument");
+    DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
+    return launch_act(*dims, *nets, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out, dueling == 1,
+                      (cudaStream_t)stream, noisy);
+}
+
+int dmdqn_sync_target_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
+                            const uint8_t* mask, double tau, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    DMDQN_CHECK_ARG(dueling == 0 || dueling == 1, "dueling=%d must be 0 or 1", dueling);
+    DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt && noisy && noisy->sigma && noisy->sigma_tgt,
+                    "sync_target_noisy: NULL network pointer");
+    dmdqn_nets sigma = *nets;
+    sigma.theta = noisy->sigma;
+    sigma.theta_tgt = noisy->sigma_tgt;
+    if ((rc = launch_sync_target(*dims, *nets, mask, tau, dueling == 1, (cudaStream_t)stream))) return rc;
+    return launch_sync_target(*dims, sigma, mask, tau, dueling == 1, (cudaStream_t)stream);
+}
+
 static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau, bool dueling,
                            void* stream) {
     int rc = validate_dims(dims);

@@ -72,6 +72,91 @@ __host__ __device__ __forceinline__ float head_project(float (&g)[4], int A) {
     return s;
 }
 
+// Noisy networks (include/dmdqn_b200.h dmdqn_noisy): Philox4x32-10 (Salmon et al. 2011, Random123's constants and round
+// order, the same function as curand_Philox4x32_10), usable on the host so that a host build can check it.
+__host__ __device__ __forceinline__ uint32_t philox_mulhi(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+    return __umulhi(a, b);
+#else
+    return (uint32_t)(((uint64_t)a * b) >> 32);
+#endif
+}
+__host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+        const uint32_t hi0 = philox_mulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = philox_mulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    }
+    return c;
+}
+
+// Offsets (floats) of the eight factor vectors inside one network's noise record for one set (include/dmdqn_b200.h
+// dmdqn_noise_record): off[2 * layer + side], layer 0..3 = W1, W2, W3, value head, side 0 = inputs, 1 = outputs; off[8]
+// is the end of the last vector, `stride` the record's stride (a network's two sets are adjacent records).
+struct NoiseRec {
+    int32_t off[9];
+    int32_t stride;
+};
+__host__ __device__ inline NoiseRec make_noise_rec(int dp, int h) {
+    const int32_t len[8] = {dp, h, h, h, h, 4, h, 4};
+    NoiseRec r;
+    r.off[0] = 0;
+    for (int v = 0; v < 8; ++v) r.off[v + 1] = r.off[v] + len[v];
+    r.stride = (r.off[8] + 31) / 32 * 32;
+    return r;
+}
+
+// f(z) of one factor entry: z = Box-Muller in float64 on the Philox words (x, y) of counter {i, layer<<2 | side<<1 | set,
+// t, "nois"} under the network's key (low word first), rounded to fp32; f(z) = sgn(z) sqrt|z| in fp32.
+__device__ __forceinline__ float noise_factor(uint64_t key, uint32_t i, int vec, int set, uint32_t t) {
+    const uint4 w = philox4x32_10(make_uint4(i, (uint32_t)((vec >> 1) << 2 | (vec & 1) << 1 | set), t, 0x6e6f6973u),
+                                  make_uint2((uint32_t)key, (uint32_t)(key >> 32)));
+    const double u1 = ((double)w.x + 0.5) * 0x1p-32, u2 = (double)w.y * 0x1p-32;
+    const float z = (float)(sqrt(-2.0 * log(u1)) * cos(6.283185307179586 * u2));
+    return z >= 0.f ? sqrtf(z) : -sqrtf(-z);
+}
+
+// The whole record of one network and set into `rec` (shared memory), every thread of the block taking part; entries for
+// padding (W1 input rows >= obs_dim, W3 output columns >= A, the value head's outputs >= 1, the tail up to the stride) are 0.
+__device__ __forceinline__ void noise_record_build(float* rec, const NoiseRec& R, int obs_dim, int n_actions, uint64_t key,
+                                                   uint32_t t, int set) {
+    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) {
+        int v = 0;
+        while (v < 8 && e >= R.off[v + 1]) ++v;
+        const int i = e - R.off[v];
+        const int valid = v == 0 ? obs_dim : v == 5 ? n_actions : v == 7 ? 1 : R.off[v + 1] - R.off[v];
+        rec[e] = v < 8 && i < valid ? noise_factor(key, (uint32_t)i, v, set, t) : 0.f;
+    }
+}
+
+// The weight noise of the four floats at offset e (a multiple of 4) of a parameter block: f_in[i] * f_out[j] for a weight,
+// f_out[j] for a bias, 0 on padding.  rec: the record of the set (include/dmdqn_b200.h: wv is the value head's input side
+// and column 0 of its output side, bv with its three pad floats takes the output side's four entries).
+__device__ __forceinline__ float4 noise_eps4(const float* rec, const NoiseRec& R, const Layout& L, int H, bool dueling, int64_t e) {
+    auto outer = [&](float fi, const float* fo) {
+        return make_float4(__fmul_rn(fi, fo[0]), __fmul_rn(fi, fo[1]), __fmul_rn(fi, fo[2]), __fmul_rn(fi, fo[3]));
+    };
+    auto vec = [](const float* f) { return make_float4(f[0], f[1], f[2], f[3]); };
+    if (e < L.b1) return outer(rec[R.off[0] + e / H], rec + R.off[1] + e % H);
+    if (e < L.w2) return vec(rec + R.off[1] + (e - L.b1));
+    if (e < L.b2) return outer(rec[R.off[2] + (e - L.w2) / H], rec + R.off[3] + (e - L.w2) % H);
+    if (e < L.w3) return vec(rec + R.off[3] + (e - L.b2));
+    if (e < L.b3) return outer(rec[R.off[4] + (e - L.w3) / 4], rec + R.off[5]);
+    if (e < L.b3 + 4) return vec(rec + R.off[5]);
+    if (dueling && e < layout_bv(L, H)) {
+        const float fo = rec[R.off[7]];
+        const float* fi = rec + R.off[6] + (e - layout_wv(L));
+        return make_float4(__fmul_rn(fi[0], fo), __fmul_rn(fi[1], fo), __fmul_rn(fi[2], fo), __fmul_rn(fi[3], fo));
+    }
+    if (dueling && e == layout_bv(L, H)) return vec(rec + R.off[7]);
+    return make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+// mu + sigma * eps as the header states it: one rounded product, then one rounded sum
+__device__ __forceinline__ float noisy_weight(float mu, float sigma, float eps) { return __fadd_rn(mu, __fmul_rn(sigma, eps)); }
+
 // Tile geometry of the fused MLP kernels for hidden width H (DESIGN.md "K3/K4 tiling").
 // A CTA owns BM batch rows and all H output columns; each thread an 8x8 register tile.
 template <int H>
@@ -261,7 +346,10 @@ int launch_featurize_alt(int32_t n, const int32_t* halting, const int32_t* phase
                          double* own_out, float* obs_out, int32_t obs_out_stride, double* reward_out, cudaStream_t s);
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
                const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,
-               cudaStream_t s);
+               cudaStream_t s, const dmdqn_noisy* noisy = nullptr);
+int launch_noisy_fold(const dmdqn_dims& d, bool dueling, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s);
+int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
+                            const float* grads, char* ws, const Workspace& w, cudaStream_t s);
 int launch_push(const dmdqn_dims& d, const dmdqn_replay& rp, const float* obs, const int32_t* act,
                 const double* rew, const float* next_obs, const uint8_t* done, int32_t in_stride,
                 const uint8_t* mask, cudaStream_t s);

@@ -624,6 +624,65 @@ __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ g
     }
 }
 
+// Noisy networks (include/dmdqn_b200.h dmdqn_noisy).  Fold: CTA (c, g, s) builds the noise record of network g and set s in
+// shared memory (every CTA of the pair builds it: a few thousand Philox draws against the ~MB it streams), CTA c == 0
+// stores it, and every CTA writes eff = mu + sigma * eps over its share of the stride.  HBM bound: 8 bytes read and 4
+// written per float.
+constexpr int kNoisyThreads = 256;
+
+__global__ void __launch_bounds__(kNoisyThreads)
+noisy_fold_kernel(Layout L, NoiseRec R, int H, int obs_dim, int n_actions, int dueling, const dmdqn_nets nets,
+                  const dmdqn_noisy nz, int64_t per) {
+    extern __shared__ __align__(16) float rec[];
+    const int g = blockIdx.y, set = blockIdx.z;
+    noise_record_build(rec, R, obs_dim, n_actions, __ldg(nz.key + g), (uint32_t)__ldg(nets.learn_step + g), set);
+    __syncthreads();
+    if (blockIdx.x == 0)
+        for (int e = threadIdx.x; e < R.stride; e += blockDim.x) nz.noise[((size_t)g * 2 + set) * R.stride + e] = rec[e];
+    const size_t base = (size_t)g * L.stride;
+    const float4* mu = reinterpret_cast<const float4*>((set ? nets.theta_tgt : nets.theta) + base);
+    const float4* sg = reinterpret_cast<const float4*>((set ? nz.sigma_tgt : nz.sigma) + base);
+    float4* out = reinterpret_cast<float4*>((set ? nz.eff_tgt : nz.eff) + base);
+    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, L.stride / 4);
+    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        const float4 m = __ldg(mu + i), s = __ldg(sg + i), e = noise_eps4(rec, R, L, H, dueling, i * 4);
+        out[i] = make_float4(noisy_weight(m.x, s.x, e.x), noisy_weight(m.y, s.y, e.y), noisy_weight(m.z, s.z, e.z),
+                             noisy_weight(m.w, s.w, e.w));
+    }
+}
+
+// Adam on mu and sigma from the effective-weight gradient g: g_mu = g, g_sigma = g * eps with set 0's record, each through
+// adam_vec4 as adam_apply_kernel applies it.  HBM bound: g once, and theta / m / v (+ target) of mu and of sigma.
+__global__ void __launch_bounds__(kNoisyThreads)
+noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, const float* __restrict__ grads, int64_t per) {
+    extern __shared__ __align__(16) float rec[];
+    const int g = blockIdx.y;
+    if (!A.active[g] || *reinterpret_cast<volatile int*>(A.error) != 0) return;
+    const float* src = nz.noise + (size_t)g * 2 * R.stride;
+    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) rec[e] = src[e];
+    __syncthreads();
+    const AdamStep k = adam_step(A, g);
+    const int H = A.d.hidden;
+    const size_t base = (size_t)g * A.L.stride;
+    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, A.L.end / 4);
+    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        const float4 g4 = *reinterpret_cast<const float4*>(grads + base + i * 4);
+        const float4 e = noise_eps4(rec, R, A.L, H, A.dueling, i * 4);
+        const float gm[4] = {g4.x, g4.y, g4.z, g4.w};
+        const float gs[4] = {__fmul_rn(g4.x, e.x), __fmul_rn(g4.y, e.y), __fmul_rn(g4.z, e.z), __fmul_rn(g4.w, e.w)};
+        const size_t o = base + i * 4;
+        adam_vec4(k, gm, A.nets.theta + o, A.nets.adam_m + o, A.nets.adam_v + o, A.nets.theta_tgt + o);
+        adam_vec4(k, gs, nz.sigma + o, nz.sigma_m + o, nz.sigma_v + o, nz.sigma_tgt + o);
+    }
+}
+
+// CTAs per network (fold: per network and set) of the two noisy kernels: enough for two waves over the SMs, each CTA
+// streaming at least 2048 float4s.
+inline int noisy_chunks(int n_sm, int64_t pairs, int64_t n4) {
+    const int64_t want = (2 * (int64_t)n_sm + pairs - 1) / pairs;
+    return (int)max((int64_t)1, min(want, (n4 + 2047) / 2048));
+}
+
 // Global-norm clipping in front of the same Adam + target sync (dmdqn_clip_adam_apply, include/dmdqn_b200.h): one
 // cluster of kClipCtas CTAs per network.  CTA r of the cluster owns float4s [r * per, (r + 1) * per) of the block
 // [0, b3 + 4): it brings them into shared memory with one bulk copy, forms their float64 sum of squares in a fixed
@@ -937,6 +996,34 @@ int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Wor
     const Layout L = make_layout(d.obs_stride, d.hidden, true);
     fold_kernel<<<dim3(d.n_nets, 2), 256, 0, s>>>(L, d.hidden, d.n_actions, nets.theta, nets.theta_tgt,
                                                   reinterpret_cast<float*>(ws + w.head));
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_noisy_fold(const dmdqn_dims& d, bool dueling, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s) {
+    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden);
+    int n_sm = 0;
+    if (int rc = device_sm_count(&n_sm)) return rc;
+    const int64_t n4 = L.stride / 4;
+    const int chunks = noisy_chunks(n_sm, 2 * (int64_t)d.n_nets, n4);
+    const int64_t per = (n4 + chunks - 1) / chunks;
+    noisy_fold_kernel<<<dim3(chunks, d.n_nets, 2), kNoisyThreads, R.stride * sizeof(float), s>>>(
+        L, R, d.hidden, d.obs_dim, d.n_actions, dueling ? 1 : 0, nets, nz, per);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
+                            const float* grads, char* ws, const Workspace& w, cudaStream_t s) {
+    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden);
+    int n_sm = 0;
+    if (int rc = device_sm_count(&n_sm)) return rc;
+    const int64_t n4 = A.L.end / 4;
+    const int chunks = noisy_chunks(n_sm, d.n_nets, n4);
+    const int64_t per = (n4 + chunks - 1) / chunks;
+    noisy_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, R, grads, per);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

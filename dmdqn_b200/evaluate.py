@@ -7,7 +7,8 @@
 The reference script drives a ``SumoTrafficEnvironment``; here ``TraciGridEnv`` offers the same four calls
 (``reset(sumo_seed)``, ``step(actions) -> (obs, rewards, done, info)``, ``get_controlled_intersection_ids()``,
 ``get_action_size(id)``) over TraCI -- real SUMO when ``traci`` imports, the seeded queue model otherwise --
-with the 89-dim observation ``DQNAgent`` is built for (order_lanes.py:502-555) and train.py's reward."""
+with the 89-dim observation ``DQNAgent`` is built for (order_lanes.py:502-555) and train.py's reward.  Noisy networks
+(``noisy: true``) are evaluated greedily on their mean weights mu, without noise."""
 from __future__ import annotations
 
 import argparse
@@ -111,7 +112,7 @@ def run_evaluation_episode(env, config, episode_seed, mode="dqn", agents=None, e
                 actions[a] = int(cyc[st["phase_idx"]][0])
                 st["time_in_phase"] += config.get("step_duration", STEP_DURATION)
         if greedy:
-            acts = env.group.act(env.obs_dev).cpu().numpy()     # eps = None: greedy for all, one launch
+            acts = env.group.act(env.obs_dev, noisy=False).cpu().numpy()     # greedy for all on mu, one launch
             for a in greedy:
                 actions[a] = int(acts[ids.index(a)])
         next_observations, rewards, done, _ = env.step(actions)

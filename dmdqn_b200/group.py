@@ -43,6 +43,9 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     "global_clipnorm": None,
     # dueling Q-networks (Wang et al. 2016): value and advantage heads on the shared trunk, Q = V + Adv - mean(Adv)
     "dueling": False,
+    # noisy networks (Fortunato et al. 2018): factorized Gaussian noise on every layer replaces epsilon-greedy exploration;
+    # sigma starts at noisy_sigma0 / sqrt(fan_in)
+    "noisy": False, "noisy_sigma0": 0.5,
 }
 
 
@@ -82,6 +85,16 @@ def keras_init(seed: int, state_size: int, hidden: int, action_size: int, duelin
     return out
 
 
+def noise_key(seed: int) -> int:
+    """The 64-bit Philox key of a noisy network from its init seed (``seed + g``, the seed ``keras_init`` takes): splitmix64,
+    so a network's noise depends on its global index only, not on how the agents are sharded."""
+    m = (1 << 64) - 1
+    z = (int(seed) + 0x9E3779B97F4A7C15) & m
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & m
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & m
+    return z ^ (z >> 31)
+
+
 class AgentGroup:
     def __init__(self, n_agents: int, config: dict | None = None, state_size: int = 89, action_size: int = 4,
                  device: str | torch.device | None = None, seed: int = 0, _parent: "AgentGroup | None" = None,
@@ -109,6 +122,16 @@ class AgentGroup:
         if cfg["dueling"] not in (True, False):
             raise ValueError(f"dueling={cfg['dueling']!r}: must be true or false")
         self.dueling = bool(cfg["dueling"])
+        if not isinstance(cfg["noisy"], (bool, np.bool_)):
+            raise ValueError(f"noisy={cfg['noisy']!r}: must be true or false")
+        self.noisy = bool(cfg["noisy"])
+        s0 = cfg["noisy_sigma0"]
+        if isinstance(s0, bool) or not isinstance(s0, numbers.Real) or not math.isfinite(s0) or s0 < 0:
+            raise ValueError(f"noisy_sigma0={s0!r}: must be a finite number >= 0")
+        self.noisy_sigma0 = float(s0)
+        if self.noisy and self.global_clipnorm is not None:
+            raise ValueError("noisy=true cannot be combined with global_clipnorm yet: the global norm over the mean and the "
+                             "sigma gradients is not implemented")
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -130,6 +153,8 @@ class AgentGroup:
         else:
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
+        self.noise_record = N.NoiseRecord()
+        N.check(self.lib.dmdqn_noise_layout(C.byref(self.dims), C.byref(self.noise_record)))
         if cfg["precision"] == "auto":   # fp32-class either way (same 1e-5 bar): tcgen05 3xTF32 where that path is built, FFMA elsewhere
             cfg["precision"] = "tf32x3" if (self.hidden == 256 and self.obs_stride in (32, 64, 96) and self.batch_size % 4 == 0
                                             and self.batch_size <= 4096) else "fp32"
@@ -143,6 +168,8 @@ class AgentGroup:
             int(cfg["per_beta_steps"]), self.n_step, dueling=int(self.dueling))
 
         dev, n, c, dp, g = self.device, self.n_agents, self.capacity, self.obs_stride, self.n_nets
+        for name in self._NOISY_PTRS:
+            setattr(self, name, None)
         if _parent is None:
             self.obs = torch.zeros((n, c, dp), dtype=torch.float32, device=dev)
             self.next_obs = torch.zeros((n, c, dp), dtype=torch.float32, device=dev)
@@ -161,6 +188,13 @@ class AgentGroup:
             # gradient clipping: the raw gradient blocks of a step and each network's norm before clipping (last step)
             self.grads = torch.zeros_like(self.theta) if self.global_clipnorm is not None else None
             self.grad_norms = torch.zeros((g,), dtype=torch.float32, device=dev) if self.global_clipnorm is not None else None
+            if self.noisy:      # sigma with its target and moments, the effective blocks, the gradient and the noise record
+                self.sigma, self.sigma_tgt = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
+                self.sigma_m, self.sigma_v = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
+                self.eff, self.eff_tgt = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
+                self.grads = torch.zeros_like(self.theta)
+                self.noise = torch.zeros((g, 2, int(self.noise_record.stride)), dtype=torch.float32, device=dev)
+                self.key = torch.zeros((g,), dtype=torch.int64, device=dev)
             self.n_written_host = np.zeros((n,), np.int64)       # host mirrors: no device sync
             self.learn_step_host = np.zeros((g,), np.int64)
         else:
@@ -176,12 +210,16 @@ class AgentGroup:
             self.learn_step = p.learn_step[j:j + 1]
             self.grads = None if p.grads is None else p.grads[j:j + 1]
             self.grad_norms = None if p.grad_norms is None else p.grad_norms[j:j + 1]
+            if self.noisy:
+                for name in self._NOISY:
+                    setattr(self, name, getattr(p, name)[j:j + 1])
             self.n_written_host = p.n_written_host[i:i + 1]
             self.learn_step_host = p.learn_step_host[j:j + 1]
         self.replay = N.Replay(_ptr(self.obs), _ptr(self.next_obs), _ptr(self.act_ring), _ptr(self.rew_ring),
                                _ptr(self.done_ring), _ptr(self.n_written), _ptr(self.priority), _ptr(self.priority_max))
         self.nets = N.Nets(_ptr(self.theta), _ptr(self.theta_tgt), _ptr(self.adam_m), _ptr(self.adam_v),
                            _ptr(self.learn_step))
+        self.noisy_ptrs = N.Noisy(*(_ptr(getattr(self, k)) for k in self._NOISY_PTRS)) if self.noisy else None
         nbytes = C.c_size_t()
         N.check(self.lib.dmdqn_workspace_bytes(C.byref(self.dims), C.byref(nbytes)))
         self.workspace = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
@@ -197,6 +235,10 @@ class AgentGroup:
         self._views: dict[int, AgentGroup] = {}
         if _parent is None:
             self.init_weights(seed)
+
+    # the noisy tensors: the dmdqn_noisy fields in order, and the gradient block of the noisy learn step
+    _NOISY_PTRS = ("sigma", "sigma_tgt", "sigma_m", "sigma_v", "eff", "eff_tgt", "noise", "key")
+    _NOISY = _NOISY_PTRS + ("grads",)
 
     # ------------------------------------------------------------------ helpers ---------
     @property
@@ -252,25 +294,52 @@ class AgentGroup:
             out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
         return out
 
+    def sigma_init(self) -> list[torch.Tensor]:
+        """Initial sigma of a noisy network in ``keras_init``'s order: noisy_sigma0 / sqrt(fan_in) for every weight and bias
+        of a layer (Fortunato et al.'s factorized rule), fan_in = state_size for layer 1 and H after it."""
+        d, h, a = self.state_size, self.hidden, self.action_size
+        s1, s2 = np.float32(self.noisy_sigma0 / math.sqrt(d)), np.float32(self.noisy_sigma0 / math.sqrt(h))
+        shapes = [((d, h), s1), ((h,), s1), ((h, h), s2), ((h,), s2), ((h, a), s2), ((a,), s2)]
+        if self.dueling:
+            shapes += [((h, 1), s2), ((1,), s2)]
+        return [torch.full(shape, float(v), dtype=torch.float32) for shape, v in shapes]
+
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
-        (dqn_agent.py:129-137)."""
+        (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
         blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, self.action_size, self.dueling))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
         self.adam_m.zero_(); self.adam_v.zero_(); self.learn_step.zero_()
         self.learn_step_host[:] = 0
+        if self.noisy:
+            sig = self.pack(self.sigma_init()).to(self.device)
+            self.sigma.copy_(sig.expand_as(self.sigma)); self.sigma_tgt.copy_(self.sigma)
+            self.sigma_m.zero_(); self.sigma_v.zero_()
+            keys = [noise_key(seed + g) for g in range(self.n_nets)]
+            self.key.copy_(torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in keys], dtype=torch.int64))
+
+    def _blocks(self, which: str) -> list[torch.Tensor]:
+        t = {"online": (self.theta, self.sigma), "target": (self.theta_tgt, self.sigma_tgt), "m": (self.adam_m, self.sigma_m),
+             "v": (self.adam_v, self.sigma_v)}[which]
+        return list(t) if self.noisy else [t[0]]
 
     def set_weights(self, net: int, weights, which: str = "online", sync_target: bool = False) -> None:
-        t = {"online": self.theta, "target": self.theta_tgt, "m": self.adam_m, "v": self.adam_v}[which]
-        t[net].copy_(self.pack(weights))
-        if sync_target:
-            self.theta_tgt[net].copy_(t[net])
+        """``weights`` as ``get_weights`` returns them: noisy networks take the mu list followed by the sigma list."""
+        weights = list(weights)
+        blocks = self._blocks(which)
+        k = len(weights) // len(blocks)
+        if k * len(blocks) != len(weights):
+            raise ValueError(f"expected {len(blocks)} equal lists of weight tensors, got {len(weights)} tensors")
+        for i, (t, tg) in enumerate(zip(blocks, self._blocks("target"))):
+            t[net].copy_(self.pack(weights[i * k:(i + 1) * k]))
+            if sync_target:
+                tg[net].copy_(t[net])
 
     def get_weights(self, net: int, which: str = "online") -> list[torch.Tensor]:
-        t = {"online": self.theta, "target": self.theta_tgt, "m": self.adam_m, "v": self.adam_v}[which]
-        return self.unpack(t[net])
+        """[W1, b1, W2, b2, W3, b3] (+ [Wv, bv] with dueling heads); noisy networks: the mu list, then the sigma list."""
+        return [w for t in self._blocks(which) for w in self.unpack(t[net])]
 
     # ------------------------------------------------------------------ K0 --------------
     @_on_device
@@ -319,11 +388,14 @@ class AgentGroup:
 
     # ------------------------------------------------------------------ K2 --------------
     @_on_device
-    def act(self, obs, eps=None, w_explore=None, w_action=None, return_q: bool = False, target: bool = False):
+    def act(self, obs, eps=None, w_explore=None, w_action=None, return_q: bool = False, target: bool = False,
+            noisy: bool | None = None):
         """Batched epsilon-greedy (dqn_agent.py:263-274).  ``eps`` None -> greedy for all.
         Draws default to the group's device generator.  Returns actions[N] int32 (device)
         and, if asked, q[N,4] (rows of exploring agents are NaN: no forward pass ran).
-        ``target=True`` runs the same kernel on the target parameters (``target_network(x)``)."""
+        ``target=True`` runs the same kernel on the target parameters (``target_network(x)``).
+        Noisy networks act on mu + sigma * eps with the online noise of the next learn step (``dmdqn_act_noisy``);
+        ``noisy=False`` acts on mu alone (greedy evaluation).  The target network is always read without noise."""
         n = self.n_agents
         obs = self._dev(obs, torch.float32)
         if obs.dim() == 3:
@@ -339,9 +411,13 @@ class AgentGroup:
         q = torch.full((n, 4), float("nan"), dtype=torch.float32, device=self.device) if return_q else None
         nets = self.nets if not target else N.Nets(_ptr(self.theta_tgt), _ptr(self.theta_tgt), _ptr(self.adam_m),
                                                    _ptr(self.adam_v), _ptr(self.learn_step))
-        act = self.lib.dmdqn_act_dueling if self.dueling else self.lib.dmdqn_act
-        N.check(act(C.byref(self.dims), C.byref(nets), _ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions),
-                    _ptr(q), self._stream))
+        args = (_ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream)
+        if self.noisy and noisy is not False and not target:
+            N.check(self.lib.dmdqn_act_noisy(C.byref(self.dims), C.byref(nets), C.byref(self.noisy_ptrs), int(self.dueling),
+                                             *args))
+        else:
+            act = self.lib.dmdqn_act_dueling if self.dueling else self.lib.dmdqn_act
+            N.check(act(C.byref(self.dims), C.byref(nets), *args))
         return (actions, q) if return_q else actions
 
     def draw_words(self, shape) -> torch.Tensor:
@@ -426,8 +502,16 @@ class AgentGroup:
     # ------------------------------------------------------------------ K1b+K3+K4 -------
     def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
         """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
-        (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``)."""
+        (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
+        ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
         ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.noisy:          # gradient of the effective weights, then Adam on mu and sigma
+            N.check(self.lib.dmdqn_learn_grads_noisy(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
+                                                     C.byref(self.noisy_ptrs), draws_ptr, mask_ptr, self.batch_size,
+                                                     _ptr(self.grads), _ptr(self.metrics), ws, nws, stream_ptr))
+            N.check(self.lib.dmdqn_noisy_adam_apply(C.byref(self.dims), C.byref(hp), C.byref(self.nets), C.byref(self.noisy_ptrs),
+                                                    _ptr(self.grads), ws, nws, stream_ptr))
+            return
         if self.global_clipnorm is None:
             N.check(self.lib.dmdqn_learn(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                          draws_ptr, mask_ptr, _ptr(self.metrics), ws, nws, stream_ptr))
@@ -504,8 +588,9 @@ class AgentGroup:
 
     def _step_host_call(self, hp, sb, stream_ptr) -> None:
         """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
-        one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy."""
-        if self.global_clipnorm is None:
+        one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy; the
+        same with ``noisy`` set and the noisy learn calls."""
+        if self.global_clipnorm is None and not self.noisy:
             N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                              C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
                                              _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
@@ -585,6 +670,8 @@ class AgentGroup:
                "active": view(v.active, torch.int32, (g,)), "tc_error": view(v.tc_error, torch.int32, (1,)),
                "is_weights": view(v.is_w, torch.float32, (g, b)),
                "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
+        if self.noisy:           # factor vectors [network][set][record] and effective blocks of the last fold
+            out["noise"], out["eff"], out["eff_tgt"] = self.noise, self.eff, self.eff_tgt
         if self.dueling:         # the folded heads W3e[H][4] | b3e[4] of the last learn step, online (0) and target (1)
             dv = N.DuelingViews()
             N.check(self.lib.dmdqn_debug_dueling(C.byref(self.dims), _ptr(self.workspace), self.workspace.numel(), C.byref(dv)))
@@ -605,5 +692,10 @@ class AgentGroup:
     def sync_target(self, mask=None, tau: float | None = None) -> None:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
+        tau = -1.0 if tau is None else float(tau)
+        if self.noisy:           # mu and sigma
+            N.check(self.lib.dmdqn_sync_target_noisy(C.byref(self.dims), C.byref(self.nets), C.byref(self.noisy_ptrs),
+                                                     int(self.dueling), _ptr(mask_t), tau, self._stream))
+            return
         sync = self.lib.dmdqn_sync_target_dueling if self.dueling else self.lib.dmdqn_sync_target
-        N.check(sync(C.byref(self.dims), C.byref(self.nets), _ptr(mask_t), -1.0 if tau is None else float(tau), self._stream))
+        N.check(sync(C.byref(self.dims), C.byref(self.nets), _ptr(mask_t), tau, self._stream))

@@ -203,7 +203,9 @@ class SharedParameterStep:
         than one rank) runs the all-reduce and Adam as one peer-memory kernel; ``fused=False`` is the NCCL
         all-reduce + ``dmdqn_adam_apply`` baseline.  A group with ``global_clipnorm`` takes the NCCL path and finishes with
         ``dmdqn_clip_adam_apply`` on the all-reduced block; ``fused=True`` is refused there.  ``exchange``: a PeerExchange
-        already connected (tests)."""
+        already connected (tests).  A ``noisy`` group takes the NCCL path too: every rank folds the same noise (same keys and
+        step counters), the effective-weight gradients are all-reduced and ``dmdqn_noisy_adam_apply`` updates mu and sigma;
+        ``fused=True`` is refused there, because the peer-memory kernel does not know sigma."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
@@ -213,8 +215,11 @@ class SharedParameterStep:
         if clip is not None and fused:
             raise ValueError("global_clipnorm is set: the fused peer-memory kernel (dmdqn_allreduce_adam) does not clip; "
                              "use fused=False (the NCCL all-reduce + dmdqn_clip_adam_apply path)")
+        if grp.noisy and fused:
+            raise ValueError("noisy=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not update sigma; use "
+                             "fused=False (the NCCL all-reduce + dmdqn_noisy_adam_apply path)")
         if fused is None:
-            fused = clip is None and (world > 1 or exchange is not None)
+            fused = clip is None and not grp.noisy and (world > 1 or exchange is not None)
         if fused and exchange is None:
             rank = dist.get_rank(group) if world > 1 else 0
             exchange = PeerExchange(grp, rank, world).connect(group)
@@ -231,9 +236,15 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                N.check(grp.lib.dmdqn_learn_grads(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay), C.byref(grp.nets),
-                                                  _ptr(d), None, int(global_batch), _ptr(out), _ptr(grp.metrics),
-                                                  _ptr(grp.workspace), grp.workspace.numel(), grp._stream))
+                if grp.noisy:
+                    N.check(grp.lib.dmdqn_learn_grads_noisy(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay),
+                                                            C.byref(grp.nets), C.byref(grp.noisy_ptrs), _ptr(d), None,
+                                                            int(global_batch), _ptr(out), _ptr(grp.metrics), _ptr(grp.workspace),
+                                                            grp.workspace.numel(), grp._stream))
+                else:
+                    N.check(grp.lib.dmdqn_learn_grads(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay), C.byref(grp.nets),
+                                                      _ptr(d), None, int(global_batch), _ptr(out), _ptr(grp.metrics),
+                                                      _ptr(grp.workspace), grp.workspace.numel(), grp._stream))
             grp.learn_step_host += 1
             return out, grp.metrics
 
@@ -259,6 +270,11 @@ class SharedParameterStep:
                     N.check(grp.lib.dmdqn_clip_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g), clip,
                                                           _ptr(grp.grad_norms), _ptr(grp.workspace), grp.workspace.numel(),
                                                           grp._stream))
+                    return
+                if grp.noisy:
+                    N.check(grp.lib.dmdqn_noisy_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets),
+                                                           C.byref(grp.noisy_ptrs), _ptr(g), _ptr(grp.workspace),
+                                                           grp.workspace.numel(), grp._stream))
                     return
                 N.check(grp.lib.dmdqn_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g),
                                                  _ptr(grp.workspace), grp.workspace.numel(), grp._stream))

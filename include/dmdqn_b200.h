@@ -452,6 +452,75 @@ int dmdqn_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint
 int dmdqn_sync_target_dueling(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask,
                               double tau, void* stream);
 
+/* Noisy networks (Fortunato et al. 2018, factorized Gaussian noise on every layer).  The learned parameters of network g
+ * are mu = nets->theta (plain or dueling layout, unchanged) and sigma, a second block of the same layout with its own
+ * target copy and Adam moments.  Layer l with p inputs and q outputs (W1 / b1, W2 / b2, W3 / b3 and, for dueling blocks,
+ * wv / bv) has factor vectors fin[p] and fout[q]; its weight noise is eps_ij = fin[i] * fout[j] (one fp32 product), its
+ * bias noise fout[j], and the effective parameters are
+ *   eff = mu + sigma * eps      (__fmul_rn, then __fadd_rn: one rounded product, one rounded sum).
+ * Factor entry i of vector (layer, side) of set s (0 = online, 1 = target) at step t is f(z), f(z) = sgn(z) sqrt|z| in fp32,
+ *   (x, y, -, -) = Philox4x32-10(key = {key[g] low word, high word}, counter = {i, layer << 2 | side << 1 | s, t, 0x6e6f6973})
+ *   z = (float)(sqrt(-2 ln((x + 0.5) 2^-32)) cos(2 pi y 2^-32))   in float64,
+ * with layer 0..3 = W1, W2, W3, the value head and side 0 = inputs, 1 = outputs.  Entries for padding are 0: W1 input rows
+ * >= obs_dim, W3 output columns >= A, the value head's outputs >= 1.  t is the network's learn_step before a learn step's
+ * sample kernel increments it: a learn step runs the online network (Q(s) and the double-DQN argmax at s') with set 0
+ * and the target network with set 1, and acting with set 0 at the current learn_step uses the noise of the next learn
+ * step's online network (the paper's rule: resample after every optimisation step).
+ *   sigma, sigma_tgt, sigma_m, sigma_v  device float [n_nets][stride]  (the layout's stride)
+ *   eff, eff_tgt                         device float [n_nets][stride], 16-byte aligned: written by dmdqn_noisy_fold
+ *   noise                                device float [n_nets][2][record.stride]: the factor vectors of set 0 and 1
+ *   key                                  device uint64 [n_nets]: each network's Philox key */
+typedef struct dmdqn_noisy {
+    float* sigma;
+    float* sigma_tgt;
+    float* sigma_m;
+    float* sigma_v;
+    float* eff;
+    float* eff_tgt;
+    float* noise;
+    const uint64_t* key;
+} dmdqn_noisy;
+
+/* Float offsets of the eight factor vectors inside one set's noise record, in this order:
+ *   w1_in[obs_stride] | w1_out[H] | w2_in[H] | w2_out[H] | w3_in[H] | w3_out[4] | v_in[H] | v_out[4]
+ * and the record's stride (a multiple of 32 floats).  The value head's vectors are there for plain blocks too. */
+typedef struct dmdqn_noise_record {
+    int64_t w1_in, w1_out, w2_in, w2_out, w3_in, w3_out, v_in, v_out, stride;
+} dmdqn_noise_record;
+int dmdqn_noise_layout(const dmdqn_dims* dims, dmdqn_noise_record* out);
+
+/* The factor vectors of both sets into noisy->noise and the effective blocks eff = mu + sigma * eps (set 0 from theta /
+ * sigma) and eff_tgt (set 1 from theta_tgt / sigma_tgt), every float of the stride, for every network at its current
+ * learn_step.  hp is read for its dueling flag only. */
+int dmdqn_noisy_fold(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                     void* stream);
+
+/* One noisy learn step up to the gradient: dmdqn_noisy_fold, then dmdqn_learn_grads with nets->theta / theta_tgt
+ * replaced by eff / eff_tgt (its dueling fold, sample, K3, K4a, K4b).  grads_out receives dL/d eff; learn_step advances as
+ * in dmdqn_learn_grads.  Finish the step with dmdqn_noisy_adam_apply. */
+int dmdqn_learn_grads_noisy(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
+                            const dmdqn_nets* nets, const dmdqn_noisy* noisy, const void* draws, const uint8_t* learn_mask,
+                            int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
+                            size_t workspace_bytes, void* stream);
+
+/* Adam on mu and sigma from the effective-weight gradient g of dmdqn_learn_grads_noisy: g_mu = g, g_sigma = g * eps (fp32,
+ * eps of set 0 from noisy->noise), each through dmdqn_adam_apply's per-element arithmetic with the step's Adam scalars
+ * (mu with adam_m / adam_v, sigma with sigma_m / sigma_v), and the target sync of both.  A network that did not learn, or
+ * any network after a tcgen05 kernel set the workspace error flag, is left untouched. */
+int dmdqn_noisy_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                           const float* grads, void* workspace, size_t workspace_bytes, void* stream);
+
+/* dmdqn_act on the noisy online network at its current learn_step (set 0): the kernel streams mu and sigma and forms
+ * mu + sigma * eps in registers, so q_out and the actions equal dmdqn_act / dmdqn_act_dueling on the eff block of a
+ * dmdqn_noisy_fold at the same learn_step, bit for bit.  dueling: the blocks are in the dueling layout. */
+int dmdqn_act_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
+                    const float* obs, int32_t obs_in_stride, const double* eps, const uint32_t* w_explore,
+                    const uint32_t* w_action, int32_t* actions_out, float* q_out, void* stream);
+
+/* dmdqn_sync_target of mu (theta -> theta_tgt) and of sigma (sigma -> sigma_tgt). */
+int dmdqn_sync_target_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
+                            const uint8_t* mask, double tau, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
