@@ -81,6 +81,17 @@ class NoiseRecord(C.Structure):
     _fields_ = [(n, C.c_int64) for n in ("w1_in", "w1_out", "w2_in", "w2_out", "w3_in", "w3_out", "v_in", "v_out", "stride")]
 
 
+class Dist(C.Structure):
+    _fields_ = [("n_atoms", C.c_int32), ("v_min", C.c_double), ("v_max", C.c_double), ("scratch", C.c_void_p),
+                ("scratch_bytes", C.c_size_t)]
+
+
+class DistViews(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("target_dist", "h2", "dlogits")]
+
+
+DIST_MAX_ATOMS = 64
+
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
 
 
@@ -141,6 +152,15 @@ SIGNATURES = {
     "dmdqn_act_noisy": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32, _P, C.c_int32, _P, _P, _P,
                                   _P, _P, _P]),
     "dmdqn_sync_target_noisy": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32, _P, C.c_double, _P]),
+    "dmdqn_param_layout_dist": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(Layout)]),
+    "dmdqn_dist_scratch_bytes": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(C.c_size_t)]),
+    "dmdqn_learn_grads_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Dist), C.POINTER(Replay),
+                                         C.POINTER(Nets), _P, _P, C.c_int32, _P, _P, _P, C.c_size_t, _P]),
+    "dmdqn_adam_apply_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P,
+                                        _P, C.c_size_t, _P]),
+    "dmdqn_act_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Dist), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    "dmdqn_sync_target_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P]),
+    "dmdqn_debug_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Dist), C.POINTER(DistViews)]),
 }
 
 _lib = None

@@ -147,6 +147,49 @@ __device__ __forceinline__ void gemv_slice_noisy(cg::cluster_group& cluster, con
     cluster.sync();
 }
 
+// The trunk on plain weights: h1 and h2 of the observation row `ob` into every CTA's h1 / h2 (xs: the padded row).
+template <int H>
+__device__ __forceinline__ void act_trunk(cg::cluster_group& cluster, const dmdqn_dims& d, const Layout& L, const float* P,
+                                          const float* __restrict__ ob, float* xs, float* h1, float* h2, float* part, int rank) {
+    const int Dp = d.obs_stride;
+    constexpr int C4 = H / kActCluster / 4, GROUPS = kActThreads / C4;
+    // The register-resident W1 slice is sized for the yaml observation (89 -> stride 96); wider observations
+    // (stride 112 / 128, accepted by validate_dims and by the learn kernels) stream layer 1 row by row instead.
+    constexpr int kRegRows = 96;
+    if constexpr (H <= 256) {
+        if (Dp <= kRegRows) {
+            float4 w1[(kRegRows + GROUPS - 1) / GROUPS], w2[(H + GROUPS - 1) / GROUPS];
+            load_slice(w1, P + L.w1, Dp, H, rank);       // 4P bytes per action: all of this CTA's share is requested here
+            load_slice(w2, P + L.w2, H, H, rank);
+            for (int c = threadIdx.x; c < Dp; c += kActThreads)
+                xs[c] = c < d.obs_dim ? ob[c] : 0.f;
+            __syncthreads();
+            gemv_slice(cluster, w1, P + L.b1, xs, h1, part, Dp, H, rank);
+            gemv_slice(cluster, w2, P + L.b2, h1, h2, part, H, H, rank);
+        } else {
+            float4 w2[(H + GROUPS - 1) / GROUPS];
+            load_slice(w2, P + L.w2, H, H, rank);
+            for (int c = threadIdx.x; c < Dp; c += kActThreads)
+                xs[c] = c < d.obs_dim ? ob[c] : 0.f;
+            __syncthreads();
+            gemv_slice_loop(cluster, P + L.w1, P + L.b1, xs, h1, part, Dp, H, rank);
+            gemv_slice(cluster, w2, P + L.b2, h1, h2, part, H, H, rank);
+        }
+    } else {                                             // H = 512: a layer's slice does not fit the register file at once
+        for (int c = threadIdx.x; c < Dp; c += kActThreads)
+            xs[c] = c < d.obs_dim ? ob[c] : 0.f;
+        __syncthreads();
+        if (Dp <= kRegRows) {
+            float4 w1[(kRegRows + GROUPS - 1) / GROUPS];
+            load_slice(w1, P + L.w1, Dp, H, rank);
+            gemv_slice(cluster, w1, P + L.b1, xs, h1, part, Dp, H, rank);
+        } else {
+            gemv_slice_loop(cluster, P + L.w1, P + L.b1, xs, h1, part, Dp, H, rank);
+        }
+        gemv_slice_loop(cluster, P + L.w2, P + L.b2, h1, h2, part, H, H, rank);
+    }
+}
+
 // DUELING: the block is in the dueling layout and the head is folded (include/dmdqn_b200.h) in registers: every CTA folds
 // its W3 rows with their wv weights, rank 0 folds the bias.
 // NOISY: the parameters are mu (theta) + sigma * eps with the online noise at the network's learn_step; every CTA builds
@@ -187,42 +230,7 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
         gemv_slice_noisy(cluster, P + L.w2, S + L.w2, P + L.b2, S + L.b2, rec + nz.R.off[2], rec + nz.R.off[3], h1, h2, part,
                          H, H, rank);
     } else {
-        constexpr int C4 = H / kActCluster / 4, GROUPS = kActThreads / C4;
-        // The register-resident W1 slice is sized for the yaml observation (89 -> stride 96); wider observations
-        // (stride 112 / 128, accepted by validate_dims and by the learn kernels) stream layer 1 row by row instead.
-        constexpr int kRegRows = 96;
-        if constexpr (H <= 256) {
-            if (Dp <= kRegRows) {
-                float4 w1[(kRegRows + GROUPS - 1) / GROUPS], w2[(H + GROUPS - 1) / GROUPS];
-                load_slice(w1, P + L.w1, Dp, H, rank);       // 4P bytes per action: all of this CTA's share is requested here
-                load_slice(w2, P + L.w2, H, H, rank);
-                for (int c = threadIdx.x; c < Dp; c += kActThreads)
-                    xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
-                __syncthreads();
-                gemv_slice(cluster, w1, P + L.b1, xs, h1, part, Dp, H, rank);
-                gemv_slice(cluster, w2, P + L.b2, h1, h2, part, H, H, rank);
-            } else {
-                float4 w2[(H + GROUPS - 1) / GROUPS];
-                load_slice(w2, P + L.w2, H, H, rank);
-                for (int c = threadIdx.x; c < Dp; c += kActThreads)
-                    xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
-                __syncthreads();
-                gemv_slice_loop(cluster, P + L.w1, P + L.b1, xs, h1, part, Dp, H, rank);
-                gemv_slice(cluster, w2, P + L.b2, h1, h2, part, H, H, rank);
-            }
-        } else {                                             // H = 512: a layer's slice does not fit the register file at once
-            for (int c = threadIdx.x; c < Dp; c += kActThreads)
-                xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
-            __syncthreads();
-            if (Dp <= kRegRows) {
-                float4 w1[(kRegRows + GROUPS - 1) / GROUPS];
-                load_slice(w1, P + L.w1, Dp, H, rank);
-                gemv_slice(cluster, w1, P + L.b1, xs, h1, part, Dp, H, rank);
-            } else {
-                gemv_slice_loop(cluster, P + L.w1, P + L.b1, xs, h1, part, Dp, H, rank);
-            }
-            gemv_slice_loop(cluster, P + L.w2, P + L.b2, h1, h2, part, H, H, rank);
-        }
+        act_trunk<H>(cluster, d, L, P, obs + (size_t)a * stride, xs, h1, h2, part, rank);
     }
 
     // layer 3: q[a] = b3[a] + sum_j h2[j] * W3[j][a]: every CTA sums its H/4 rows (warp butterfly, warps in
@@ -289,7 +297,86 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
     }
 }
 
+// Distributional heads (include/dmdqn_b200.h dmdqn_dist): the plain trunk, then CTA `rank` computes action rank's Np
+// logits (thread j < Np owns column j, four thread groups split the H rows k = grp, grp + 4, ..., their partials added
+// to b3 in group order), their softmax and the expected Q; the four Q values meet on rank 0 over DSMEM for the argmax.
+template <int H>
+__global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads, 4)
+act_dist_kernel(dmdqn_dims d, Layout L, int n_atoms, double v_min, double dz64, const float* __restrict__ theta,
+                const float* __restrict__ obs, int stride, const double* __restrict__ eps, const uint32_t* __restrict__ w_explore,
+                const uint32_t* __restrict__ w_action, int32_t* __restrict__ actions, float* __restrict__ q_out) {
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int a = blockIdx.x / kActCluster, rank = (int)cluster.block_rank();
+    const bool explore = (double)w_explore[a] < eps[a] * 4294967296.0;
+    if (explore) {
+        if (threadIdx.x == 0 && rank == 0) actions[a] = (int32_t)__umulhi(w_action[a], (uint32_t)d.n_actions);
+        return;
+    }
+    float* xs = smem;                        // [Dp]
+    float* h1 = xs + d.obs_stride;           // [H]
+    float* h2 = h1 + H;                      // [H]
+    float* part = h2 + H;                    // [1024]: trunk partials, then head partials [4][64] and rank 0's Q[4] at 512
+    float* lg = part + kActThreads * 4;      // [64] logits
+    float* zs = lg + kDistMaxAtoms;          // [64] support
+    const int net = d.n_nets == 1 ? 0 : a;
+    const float* P = theta + (size_t)net * L.stride;
+    act_trunk<H>(cluster, d, L, P, obs + (size_t)a * stride, xs, h1, h2, part, rank);
+
+    const int np = (n_atoms + 3) / 4 * 4, nh = 4 * np;
+    const int j = threadIdx.x & 63, grp = threadIdx.x >> 6;
+    const bool mine = rank < d.n_actions;
+    if (mine && j < np) {
+        const float* w = P + L.w3 + rank * np + j;
+        float s = 0.f;
+        for (int k = grp; k < H; k += 4) s = fmaf(h2[k], __ldg(w + (size_t)k * nh), s);
+        part[grp * 64 + j] = s;
+    }
+    if (threadIdx.x < n_atoms) zs[threadIdx.x] = dist_z(v_min, dz64, threadIdx.x);
+    __syncthreads();
+    if (mine && threadIdx.x < n_atoms) {
+        float x = __ldg(P + L.b3 + rank * np + threadIdx.x);
+        for (int g = 0; g < 4; ++g) x += part[g * 64 + threadIdx.x];
+        lg[threadIdx.x] = x;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float mx, s;
+        cluster.map_shared_rank(part, 0)[512 + rank] = mine ? dist_expect(lg, n_atoms, zs, mx, s) : 0.f;
+    }
+    cluster.sync();
+    if (threadIdx.x == 0 && rank == 0) {
+        const float* q = part + 512;
+        int best = 0;                                   // ties -> lowest index
+        for (int k = 1; k < d.n_actions; ++k) if (q[k] > q[best]) best = k;
+        actions[a] = best;
+        if (q_out)
+            for (int k = 0; k < 4; ++k) q_out[(size_t)a * 4 + k] = q[k];
+    }
+}
+
 }  // namespace
+
+int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
+                    const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s) {
+    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(ds.n_atoms));
+    const double dz64 = (ds.v_max - ds.v_min) / (ds.n_atoms - 1);
+    const size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + 2 * kDistMaxAtoms) * sizeof(float);
+    const dim3 grid(d.n_agents * kActCluster);
+    auto run = [&](auto kernel) {
+        kernel<<<grid, kActThreads, smem, s>>>(d, L, ds.n_atoms, ds.v_min, dz64, nets.theta, obs, stride, eps, w1, w2, actions,
+                                               q_out);
+    };
+    switch (d.hidden) {
+        case 64: run(act_dist_kernel<64>); break;
+        case 128: run(act_dist_kernel<128>); break;
+        case 256: run(act_dist_kernel<256>); break;
+        case 512: run(act_dist_kernel<512>); break;
+        default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
+    }
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
 
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
                const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,

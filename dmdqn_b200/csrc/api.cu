@@ -535,6 +535,132 @@ int dmdqn_sync_target_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, cons
     return launch_sync_target(*dims, sigma, mask, tau, dueling == 1, (cudaStream_t)stream);
 }
 
+// Distributional calls (include/dmdqn_b200.h dmdqn_dist): the atom count, the support and, where the call reads it, the
+// scratch; every check runs before anything is launched.
+static int check_atoms(int32_t n_atoms) {
+    DMDQN_CHECK_ARG(n_atoms >= 2 && n_atoms <= DMDQN_DIST_MAX_ATOMS, "n_atoms=%d must be in [2, %d]", n_atoms,
+                    DMDQN_DIST_MAX_ATOMS);
+    return DMDQN_OK;
+}
+
+static bool aligned16(const void* p) { return (uintptr_t)p % 16 == 0; }
+
+static int check_dist(const dmdqn_dims* dims, const dmdqn_dist* ds, bool scratch) {
+    DMDQN_CHECK_ARG(ds != nullptr, "dist is NULL");
+    if (int rc = check_atoms(ds->n_atoms)) return rc;
+    DMDQN_CHECK_ARG(isfinite(ds->v_min) && isfinite(ds->v_max) && ds->v_min < ds->v_max,
+                    "v_min=%g v_max=%g: the support needs finite v_min < v_max", ds->v_min, ds->v_max);
+    if (scratch) {
+        DMDQN_CHECK_ARG(ds->scratch && aligned16(ds->scratch), "dist: scratch is NULL or not 16-byte aligned");
+        const size_t need = make_dist_scratch(*dims, dist_np(ds->n_atoms)).total;
+        DMDQN_CHECK_ARG(ds->scratch_bytes >= need, "dist: scratch has %zu bytes, %zu needed", ds->scratch_bytes, need);
+    }
+    return DMDQN_OK;
+}
+
+static int check_dist_hp(const dmdqn_hparams* hp) {
+    DMDQN_CHECK_ARG(hp != nullptr, "dist: hp is NULL");
+    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32,
+                    "precision=%d: distributional networks run the fp32 (FFMA) path only", hp->precision);
+    DMDQN_CHECK_ARG(hp->dueling == 0, "dueling=%d: dueling heads are not supported with distributional networks", hp->dueling);
+    return DMDQN_OK;
+}
+
+static int check_dist_nets(const dmdqn_nets* nets, bool adam) {
+    DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt, "dist: NULL network pointer");
+    if (adam) DMDQN_CHECK_ARG(nets->adam_m && nets->adam_v && nets->learn_step, "dist: NULL Adam pointer");
+    const void* p[] = {nets->theta, nets->theta_tgt, adam ? nets->adam_m : nets->theta, adam ? nets->adam_v : nets->theta};
+    for (const void* q : p) DMDQN_CHECK_ARG(aligned16(q), "dist: pointer %p is not 16-byte aligned", q);
+    return DMDQN_OK;
+}
+
+int dmdqn_param_layout_dist(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_layout* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const Layout l = make_layout_dist(dims->obs_stride, dims->hidden, dist_np(n_atoms));
+    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
+    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
+    return DMDQN_OK;
+}
+
+int dmdqn_dist_scratch_bytes(const dmdqn_dims* dims, int32_t n_atoms, size_t* out_bytes) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    DMDQN_CHECK_ARG(out_bytes != nullptr, "out_bytes is NULL");
+    *out_bytes = make_dist_scratch(*dims, dist_np(n_atoms)).total;
+    return DMDQN_OK;
+}
+
+int dmdqn_learn_grads_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_dist* dist, const dmdqn_replay* replay,
+                           const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
+                           float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    if ((rc = check_dist_hp(hp))) return rc;
+    if ((rc = check_dist(dims, dist, true))) return rc;
+    if ((rc = check_dist_nets(nets, true))) return rc;
+    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
+    return launch_learn_dist(*dims, *hp, *replay, *nets, *dist, metrics_out, (char*)workspace, w, grads_out, global_batch, s);
+}
+
+int dmdqn_adam_apply_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, int32_t n_atoms,
+                          const float* grads, double global_clipnorm, float* norms_out, void* workspace, size_t workspace_bytes,
+                          void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_dist_hp(hp))) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    if ((rc = check_dist_nets(nets, true))) return rc;
+    DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_dist: grads is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_clipnorm >= 0.0 && isfinite(global_clipnorm),
+                    "global_clipnorm=%g must be 0 (no clipping) or a positive finite number", global_clipnorm);
+    return launch_adam_apply_dist(*dims, *hp, *nets, n_atoms, grads, global_clipnorm, norms_out, (char*)workspace, w,
+                                  (cudaStream_t)stream);
+}
+
+int dmdqn_act_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_dist* dist, const float* obs,
+                   int32_t obs_in_stride, const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
+                   int32_t* actions_out, float* q_out, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_dist(dims, dist, false))) return rc;
+    DMDQN_CHECK_ARG(nets && nets->theta && aligned16(nets->theta), "act_dist: theta is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(obs && eps && w_explore && w_action && actions_out, "act_dist: NULL argument");
+    DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
+    return launch_act_dist(*dims, *nets, *dist, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out,
+                           (cudaStream_t)stream);
+}
+
+int dmdqn_sync_target_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, int32_t n_atoms, const uint8_t* mask, double tau,
+                           void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    if ((rc = check_dist_nets(nets, false))) return rc;
+    return launch_sync_target_dist(*dims, *nets, n_atoms, mask, tau, (cudaStream_t)stream);
+}
+
+int dmdqn_debug_dist(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_dist_views* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_dist(dims, dist, true))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const DistArgs D = make_dist_args(*dims, *dist);
+    out->target_dist = D.m;
+    out->h2 = D.h2;
+    out->dlogits = D.dx;
+    return DMDQN_OK;
+}
+
 static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau, bool dueling,
                            void* stream) {
     int rc = validate_dims(dims);

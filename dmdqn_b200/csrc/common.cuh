@@ -157,6 +157,76 @@ __device__ __forceinline__ float4 noise_eps4(const float* rec, const NoiseRec& R
 // mu + sigma * eps as the header states it: one rounded product, then one rounded sum
 __device__ __forceinline__ float noisy_weight(float mu, float sigma, float eps) { return __fadd_rn(mu, __fmul_rn(sigma, eps)); }
 
+// Distributional (C51) networks (include/dmdqn_b200.h dmdqn_dist).  The head is W3[H][4 * Np] | b3[4 * Np], Np = N rounded
+// up to a multiple of 4, column a * Np + j = atom j of action a; the Adam range ends after b3.
+constexpr int kDistMaxAtoms = 64;
+inline int dist_np(int n_atoms) { return (n_atoms + 3) / 4 * 4; }
+__host__ __device__ inline Layout make_layout_dist(int dp, int h, int np) {
+    Layout l = make_layout(dp, h);
+    l.b3 = l.w3 + (int64_t)h * 4 * np;
+    l.end = l.b3 + 4 * np;
+    l.stride = (l.end + 31) / 32 * 32;
+    return l;
+}
+// The caller-owned scratch of the distributional learn kernels, byte offsets (256-aligned): the projected target
+// distribution m [n_nets][B][Np], h2 [n_nets][B][H] and the logit gradient dX [n_nets][B][4 * Np].
+struct DistScratch {
+    size_t m, h2, dx, total;
+};
+inline DistScratch make_dist_scratch(const dmdqn_dims& d, int np) {
+    DistScratch s;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t nb = (size_t)d.n_nets * d.batch;
+    s.m = take(nb * np * 4);
+    s.h2 = take(nb * d.hidden * 4);
+    s.dx = take(nb * 4 * np * 4);
+    s.total = off;
+    return s;
+}
+// What the distributional kernels take beyond LearnArgs: the support and the scratch pointers.
+struct DistArgs {
+    int n_atoms, np, nh;              // N, Np, 4 * Np
+    float lo, hi, dz;                 // (float)v_min, (float)v_max, (float)dz64
+    double v_min, dz64;               // dz64 = (v_max - v_min) / (N - 1) in float64
+    float *m, *h2, *dx;
+};
+inline DistArgs make_dist_args(const dmdqn_dims& d, const dmdqn_dist& ds) {
+    DistArgs D;
+    D.n_atoms = ds.n_atoms;
+    D.np = dist_np(ds.n_atoms);
+    D.nh = 4 * D.np;
+    D.v_min = ds.v_min;
+    D.dz64 = (ds.v_max - ds.v_min) / (ds.n_atoms - 1);
+    D.lo = (float)ds.v_min;
+    D.hi = (float)ds.v_max;
+    D.dz = (float)D.dz64;
+    const DistScratch s = make_dist_scratch(d, D.np);
+    char* p = static_cast<char*>(ds.scratch);
+    D.m = p ? reinterpret_cast<float*>(p + s.m) : nullptr;
+    D.h2 = p ? reinterpret_cast<float*>(p + s.h2) : nullptr;
+    D.dx = p ? reinterpret_cast<float*>(p + s.dx) : nullptr;
+    return D;
+}
+// z_j = (float)(v_min + j * dz64): one rounded float64 product, one rounded sum, then rounded to float
+__device__ __forceinline__ float dist_z(double v_min, double dz64, int j) { return (float)__dadd_rn(v_min, __dmul_rn((double)j, dz64)); }
+// Softmax statistics of one action's logits x[0..n): mx = max_j x_j, s = sum_j expf(x_j - mx) in j order
+__device__ __forceinline__ void dist_stats(const float* x, int n, float& mx, float& s) {
+    float m = x[0];
+    for (int j = 1; j < n; ++j) m = fmaxf(m, x[j]);
+    float t = 0.f;
+    for (int j = 0; j < n; ++j) t = __fadd_rn(t, expf(__fsub_rn(x[j], m)));
+    mx = m;
+    s = t;
+}
+// The expected value Q = sum_j p_j z_j (fmaf in j order), p_j = expf(x_j - mx) / s
+__device__ __forceinline__ float dist_expect(const float* x, int n, const float* z, float& mx, float& s) {
+    dist_stats(x, n, mx, s);
+    float q = 0.f;
+    for (int j = 0; j < n; ++j) q = fmaf(__fdiv_rn(expf(__fsub_rn(x[j], mx)), s), z[j], q);
+    return q;
+}
+
 // Tile geometry of the fused MLP kernels for hidden width H (DESIGN.md "K3/K4 tiling").
 // A CTA owns BM batch rows and all H output columns; each thread an 8x8 register tile.
 template <int H>
@@ -372,5 +442,14 @@ int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_
 int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Workspace& w, cudaStream_t s);
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,
                      const float* my_loss_src, float* loss_out, char* ws, const Workspace& w, cudaStream_t s);
+int launch_learn_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                      const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                      cudaStream_t s);
+int launch_adam_apply_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_atoms, const float* grads,
+                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
+int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_atoms, const uint8_t* mask, double tau,
+                            cudaStream_t s);
+int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
+                    const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
 
 }  // namespace dmdqn

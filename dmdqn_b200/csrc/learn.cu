@@ -11,6 +11,8 @@
 // thread owns an 8x8 register tile (rows split 4+4, columns split 4+4 so that every
 // 16-byte shared-memory access of a quarter-warp is conflict-free).  All sums run in a
 // fixed order: results are deterministic run to run.
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace dmdqn {
@@ -55,15 +57,17 @@ __device__ __forceinline__ void cp_async4(float* smem_dst, const float* gsrc) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;\n" ::: "memory"); }
 
+// ncol (direct only): columns >= ncol of the chunk are zero-filled and not read (the distributional head's last slab).
 template <int H, bool TRANS>
-__device__ __forceinline__ void chunk_issue(float* Ws, const float* __restrict__ W, int ldw, int k0) {
+__device__ __forceinline__ void chunk_issue(float* Ws, const float* __restrict__ W, int ldw, int k0, int ncol = H) {
     using T = Tile<H>;
     if (!TRANS) {
 #pragma unroll
         for (int r = 0; r < T::KC * H / 4 / T::NT; ++r) {
             const int f = threadIdx.x + r * T::NT;
             const int kk = f / (H / 4), n4 = f % (H / 4);
-            cp_async16(Ws + kk * T::LDW + n4 * 4, W + (size_t)(k0 + kk) * ldw + n4 * 4);
+            const bool ok = n4 * 4 < ncol;
+            cp_async16(Ws + kk * T::LDW + n4 * 4, ok ? W + (size_t)(k0 + kk) * ldw + n4 * 4 : W, ok);
         }
     } else {
 #pragma unroll
@@ -87,19 +91,19 @@ __device__ __forceinline__ void fma8(float (&acc)[8], float a, const float4& b0,
 // Ends with a __syncthreads(): As and Ws may be overwritten right after it returns.
 template <int H, bool TRANS>
 __device__ __forceinline__ void gemm_rowA(float (&acc)[8][8], const Coord<H>& c, const float* As, int lda,
-                                          const float* __restrict__ W, int ldw, int K, float* Ws) {
+                                          const float* __restrict__ W, int ldw, int K, float* Ws, int ncol = H) {
     using T = Tile<H>;
 #pragma unroll
     for (int i = 0; i < 8; ++i)
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-    chunk_issue<H, TRANS>(Ws, W, ldw, 0);
+    chunk_issue<H, TRANS>(Ws, W, ldw, 0, ncol);
     cp_async_wait_all();
     __syncthreads();
     int buf = 0;
     for (int k0 = 0; k0 < K; k0 += T::KC) {
         const bool more = k0 + T::KC < K;
-        if (more) chunk_issue<H, TRANS>(Ws + (buf ^ 1) * (T::KC * T::LDW), W, ldw, k0 + T::KC);
+        if (more) chunk_issue<H, TRANS>(Ws + (buf ^ 1) * (T::KC * T::LDW), W, ldw, k0 + T::KC, ncol);
         const float* Wb = Ws + buf * (T::KC * T::LDW);
 #pragma unroll
         for (int kk = 0; kk < T::KC; kk += 4) {
@@ -858,6 +862,427 @@ peer_reduce_adam_kernel(const LearnArgs A, const dmdqn_peers P, const float* __r
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// Distributional (C51) learn step, fp32 (include/dmdqn_b200.h dmdqn_dist): K3 / K4a / K4b written for a head of
+// nh = 4 * Np logits.  The trunk runs the kernels above; the head is a [BM x H] x [H x nh] GEMM in column slabs of H (the
+// last slab zero-filled past nh).  Its logits Ls[BM][nh + 4] take the place of Hs1 (the target kernel needs h1 no longer;
+// the online kernel reloads it from the workspace for relu'(h1)).
+// ------------------------------------------------------------------------------------------
+template <int H>
+struct DistSmem {
+    using T = Tile<H>;
+    float *Xs, *Hs1, *Ls, *Hs2, *Ws, *qs0, *qs1, *terms, *zs;
+    int* as;
+    int ldx, ldl;
+    __device__ __forceinline__ DistSmem(float* base, int Dp, int nh) {
+        ldx = Dp + 4;
+        ldl = nh + 4;
+        Xs = base;
+        Hs1 = Ls = Xs + T::BM * ldx;
+        Hs2 = Hs1 + T::BM * max(T::LDH, ldl);
+        Ws = Hs2 + T::BM * T::LDH;
+        qs0 = Ws + 2 * T::KC * T::LDW;
+        qs1 = qs0 + T::BM * 4;
+        terms = qs1 + T::BM * 4;
+        zs = terms + T::BM;
+        as = reinterpret_cast<int*>(zs + kDistMaxAtoms);
+    }
+    static size_t bytes(int Dp, int nh) {
+        return sizeof(float) * ((size_t)T::BM * (Dp + 4) + (size_t)T::BM * std::max(T::LDH, nh + 4) + (size_t)T::BM * T::LDH +
+                                2 * (size_t)T::KC * T::LDW + 10 * (size_t)T::BM + kDistMaxAtoms);
+    }
+};
+
+// Ls[i][col] = (Hs2[i] . W3[:, col]) + b3[col] for col < nh.  Caller syncs before (store_relu into Hs2); ends synced.
+template <int H>
+__device__ __forceinline__ void dist_head(float (&acc)[8][8], const Coord<H>& c, const DistSmem<H>& S, const float* P,
+                                          const Layout& L, int nh) {
+    using T = Tile<H>;
+    for (int c0 = 0; c0 < nh; c0 += H) {
+        gemm_rowA<H, false>(acc, c, S.Hs2, T::LDH, P + L.w3 + c0, nh, H, S.Ws, nh - c0);
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+            const int col = c0 + c.col0(half);
+            if (col >= nh) continue;
+            const float4 b = __ldg(reinterpret_cast<const float4*>(P + L.b3 + col));
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+                *reinterpret_cast<float4*>(S.Ls + c.row(i) * S.ldl + col) =
+                    make_float4(acc[i][half * 4 + 0] + b.x, acc[i][half * 4 + 1] + b.y, acc[i][half * 4 + 2] + b.z,
+                                acc[i][half * 4 + 3] + b.w);
+        }
+    }
+    __syncthreads();
+}
+
+// The projection of the target distribution p = softmax(x) (stats mx, s) of one row onto the support, into m[0..Np)
+// (include/dmdqn_b200.h: j in order, every product and sum rounded on its own).  t is clamped to [lo, hi], so
+// 0 <= l <= u <= N - 1 for every input, a NaN return included.
+__device__ __forceinline__ void dist_project(float* m, const float* x, float mx, float s, const float* z, float R, float d,
+                                             const DistArgs& D) {
+    for (int j = 0; j < D.np; ++j) m[j] = 0.f;
+    const float last = (float)(D.n_atoms - 1);
+    for (int j = 0; j < D.n_atoms; ++j) {
+        const float p = __fdiv_rn(expf(__fsub_rn(x[j], mx)), s);
+        const float t = fminf(fmaxf(__fadd_rn(R, __fmul_rn(d, z[j])), D.lo), D.hi);
+        const float b = fminf(__fdiv_rn(__fsub_rn(t, D.lo), D.dz), last);
+        const float l = floorf(b), u = ceilf(b);
+        const int li = (int)l, ui = (int)u;
+        if (li == ui) {
+            m[li] = __fadd_rn(m[li], p);
+        } else {
+            m[li] = __fadd_rn(m[li], __fmul_rn(p, __fsub_rn(u, b)));
+            m[ui] = __fadd_rn(m[ui], __fmul_rn(p, __fsub_rn(b, l)));
+        }
+    }
+}
+
+// Distributional K3: online and target trunk + head on s', expected Q, a*, the projected target distribution -> D.m.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const LearnArgs A, const DistArgs D) {
+    using T = Tile<H>;
+    extern __shared__ __align__(16) float smem[];
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
+    if (!A.active[g]) return;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, n = D.n_atoms, np = D.np;
+    DistSmem<H> S(smem, Dp, D.nh);
+    const Coord<H> c;
+    for (int j = threadIdx.x; j < n; j += T::NT) S.zs[j] = dist_z(D.v_min, D.dz64, j);
+    gather_tile<H>(S.Xs, S.ldx, A.rp.next_obs, A.nrows + (size_t)g * B, r0, B, Dp);
+
+    float acc[8][8];
+#pragma unroll 1
+    for (int pass = 0; pass < 2; ++pass) {          // 0: online(s')  1: target(s'); the target's logits stay in Ls
+        const float* P = (pass == 0 ? A.nets.theta : A.nets.theta_tgt) + (size_t)g * A.L.stride;
+        gemm_rowA<H, false>(acc, c, S.Xs, S.ldx, P + A.L.w1, H, Dp, S.Ws);
+        store_relu<H>(acc, c, P + A.L.b1, S.Hs1, nullptr, r0, B);
+        gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
+        store_relu<H>(acc, c, P + A.L.b2, S.Hs2, nullptr, r0, B);
+        dist_head<H>(acc, c, S, P, A.L, D.nh);
+        float* qs = pass == 0 ? S.qs0 : S.qs1;
+        for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {   // one thread per (row, action)
+            const int i = f >> 2, a = f & 3;
+            float mx, s;
+            qs[f] = a < nA && r0 + i < B ? dist_expect(S.Ls + i * S.ldl + a * np, n, S.zs, mx, s) : 0.f;
+        }
+        __syncthreads();
+    }
+    for (int i = threadIdx.x; i < T::BM; i += T::NT) {      // one thread per row; m is built in Hs2 (free now)
+        const int gr = r0 + i;
+        if (gr >= B) continue;
+        const float* qo = S.qs0 + i * 4;
+        const float* qt = S.qs1 + i * 4;
+        const float* qa = A.double_dqn ? qo : qt;
+        int best = 0;                               // ties -> lowest index
+        for (int k = 1; k < nA; ++k)
+            if (qa[k] > qa[best]) best = k;
+        const size_t o = (size_t)g * B + gr;
+        const float* x = S.Ls + i * S.ldl + best * np;
+        float mx, s;
+        dist_stats(x, n, mx, s);
+        dist_project(S.Hs2 + i * T::LDH, x, mx, s, S.zs, A.r_hat[o], A.disc_b[o], D);
+        for (int k = 0; k < 4; ++k) {
+            A.q_next[o * 4 + k] = qo[k];
+            A.tq_all[o * 4 + k] = qt[k];
+        }
+    }
+    __syncthreads();
+    for (int f = threadIdx.x; f < T::BM * np; f += T::NT) {
+        const int i = f / np, j = f % np;
+        if (r0 + i < B) D.m[((size_t)g * B + r0 + i) * np + j] = S.Hs2[i * T::LDH + j];
+    }
+}
+
+// Distributional K4a: forward on s (h1 -> workspace, h2 -> scratch), every action's expected Q, the cross-entropy of a_i
+// against m, the logit gradient dX (-> scratch), dh2 = (dX W3^T) * relu'(h2), dh1, and the per-tile partials.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const LearnArgs A, const DistArgs D) {
+    using T = Tile<H>;
+    extern __shared__ __align__(16) float smem[];
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
+    if (!A.active[g]) return;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, n = D.n_atoms, np = D.np, nh = D.nh;
+    DistSmem<H> S(smem, Dp, nh);
+    const Coord<H> c;
+    const int32_t* rows = A.rows + (size_t)g * B;
+    const float* P = A.nets.theta + (size_t)g * A.L.stride;
+    const size_t sb = (size_t)g * B;
+    for (int j = threadIdx.x; j < n; j += T::NT) S.zs[j] = dist_z(D.v_min, D.dz64, j);
+    gather_tile<H>(S.Xs, S.ldx, A.rp.obs, rows, r0, B, Dp);
+
+    float acc[8][8];
+    gemm_rowA<H, false>(acc, c, S.Xs, S.ldx, P + A.L.w1, H, Dp, S.Ws);
+    store_relu<H>(acc, c, P + A.L.b1, S.Hs1, A.h1 + sb * H, r0, B);
+    gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
+    store_relu<H>(acc, c, P + A.L.b2, S.Hs2, D.h2 + sb * H, r0, B);
+    dist_head<H>(acc, c, S, P, A.L, nh);
+
+    // one thread per (row, action): expected Q; the thread of the taken action also the loss term, the priority and the
+    // gradient of its Np logits (in place); every other block of the row's logit gradient is 0
+    for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {
+        const int i = f >> 2, a = f & 3, gr = r0 + i;
+        const bool row_ok = gr < B;
+        const int ai = row_ok ? A.act_b[sb + gr] : 0;
+        float* x = S.Ls + i * S.ldl + a * np;
+        float q = 0.f;
+        bool taken = false;
+        if (row_ok && a < nA) {
+            float mx, s;
+            q = dist_expect(x, n, S.zs, mx, s);
+            A.q_all[(sb + gr) * 4 + a] = q;
+            if (a == ai) {
+                taken = true;
+                const float* m = D.m + (sb + gr) * np;
+                const float wi = A.per ? A.is_w[sb + gr] : 1.f;
+                const float ls = logf(s);
+                float ce = 0.f;
+                for (int j = 0; j < n; ++j) {
+                    const float xm = __fsub_rn(x[j], mx), mj = m[j];
+                    ce = fmaf(mj, __fsub_rn(xm, ls), ce);
+                    x[j] = __fdiv_rn(__fmul_rn(wi, __fsub_rn(__fdiv_rn(expf(xm), s), mj)), (float)A.loss_batch);
+                }
+                for (int j = n; j < np; ++j) x[j] = 0.f;
+                ce = -ce;
+                if (A.per) per_store_priority(A, rows[gr], ce);
+                S.terms[i] = __fmul_rn(wi, ce);
+            }
+        } else if (row_ok) {
+            A.q_all[(sb + gr) * 4 + a] = 0.f;
+        }
+        if (!taken)
+            for (int j = 0; j < np; ++j) x[j] = 0.f;
+        if (a == 0) {
+            S.as[i] = ai;
+            if (!row_ok) S.terms[i] = 0.f;
+        }
+        S.qs0[f] = q;
+    }
+    __syncthreads();
+    const size_t pt = (size_t)g * A.ws_tiles + rt;   // partial slot of this (network, row tile)
+    if (threadIdx.x == 0) {                          // per-tile loss / metric partials, rows in order
+        float ls = 0.f, qsum = 0.f, qsq = 0.f, hist[4] = {0.f, 0.f, 0.f, 0.f};
+        for (int i = 0; i < T::BM && r0 + i < B; ++i) {
+            ls += S.terms[i];
+            for (int k = 0; k < nA; ++k) {
+                const float q = S.qs0[i * 4 + k];
+                qsum += q;
+                qsq = fmaf(q, q, qsq);
+            }
+            hist[S.as[i]] += 1.f;
+        }
+        float* pl = A.part_loss + pt * 8;
+        pl[0] = ls; pl[1] = qsum; pl[2] = qsq;
+        pl[3] = hist[0]; pl[4] = hist[1]; pl[5] = hist[2]; pl[6] = hist[3]; pl[7] = 0.f;
+    }
+    for (int f = threadIdx.x; f < T::BM * (nh / 4); f += T::NT) {   // dX tile -> scratch, coalesced
+        const int i = f / (nh / 4), c4 = f % (nh / 4);
+        if (r0 + i < B)
+            reinterpret_cast<float4*>(D.dx + (sb + r0 + i) * nh)[c4] = *reinterpret_cast<const float4*>(S.Ls + i * S.ldl + c4 * 4);
+    }
+    // dh2 = (dX W3^T) * relu'(h2), in place over h2
+    gemm_rowA<H, true>(acc, c, S.Ls, S.ldl, P + A.L.w3, nh, nh, S.Ws);
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int col = c.col0(half);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int row = c.row(i);
+            float4* hp = reinterpret_cast<float4*>(S.Hs2 + row * T::LDH + col);
+            const float4 h = *hp;
+            float4 v;
+            v.x = h.x > 0.f ? acc[i][half * 4 + 0] : 0.f;
+            v.y = h.y > 0.f ? acc[i][half * 4 + 1] : 0.f;
+            v.z = h.z > 0.f ? acc[i][half * 4 + 2] : 0.f;
+            v.w = h.w > 0.f ? acc[i][half * 4 + 3] : 0.f;
+            *hp = v;
+            if (r0 + row < B) *reinterpret_cast<float4*>(A.dh2 + (sb + r0 + row) * H + col) = v;
+        }
+    }
+    for (int f = threadIdx.x; f < T::BM * (H / 4); f += T::NT) {    // h1 back over the logits (rows past the batch: 0)
+        const int i = f / (H / 4), c4 = f % (H / 4);
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (r0 + i < B) v = reinterpret_cast<const float4*>(A.h1 + (sb + r0 + i) * H)[c4];
+        *reinterpret_cast<float4*>(S.Hs1 + i * T::LDH + c4 * 4) = v;
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < H; j += T::NT) {   // db2 partial
+        float s = 0.f;
+        for (int i = 0; i < T::BM; ++i) s += S.Hs2[i * T::LDH + j];
+        A.part_b2[pt * H + j] = s;
+    }
+    // dh1 = (dh2 W2^T) * relu'(h1), in place over h1
+    gemm_rowA<H, true>(acc, c, S.Hs2, T::LDH, P + A.L.w2, H, H, S.Ws);
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int col = c.col0(half);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int row = c.row(i);
+            float4* hp = reinterpret_cast<float4*>(S.Hs1 + row * T::LDH + col);
+            const float4 h = *hp;
+            float4 v;
+            v.x = h.x > 0.f ? acc[i][half * 4 + 0] : 0.f;
+            v.y = h.y > 0.f ? acc[i][half * 4 + 1] : 0.f;
+            v.z = h.z > 0.f ? acc[i][half * 4 + 2] : 0.f;
+            v.w = h.w > 0.f ? acc[i][half * 4 + 3] : 0.f;
+            *hp = v;
+            if (r0 + row < B) *reinterpret_cast<float4*>(A.dh1 + (sb + r0 + row) * H + col) = v;
+        }
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < H; j += T::NT) {   // db1 partial
+        float s = 0.f;
+        for (int i = 0; i < T::BM; ++i) s += S.Hs1[i * T::LDH + j];
+        A.part_b1[pt * H + j] = s;
+    }
+}
+
+// Distributional K4b, gradients only (A.grads): dW2 = h1^T dh2, dW1 = s^T dh1 and dW3 = h2^T dX (column slabs of H) tiles
+// in wgrad_adam_kernel's tile form, and a misc tile for b1 / b2 (partials in tile order), b3 (column sums of dX in row
+// order) and the metrics.  Pad columns of dX are 0, so their W3 / b3 gradients are 0.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT) dist_wgrad_kernel(const LearnArgs A, const DistArgs D) {
+    using T = Tile<H>;
+    constexpr int LDA = T::BM + 4;
+    extern __shared__ __align__(16) float smem[];
+    float (*As)[T::KC * LDA] = reinterpret_cast<float (*)[T::KC * LDA]>(smem);
+    float (*Bs)[T::KC * T::LDW] = reinterpret_cast<float (*)[T::KC * T::LDW]>(smem + 2 * T::KC * LDA);
+    const int B = A.d.batch, Dp = A.d.obs_stride, nh = D.nh;
+    const int tiles_w2 = H / T::BM, tiles_w1 = (Dp + T::BM - 1) / T::BM, slabs = (nh + H - 1) / H;
+    const int per_net = tiles_w2 + tiles_w1 + tiles_w2 * slabs + 1;
+    const int g = blockIdx.x / per_net, t = blockIdx.x % per_net;
+    const size_t sb = (size_t)g * B;
+    float* gout = A.grads + (size_t)g * A.L.stride;
+
+    if (t == per_net - 1) {
+        if (!A.active[g]) {
+            if (threadIdx.x < DMDQN_METRICS_STRIDE && A.metrics) A.metrics[g * DMDQN_METRICS_STRIDE + threadIdx.x] = 0.f;
+            return;
+        }
+        const size_t p0 = (size_t)g * A.ws_tiles;
+        for (int e = threadIdx.x; e < 2 * H + nh; e += T::NT) {
+            float gsum = 0.f;
+            if (e < 2 * H) {
+                const float* part = e < H ? A.part_b1 : A.part_b2;
+                const int j = e < H ? e : e - H;
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += part[(p0 + r) * H + j];
+                gout[(e < H ? A.L.b1 : A.L.b2) + j] = gsum;
+            } else {
+                const int j = e - 2 * H;
+                for (int k = 0; k < B; ++k) gsum += D.dx[(sb + k) * nh + j];
+                gout[A.L.b3 + j] = gsum;
+            }
+        }
+        if (threadIdx.x == 0 && A.metrics) finish_metrics(A, g, A.ws_tiles, [](const float* p) { return *p; });
+        return;
+    }
+    if (!A.active[g]) return;
+
+    // tile kinds: W2 (A = h1, D = dh2), W1 (A = gathered s, D = dh1), W3 slab (A = h2, D = dX columns c0 .. c0 + H)
+    const bool is_w2 = t < tiles_w2, is_w1 = !is_w2 && t < tiles_w2 + tiles_w1;
+    const int u = t - tiles_w2 - tiles_w1;
+    const int m0 = (is_w2 ? t : is_w1 ? t - tiles_w2 : u % tiles_w2) * T::BM;
+    const int c0 = is_w2 || is_w1 ? 0 : (u / tiles_w2) * H;
+    const int m_valid = is_w1 ? Dp : H;
+    const float* Asrc = is_w2 ? A.h1 + sb * H : is_w1 ? A.rp.obs : D.h2 + sb * H;
+    const int lda_src = is_w1 ? Dp : H;
+    const float* Dsrc = is_w2 ? A.dh2 + sb * H : is_w1 ? A.dh1 + sb * H : D.dx + sb * nh + c0;
+    const int ldd = is_w2 || is_w1 ? H : nh, ncol = is_w2 || is_w1 ? H : nh - c0;
+    const int32_t* rows = A.rows + sb;
+    const Coord<H> c;
+
+    constexpr int A4 = T::KC * T::BM / 4;            // 16-byte pieces in an A chunk
+    constexpr int NA = (A4 + T::NT - 1) / T::NT;
+    auto issue = [&](int k0, int buf) {
+#pragma unroll
+        for (int r = 0; r < NA; ++r) {
+            const int f = threadIdx.x + r * T::NT;
+            if (f < A4) {
+                const int kk = f / (T::BM / 4), m4 = f % (T::BM / 4);
+                const int kr = k0 + kk, m = m0 + m4 * 4;
+                const bool ok = kr < B && m < m_valid;
+                const size_t src_row = ok ? (is_w1 ? (size_t)rows[kr] : (size_t)kr) : 0;
+                cp_async16(&As[buf][kk * LDA + m4 * 4], Asrc + src_row * lda_src + (ok ? m : 0), ok);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < T::KC * H / 4 / T::NT; ++r) {
+            const int f = threadIdx.x + r * T::NT;
+            const int kk = f / (H / 4), n4 = f % (H / 4);
+            const bool ok = k0 + kk < B && n4 * 4 < ncol;
+            cp_async16(&Bs[buf][kk * T::LDW + n4 * 4], Dsrc + (ok ? (size_t)(k0 + kk) * ldd + n4 * 4 : 0), ok);
+        }
+        cp_async_commit();
+    };
+
+    float acc[8][8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+    issue(0, 0);
+    cp_async_wait_all();
+    __syncthreads();
+    int buf = 0;
+    for (int k0 = 0; k0 < B; k0 += T::KC) {
+        const bool more = k0 + T::KC < B;
+        if (more) issue(k0 + T::KC, buf ^ 1);
+#pragma unroll
+        for (int kk = 0; kk < T::KC; ++kk) {
+            const float4 a0 = *reinterpret_cast<const float4*>(&As[buf][kk * LDA + c.wm * 32 + c.lm * 4]);
+            const float4 a1 = *reinterpret_cast<const float4*>(&As[buf][kk * LDA + c.wm * 32 + 16 + c.lm * 4]);
+            const float4 b0 = *reinterpret_cast<const float4*>(&Bs[buf][kk * T::LDW + c.col0(0)]);
+            const float4 b1 = *reinterpret_cast<const float4*>(&Bs[buf][kk * T::LDW + c.col0(1)]);
+            fma8(acc[0], a0.x, b0, b1); fma8(acc[1], a0.y, b0, b1);
+            fma8(acc[2], a0.z, b0, b1); fma8(acc[3], a0.w, b0, b1);
+            fma8(acc[4], a1.x, b0, b1); fma8(acc[5], a1.y, b0, b1);
+            fma8(acc[6], a1.z, b0, b1); fma8(acc[7], a1.w, b0, b1);
+        }
+        if (more) cp_async_wait_all();
+        __syncthreads();
+        buf ^= 1;
+    }
+
+    const int64_t wbase = is_w2 ? A.L.w2 : is_w1 ? A.L.w1 : A.L.w3 + c0;
+    const int ldo = is_w2 || is_w1 ? H : nh;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const int m = m0 + c.row(i);
+        if (m >= m_valid) continue;
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+            const int col = c.col0(half);
+            if (col < ncol)
+                *reinterpret_cast<float4*>(gout + wbase + (int64_t)m * ldo + col) =
+                    make_float4(acc[i][half * 4], acc[i][half * 4 + 1], acc[i][half * 4 + 2], acc[i][half * 4 + 3]);
+        }
+    }
+}
+
+template <int H>
+int launch_learn_dist_h(const LearnArgs& A, const DistArgs& D, cudaStream_t s) {
+    using T = Tile<H>;
+    const size_t smem = DistSmem<H>::bytes(A.d.obs_stride, D.nh);
+    const size_t smem_w = sizeof(float) * 2 * T::KC * ((T::BM + 4) + T::LDW);
+    static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_target_kernel<H>), smem, cfg_t)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_online_kernel<H>), smem, cfg_o)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_wgrad_kernel<H>), smem_w, cfg_w)) return rc;
+    const int grid = A.d.n_nets * A.ws_tiles;
+    dist_target_kernel<H><<<grid, T::NT, smem, s>>>(A, D);
+    DMDQN_CUDA(cudaGetLastError());
+    dist_online_kernel<H><<<grid, T::NT, smem, s>>>(A, D);
+    DMDQN_CUDA(cudaGetLastError());
+    const int per_net = H / T::BM + (A.d.obs_stride + T::BM - 1) / T::BM + (H / T::BM) * ((D.nh + H - 1) / H) + 1;
+    dist_wgrad_kernel<H><<<A.d.n_nets * per_net, T::NT, smem_w, s>>>(A, D);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+// One dynamic shared-memory opt-in record for clip_adam_apply_kernel, whichever layout the launch carries (the attribute
+// belongs to the kernel: a smaller request after a larger one must not lower it below what the larger launch needs).
+size_t g_clip_smem_cfg[kMaxDevices] = {};
+
 template <int H, bool DUELING>
 int launch_learn_h(const LearnArgs& A, int stages, cudaStream_t s) {
     using T = Tile<H>;
@@ -977,9 +1402,50 @@ int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const d
     const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
     const int64_t per = clip_per_cta(A.L);
     const size_t smem = (size_t)per * 16;
-    static size_t cfg[kMaxDevices] = {};
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, cfg)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
     clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_learn_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                      const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                      cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    const DistArgs D = make_dist_args(d, ds);
+    A.L = make_layout_dist(d.obs_stride, d.hidden, D.np);
+    switch (d.hidden) {
+        case 64: return launch_learn_dist_h<64>(A, D, s);
+        case 128: return launch_learn_dist_h<128>(A, D, s);
+        case 256: return launch_learn_dist_h<256>(A, D, s);
+        case 512: return launch_learn_dist_h<512>(A, D, s);
+    }
+    set_error("unsupported hidden width %d", d.hidden);
+    return DMDQN_ERR_ARG;
+}
+
+// adam_apply_kernel (clipnorm == 0) or clip_adam_apply_kernel on the distributional layout: the same arithmetic over [0, end)
+int launch_adam_apply_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_atoms, const float* grads,
+                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    A.L = make_layout_dist(d.obs_stride, d.hidden, dist_np(n_atoms));
+    if (clipnorm == 0.0) {
+        adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
+        DMDQN_CUDA(cudaGetLastError());
+        return DMDQN_OK;
+    }
+    const int64_t per = clip_per_cta(A.L);
+    const size_t smem = (size_t)per * 16;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
+    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_atoms, const uint8_t* mask, double tau,
+                            cudaStream_t s) {
+    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(n_atoms));
+    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

@@ -46,7 +46,40 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # noisy networks (Fortunato et al. 2018): factorized Gaussian noise on every layer replaces epsilon-greedy exploration;
     # sigma starts at noisy_sigma0 / sqrt(fan_in)
     "noisy": False, "noisy_sigma0": 0.5,
+    # distributional Q-learning (C51, Bellemare et al. 2017): a categorical return distribution over num_atoms atoms of
+    # [v_min, v_max] per action, projected Bellman targets and a cross-entropy loss
+    "distributional": False, "num_atoms": 51, "v_min": -10.0, "v_max": 10.0,
 }
+
+
+def dist_config(cfg: dict) -> dict:
+    """Validate the distributional keys of ``cfg`` and resolve its precision (in place; returns ``cfg``).  With
+    ``distributional: true`` the learn step runs the fp32 (FFMA) kernels only, so ``precision: auto`` becomes fp32 and an
+    explicit tcgen05 precision, dueling heads, noisy networks and the Huber loss are refused."""
+    if not isinstance(cfg["distributional"], (bool, np.bool_)):
+        raise ValueError(f"distributional={cfg['distributional']!r}: must be true or false")
+    if not cfg["distributional"]:
+        return cfg
+    n = cfg["num_atoms"]
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 2 <= n <= N.DIST_MAX_ATOMS:
+        raise ValueError(f"num_atoms={n!r}: must be an integer in [2, {N.DIST_MAX_ATOMS}]")
+    lo, hi = cfg["v_min"], cfg["v_max"]
+    if any(isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v) for v in (lo, hi)) or lo >= hi:
+        raise ValueError(f"v_min={lo!r}, v_max={hi!r}: the support needs finite numbers with v_min < v_max")
+    if cfg["precision"] not in ("auto", "fp32"):
+        raise ValueError(f"precision={cfg['precision']!r}: distributional networks run the fp32 (FFMA) learn path only; the "
+                         "tcgen05 distributional kernels are not built yet (use precision: auto or fp32)")
+    if cfg["dueling"]:
+        raise ValueError("distributional=true cannot be combined with dueling=true yet: the per-atom dueling fold is not "
+                         "implemented")
+    if cfg["noisy"]:
+        raise ValueError("distributional=true cannot be combined with noisy=true yet: noisy distributional heads are not "
+                         "implemented")
+    if cfg["loss"] != "mse":
+        raise ValueError(f"loss={cfg['loss']!r}: distributional networks minimise the cross-entropy of the projected target; "
+                         "the loss key does not apply (leave it at mse)")
+    cfg["precision"] = "fp32"
+    return cfg
 
 
 def _ptr(t: torch.Tensor | None) -> int | None:
@@ -132,6 +165,9 @@ class AgentGroup:
         if self.noisy and self.global_clipnorm is not None:
             raise ValueError("noisy=true cannot be combined with global_clipnorm yet: the global norm over the mean and the "
                              "sigma gradients is not implemented")
+        dist_config(cfg)
+        self.distributional = bool(cfg["distributional"])
+        self.num_atoms = int(cfg["num_atoms"]) if self.distributional else 0
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -150,6 +186,10 @@ class AgentGroup:
         if self.dueling:        # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
             self.layout = N.DuelingLayout()
             N.check(self.lib.dmdqn_param_layout_dueling(C.byref(self.dims), C.byref(self.layout)))
+        elif self.distributional:   # the head W3[H][4 * Np] | b3[4 * Np]
+            self.layout = N.Layout()
+            N.check(self.lib.dmdqn_param_layout_dist(C.byref(self.dims), self.num_atoms, C.byref(self.layout)))
+            self.atom_stride = (self.num_atoms + 3) // 4 * 4
         else:
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
@@ -188,6 +228,8 @@ class AgentGroup:
             # gradient clipping: the raw gradient blocks of a step and each network's norm before clipping (last step)
             self.grads = torch.zeros_like(self.theta) if self.global_clipnorm is not None else None
             self.grad_norms = torch.zeros((g,), dtype=torch.float32, device=dev) if self.global_clipnorm is not None else None
+            if self.distributional:     # the gradient block between dmdqn_learn_grads_dist and dmdqn_adam_apply_dist
+                self.grads = torch.zeros_like(self.theta)
             if self.noisy:      # sigma with its target and moments, the effective blocks, the gradient and the noise record
                 self.sigma, self.sigma_tgt = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
                 self.sigma_m, self.sigma_v = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
@@ -220,6 +262,12 @@ class AgentGroup:
         self.nets = N.Nets(_ptr(self.theta), _ptr(self.theta_tgt), _ptr(self.adam_m), _ptr(self.adam_v),
                            _ptr(self.learn_step))
         self.noisy_ptrs = N.Noisy(*(_ptr(getattr(self, k)) for k in self._NOISY_PTRS)) if self.noisy else None
+        self.dist_scratch, self.dist = None, None
+        if self.distributional:     # per group, like the workspace: what the distributional kernels of one step pass on
+            nbytes = C.c_size_t()
+            N.check(self.lib.dmdqn_dist_scratch_bytes(C.byref(self.dims), self.num_atoms, C.byref(nbytes)))
+            self.dist_scratch = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
+            self.dist = N.Dist(self.num_atoms, float(cfg["v_min"]), float(cfg["v_max"]), _ptr(self.dist_scratch), nbytes.value)
         nbytes = C.c_size_t()
         N.check(self.lib.dmdqn_workspace_bytes(C.byref(self.dims), C.byref(nbytes)))
         self.workspace = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
@@ -276,6 +324,11 @@ class AgentGroup:
         blk[L.b1:L.b1 + H] = b1
         blk[L.w2:L.w2 + H * H] = w2.reshape(-1)
         blk[L.b2:L.b2 + H] = b2
+        if getattr(self, "distributional", False):     # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
+            n, npad = self.num_atoms, self.atom_stride
+            blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n] = w3.reshape(H, A, n)
+            blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n] = b3.reshape(A, n)
+            return blk
         blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A] = w3
         blk[L.b3:L.b3 + A] = b3
         if self.dueling:
@@ -287,9 +340,12 @@ class AgentGroup:
         L, H, A = self.layout, self.hidden, self.action_size
         blk = blk.detach().cpu()
         out = [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
-               blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(),
-               blk[L.b2:L.b2 + H].clone(), blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(),
-               blk[L.b3:L.b3 + A].clone()]
+               blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(), blk[L.b2:L.b2 + H].clone()]
+        if getattr(self, "distributional", False):
+            n, npad = self.num_atoms, self.atom_stride
+            return out + [blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
+                          blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
+        out += [blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(), blk[L.b3:L.b3 + A].clone()]
         if self.dueling:
             out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
         return out
@@ -307,7 +363,8 @@ class AgentGroup:
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
         (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
-        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, self.action_size, self.dueling))
+        head = self.action_size * self.num_atoms if self.distributional else self.action_size   # dist: W3 GlorotUniform over [H, A*N]
+        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, self.dueling))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
@@ -412,7 +469,9 @@ class AgentGroup:
         nets = self.nets if not target else N.Nets(_ptr(self.theta_tgt), _ptr(self.theta_tgt), _ptr(self.adam_m),
                                                    _ptr(self.adam_v), _ptr(self.learn_step))
         args = (_ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream)
-        if self.noisy and noisy is not False and not target:
+        if self.distributional:
+            N.check(self.lib.dmdqn_act_dist(C.byref(self.dims), C.byref(nets), C.byref(self.dist), *args))
+        elif self.noisy and noisy is not False and not target:
             N.check(self.lib.dmdqn_act_noisy(C.byref(self.dims), C.byref(nets), C.byref(self.noisy_ptrs), int(self.dueling),
                                              *args))
         else:
@@ -505,6 +564,14 @@ class AgentGroup:
         (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
         ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
         ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.distributional:     # the C51 gradient, then Adam (clipped when global_clipnorm is set)
+            N.check(self.lib.dmdqn_learn_grads_dist(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
+                                                    C.byref(self.nets), draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads),
+                                                    _ptr(self.metrics), ws, nws, stream_ptr))
+            N.check(self.lib.dmdqn_adam_apply_dist(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.num_atoms,
+                                                   _ptr(self.grads), self.global_clipnorm or 0.0, _ptr(self.grad_norms), ws, nws,
+                                                   stream_ptr))
+            return
         if self.noisy:          # gradient of the effective weights, then Adam on mu and sigma
             N.check(self.lib.dmdqn_learn_grads_noisy(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                                      C.byref(self.noisy_ptrs), draws_ptr, mask_ptr, self.batch_size,
@@ -590,7 +657,7 @@ class AgentGroup:
         """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
         one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy; the
         same with ``noisy`` set and the noisy learn calls."""
-        if self.global_clipnorm is None and not self.noisy:
+        if self.global_clipnorm is None and not self.noisy and not self.distributional:
             N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                              C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
                                              _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
@@ -672,6 +739,14 @@ class AgentGroup:
                "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
         if self.noisy:           # factor vectors [network][set][record] and effective blocks of the last fold
             out["noise"], out["eff"], out["eff_tgt"] = self.noise, self.eff, self.eff_tgt
+        if self.distributional:  # the projected target distributions m [network][row][Np] of the last learn step
+            dv = N.DistViews()
+            N.check(self.lib.dmdqn_debug_dist(C.byref(self.dims), C.byref(self.dist), C.byref(dv)))
+            sbase = self.dist_scratch.data_ptr()
+            for key, ptr, width in (("target_dist", dv.target_dist, self.atom_stride), ("h2", dv.h2, self.hidden),
+                                    ("dlogits", dv.dlogits, 4 * self.atom_stride)):
+                off = ptr - sbase
+                out[key] = self.dist_scratch[off:off + g * b * width * 4].view(torch.float32).view(g, b, width)
         if self.dueling:         # the folded heads W3e[H][4] | b3e[4] of the last learn step, online (0) and target (1)
             dv = N.DuelingViews()
             N.check(self.lib.dmdqn_debug_dueling(C.byref(self.dims), _ptr(self.workspace), self.workspace.numel(), C.byref(dv)))
@@ -693,6 +768,10 @@ class AgentGroup:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
         tau = -1.0 if tau is None else float(tau)
+        if self.distributional:
+            N.check(self.lib.dmdqn_sync_target_dist(C.byref(self.dims), C.byref(self.nets), self.num_atoms, _ptr(mask_t), tau,
+                                                    self._stream))
+            return
         if self.noisy:           # mu and sigma
             N.check(self.lib.dmdqn_sync_target_noisy(C.byref(self.dims), C.byref(self.nets), C.byref(self.noisy_ptrs),
                                                      int(self.dueling), _ptr(mask_t), tau, self._stream))

@@ -205,7 +205,9 @@ class SharedParameterStep:
         ``dmdqn_clip_adam_apply`` on the all-reduced block; ``fused=True`` is refused there.  ``exchange``: a PeerExchange
         already connected (tests).  A ``noisy`` group takes the NCCL path too: every rank folds the same noise (same keys and
         step counters), the effective-weight gradients are all-reduced and ``dmdqn_noisy_adam_apply`` updates mu and sigma;
-        ``fused=True`` is refused there, because the peer-memory kernel does not know sigma."""
+        ``fused=True`` is refused there, because the peer-memory kernel does not know sigma.  A ``distributional`` group takes
+        the NCCL path as well: ``dmdqn_learn_grads_dist``, the all-reduce of its gradient block, then ``dmdqn_adam_apply_dist``
+        (clipped when ``global_clipnorm`` is set); ``fused=True`` is refused there."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
@@ -218,8 +220,11 @@ class SharedParameterStep:
         if grp.noisy and fused:
             raise ValueError("noisy=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not update sigma; use "
                              "fused=False (the NCCL all-reduce + dmdqn_noisy_adam_apply path)")
+        if grp.distributional and fused:
+            raise ValueError("distributional=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the "
+                             "distributional layout; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_dist path)")
         if fused is None:
-            fused = clip is None and not grp.noisy and (world > 1 or exchange is not None)
+            fused = clip is None and not grp.noisy and not grp.distributional and (world > 1 or exchange is not None)
         if fused and exchange is None:
             rank = dist.get_rank(group) if world > 1 else 0
             exchange = PeerExchange(grp, rank, world).connect(group)
@@ -236,7 +241,12 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                if grp.noisy:
+                if grp.distributional:
+                    N.check(grp.lib.dmdqn_learn_grads_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.dist),
+                                                           C.byref(grp.replay), C.byref(grp.nets), _ptr(d), None,
+                                                           int(global_batch), _ptr(out), _ptr(grp.metrics), _ptr(grp.workspace),
+                                                           grp.workspace.numel(), grp._stream))
+                elif grp.noisy:
                     N.check(grp.lib.dmdqn_learn_grads_noisy(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay),
                                                             C.byref(grp.nets), C.byref(grp.noisy_ptrs), _ptr(d), None,
                                                             int(global_batch), _ptr(out), _ptr(grp.metrics), _ptr(grp.workspace),
@@ -266,6 +276,11 @@ class SharedParameterStep:
 
         def apply(g: torch.Tensor):
             with torch.cuda.device(grp.device):
+                if grp.distributional:          # clipped (the norm of the all-reduced block) when global_clipnorm is set
+                    N.check(grp.lib.dmdqn_adam_apply_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.num_atoms,
+                                                          _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),
+                                                          grp.workspace.numel(), grp._stream))
+                    return
                 if clip is not None:            # the norm of the all-reduced block: the same scale on every replica
                     N.check(grp.lib.dmdqn_clip_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g), clip,
                                                           _ptr(grp.grad_norms), _ptr(grp.workspace), grp.workspace.numel(),

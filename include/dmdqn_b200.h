@@ -40,6 +40,8 @@
  *   (Wang et al. 2016), which is the plain 4-wide head with the effective weights
  *     W3e[k][a] = (W3[k][a] - mean_{b<A} W3[k][b]) + wv[k]  (a < A; 0 for a >= A),  b3e[a] = (b3[a] - mean_{b<A} b3[b]) + bv
  *   each mean summed left to right in fp32 and divided by A (IEEE division).  Advantage columns >= A keep gradient 0.
+ *   distributional networks (C51; dmdqn_param_layout_dist, see dmdqn_dist below) widen the head to 4 * Np columns:
+ *     W1 | b1 | W2 | b2 | W3[H][4 * Np] | b3[4 * Np] | pad
  */
 #ifndef DMDQN_B200_H
 #define DMDQN_B200_H
@@ -520,6 +522,79 @@ int dmdqn_act_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_
 /* dmdqn_sync_target of mu (theta -> theta_tgt) and of sigma (sigma -> sigma_tgt). */
 int dmdqn_sync_target_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
                             const uint8_t* mask, double tau, void* stream);
+
+/* Distributional Q-learning (C51, Bellemare, Dabney & Munos 2017), fp32 (FFMA) path only.  Each action's return is a
+ * categorical distribution over N = n_atoms atoms (2 <= N <= 64) of the fixed support
+ *   dz64 = (v_max - v_min) / (N - 1) (float64),  z_j = (float)(v_min + j * dz64),  dz = (float)dz64,
+ *   lo = (float)v_min,  hi = (float)v_max                          (v_min < v_max, both finite).
+ * Parameter block (dmdqn_param_layout_dist fills a dmdqn_layout):
+ *   W1[obs_stride][H] | b1[H] | W2[H][H] | b2[H] | W3[H][4 * Np] | b3[4 * Np] | pad
+ * with Np = N rounded up to a multiple of 4 and column a * Np + j holding atom j of action a.  Columns with a >= A or
+ * j >= N are 0 and keep gradient 0.  Adam updates [0, b3 + 4 * Np); the stride is rounded up to 32 floats.
+ * Head: for action a the logits are x_a = h2 . W3[:, a*Np .. a*Np + N) + b3[a*Np ..], and per action
+ *   mx = max_j x_j,  e_j = expf(x_j - mx),  S = sum_j e_j (j order),  p_j = e_j / S,  log p_j = (x_j - mx) - logf(S)
+ *   Q(s, a) = sum_j p_j z_j   (fmaf, j order)
+ * with the accurate expf / logf and IEEE division.  Expected-Q outputs hold 0 for actions a >= A.
+ * Target of sampled row i (R, discount d and the bootstrap row as dmdqn_sample forms them, so n-step returns and done
+ * apply): a* = argmax of the online (double_dqn = 1) or the target (double_dqn = 0) network's expected Q at s', ties to
+ * the lowest index; p = softmax of the target network's logits of a* at s'; m = 0, then for j = 0 .. N - 1 in order
+ *   t = min(max(R + d * z_j, lo), hi)    (product and sum rounded separately)
+ *   b = min((t - lo) / dz, N - 1),  l = floor(b),  u = ceil(b)
+ *   l == u:  m[l] += p_j      else:  m[l] += p_j * (u - b);  m[u] += p_j * (b - l)
+ * Loss of row i with action a_i: L_i = -sum_j m_j log p_j(s_i, a_i) (the sum as fmaf in j order, then negated); the loss
+ * term is w_i * L_i with w_i the importance weight of prioritized replay (1 otherwise), and prioritized replay stores
+ * priority = (float)pow(L_i + per_eps, per_alpha) (the unweighted cross-entropy).  The gradient of the logits of a_i is
+ * (w_i * (p_j - m_j)) / loss_batch and 0 for every other column.  hp->loss is not read.
+ * Metrics row: [0] the weighted batch-mean cross-entropy, [1] / [2] the mean and std of the online expected Q over
+ * a < A, the action histogram and the learned flag.  dmdqn_debug's q_all / q_next / tq_all hold expected Q values; y is
+ * not written.
+ *   scratch   caller-owned device memory of at least dmdqn_dist_scratch_bytes, 16-byte aligned: the projected target
+ *             distribution m [n_nets][B][Np], h2 [n_nets][B][H] and the logit gradient [n_nets][B][4 * Np].
+ * Every call below refuses, before anything is launched: n_atoms outside [2, 64], v_min >= v_max or either non-finite,
+ * hp->precision other than DMDQN_PRECISION_FP32, hp->dueling != 0, NULL or misaligned pointers and a scratch smaller
+ * than the query returns. */
+typedef struct dmdqn_dist {
+    int32_t n_atoms;
+    double v_min, v_max;
+    void* scratch;
+    size_t scratch_bytes;
+} dmdqn_dist;
+#define DMDQN_DIST_MAX_ATOMS 64
+int dmdqn_param_layout_dist(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_layout* out);
+int dmdqn_dist_scratch_bytes(const dmdqn_dims* dims, int32_t n_atoms, size_t* out_bytes);
+
+/* One distributional learn step up to the gradient: the sample kernel of dmdqn_learn (learn_step, Adam scalars, n-step
+ * and prioritized rows), then the distributional target, online and weight-gradient kernels.  grads_out[n_nets][stride]
+ * receives dL/dtheta for every float of [0, b3 + 4 * Np) with the loss mean over global_batch (>= batch).  Finish the step
+ * with dmdqn_adam_apply_dist. */
+int dmdqn_learn_grads_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_dist* dist, const dmdqn_replay* replay,
+                           const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
+                           float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Adam + target sync on distributional blocks from a gradient block: global_clipnorm == 0 is dmdqn_adam_apply's arithmetic,
+ * global_clipnorm > 0 (finite) dmdqn_clip_adam_apply's (the norm over [0, b3 + 4 * Np), norms_out as there); a negative,
+ * NaN or infinite global_clipnorm is refused. */
+int dmdqn_adam_apply_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, int32_t n_atoms,
+                          const float* grads, double global_clipnorm, float* norms_out, void* workspace, size_t workspace_bytes,
+                          void* stream);
+
+/* dmdqn_act on distributional blocks: q_out holds the expected Q values (0 for a >= A), the action is their argmax under
+ * dmdqn_act's epsilon rule, and exploring agents skip the forward pass (their q_out rows are untouched).  dist->scratch is
+ * not used and may be NULL. */
+int dmdqn_act_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_dist* dist, const float* obs,
+                   int32_t obs_in_stride, const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
+                   int32_t* actions_out, float* q_out, void* stream);
+
+/* dmdqn_sync_target over the whole distributional stride. */
+int dmdqn_sync_target_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, int32_t n_atoms, const uint8_t* mask, double tau,
+                           void* stream);
+
+/* The scratch's views after dmdqn_learn_grads_dist: target_dist float[n_nets][B][Np] (the projected m of every row),
+ * h2 float[n_nets][B][H], dlogits float[n_nets][B][4 * Np] (the logit gradient). */
+typedef struct dmdqn_dist_views {
+    const float* target_dist; const float* h2; const float* dlogits;
+} dmdqn_dist_views;
+int dmdqn_debug_dist(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_dist_views* out);
 
 #ifdef __cplusplus
 }
