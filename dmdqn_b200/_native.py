@@ -90,6 +90,10 @@ class DistViews(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("target_dist", "h2", "dlogits")]
 
 
+class Quantile(C.Structure):
+    _fields_ = [("n_quantiles", C.c_int32), ("kappa", C.c_double), ("scratch", C.c_void_p), ("scratch_bytes", C.c_size_t)]
+
+
 DIST_MAX_ATOMS = 64
 
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
@@ -161,6 +165,11 @@ SIGNATURES = {
     "dmdqn_act_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Dist), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "dmdqn_sync_target_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P]),
     "dmdqn_debug_dist": (C.c_int, [C.POINTER(Dims), C.POINTER(Dist), C.POINTER(DistViews)]),
+    "dmdqn_learn_grads_quantile": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Quantile), C.POINTER(Replay),
+                                             C.POINTER(Nets), _P, _P, C.c_int32, _P, _P, _P, C.c_size_t, _P]),
+    "dmdqn_act_quantile": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Quantile), _P, C.c_int32, _P, _P, _P, _P, _P,
+                                     _P]),
+    "dmdqn_debug_quantile": (C.c_int, [C.POINTER(Dims), C.POINTER(Quantile), C.POINTER(DistViews)]),
 }
 
 _lib = None

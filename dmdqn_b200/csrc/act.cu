@@ -355,6 +355,61 @@ act_dist_kernel(dmdqn_dims d, Layout L, int n_atoms, double v_min, double dz64, 
     }
 }
 
+// Quantile heads (include/dmdqn_b200.h dmdqn_quantile): act_dist_kernel's scheme with the mean of the quantiles in place of
+// the softmax expectation: the plain trunk, CTA `rank` computes action rank's Np quantiles (thread j < Np owns column j,
+// four thread groups split the H rows, partials added to b3 in group order) and their mean; the four Q values meet on
+// rank 0 over DSMEM for the argmax.  (act_dist_kernel keeps its own head: compiled through a head shared with this
+// kernel, its register allocation changes.)
+template <int H>
+__global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads, 4)
+act_quantile_kernel(dmdqn_dims d, Layout L, int n_quantiles, const float* __restrict__ theta, const float* __restrict__ obs,
+                    int stride, const double* __restrict__ eps, const uint32_t* __restrict__ w_explore,
+                    const uint32_t* __restrict__ w_action, int32_t* __restrict__ actions, float* __restrict__ q_out) {
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int a = blockIdx.x / kActCluster, rank = (int)cluster.block_rank();
+    const bool explore = (double)w_explore[a] < eps[a] * 4294967296.0;
+    if (explore) {
+        if (threadIdx.x == 0 && rank == 0) actions[a] = (int32_t)__umulhi(w_action[a], (uint32_t)d.n_actions);
+        return;
+    }
+    float* xs = smem;                        // [Dp]
+    float* h1 = xs + d.obs_stride;           // [H]
+    float* h2 = h1 + H;                      // [H]
+    float* part = h2 + H;                    // [1024]: trunk partials, then head partials [4][64] and rank 0's Q[4] at 512
+    float* th = part + kActThreads * 4;      // [64] quantiles
+    const int net = d.n_nets == 1 ? 0 : a;
+    const float* P = theta + (size_t)net * L.stride;
+    act_trunk<H>(cluster, d, L, P, obs + (size_t)a * stride, xs, h1, h2, part, rank);
+
+    const int np = (n_quantiles + 3) / 4 * 4, nh = 4 * np;
+    const int j = threadIdx.x & 63, grp = threadIdx.x >> 6;
+    const bool mine = rank < d.n_actions;
+    if (mine && j < np) {
+        const float* w = P + L.w3 + rank * np + j;
+        float s = 0.f;
+        for (int k = grp; k < H; k += 4) s = fmaf(h2[k], __ldg(w + (size_t)k * nh), s);
+        part[grp * 64 + j] = s;
+    }
+    __syncthreads();
+    if (mine && threadIdx.x < n_quantiles) {
+        float x = __ldg(P + L.b3 + rank * np + threadIdx.x);
+        for (int g = 0; g < 4; ++g) x += part[g * 64 + threadIdx.x];
+        th[threadIdx.x] = x;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) cluster.map_shared_rank(part, 0)[512 + rank] = mine ? quantile_mean(th, n_quantiles) : 0.f;
+    cluster.sync();
+    if (threadIdx.x == 0 && rank == 0) {
+        const float* q = part + 512;
+        int best = 0;                                   // ties -> lowest index
+        for (int k = 1; k < d.n_actions; ++k) if (q[k] > q[best]) best = k;
+        actions[a] = best;
+        if (q_out)
+            for (int k = 0; k < 4; ++k) q_out[(size_t)a * 4 + k] = q[k];
+    }
+}
+
 }  // namespace
 
 int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
@@ -372,6 +427,26 @@ int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dis
         case 128: run(act_dist_kernel<128>); break;
         case 256: run(act_dist_kernel<256>); break;
         case 512: run(act_dist_kernel<512>); break;
+        default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
+    }
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_quantile& qs, const float* obs, int32_t stride,
+                        const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
+                        cudaStream_t s) {
+    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(qs.n_quantiles));
+    const size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + kDistMaxAtoms) * sizeof(float);
+    const dim3 grid(d.n_agents * kActCluster);
+    auto run = [&](auto kernel) {
+        kernel<<<grid, kActThreads, smem, s>>>(d, L, qs.n_quantiles, nets.theta, obs, stride, eps, w1, w2, actions, q_out);
+    };
+    switch (d.hidden) {
+        case 64: run(act_quantile_kernel<64>); break;
+        case 128: run(act_quantile_kernel<128>); break;
+        case 256: run(act_quantile_kernel<256>); break;
+        case 512: run(act_quantile_kernel<512>); break;
         default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
     }
     DMDQN_CUDA(cudaGetLastError());

@@ -661,6 +661,65 @@ int dmdqn_debug_dist(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_dist_
     return DMDQN_OK;
 }
 
+// Quantile calls (include/dmdqn_b200.h dmdqn_quantile): the quantile count, kappa and, where the call reads it, the scratch;
+// the hparams and network checks are those of the distributional calls.
+static int check_quantile(const dmdqn_dims* dims, const dmdqn_quantile* qs, bool scratch) {
+    DMDQN_CHECK_ARG(qs != nullptr, "quantile is NULL");
+    DMDQN_CHECK_ARG(qs->n_quantiles >= 2 && qs->n_quantiles <= DMDQN_DIST_MAX_ATOMS, "n_quantiles=%d must be in [2, %d]",
+                    qs->n_quantiles, DMDQN_DIST_MAX_ATOMS);
+    DMDQN_CHECK_ARG(isfinite(qs->kappa) && qs->kappa >= 0.0, "kappa=%g must be finite and >= 0", qs->kappa);
+    if (scratch) {
+        DMDQN_CHECK_ARG(qs->scratch && aligned16(qs->scratch), "quantile: scratch is NULL or not 16-byte aligned");
+        const size_t need = make_dist_scratch(*dims, dist_np(qs->n_quantiles)).total;
+        DMDQN_CHECK_ARG(qs->scratch_bytes >= need, "quantile: scratch has %zu bytes, %zu needed", qs->scratch_bytes, need);
+    }
+    return DMDQN_OK;
+}
+
+int dmdqn_learn_grads_quantile(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_quantile* quantile,
+                               const dmdqn_replay* replay, const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
+                               int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    if ((rc = check_dist_hp(hp))) return rc;
+    if ((rc = check_quantile(dims, quantile, true))) return rc;
+    if ((rc = check_dist_nets(nets, true))) return rc;
+    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
+    return launch_learn_quantile(*dims, *hp, *replay, *nets, *quantile, metrics_out, (char*)workspace, w, grads_out,
+                                 global_batch, s);
+}
+
+int dmdqn_act_quantile(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_quantile* quantile, const float* obs,
+                       int32_t obs_in_stride, const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
+                       int32_t* actions_out, float* q_out, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_quantile(dims, quantile, false))) return rc;
+    DMDQN_CHECK_ARG(nets && nets->theta && aligned16(nets->theta), "act_quantile: theta is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(obs && eps && w_explore && w_action && actions_out, "act_quantile: NULL argument");
+    DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
+    return launch_act_quantile(*dims, *nets, *quantile, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out,
+                               (cudaStream_t)stream);
+}
+
+int dmdqn_debug_quantile(const dmdqn_dims* dims, const dmdqn_quantile* quantile, dmdqn_dist_views* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_quantile(dims, quantile, true))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const QuantArgs Q = make_quantile_args(*dims, *quantile);
+    out->target_dist = Q.m;
+    out->h2 = Q.h2;
+    out->dlogits = Q.dx;
+    return DMDQN_OK;
+}
+
 static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau, bool dueling,
                            void* stream) {
     int rc = validate_dims(dims);

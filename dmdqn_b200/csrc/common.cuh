@@ -227,6 +227,33 @@ __device__ __forceinline__ float dist_expect(const float* x, int n, const float*
     return q;
 }
 
+// Quantile (QR-DQN) networks (include/dmdqn_b200.h dmdqn_quantile): the C51 head layout, scratch and Adam range for
+// N = n_quantiles atoms; the scratch's m region holds the target samples T.  What the kernels take beyond LearnArgs:
+struct QuantArgs {
+    int n_atoms, np, nh;              // N, Np, 4 * Np
+    float kappa;                      // (float)kappa
+    float *m, *h2, *dx;
+};
+inline QuantArgs make_quantile_args(const dmdqn_dims& d, const dmdqn_quantile& qs) {
+    QuantArgs D;
+    D.n_atoms = qs.n_quantiles;
+    D.np = dist_np(qs.n_quantiles);
+    D.nh = 4 * D.np;
+    D.kappa = (float)qs.kappa;
+    const DistScratch s = make_dist_scratch(d, D.np);
+    char* p = static_cast<char*>(qs.scratch);
+    D.m = p ? reinterpret_cast<float*>(p + s.m) : nullptr;
+    D.h2 = p ? reinterpret_cast<float*>(p + s.h2) : nullptr;
+    D.dx = p ? reinterpret_cast<float*>(p + s.dx) : nullptr;
+    return D;
+}
+// The expected value Q = (sum_i x_i, fp32 adds in i order) / N
+__device__ __forceinline__ float quantile_mean(const float* x, int n) {
+    float s = 0.f;
+    for (int i = 0; i < n; ++i) s = __fadd_rn(s, x[i]);
+    return __fdiv_rn(s, (float)n);
+}
+
 // Tile geometry of the fused MLP kernels for hidden width H (DESIGN.md "K3/K4 tiling").
 // A CTA owns BM batch rows and all H output columns; each thread an 8x8 register tile.
 template <int H>
@@ -451,5 +478,11 @@ int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_a
                             cudaStream_t s);
 int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
                     const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
+int launch_learn_quantile(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                          const dmdqn_quantile& qs, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                          cudaStream_t s);
+int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_quantile& qs, const float* obs, int32_t stride,
+                        const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
+                        cudaStream_t s);
 
 }  // namespace dmdqn

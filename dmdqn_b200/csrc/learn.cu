@@ -937,17 +937,52 @@ __device__ __forceinline__ void dist_project(float* m, const float* x, float mx,
     }
 }
 
-// Distributional K3: online and target trunk + head on s', expected Q, a*, the projected target distribution -> D.m.
+// The head-specific parts of the distributional kernels, chosen by the argument type: DistArgs (C51) or QuantArgs
+// (QR-DQN, include/dmdqn_b200.h dmdqn_quantile).  head_prologue: the C51 support into zs.
 template <int H>
-__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const LearnArgs A, const DistArgs D) {
+__device__ __forceinline__ void head_prologue(const DistSmem<H>& S, const DistArgs& D) {
+    for (int j = threadIdx.x; j < D.n_atoms; j += Tile<H>::NT) S.zs[j] = dist_z(D.v_min, D.dz64, j);
+}
+template <int H>
+__device__ __forceinline__ void head_prologue(const DistSmem<H>&, const QuantArgs&) {}
+
+// head_q: the expected Q of one action's Np head outputs x
+template <int H>
+__device__ __forceinline__ float head_q(const float* x, const DistSmem<H>& S, const DistArgs& D) {
+    float mx, s;
+    return dist_expect(x, D.n_atoms, S.zs, mx, s);
+}
+template <int H>
+__device__ __forceinline__ float head_q(const float* x, const DistSmem<H>&, const QuantArgs& D) {
+    return quantile_mean(x, D.n_atoms);
+}
+
+// head_target: the target of one row into m[0..Np) from the target network's outputs x of a*, return R, discount d
+template <int H>
+__device__ __forceinline__ void head_target(float* m, const float* x, const DistSmem<H>& S, float R, float d,
+                                            const DistArgs& D) {
+    float mx, s;
+    dist_stats(x, D.n_atoms, mx, s);
+    dist_project(m, x, mx, s, S.zs, R, d, D);
+}
+template <int H>
+__device__ __forceinline__ void head_target(float* m, const float* x, const DistSmem<H>&, float R, float d,
+                                            const QuantArgs& D) {
+    for (int j = 0; j < D.np; ++j) m[j] = j < D.n_atoms ? __fadd_rn(R, __fmul_rn(d, x[j])) : 0.f;
+}
+
+// Distributional K3: online and target trunk + head on s', expected Q, a*, the head's target (C51: the projected
+// distribution, QR-DQN: the target samples) -> D.m.
+template <int H, class DA>
+__device__ __forceinline__ void dist_target_body(const LearnArgs& A, const DA& D) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
     const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
     if (!A.active[g]) return;
-    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, n = D.n_atoms, np = D.np;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, np = D.np;
     DistSmem<H> S(smem, Dp, D.nh);
     const Coord<H> c;
-    for (int j = threadIdx.x; j < n; j += T::NT) S.zs[j] = dist_z(D.v_min, D.dz64, j);
+    head_prologue<H>(S, D);
     gather_tile<H>(S.Xs, S.ldx, A.rp.next_obs, A.nrows + (size_t)g * B, r0, B, Dp);
 
     float acc[8][8];
@@ -962,8 +997,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const Learn
         float* qs = pass == 0 ? S.qs0 : S.qs1;
         for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {   // one thread per (row, action)
             const int i = f >> 2, a = f & 3;
-            float mx, s;
-            qs[f] = a < nA && r0 + i < B ? dist_expect(S.Ls + i * S.ldl + a * np, n, S.zs, mx, s) : 0.f;
+            qs[f] = a < nA && r0 + i < B ? head_q<H>(S.Ls + i * S.ldl + a * np, S, D) : 0.f;
         }
         __syncthreads();
     }
@@ -978,9 +1012,7 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const Learn
             if (qa[k] > qa[best]) best = k;
         const size_t o = (size_t)g * B + gr;
         const float* x = S.Ls + i * S.ldl + best * np;
-        float mx, s;
-        dist_stats(x, n, mx, s);
-        dist_project(S.Hs2 + i * T::LDH, x, mx, s, S.zs, A.r_hat[o], A.disc_b[o], D);
+        head_target<H>(S.Hs2 + i * T::LDH, x, S, A.r_hat[o], A.disc_b[o], D);
         for (int k = 0; k < 4; ++k) {
             A.q_next[o * 4 + k] = qo[k];
             A.tq_all[o * 4 + k] = qt[k];
@@ -993,32 +1025,26 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const Learn
     }
 }
 
-// Distributional K4a: forward on s (h1 -> workspace, h2 -> scratch), every action's expected Q, the cross-entropy of a_i
-// against m, the logit gradient dX (-> scratch), dh2 = (dX W3^T) * relu'(h2), dh1, and the per-tile partials.
 template <int H>
-__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const LearnArgs A, const DistArgs D) {
+__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const LearnArgs A, const DistArgs D) {
+    dist_target_body<H>(A, D);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) quantile_target_kernel(const LearnArgs A, const QuantArgs D) {
+    dist_target_body<H>(A, D);
+}
+
+// head_loss: the per-row loss of the online kernel over the logits Ls of the tile.  It leaves every action's expected Q
+// in qs0 (and q_all), the taken action in as, the loss term in terms (the priority stored), and the logit gradient in
+// Ls: the taken action's block holds it, every other block is 0.  Ends synced.
+// C51: one thread per (row, action); the thread of the taken action also forms the cross-entropy and the gradient of
+// its Np logits in place.
+template <int H>
+__device__ __forceinline__ void head_loss(const LearnArgs& A, const DistArgs& D, const DistSmem<H>& S, int r0, size_t sb,
+                                          const int32_t* rows) {
     using T = Tile<H>;
-    extern __shared__ __align__(16) float smem[];
-    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
-    if (!A.active[g]) return;
-    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, n = D.n_atoms, np = D.np, nh = D.nh;
-    DistSmem<H> S(smem, Dp, nh);
-    const Coord<H> c;
-    const int32_t* rows = A.rows + (size_t)g * B;
-    const float* P = A.nets.theta + (size_t)g * A.L.stride;
-    const size_t sb = (size_t)g * B;
-    for (int j = threadIdx.x; j < n; j += T::NT) S.zs[j] = dist_z(D.v_min, D.dz64, j);
-    gather_tile<H>(S.Xs, S.ldx, A.rp.obs, rows, r0, B, Dp);
-
-    float acc[8][8];
-    gemm_rowA<H, false>(acc, c, S.Xs, S.ldx, P + A.L.w1, H, Dp, S.Ws);
-    store_relu<H>(acc, c, P + A.L.b1, S.Hs1, A.h1 + sb * H, r0, B);
-    gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
-    store_relu<H>(acc, c, P + A.L.b2, S.Hs2, D.h2 + sb * H, r0, B);
-    dist_head<H>(acc, c, S, P, A.L, nh);
-
-    // one thread per (row, action): expected Q; the thread of the taken action also the loss term, the priority and the
-    // gradient of its Np logits (in place); every other block of the row's logit gradient is 0
+    const int B = A.d.batch, nA = A.d.n_actions, n = D.n_atoms, np = D.np;
     for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {
         const int i = f >> 2, a = f & 3, gr = r0 + i;
         const bool row_ok = gr < B;
@@ -1058,6 +1084,108 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const Learn
         S.qs0[f] = q;
     }
     __syncthreads();
+}
+
+// QR-DQN: the N^2 pair terms of a row are spread over one thread per (row, quantile i), each summing over j.  While
+// they run, the row's block after the taken action's holds T and the block two after it the per-quantile loss sums
+// (both are 0 in the gradient, and are cleared again by the row pass that forms L_r in i order).
+template <int H>
+__device__ __forceinline__ void head_loss(const LearnArgs& A, const QuantArgs& D, const DistSmem<H>& S, int r0, size_t sb,
+                                          const int32_t* rows) {
+    using T = Tile<H>;
+    const int B = A.d.batch, nA = A.d.n_actions, n = D.n_atoms, np = D.np;
+    for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {   // one thread per (row, action)
+        const int i = f >> 2, a = f & 3, gr = r0 + i;
+        const bool row_ok = gr < B;
+        const int ai = row_ok ? A.act_b[sb + gr] : 0;
+        float* x = S.Ls + i * S.ldl + a * np;
+        const float q = row_ok && a < nA ? quantile_mean(x, n) : 0.f;
+        if (row_ok) A.q_all[(sb + gr) * 4 + a] = q;
+        if (a != ai) {
+            const bool tb = row_ok && a == ((ai + 1) & 3);
+            const float* t = D.m + (sb + (tb ? gr : 0)) * np;
+            for (int j = 0; j < np; ++j) x[j] = tb ? t[j] : 0.f;
+        }
+        if (a == 0) S.as[i] = ai;
+        S.qs0[f] = q;
+    }
+    __syncthreads();
+    const float k = D.kappa;
+    for (int f = threadIdx.x; f < T::BM * np; f += T::NT) {   // one thread per (row, quantile i)
+        const int i = f / np, qi = f % np, gr = r0 + i, ai = S.as[i];
+        float* row = S.Ls + i * S.ldl;
+        float g = 0.f, l = 0.f;
+        if (gr < B && qi < n) {
+            const float* t = row + ((ai + 1) & 3) * np;
+            const float th = row[ai * np + qi];
+            const float tau = (float)((2.0 * qi + 1.0) / (2.0 * n)), omt = __fsub_rn(1.f, tau);
+            float gs = 0.f;
+            for (int j = 0; j < n; ++j) {
+                const float u = __fsub_rn(t[j], th);
+                const float w = u < 0.f ? omt : tau;
+                float rho, dr;
+                if (k > 0.f) {
+                    const float au = fabsf(u);
+                    rho = __fmul_rn(w, au <= k ? __fdiv_rn(__fmul_rn(0.5f, __fmul_rn(u, u)), k) : __fsub_rn(au, __fmul_rn(0.5f, k)));
+                    dr = __fdiv_rn(__fmul_rn(-w, fminf(fmaxf(u, -k), k)), k);
+                } else {
+                    rho = __fmul_rn(w, fabsf(u));
+                    dr = u > 0.f ? -w : (u < 0.f ? w : 0.f);
+                }
+                l = __fadd_rn(l, rho);
+                gs = __fadd_rn(gs, dr);
+            }
+            const float wi = A.per ? A.is_w[sb + gr] : 1.f;
+            g = __fdiv_rn(__fmul_rn(wi, __fdiv_rn(gs, (float)n)), (float)A.loss_batch);
+        }
+        row[ai * np + qi] = g;
+        row[((ai + 2) & 3) * np + qi] = l;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < T::BM; i += T::NT) {       // one thread per row: L_r, the loss term, the priority
+        const int gr = r0 + i, ai = S.as[i];
+        float* t = S.Ls + i * S.ldl + ((ai + 1) & 3) * np;
+        float* ls = S.Ls + i * S.ldl + ((ai + 2) & 3) * np;
+        float L = 0.f;
+        for (int j = 0; j < n; ++j) L = __fadd_rn(L, ls[j]);
+        for (int j = 0; j < np; ++j) t[j] = ls[j] = 0.f;
+        float term = 0.f;
+        if (gr < B) {
+            L = __fdiv_rn(L, (float)n);
+            if (A.per) per_store_priority(A, rows[gr], L);
+            term = __fmul_rn(A.per ? A.is_w[sb + gr] : 1.f, L);
+        }
+        S.terms[i] = term;
+    }
+    __syncthreads();
+}
+
+// Distributional K4a: forward on s (h1 -> workspace, h2 -> scratch), every action's expected Q, the head's loss (C51:
+// the cross-entropy of a_i against m, QR-DQN: the quantile Huber loss against T), the logit gradient dX (-> scratch),
+// dh2 = (dX W3^T) * relu'(h2), dh1, and the per-tile partials.
+template <int H, class DA>
+__device__ __forceinline__ void dist_online_body(const LearnArgs& A, const DA& D) {
+    using T = Tile<H>;
+    extern __shared__ __align__(16) float smem[];
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
+    if (!A.active[g]) return;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, nh = D.nh;
+    DistSmem<H> S(smem, Dp, nh);
+    const Coord<H> c;
+    const int32_t* rows = A.rows + (size_t)g * B;
+    const float* P = A.nets.theta + (size_t)g * A.L.stride;
+    const size_t sb = (size_t)g * B;
+    head_prologue<H>(S, D);
+    gather_tile<H>(S.Xs, S.ldx, A.rp.obs, rows, r0, B, Dp);
+
+    float acc[8][8];
+    gemm_rowA<H, false>(acc, c, S.Xs, S.ldx, P + A.L.w1, H, Dp, S.Ws);
+    store_relu<H>(acc, c, P + A.L.b1, S.Hs1, A.h1 + sb * H, r0, B);
+    gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
+    store_relu<H>(acc, c, P + A.L.b2, S.Hs2, D.h2 + sb * H, r0, B);
+    dist_head<H>(acc, c, S, P, A.L, nh);
+    head_loss<H>(A, D, S, r0, sb, rows);
+
     const size_t pt = (size_t)g * A.ws_tiles + rt;   // partial slot of this (network, row tile)
     if (threadIdx.x == 0) {                          // per-tile loss / metric partials, rows in order
         float ls = 0.f, qsum = 0.f, qsq = 0.f, hist[4] = {0.f, 0.f, 0.f, 0.f};
@@ -1135,6 +1263,16 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const Learn
         for (int i = 0; i < T::BM; ++i) s += S.Hs1[i * T::LDH + j];
         A.part_b1[pt * H + j] = s;
     }
+}
+
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const LearnArgs A, const DistArgs D) {
+    dist_online_body<H>(A, D);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) quantile_online_kernel(const LearnArgs A, const QuantArgs D) {
+    dist_online_body<H>(A, D);
 }
 
 // Distributional K4b, gradients only (A.grads): dW2 = h1^T dh2, dW1 = s^T dh1 and dW3 = h2^T dX (column slabs of H) tiles
@@ -1259,22 +1397,27 @@ __global__ void __launch_bounds__(Tile<H>::NT) dist_wgrad_kernel(const LearnArgs
     }
 }
 
-template <int H>
-int launch_learn_dist_h(const LearnArgs& A, const DistArgs& D, cudaStream_t s) {
+// The target and online kernels of the head of DA (C51 or QR-DQN), then dist_wgrad_kernel on Dw, the same head width
+// and scratch as DistArgs.
+template <int H, class DA>
+int launch_learn_dist_h(const LearnArgs& A, const DA& D, const DistArgs& Dw, cudaStream_t s) {
     using T = Tile<H>;
+    constexpr bool qr = std::is_same<DA, QuantArgs>::value;
+    const auto target = [] { if constexpr (qr) return quantile_target_kernel<H>; else return dist_target_kernel<H>; }();
+    const auto online = [] { if constexpr (qr) return quantile_online_kernel<H>; else return dist_online_kernel<H>; }();
     const size_t smem = DistSmem<H>::bytes(A.d.obs_stride, D.nh);
     const size_t smem_w = sizeof(float) * 2 * T::KC * ((T::BM + 4) + T::LDW);
     static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_target_kernel<H>), smem, cfg_t)) return rc;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_online_kernel<H>), smem, cfg_o)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(target), smem, cfg_t)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(online), smem, cfg_o)) return rc;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(dist_wgrad_kernel<H>), smem_w, cfg_w)) return rc;
     const int grid = A.d.n_nets * A.ws_tiles;
-    dist_target_kernel<H><<<grid, T::NT, smem, s>>>(A, D);
+    target<<<grid, T::NT, smem, s>>>(A, D);
     DMDQN_CUDA(cudaGetLastError());
-    dist_online_kernel<H><<<grid, T::NT, smem, s>>>(A, D);
+    online<<<grid, T::NT, smem, s>>>(A, D);
     DMDQN_CUDA(cudaGetLastError());
     const int per_net = H / T::BM + (A.d.obs_stride + T::BM - 1) / T::BM + (H / T::BM) * ((D.nh + H - 1) / H) + 1;
-    dist_wgrad_kernel<H><<<A.d.n_nets * per_net, T::NT, smem_w, s>>>(A, D);
+    dist_wgrad_kernel<H><<<A.d.n_nets * per_net, T::NT, smem_w, s>>>(A, Dw);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
@@ -1415,10 +1558,29 @@ int launch_learn_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_
     const DistArgs D = make_dist_args(d, ds);
     A.L = make_layout_dist(d.obs_stride, d.hidden, D.np);
     switch (d.hidden) {
-        case 64: return launch_learn_dist_h<64>(A, D, s);
-        case 128: return launch_learn_dist_h<128>(A, D, s);
-        case 256: return launch_learn_dist_h<256>(A, D, s);
-        case 512: return launch_learn_dist_h<512>(A, D, s);
+        case 64: return launch_learn_dist_h<64>(A, D, D, s);
+        case 128: return launch_learn_dist_h<128>(A, D, D, s);
+        case 256: return launch_learn_dist_h<256>(A, D, D, s);
+        case 512: return launch_learn_dist_h<512>(A, D, D, s);
+    }
+    set_error("unsupported hidden width %d", d.hidden);
+    return DMDQN_ERR_ARG;
+}
+
+int launch_learn_quantile(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                          const dmdqn_quantile& qs, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                          cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    const QuantArgs Q = make_quantile_args(d, qs);
+    A.L = make_layout_dist(d.obs_stride, d.hidden, Q.np);
+    DistArgs D = {};                                 // what dist_wgrad_kernel reads: the head width and the scratch
+    D.n_atoms = Q.n_atoms; D.np = Q.np; D.nh = Q.nh;
+    D.m = Q.m; D.h2 = Q.h2; D.dx = Q.dx;
+    switch (d.hidden) {
+        case 64: return launch_learn_dist_h<64>(A, Q, D, s);
+        case 128: return launch_learn_dist_h<128>(A, Q, D, s);
+        case 256: return launch_learn_dist_h<256>(A, Q, D, s);
+        case 512: return launch_learn_dist_h<512>(A, Q, D, s);
     }
     set_error("unsupported hidden width %d", d.hidden);
     return DMDQN_ERR_ARG;

@@ -49,6 +49,9 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # distributional Q-learning (C51, Bellemare et al. 2017): a categorical return distribution over num_atoms atoms of
     # [v_min, v_max] per action, projected Bellman targets and a cross-entropy loss
     "distributional": False, "num_atoms": 51, "v_min": -10.0, "v_max": 10.0,
+    # quantile regression DQN (QR-DQN, Dabney et al. 2018): num_quantiles learned return quantiles per action at the
+    # midpoints (2i + 1) / 2N, the quantile Huber loss with threshold quantile_kappa (0: the pure quantile loss)
+    "quantile": False, "num_quantiles": 50, "quantile_kappa": 1.0,
 }
 
 
@@ -78,6 +81,37 @@ def dist_config(cfg: dict) -> dict:
     if cfg["loss"] != "mse":
         raise ValueError(f"loss={cfg['loss']!r}: distributional networks minimise the cross-entropy of the projected target; "
                          "the loss key does not apply (leave it at mse)")
+    cfg["precision"] = "fp32"
+    return cfg
+
+
+def quantile_config(cfg: dict) -> dict:
+    """Validate the quantile keys of ``cfg`` and resolve its precision (in place; returns ``cfg``).  With ``quantile: true``
+    the learn step runs the fp32 (FFMA) kernels only, so ``precision: auto`` becomes fp32 and an explicit tcgen05
+    precision, C51, dueling heads, noisy networks and the Huber loss key are refused."""
+    if not isinstance(cfg["quantile"], (bool, np.bool_)):
+        raise ValueError(f"quantile={cfg['quantile']!r}: must be true or false")
+    if not cfg["quantile"]:
+        return cfg
+    n = cfg["num_quantiles"]
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 2 <= n <= N.DIST_MAX_ATOMS:
+        raise ValueError(f"num_quantiles={n!r}: must be an integer in [2, {N.DIST_MAX_ATOMS}]")
+    k = cfg["quantile_kappa"]
+    if isinstance(k, bool) or not isinstance(k, numbers.Real) or not math.isfinite(k) or k < 0:
+        raise ValueError(f"quantile_kappa={k!r}: must be a finite number >= 0 (0 = the pure quantile loss)")
+    if cfg["distributional"]:
+        raise ValueError("quantile=true cannot be combined with distributional=true: QR-DQN and C51 are two different "
+                         "distributional heads; choose one")
+    if cfg["precision"] not in ("auto", "fp32"):
+        raise ValueError(f"precision={cfg['precision']!r}: quantile networks run the fp32 (FFMA) learn path only; the "
+                         "tcgen05 quantile kernels are not built yet (use precision: auto or fp32)")
+    if cfg["dueling"]:
+        raise ValueError("quantile=true cannot be combined with dueling=true yet: dueling quantile heads are not implemented")
+    if cfg["noisy"]:
+        raise ValueError("quantile=true cannot be combined with noisy=true yet: noisy quantile heads are not implemented")
+    if cfg["loss"] != "mse":
+        raise ValueError(f"loss={cfg['loss']!r}: quantile networks minimise the quantile Huber loss, whose threshold is "
+                         "quantile_kappa; the loss key does not apply (leave it at mse)")
     cfg["precision"] = "fp32"
     return cfg
 
@@ -166,8 +200,14 @@ class AgentGroup:
             raise ValueError("noisy=true cannot be combined with global_clipnorm yet: the global norm over the mean and the "
                              "sigma gradients is not implemented")
         dist_config(cfg)
-        self.distributional = bool(cfg["distributional"])
+        quantile_config(cfg)
+        self.distributional = bool(cfg["distributional"])     # C51
         self.num_atoms = int(cfg["num_atoms"]) if self.distributional else 0
+        self.quantile = bool(cfg["quantile"])                 # QR-DQN
+        self.num_quantiles = int(cfg["num_quantiles"]) if self.quantile else 0
+        # either head uses the distributional layout W3[H][4 * Np] | b3[4 * Np] of N = head_atoms atoms or quantiles
+        self.dist_layout = self.distributional or self.quantile
+        self.head_atoms = self.num_atoms or self.num_quantiles
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -186,10 +226,10 @@ class AgentGroup:
         if self.dueling:        # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
             self.layout = N.DuelingLayout()
             N.check(self.lib.dmdqn_param_layout_dueling(C.byref(self.dims), C.byref(self.layout)))
-        elif self.distributional:   # the head W3[H][4 * Np] | b3[4 * Np]
+        elif self.dist_layout:      # the head W3[H][4 * Np] | b3[4 * Np]
             self.layout = N.Layout()
-            N.check(self.lib.dmdqn_param_layout_dist(C.byref(self.dims), self.num_atoms, C.byref(self.layout)))
-            self.atom_stride = (self.num_atoms + 3) // 4 * 4
+            N.check(self.lib.dmdqn_param_layout_dist(C.byref(self.dims), self.head_atoms, C.byref(self.layout)))
+            self.atom_stride = (self.head_atoms + 3) // 4 * 4
         else:
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
@@ -228,7 +268,7 @@ class AgentGroup:
             # gradient clipping: the raw gradient blocks of a step and each network's norm before clipping (last step)
             self.grads = torch.zeros_like(self.theta) if self.global_clipnorm is not None else None
             self.grad_norms = torch.zeros((g,), dtype=torch.float32, device=dev) if self.global_clipnorm is not None else None
-            if self.distributional:     # the gradient block between dmdqn_learn_grads_dist and dmdqn_adam_apply_dist
+            if self.dist_layout:        # the gradient block between the dist / quantile learn_grads and dmdqn_adam_apply_dist
                 self.grads = torch.zeros_like(self.theta)
             if self.noisy:      # sigma with its target and moments, the effective blocks, the gradient and the noise record
                 self.sigma, self.sigma_tgt = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
@@ -262,12 +302,16 @@ class AgentGroup:
         self.nets = N.Nets(_ptr(self.theta), _ptr(self.theta_tgt), _ptr(self.adam_m), _ptr(self.adam_v),
                            _ptr(self.learn_step))
         self.noisy_ptrs = N.Noisy(*(_ptr(getattr(self, k)) for k in self._NOISY_PTRS)) if self.noisy else None
-        self.dist_scratch, self.dist = None, None
-        if self.distributional:     # per group, like the workspace: what the distributional kernels of one step pass on
+        self.dist_scratch, self.dist, self.qr = None, None, None
+        if self.dist_layout:        # per group, like the workspace: what the distributional kernels of one step pass on
             nbytes = C.c_size_t()
-            N.check(self.lib.dmdqn_dist_scratch_bytes(C.byref(self.dims), self.num_atoms, C.byref(nbytes)))
+            N.check(self.lib.dmdqn_dist_scratch_bytes(C.byref(self.dims), self.head_atoms, C.byref(nbytes)))
             self.dist_scratch = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
-            self.dist = N.Dist(self.num_atoms, float(cfg["v_min"]), float(cfg["v_max"]), _ptr(self.dist_scratch), nbytes.value)
+            if self.quantile:
+                self.qr = N.Quantile(self.num_quantiles, float(cfg["quantile_kappa"]), _ptr(self.dist_scratch), nbytes.value)
+            else:
+                self.dist = N.Dist(self.num_atoms, float(cfg["v_min"]), float(cfg["v_max"]), _ptr(self.dist_scratch),
+                                   nbytes.value)
         nbytes = C.c_size_t()
         N.check(self.lib.dmdqn_workspace_bytes(C.byref(self.dims), C.byref(nbytes)))
         self.workspace = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
@@ -324,8 +368,8 @@ class AgentGroup:
         blk[L.b1:L.b1 + H] = b1
         blk[L.w2:L.w2 + H * H] = w2.reshape(-1)
         blk[L.b2:L.b2 + H] = b2
-        if getattr(self, "distributional", False):     # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
-            n, npad = self.num_atoms, self.atom_stride
+        if getattr(self, "dist_layout", False):     # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
+            n, npad = self.head_atoms, self.atom_stride
             blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n] = w3.reshape(H, A, n)
             blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n] = b3.reshape(A, n)
             return blk
@@ -341,8 +385,8 @@ class AgentGroup:
         blk = blk.detach().cpu()
         out = [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
                blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(), blk[L.b2:L.b2 + H].clone()]
-        if getattr(self, "distributional", False):
-            n, npad = self.num_atoms, self.atom_stride
+        if getattr(self, "dist_layout", False):
+            n, npad = self.head_atoms, self.atom_stride
             return out + [blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
                           blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
         out += [blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(), blk[L.b3:L.b3 + A].clone()]
@@ -363,7 +407,7 @@ class AgentGroup:
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
         (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
-        head = self.action_size * self.num_atoms if self.distributional else self.action_size   # dist: W3 GlorotUniform over [H, A*N]
+        head = self.action_size * self.head_atoms if self.dist_layout else self.action_size   # dist: W3 GlorotUniform over [H, A*N]
         blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, self.dueling))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
@@ -471,6 +515,8 @@ class AgentGroup:
         args = (_ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream)
         if self.distributional:
             N.check(self.lib.dmdqn_act_dist(C.byref(self.dims), C.byref(nets), C.byref(self.dist), *args))
+        elif self.quantile:
+            N.check(self.lib.dmdqn_act_quantile(C.byref(self.dims), C.byref(nets), C.byref(self.qr), *args))
         elif self.noisy and noisy is not False and not target:
             N.check(self.lib.dmdqn_act_noisy(C.byref(self.dims), C.byref(nets), C.byref(self.noisy_ptrs), int(self.dueling),
                                              *args))
@@ -559,16 +605,27 @@ class AgentGroup:
         return states, actions, rewards, next_states, dones, active
 
     # ------------------------------------------------------------------ K1b+K3+K4 -------
+    def _dist_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
+        """The gradient half of a distributional-layout learn step: ``dmdqn_learn_grads_dist`` (C51) or
+        ``dmdqn_learn_grads_quantile`` (QR-DQN) into ``grads_ptr``, the loss mean over ``global_batch``."""
+        ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.quantile:
+            N.check(self.lib.dmdqn_learn_grads_quantile(C.byref(self.dims), C.byref(hp), C.byref(self.qr), C.byref(self.replay),
+                                                        C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
+                                                        _ptr(self.metrics), ws, nws, stream_ptr))
+        else:
+            N.check(self.lib.dmdqn_learn_grads_dist(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
+                                                    C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
+                                                    _ptr(self.metrics), ws, nws, stream_ptr))
+
     def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
         """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
         (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
         ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
         ws, nws = _ptr(self.workspace), self.workspace.numel()
-        if self.distributional:     # the C51 gradient, then Adam (clipped when global_clipnorm is set)
-            N.check(self.lib.dmdqn_learn_grads_dist(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
-                                                    C.byref(self.nets), draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads),
-                                                    _ptr(self.metrics), ws, nws, stream_ptr))
-            N.check(self.lib.dmdqn_adam_apply_dist(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.num_atoms,
+        if self.dist_layout:        # the C51 / QR-DQN gradient, then Adam (clipped when global_clipnorm is set)
+            self._dist_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
+            N.check(self.lib.dmdqn_adam_apply_dist(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.head_atoms,
                                                    _ptr(self.grads), self.global_clipnorm or 0.0, _ptr(self.grad_norms), ws, nws,
                                                    stream_ptr))
             return
@@ -657,7 +714,7 @@ class AgentGroup:
         """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
         one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy; the
         same with ``noisy`` set and the noisy learn calls."""
-        if self.global_clipnorm is None and not self.noisy and not self.distributional:
+        if self.global_clipnorm is None and not self.noisy and not self.dist_layout:
             N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                              C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
                                              _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
@@ -739,9 +796,12 @@ class AgentGroup:
                "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
         if self.noisy:           # factor vectors [network][set][record] and effective blocks of the last fold
             out["noise"], out["eff"], out["eff_tgt"] = self.noise, self.eff, self.eff_tgt
-        if self.distributional:  # the projected target distributions m [network][row][Np] of the last learn step
+        if self.dist_layout:     # the targets [network][row][Np] of the last learn step: C51's projected m, QR-DQN's T
             dv = N.DistViews()
-            N.check(self.lib.dmdqn_debug_dist(C.byref(self.dims), C.byref(self.dist), C.byref(dv)))
+            if self.quantile:
+                N.check(self.lib.dmdqn_debug_quantile(C.byref(self.dims), C.byref(self.qr), C.byref(dv)))
+            else:
+                N.check(self.lib.dmdqn_debug_dist(C.byref(self.dims), C.byref(self.dist), C.byref(dv)))
             sbase = self.dist_scratch.data_ptr()
             for key, ptr, width in (("target_dist", dv.target_dist, self.atom_stride), ("h2", dv.h2, self.hidden),
                                     ("dlogits", dv.dlogits, 4 * self.atom_stride)):
@@ -768,8 +828,8 @@ class AgentGroup:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
         tau = -1.0 if tau is None else float(tau)
-        if self.distributional:
-            N.check(self.lib.dmdqn_sync_target_dist(C.byref(self.dims), C.byref(self.nets), self.num_atoms, _ptr(mask_t), tau,
+        if self.dist_layout:
+            N.check(self.lib.dmdqn_sync_target_dist(C.byref(self.dims), C.byref(self.nets), self.head_atoms, _ptr(mask_t), tau,
                                                     self._stream))
             return
         if self.noisy:           # mu and sigma

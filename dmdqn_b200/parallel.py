@@ -207,7 +207,8 @@ class SharedParameterStep:
         step counters), the effective-weight gradients are all-reduced and ``dmdqn_noisy_adam_apply`` updates mu and sigma;
         ``fused=True`` is refused there, because the peer-memory kernel does not know sigma.  A ``distributional`` group takes
         the NCCL path as well: ``dmdqn_learn_grads_dist``, the all-reduce of its gradient block, then ``dmdqn_adam_apply_dist``
-        (clipped when ``global_clipnorm`` is set); ``fused=True`` is refused there."""
+        (clipped when ``global_clipnorm`` is set); ``fused=True`` is refused there.  A ``quantile`` (QR-DQN) group does the
+        same with ``dmdqn_learn_grads_quantile``."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
@@ -223,8 +224,11 @@ class SharedParameterStep:
         if grp.distributional and fused:
             raise ValueError("distributional=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the "
                              "distributional layout; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_dist path)")
+        if grp.quantile and fused:
+            raise ValueError("quantile=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the quantile "
+                             "head's layout; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_dist path)")
         if fused is None:
-            fused = clip is None and not grp.noisy and not grp.distributional and (world > 1 or exchange is not None)
+            fused = clip is None and not grp.noisy and not grp.dist_layout and (world > 1 or exchange is not None)
         if fused and exchange is None:
             rank = dist.get_rank(group) if world > 1 else 0
             exchange = PeerExchange(grp, rank, world).connect(group)
@@ -241,11 +245,8 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                if grp.distributional:
-                    N.check(grp.lib.dmdqn_learn_grads_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.dist),
-                                                           C.byref(grp.replay), C.byref(grp.nets), _ptr(d), None,
-                                                           int(global_batch), _ptr(out), _ptr(grp.metrics), _ptr(grp.workspace),
-                                                           grp.workspace.numel(), grp._stream))
+                if grp.dist_layout:             # C51 or QR-DQN
+                    grp._dist_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
                 elif grp.noisy:
                     N.check(grp.lib.dmdqn_learn_grads_noisy(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay),
                                                             C.byref(grp.nets), C.byref(grp.noisy_ptrs), _ptr(d), None,
@@ -276,8 +277,8 @@ class SharedParameterStep:
 
         def apply(g: torch.Tensor):
             with torch.cuda.device(grp.device):
-                if grp.distributional:          # clipped (the norm of the all-reduced block) when global_clipnorm is set
-                    N.check(grp.lib.dmdqn_adam_apply_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.num_atoms,
+                if grp.dist_layout:             # clipped (the norm of the all-reduced block) when global_clipnorm is set
+                    N.check(grp.lib.dmdqn_adam_apply_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.head_atoms,
                                                           _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),
                                                           grp.workspace.numel(), grp._stream))
                     return

@@ -42,6 +42,7 @@
  *   each mean summed left to right in fp32 and divided by A (IEEE division).  Advantage columns >= A keep gradient 0.
  *   distributional networks (C51; dmdqn_param_layout_dist, see dmdqn_dist below) widen the head to 4 * Np columns:
  *     W1 | b1 | W2 | b2 | W3[H][4 * Np] | b3[4 * Np] | pad
+ *   quantile networks (QR-DQN, see dmdqn_quantile below) use the same block with N quantiles in place of N atoms.
  */
 #ifndef DMDQN_B200_H
 #define DMDQN_B200_H
@@ -595,6 +596,64 @@ typedef struct dmdqn_dist_views {
     const float* target_dist; const float* h2; const float* dlogits;
 } dmdqn_dist_views;
 int dmdqn_debug_dist(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_dist_views* out);
+
+/* Quantile regression DQN (QR-DQN, Dabney, Rowland, Bellemare & Munos 2018), fp32 (FFMA) path only.  Each action's
+ * return is N = n_quantiles quantiles (2 <= N <= DMDQN_DIST_MAX_ATOMS) at the fixed midpoints
+ *   tau_i = (float)((2 i + 1) / (2.0 N))   (float64 division, then rounded)
+ * and the values of the quantiles are learned, so there is no support to choose.  The parameter block, its padding and
+ * the Adam range are those of dmdqn_dist with N atoms (dmdqn_param_layout_dist(dims, N)); column a * Np + i holds
+ * quantile i of action a.  After the head, every operation below is one rounded fp32 operation unless stated, and none
+ * is fused (no FMA).
+ * Head: theta_{a,i}(s) = h2 . W3[:, a*Np + i] + b3[a*Np + i] (the C51 logits, computed as C51 computes them), and
+ *   Q(s, a) = (sum_i theta_{a,i}, adds in i order from 0) / (float)N      (IEEE division; 0 for actions a >= A)
+ * Target of sampled row r (R, discount d and the bootstrap row as dmdqn_sample forms them, so n-step returns and done
+ * apply): a* = argmax of the online (double_dqn = 1) or the target (double_dqn = 0) network's Q at s', ties to the
+ * lowest index, and for j < N
+ *   T_j = R + d * theta^tgt_{a*, j}(s')   (product and sum rounded separately; not differentiated)
+ * Loss of row r with action a_r, k = (float)kappa: for each pair (i, j), theta_i = theta_{a_r,i}(s),
+ *   u = T_j - theta_i,  w = u < 0 ? 1 - tau_i : tau_i
+ *   k > 0:  rho = w * (|u| <= k ? (0.5 * (u * u)) / k : |u| - 0.5 * k),   drho = (-w * min(max(u, -k), k)) / k
+ *   k = 0:  rho = w * |u|,   drho = u > 0 ? -w : u < 0 ? w : 0
+ *   L_r = (sum_i (sum_j rho_ij, j order) in i order) / (float)N,   g_i = (sum_j drho_ij, j order) / (float)N
+ * every sum an fp32 add from 0.  The loss term is w_r * L_r with w_r the importance weight of prioritized replay (1
+ * otherwise), prioritized replay stores priority = (float)pow(L_r + per_eps, per_alpha) (the unweighted loss), and the
+ * gradient of column a_r * Np + i is (w_r * g_i) / loss_batch (0 for i >= N and for every other action's columns).
+ * hp->loss is not read.
+ * Metrics row: [0] the weighted batch-mean loss, [1] / [2] the mean and std of the online Q over a < A, the action
+ * histogram and the learned flag.  dmdqn_debug's q_all / q_next / tq_all hold expected Q values; y is not written.
+ *   kappa     the Huber threshold: finite and >= 0; 0 is the pure quantile loss (QR-DQN-0).
+ *   scratch   caller-owned device memory of at least dmdqn_dist_scratch_bytes(dims, N), 16-byte aligned, with the regions
+ *             of dmdqn_dist: the target samples T [n_nets][B][Np] (0 for j >= N), h2 and the logit gradient.
+ * Every call below refuses, before anything is launched: n_quantiles outside [2, 64], kappa negative, NaN or infinite,
+ * hp->precision other than DMDQN_PRECISION_FP32, hp->dueling != 0, NULL or misaligned pointers and a scratch smaller
+ * than the query returns.  Adam, clipping and the target sync are dmdqn_adam_apply_dist and dmdqn_sync_target_dist with
+ * n_atoms = N. */
+typedef struct dmdqn_quantile {
+    int32_t n_quantiles;
+    double kappa;
+    void* scratch;
+    size_t scratch_bytes;
+} dmdqn_quantile;
+
+/* One quantile learn step up to the gradient: the sample kernel of dmdqn_learn (learn_step, Adam scalars, n-step and
+ * prioritized rows), then the quantile target, online and (C51) weight-gradient kernels.  grads_out[n_nets][stride]
+ * receives dL/dtheta for every float of [0, b3 + 4 * Np) with the loss mean over global_batch (>= batch).  Finish the step
+ * with dmdqn_adam_apply_dist(..., N, ...). */
+int dmdqn_learn_grads_quantile(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_quantile* quantile,
+                               const dmdqn_replay* replay, const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask,
+                               int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
+                               size_t workspace_bytes, void* stream);
+
+/* dmdqn_act on quantile blocks: q_out holds the expected Q values (0 for a >= A), the action is their argmax under
+ * dmdqn_act's epsilon rule, and exploring agents skip the forward pass (their q_out rows are untouched).
+ * quantile->scratch and kappa are not used; the scratch may be NULL. */
+int dmdqn_act_quantile(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_quantile* quantile, const float* obs,
+                       int32_t obs_in_stride, const double* eps, const uint32_t* w_explore, const uint32_t* w_action,
+                       int32_t* actions_out, float* q_out, void* stream);
+
+/* The scratch's views after dmdqn_learn_grads_quantile: target_dist holds the target samples T [n_nets][B][Np]; h2 and
+ * dlogits are as in dmdqn_debug_dist. */
+int dmdqn_debug_quantile(const dmdqn_dims* dims, const dmdqn_quantile* quantile, dmdqn_dist_views* out);
 
 #ifdef __cplusplus
 }
