@@ -96,6 +96,23 @@ class Quantile(C.Structure):
 
 DIST_MAX_ATOMS = 64
 
+
+class Iqn(C.Structure):
+    _fields_ = [("n_tau", C.c_int32), ("n_tau_prime", C.c_int32), ("n_policy", C.c_int32), ("n_cos", C.c_int32),
+                ("kappa", C.c_double), ("row_base", C.c_int64), ("key", C.c_void_p), ("scratch", C.c_void_p),
+                ("scratch_bytes", C.c_size_t)]
+
+
+class IqnLayout(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "w2", "b2", "w3", "b3", "wphi", "bphi", "end", "stride")]
+
+
+class IqnViews(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("tau", "tau_prime", "target", "theta", "grad", "dh2", "dphi")]
+
+
+IQN_MAX_TAU, IQN_MAX_COS = 64, 128
+
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
 
 
@@ -170,6 +187,15 @@ SIGNATURES = {
     "dmdqn_act_quantile": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Quantile), _P, C.c_int32, _P, _P, _P, _P, _P,
                                      _P]),
     "dmdqn_debug_quantile": (C.c_int, [C.POINTER(Dims), C.POINTER(Quantile), C.POINTER(DistViews)]),
+    "dmdqn_param_layout_iqn": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(IqnLayout)]),
+    "dmdqn_iqn_scratch_bytes": (C.c_int, [C.POINTER(Dims), C.POINTER(Iqn), C.POINTER(C.c_size_t)]),
+    "dmdqn_learn_grads_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Iqn), C.POINTER(Replay),
+                                        C.POINTER(Nets), _P, _P, C.c_int32, _P, _P, _P, C.c_size_t, _P]),
+    "dmdqn_adam_apply_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P,
+                                       _P, C.c_size_t, _P]),
+    "dmdqn_act_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Iqn), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    "dmdqn_sync_target_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P]),
+    "dmdqn_debug_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Iqn), C.POINTER(IqnViews)]),
 }
 
 _lib = None

@@ -12,6 +12,8 @@
 // agents): an agent is a chain of two HBM latencies, three cluster barriers and serial reductions, so the number of
 // agents in flight matters more than the number of loads each thread keeps in flight.
 // Exploring agents skip the forward pass, as the reference does.
+#include <algorithm>
+
 #include <cooperative_groups.h>
 #include "common.cuh"
 
@@ -410,7 +412,134 @@ act_quantile_kernel(dmdqn_dims d, Layout L, int n_quantiles, const float* __rest
     }
 }
 
+// Implicit quantile networks (include/dmdqn_b200.h dmdqn_iqn): layer 1 as a column-split GEMV (h1 in every CTA), then CTA
+// `rank` forms phi of its H/4 columns at the K midpoints and broadcasts z = h1 * phi [K][H] over DSMEM; layer 2 is a small
+// GEMM per CTA (its H/4 columns for all K rows: every W2 row is loaded once per CTA and used for the K rows, FFMA in k
+// order), the head partials of its columns meet on rank 0, which adds them in rank order to b3, averages the K values of
+// each action in k order and takes the argmax.
+constexpr int kIqnActRows = 8;                       // K rows per thread of the layer-2 GEMM at H = 512 (K <= 64)
+template <int H>
+__global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads)
+act_iqn_kernel(dmdqn_dims d, Layout L, int64_t wphi, int64_t bphi, int K, int n_cos, const float* __restrict__ theta,
+               const float* __restrict__ obs, int stride, const double* __restrict__ eps, const uint32_t* __restrict__ w_explore,
+               const uint32_t* __restrict__ w_action, int32_t* __restrict__ actions, float* __restrict__ q_out) {
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int a = blockIdx.x / kActCluster, rank = (int)cluster.block_rank();
+    const bool explore = (double)w_explore[a] < eps[a] * 4294967296.0;
+    if (explore) {
+        if (threadIdx.x == 0 && rank == 0) actions[a] = (int32_t)__umulhi(w_action[a], (uint32_t)d.n_actions);
+        return;
+    }
+    constexpr int Hs = H / kActCluster, C4 = Hs / 4, RG = kActThreads / C4;
+    const int Dp = d.obs_stride, tw = max(n_cos, Hs);
+    float* xs = smem;                        // [Dp]
+    float* h1 = xs + Dp;                     // [H]
+    float* part = h1 + H;                    // [1024]: layer-1 partials, then rank 0's Q[4]
+    float* z = part + kActThreads * 4;       // [K][H]
+    float* tab = z + (size_t)K * H;          // [K][tw]: cosine features, then this CTA's h2 columns [K][Hs]
+    float* heads = tab + (size_t)K * tw;     // [4 ranks][K][4] on rank 0
+    const int net = d.n_nets == 1 ? 0 : a;
+    const float* P = theta + (size_t)net * L.stride;
+    for (int c = threadIdx.x; c < Dp; c += kActThreads) xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
+    for (int f = threadIdx.x; f < K * n_cos; f += kActThreads) tab[f] = iqn_cos(f % n_cos, iqn_midpoint(f / n_cos, K));
+    __syncthreads();
+    gemv_slice_loop(cluster, P + L.w1, P + L.b1, xs, h1, part, Dp, H, rank);
+
+    for (int f = threadIdx.x; f < K * Hs; f += kActThreads) {   // phi and z of this CTA's columns
+        const int k = f / Hs, col = rank * Hs + f % Hs;
+        float s = 0.f;
+        for (int m = 0; m < n_cos; ++m) s = fmaf(tab[k * n_cos + m], __ldg(P + wphi + (size_t)m * H + col), s);
+        const float zv = __fmul_rn(h1[col], fmaxf(s + __ldg(P + bphi + col), 0.f));
+#pragma unroll
+        for (int r = 0; r < kActCluster; ++r) cluster.map_shared_rank(z, r)[(size_t)k * H + col] = zv;
+    }
+    cluster.sync();
+
+    const int col4 = threadIdx.x % C4, rg = threadIdx.x / C4;
+    float4 acc[kIqnActRows];
+#pragma unroll
+    for (int t = 0; t < kIqnActRows; ++t) acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4* Wv = reinterpret_cast<const float4*>(P + L.w2 + rank * Hs) + col4;
+#pragma unroll 4
+    for (int m = 0; m < H; ++m) {
+        const float4 w = __ldg(Wv + (size_t)m * (H / 4));
+#pragma unroll
+        for (int t = 0; t < kIqnActRows; ++t) {
+            const int k = rg + t * RG;
+            if (t * RG < K && k < K) {
+                const float zv = z[(size_t)k * H + m];
+                acc[t].x = fmaf(zv, w.x, acc[t].x); acc[t].y = fmaf(zv, w.y, acc[t].y);
+                acc[t].z = fmaf(zv, w.z, acc[t].z); acc[t].w = fmaf(zv, w.w, acc[t].w);
+            }
+        }
+    }
+    const float4 b2 = __ldg(reinterpret_cast<const float4*>(P + L.b2 + rank * Hs) + col4);
+#pragma unroll
+    for (int t = 0; t < kIqnActRows; ++t) {
+        const int k = rg + t * RG;
+        if (k < K)
+            *reinterpret_cast<float4*>(tab + (size_t)k * Hs + col4 * 4) =
+                make_float4(fmaxf(acc[t].x + b2.x, 0.f), fmaxf(acc[t].y + b2.y, 0.f), fmaxf(acc[t].z + b2.z, 0.f),
+                            fmaxf(acc[t].w + b2.w, 0.f));
+    }
+    __syncthreads();
+    for (int f = threadIdx.x; f < K * 4; f += kActThreads) {    // head partial of this CTA's columns, column order
+        const int k = f >> 2, q = f & 3;
+        float s = 0.f;
+        for (int j = 0; j < Hs; ++j) s = fmaf(tab[k * Hs + j], __ldg(P + L.w3 + (size_t)(rank * Hs + j) * 4 + q), s);
+        cluster.map_shared_rank(heads, 0)[(rank * K + k) * 4 + q] = s;
+    }
+    cluster.sync();
+    if (rank != 0) return;
+    if (threadIdx.x < 4) {
+        const int q = threadIdx.x;
+        float sum = 0.f;
+        for (int k = 0; k < K; ++k) {
+            float v = __ldg(P + L.b3 + q);
+            for (int r = 0; r < kActCluster; ++r) v += heads[(r * K + k) * 4 + q];
+            sum = __fadd_rn(sum, v);
+        }
+        part[q] = q < d.n_actions ? __fdiv_rn(sum, (float)K) : 0.f;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int best = 0;                                   // ties -> lowest index
+        for (int k = 1; k < d.n_actions; ++k) if (part[k] > part[best]) best = k;
+        actions[a] = best;
+        if (q_out)
+            for (int k = 0; k < 4; ++k) q_out[(size_t)a * 4 + k] = part[k];
+    }
+}
+
 }  // namespace
+
+int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn& q, const float* obs, int32_t stride,
+                   const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s) {
+    const IqnLayout L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos);
+    const int K = q.n_policy, tw = std::max(q.n_cos, d.hidden / kActCluster);
+    const size_t smem = ((size_t)d.obs_stride + d.hidden + kActThreads * 4 + (size_t)K * d.hidden + (size_t)K * tw +
+                         (size_t)kActCluster * K * 4) * sizeof(float);
+    const dim3 grid(d.n_agents * kActCluster);
+    static size_t cfg[4][kMaxDevices] = {};
+    auto run = [&](auto kernel, size_t (&c)[kMaxDevices]) {
+        if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kernel), smem, c)) return rc;
+        kernel<<<grid, kActThreads, smem, s>>>(d, L.L, L.wphi, L.bphi, K, q.n_cos, nets.theta, obs, stride, eps, w1, w2, actions,
+                                               q_out);
+        return 0;
+    };
+    int rc = 0;
+    switch (d.hidden) {
+        case 64: rc = run(act_iqn_kernel<64>, cfg[0]); break;
+        case 128: rc = run(act_iqn_kernel<128>, cfg[1]); break;
+        case 256: rc = run(act_iqn_kernel<256>, cfg[2]); break;
+        case 512: rc = run(act_iqn_kernel<512>, cfg[3]); break;
+        default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
+    }
+    if (rc) return rc;
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
 
 int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
                     const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s) {

@@ -720,6 +720,128 @@ int dmdqn_debug_quantile(const dmdqn_dims* dims, const dmdqn_quantile* quantile,
     return DMDQN_OK;
 }
 
+// IQN calls (include/dmdqn_b200.h dmdqn_iqn): the counts, n_cos, kappa, row_base and, where the call reads them, the key and
+// the scratch; every check runs before anything is launched.
+static int check_n_cos(int32_t n_cos) {
+    DMDQN_CHECK_ARG(n_cos >= 4 && n_cos <= DMDQN_IQN_MAX_COS && n_cos % 4 == 0, "n_cos=%d must be a multiple of 4 in [4, %d]",
+                    n_cos, DMDQN_IQN_MAX_COS);
+    return DMDQN_OK;
+}
+
+static int check_iqn(const dmdqn_dims* dims, const dmdqn_iqn* q, bool learn) {
+    DMDQN_CHECK_ARG(q != nullptr, "iqn is NULL");
+    const int32_t counts[3] = {q->n_tau, q->n_tau_prime, q->n_policy};
+    const char* names[3] = {"n_tau", "n_tau_prime", "n_policy"};
+    for (int i = 0; i < 3; ++i)
+        DMDQN_CHECK_ARG(counts[i] >= 1 && counts[i] <= DMDQN_IQN_MAX_TAU, "%s=%d must be in [1, %d]", names[i], counts[i],
+                        DMDQN_IQN_MAX_TAU);
+    if (int rc = check_n_cos(q->n_cos)) return rc;
+    DMDQN_CHECK_ARG(isfinite(q->kappa) && q->kappa >= 0.0, "kappa=%g must be finite and >= 0", q->kappa);
+    DMDQN_CHECK_ARG(q->row_base >= 0, "row_base=%lld must be >= 0", (long long)q->row_base);
+    if (learn) {
+        DMDQN_CHECK_ARG(q->key != nullptr, "iqn: key is NULL");
+        DMDQN_CHECK_ARG(q->scratch && aligned16(q->scratch), "iqn: scratch is NULL or not 16-byte aligned");
+        const size_t need = make_iqn_scratch(*dims, q->n_tau, q->n_tau_prime, q->n_cos).total;
+        DMDQN_CHECK_ARG(q->scratch_bytes >= need, "iqn: scratch has %zu bytes, %zu needed", q->scratch_bytes, need);
+    }
+    return DMDQN_OK;
+}
+
+static int check_iqn_hp(const dmdqn_hparams* hp) {
+    DMDQN_CHECK_ARG(hp != nullptr, "iqn: hp is NULL");
+    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32, "precision=%d: IQN networks run the fp32 (FFMA) path only",
+                    hp->precision);
+    DMDQN_CHECK_ARG(hp->dueling == 0, "dueling=%d: dueling heads are not supported with IQN networks", hp->dueling);
+    return DMDQN_OK;
+}
+
+int dmdqn_param_layout_iqn(const dmdqn_dims* dims, int32_t n_cos, dmdqn_iqn_layout* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_n_cos(n_cos))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const IqnLayout q = make_layout_iqn(dims->obs_stride, dims->hidden, n_cos);
+    out->w1 = q.L.w1; out->b1 = q.L.b1; out->w2 = q.L.w2; out->b2 = q.L.b2; out->w3 = q.L.w3; out->b3 = q.L.b3;
+    out->wphi = q.wphi; out->bphi = q.bphi; out->end = q.L.end; out->stride = q.L.stride;
+    return DMDQN_OK;
+}
+
+int dmdqn_iqn_scratch_bytes(const dmdqn_dims* dims, const dmdqn_iqn* iqn, size_t* out_bytes) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_iqn(dims, iqn, false))) return rc;
+    DMDQN_CHECK_ARG(out_bytes != nullptr, "out_bytes is NULL");
+    *out_bytes = make_iqn_scratch(*dims, iqn->n_tau, iqn->n_tau_prime, iqn->n_cos).total;
+    return DMDQN_OK;
+}
+
+int dmdqn_learn_grads_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_iqn* iqn, const dmdqn_replay* replay,
+                          const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
+                          float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    if ((rc = check_iqn_hp(hp))) return rc;
+    if ((rc = check_iqn(dims, iqn, true))) return rc;
+    if ((rc = check_dist_nets(nets, true))) return rc;
+    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
+    return launch_learn_iqn(*dims, *hp, *replay, *nets, *iqn, metrics_out, (char*)workspace, w, grads_out, global_batch, s);
+}
+
+int dmdqn_adam_apply_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, int32_t n_cos,
+                         const float* grads, double global_clipnorm, float* norms_out, void* workspace, size_t workspace_bytes,
+                         void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_iqn_hp(hp))) return rc;
+    if ((rc = check_n_cos(n_cos))) return rc;
+    if ((rc = check_dist_nets(nets, true))) return rc;
+    DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_iqn: grads is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_clipnorm >= 0.0 && isfinite(global_clipnorm),
+                    "global_clipnorm=%g must be 0 (no clipping) or a positive finite number", global_clipnorm);
+    return launch_adam_apply_iqn(*dims, *hp, *nets, n_cos, grads, global_clipnorm, norms_out, (char*)workspace, w,
+                                 (cudaStream_t)stream);
+}
+
+int dmdqn_act_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_iqn* iqn, const float* obs, int32_t obs_in_stride,
+                  const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out, float* q_out,
+                  void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_iqn(dims, iqn, false))) return rc;
+    DMDQN_CHECK_ARG(nets && nets->theta && aligned16(nets->theta), "act_iqn: theta is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(obs && eps && w_explore && w_action && actions_out, "act_iqn: NULL argument");
+    DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
+    return launch_act_iqn(*dims, *nets, *iqn, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out,
+                          (cudaStream_t)stream);
+}
+
+int dmdqn_sync_target_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, int32_t n_cos, const uint8_t* mask, double tau,
+                          void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_n_cos(n_cos))) return rc;
+    if ((rc = check_dist_nets(nets, false))) return rc;
+    return launch_sync_target_iqn(*dims, *nets, n_cos, mask, tau, (cudaStream_t)stream);
+}
+
+int dmdqn_debug_iqn(const dmdqn_dims* dims, const dmdqn_iqn* iqn, dmdqn_iqn_views* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_iqn(dims, iqn, false))) return rc;
+    DMDQN_CHECK_ARG(iqn->scratch && aligned16(iqn->scratch), "iqn: scratch is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const IqnArgs Q = make_iqn_args(*dims, *iqn);
+    out->tau = Q.tau; out->tau_prime = Q.tau_p; out->target = Q.t; out->theta = Q.theta; out->grad = Q.grad;
+    out->dh2 = Q.h2; out->dphi = Q.phi;
+    return DMDQN_OK;
+}
+
 static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau, bool dueling,
                            void* stream) {
     int rc = validate_dims(dims);

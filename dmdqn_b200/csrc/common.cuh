@@ -254,6 +254,46 @@ __device__ __forceinline__ float quantile_mean(const float* x, int n) {
     return __fdiv_rn(s, (float)n);
 }
 
+// Implicit quantile networks (include/dmdqn_b200.h dmdqn_iqn).  The block is the plain one with the cosine embedding
+// Wphi[n_cos][H] | bphi[H] after b3; Adam covers all of it.
+struct IqnLayout {
+    Layout L;                         // L.end = bphi + H
+    int64_t wphi, bphi;
+};
+__host__ __device__ inline IqnLayout make_layout_iqn(int dp, int h, int n_cos) {
+    IqnLayout q;
+    q.L = make_layout(dp, h);
+    q.wphi = q.L.b3 + 4;
+    q.bphi = q.wphi + (int64_t)n_cos * h;
+    q.L.end = q.bphi + h;
+    q.L.stride = (q.L.end + 31) / 32 * 32;
+    return q;
+}
+// Fraction i of sampled row `row` (row_base + r), set 0 (tau) or 1 (tau') at step t: the top 23 bits of the first Philox
+// word, ((x >> 9) + 0.5) * 2^-23, exact in fp32 and strictly inside (0, 1).
+__host__ __device__ __forceinline__ float iqn_tau(uint64_t key, uint32_t row, uint32_t i, uint32_t t, int set) {
+    const uint4 w = philox4x32_10(make_uint4(row, i, t, 0x69716e00u | (uint32_t)set), make_uint2((uint32_t)key, (uint32_t)(key >> 32)));
+    return ((float)(w.x >> 9) + 0.5f) * 0x1p-23f;
+}
+// Midpoint k of K: (float)((2k + 1) / (2.0 K)), as QR-DQN forms its quantile fractions
+__host__ __device__ __forceinline__ float iqn_midpoint(int k, int K) { return (float)((2.0 * k + 1.0) / (2.0 * K)); }
+// Cosine feature m of fraction tau: cos(pi * m * tau) in float64, rounded to float
+__device__ __forceinline__ float iqn_cos(int m, float tau) { return (float)cos(3.141592653589793 * (double)m * (double)tau); }
+
+// The quantile Huber pair term of one (i, j) pair (include/dmdqn_b200.h dmdqn_quantile): u = T_j - theta_i, fraction tau_i
+// with omt = 1 - tau_i, k = (float)kappa.  rho -> the loss term, dr -> its derivative in theta_i.
+__device__ __forceinline__ void quantile_pair(float u, float tau, float omt, float k, float& rho, float& dr) {
+    const float w = u < 0.f ? omt : tau;
+    if (k > 0.f) {
+        const float au = fabsf(u);
+        rho = __fmul_rn(w, au <= k ? __fdiv_rn(__fmul_rn(0.5f, __fmul_rn(u, u)), k) : __fsub_rn(au, __fmul_rn(0.5f, k)));
+        dr = __fdiv_rn(__fmul_rn(-w, fminf(fmaxf(u, -k), k)), k);
+    } else {
+        rho = __fmul_rn(w, fabsf(u));
+        dr = u > 0.f ? -w : (u < 0.f ? w : 0.f);
+    }
+}
+
 // Tile geometry of the fused MLP kernels for hidden width H (DESIGN.md "K3/K4 tiling").
 // A CTA owns BM batch rows and all H output columns; each thread an 8x8 register tile.
 template <int H>
@@ -334,6 +374,62 @@ inline Workspace make_workspace(const dmdqn_dims& d) {
     return w;
 }
 
+// The caller-owned scratch of the IQN learn kernels, byte offsets (256-aligned).  Debug views are [n_nets][B][count]; the
+// per-(row, fraction) buffers are fraction-major per network, [n_nets][N][B][width], so that one pass of a row tile writes
+// rows of stride width and the weight-gradient GEMMs of network g run over its N * B consecutive rows.
+struct IqnScratch {
+    size_t tau, tau_p, t, theta, grad;    // [nb][N], [nb][N'], [nb][N'], [nb][N], [nb][N]
+    size_t h1n;                           // [2][nb][H]: h1 at s' of the online and the target network
+    size_t c;                             // [n_nets][N][B][n_cos]: cosine features of the sampled fractions at s
+    size_t z, h2, phi;                    // [n_nets][N][B][H]: z, h2 (then dh2), phi (then dphi) at s
+    size_t part_bphi;                     // [n_nets][T][H]: dbphi partials of the online kernel's row tiles
+    size_t total;
+};
+inline IqnScratch make_iqn_scratch(const dmdqn_dims& d, int n, int n_p, int n_cos) {
+    IqnScratch s;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t nb = (size_t)d.n_nets * d.batch, h = d.hidden;
+    const int tiles = row_tiles(d.batch, tile_bm(d.hidden));        // Workspace::tiles: part_bphi is indexed as part_b1
+    s.tau = take(nb * n * 4);
+    s.tau_p = take(nb * n_p * 4);
+    s.t = take(nb * n_p * 4);
+    s.theta = take(nb * n * 4);
+    s.grad = take(nb * n * 4);
+    s.h1n = take(2 * nb * h * 4);
+    s.c = take(nb * n * n_cos * 4);
+    s.z = take(nb * n * h * 4);
+    s.h2 = take(nb * n * h * 4);
+    s.phi = take(nb * n * h * 4);
+    s.part_bphi = take((size_t)d.n_nets * tiles * h * 4);
+    s.total = off;
+    return s;
+}
+// What the IQN kernels take beyond LearnArgs
+struct IqnArgs {
+    int n, n_p, k, n_cos, ncp;        // N, N', K, n_cos, n_cos rounded up to 16 (the cosine tile's used width)
+    float kappa;
+    int64_t row_base;
+    const uint64_t* key;
+    int64_t wphi, bphi;
+    float *tau, *tau_p, *t, *theta, *grad, *h1n, *c, *z, *h2, *phi, *part_bphi;
+};
+inline IqnArgs make_iqn_args(const dmdqn_dims& d, const dmdqn_iqn& q) {
+    IqnArgs Q;
+    Q.n = q.n_tau; Q.n_p = q.n_tau_prime; Q.k = q.n_policy; Q.n_cos = q.n_cos;
+    Q.ncp = (q.n_cos + 15) / 16 * 16;
+    Q.kappa = (float)q.kappa;
+    Q.row_base = q.row_base;
+    Q.key = q.key;
+    const IqnLayout L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos);
+    Q.wphi = L.wphi; Q.bphi = L.bphi;
+    const IqnScratch s = make_iqn_scratch(d, q.n_tau, q.n_tau_prime, q.n_cos);
+    char* p = static_cast<char*>(q.scratch);
+    auto at = [&](size_t o) { return p ? reinterpret_cast<float*>(p + o) : nullptr; };
+    Q.tau = at(s.tau); Q.tau_p = at(s.tau_p); Q.t = at(s.t); Q.theta = at(s.theta); Q.grad = at(s.grad);
+    Q.h1n = at(s.h1n); Q.c = at(s.c); Q.z = at(s.z); Q.h2 = at(s.h2); Q.phi = at(s.phi); Q.part_bphi = at(s.part_bphi);
+    return Q;
+}
 int validate_dims(const dmdqn_dims* d);
 
 constexpr int kAllStages = DMDQN_STAGE_SAMPLE | DMDQN_STAGE_TARGET | DMDQN_STAGE_ONLINE | DMDQN_STAGE_WGRAD;   // dmdqn_learn
@@ -484,5 +580,12 @@ int launch_learn_quantile(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
 int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_quantile& qs, const float* obs, int32_t stride,
                         const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
                         cudaStream_t s);
+int launch_learn_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                     const dmdqn_iqn& q, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch, cudaStream_t s);
+int launch_adam_apply_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_cos, const float* grads,
+                          double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
+int launch_sync_target_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, int n_cos, const uint8_t* mask, double tau, cudaStream_t s);
+int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn& q, const float* obs, int32_t stride,
+                   const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
 
 }  // namespace dmdqn

@@ -1121,17 +1121,8 @@ __device__ __forceinline__ void head_loss(const LearnArgs& A, const QuantArgs& D
             const float tau = (float)((2.0 * qi + 1.0) / (2.0 * n)), omt = __fsub_rn(1.f, tau);
             float gs = 0.f;
             for (int j = 0; j < n; ++j) {
-                const float u = __fsub_rn(t[j], th);
-                const float w = u < 0.f ? omt : tau;
                 float rho, dr;
-                if (k > 0.f) {
-                    const float au = fabsf(u);
-                    rho = __fmul_rn(w, au <= k ? __fdiv_rn(__fmul_rn(0.5f, __fmul_rn(u, u)), k) : __fsub_rn(au, __fmul_rn(0.5f, k)));
-                    dr = __fdiv_rn(__fmul_rn(-w, fminf(fmaxf(u, -k), k)), k);
-                } else {
-                    rho = __fmul_rn(w, fabsf(u));
-                    dr = u > 0.f ? -w : (u < 0.f ? w : 0.f);
-                }
+                quantile_pair(__fsub_rn(t[j], th), tau, omt, k, rho, dr);
                 l = __fadd_rn(l, rho);
                 gs = __fadd_rn(gs, dr);
             }
@@ -1422,6 +1413,601 @@ int launch_learn_dist_h(const LearnArgs& A, const DA& D, const DistArgs& Dw, cud
     return DMDQN_OK;
 }
 
+// ------------------------------------------------------------------------------------------
+// Implicit quantile networks, fp32 (include/dmdqn_b200.h dmdqn_iqn).  A CTA owns BM transitions of one network, as the
+// plain kernels do, and runs one pass per fraction: the BM rows of a pass are its transitions at that fraction, so every
+// pass is a [BM x H] x [H x H] layer-2 GEMM on z = h1 * phi(tau) (h1 computed once per transition and kept in the scratch)
+// with the plain head after it.  Midpoint passes share one phi vector across the rows; sampled passes form phi as a
+// [BM x n_cos] x [n_cos x H] GEMM on the rows' cosine features.
+// ------------------------------------------------------------------------------------------
+template <int H>
+struct IqnSmem {
+    using T = Tile<H>;
+    float *Cs, *Zs, *Ws, *th, *lr, *qs, *qsum, *terms, *tv, *cv, *phv;
+    int* as;
+    int ldc;
+    __device__ __forceinline__ IqnSmem(float* base, int Dp, int ncp, int n) {
+        ldc = max(Dp, ncp) + 4;
+        Cs = base;                               // gathered observations, then the cosine features [BM][ncp]
+        Zs = Cs + T::BM * ldc;                   // z, h2, dh2, dphi of the current pass
+        Ws = Zs + T::BM * T::LDH;
+        th = Ws + 2 * T::KC * T::LDW;            // [BM][N]: theta_i, then the gradients
+        lr = th + T::BM * n;                     // [BM][N]: per-fraction loss sums
+        qs = lr + T::BM * n;                     // [BM][4] head outputs of a pass
+        qsum = qs + T::BM * 4;                   // [BM][4] sums over the passes
+        terms = qsum + T::BM * 4;
+        tv = terms + T::BM;                      // [BM] the fraction of each row in this pass
+        cv = tv + T::BM;                         // [DMDQN_IQN_MAX_COS] cosine features of a midpoint
+        phv = cv + DMDQN_IQN_MAX_COS;            // [H] phi of a midpoint
+        as = reinterpret_cast<int*>(phv + H);
+    }
+    static size_t bytes(int Dp, int ncp, int n) {
+        return sizeof(float) * ((size_t)T::BM * (std::max(Dp, ncp) + 4) + (size_t)T::BM * T::LDH + 2 * (size_t)T::KC * T::LDW +
+                                2 * (size_t)T::BM * n + 12 * (size_t)T::BM + DMDQN_IQN_MAX_COS + H);
+    }
+};
+
+// acc = Cs[BM][ncp] x Wphi[n_cos][H]: gemm_rowA's FFMA order (k ascending) with the weight chunks staged by plain loads,
+// rows >= n_cos zero-filled (the cosine tile's columns >= n_cos are 0 too).  Ends synced.
+template <int H>
+__device__ __forceinline__ void gemm_phi(float (&acc)[8][8], const Coord<H>& c, const float* Cs, int ldc,
+                                         const float* __restrict__ W, int n_cos, float* Ws) {
+    using T = Tile<H>;
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+    for (int k0 = 0; k0 < n_cos; k0 += T::KC) {
+        for (int f = threadIdx.x; f < T::KC * H / 4; f += T::NT) {
+            const int kk = f / (H / 4), n4 = f % (H / 4);
+            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (k0 + kk < n_cos) v = __ldg(reinterpret_cast<const float4*>(W + (size_t)(k0 + kk) * H) + n4);
+            *reinterpret_cast<float4*>(Ws + kk * T::LDW + n4 * 4) = v;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < T::KC; kk += 4) {
+            float4 a[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) a[i] = *reinterpret_cast<const float4*>(Cs + c.row(i) * ldc + k0 + kk);
+#pragma unroll
+            for (int s = 0; s < 4; ++s) {
+                const float4 b0 = *reinterpret_cast<const float4*>(Ws + (kk + s) * T::LDW + c.col0(0));
+                const float4 b1 = *reinterpret_cast<const float4*>(Ws + (kk + s) * T::LDW + c.col0(1));
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const float av = s == 0 ? a[i].x : s == 1 ? a[i].y : s == 2 ? a[i].z : a[i].w;
+                    fma8(acc[i], av, b0, b1);
+                }
+            }
+        }
+        __syncthreads();
+    }
+}
+
+// The cosine features of the rows' fractions S.tv (rows past the batch: 0) into Cs, and to gc (row stride n_cos) if set
+template <int H>
+__device__ __forceinline__ void iqn_cos_tile(const IqnSmem<H>& S, const IqnArgs& Q, int r0, int B, float* gc) {
+    for (int f = threadIdx.x; f < Tile<H>::BM * Q.ncp; f += Tile<H>::NT) {
+        const int i = f / Q.ncp, m = f % Q.ncp;
+        float v = 0.f;
+        if (r0 + i < B && m < Q.n_cos) {
+            v = iqn_cos(m, S.tv[i]);
+            if (gc) gc[(size_t)(r0 + i) * Q.n_cos + m] = v;
+        }
+        S.Cs[i * S.ldc + m] = v;
+    }
+    __syncthreads();
+}
+
+// z = h1 * relu(acc + bphi) into Zs (h1: the rows' layer-1 outputs, row stride H; rows past the batch give 0); phi and z
+// also to gphi / gz (row stride H) when set
+template <int H>
+__device__ __forceinline__ void store_z(const float (&acc)[8][8], const Coord<H>& c, const float* __restrict__ bphi,
+                                        const float* h1, float* Zs, float* gphi, float* gz, int r0, int B) {
+    using T = Tile<H>;
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+        const int col = c.col0(half);
+        const float4 b = __ldg(reinterpret_cast<const float4*>(bphi + col));
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int row = c.row(i);
+            const bool ok = r0 + row < B;
+            float4 p, z;
+            p.x = fmaxf(acc[i][half * 4 + 0] + b.x, 0.f);
+            p.y = fmaxf(acc[i][half * 4 + 1] + b.y, 0.f);
+            p.z = fmaxf(acc[i][half * 4 + 2] + b.z, 0.f);
+            p.w = fmaxf(acc[i][half * 4 + 3] + b.w, 0.f);
+            const float4 h = ok ? *reinterpret_cast<const float4*>(h1 + (size_t)(r0 + row) * H + col) : make_float4(0.f, 0.f, 0.f, 0.f);
+            z.x = __fmul_rn(h.x, p.x); z.y = __fmul_rn(h.y, p.y); z.z = __fmul_rn(h.z, p.z); z.w = __fmul_rn(h.w, p.w);
+            *reinterpret_cast<float4*>(Zs + row * T::LDH + col) = z;
+            if (ok && gphi) *reinterpret_cast<float4*>(gphi + (size_t)(r0 + row) * H + col) = p;
+            if (ok && gz) *reinterpret_cast<float4*>(gz + (size_t)(r0 + row) * H + col) = z;
+        }
+    }
+}
+
+// One pass through layer 2 and the head of the z tile in Zs: head outputs -> S.qs; h2 -> gh2 (row stride H) if set.
+// Caller syncs before (Zs complete); ends synced.
+template <int H>
+__device__ __forceinline__ void iqn_layer2_head(float (&acc)[8][8], const Coord<H>& c, const IqnSmem<H>& S, const float* P,
+                                                const Layout& L, float* gh2, int r0, int B) {
+    gemm_rowA<H, false>(acc, c, S.Zs, Tile<H>::LDH, P + L.w2, H, H, S.Ws);
+    store_relu<H>(acc, c, P + L.b2, S.Zs, gh2, r0, B);
+    __syncthreads();
+    layer3<H>(S.Zs, P + L.w3, P + L.b3, S.qs, S.Ws);
+}
+
+// IQN K3: at s', layer 1 of the online (double DQN) and the target network, the K midpoint passes of the network that picks
+// a*, then the N' sampled passes of the target network: T, q_next, tq_all.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) iqn_target_kernel(const LearnArgs A, const IqnArgs Q) {
+    using T = Tile<H>;
+    extern __shared__ __align__(16) float smem[];
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
+    if (!A.active[g]) return;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions;
+    IqnSmem<H> S(smem, Dp, Q.ncp, 0);
+    const Coord<H> c;
+    const size_t sb = (size_t)g * B, nb = (size_t)A.d.n_nets * B;
+    const uint64_t key = Q.key[g];
+    const uint32_t step = (uint32_t)(A.nets.learn_step[g] - 1);     // learn_step before the sample kernel's increment
+    gather_tile<H>(S.Cs, S.ldc, A.rp.next_obs, A.nrows + sb, r0, B, Dp);
+
+    float acc[8][8];
+    const int na = A.double_dqn ? 0 : 1;            // the network that picks a*
+#pragma unroll 1
+    for (int net = na; net < 2; ++net) {
+        const float* P = (net ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride;
+        gemm_rowA<H, false>(acc, c, S.Cs, S.ldc, P + A.L.w1, H, Dp, S.Ws);
+        store_relu<H>(acc, c, P + A.L.b1, S.Zs, Q.h1n + ((size_t)net * nb + sb) * H, r0, B);
+    }
+    __syncthreads();
+
+    const float* Pa = (na ? A.nets.theta_tgt : A.nets.theta) + (size_t)g * A.L.stride;
+    const float* h1a = Q.h1n + ((size_t)na * nb + sb) * H;
+    for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) S.qsum[f] = 0.f;
+#pragma unroll 1
+    for (int k = 0; k < Q.k; ++k) {                 // midpoint passes: one phi vector for every row
+        const float tk = iqn_midpoint(k, Q.k);
+        for (int m = threadIdx.x; m < Q.n_cos; m += T::NT) S.cv[m] = iqn_cos(m, tk);
+        __syncthreads();
+        for (int col = threadIdx.x; col < H; col += T::NT) {
+            float s = 0.f;
+            for (int m = 0; m < Q.n_cos; ++m) s = fmaf(S.cv[m], __ldg(Pa + Q.wphi + (size_t)m * H + col), s);
+            S.phv[col] = fmaxf(s + __ldg(Pa + Q.bphi + col), 0.f);
+        }
+        __syncthreads();
+        for (int f = threadIdx.x; f < T::BM * (H / 4); f += T::NT) {
+            const int i = f / (H / 4), c4 = f % (H / 4);
+            float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (r0 + i < B) {
+                const float4 h = *reinterpret_cast<const float4*>(h1a + (size_t)(r0 + i) * H + c4 * 4);
+                const float4 p = *reinterpret_cast<const float4*>(S.phv + c4 * 4);
+                z = make_float4(__fmul_rn(h.x, p.x), __fmul_rn(h.y, p.y), __fmul_rn(h.z, p.z), __fmul_rn(h.w, p.w));
+            }
+            *reinterpret_cast<float4*>(S.Zs + i * T::LDH + c4 * 4) = z;
+        }
+        __syncthreads();
+        iqn_layer2_head<H>(acc, c, S, Pa, A.L, nullptr, r0, B);
+        for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) S.qsum[f] = __fadd_rn(S.qsum[f], S.qs[f]);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < T::BM; i += T::NT) {          // a* and q_next
+        const int gr = r0 + i;
+        int best = 0;
+        float q[4];
+        for (int a = 0; a < 4; ++a) q[a] = a < nA ? __fdiv_rn(S.qsum[i * 4 + a], (float)Q.k) : 0.f;
+        for (int a = 1; a < nA; ++a)
+            if (q[a] > q[best]) best = a;
+        S.as[i] = best;
+        if (gr < B)
+            for (int a = 0; a < 4; ++a) A.q_next[(sb + gr) * 4 + a] = q[a];
+        for (int a = 0; a < 4; ++a) S.qsum[i * 4 + a] = 0.f;
+    }
+    __syncthreads();
+
+    const float* Pt = A.nets.theta_tgt + (size_t)g * A.L.stride;
+    const float* h1t = Q.h1n + (nb + sb) * H;
+#pragma unroll 1
+    for (int j = 0; j < Q.n_p; ++j) {               // sampled passes of the target network
+        for (int i = threadIdx.x; i < T::BM; i += T::NT) {
+            const int gr = r0 + i;
+            float tau = 0.f;
+            if (gr < B) {
+                tau = iqn_tau(key, (uint32_t)(Q.row_base + gr), (uint32_t)j, step, 1);
+                Q.tau_p[(sb + gr) * Q.n_p + j] = tau;
+            }
+            S.tv[i] = tau;
+        }
+        __syncthreads();
+        iqn_cos_tile<H>(S, Q, r0, B, nullptr);
+        gemm_phi<H>(acc, c, S.Cs, S.ldc, Pt + Q.wphi, Q.n_cos, S.Ws);
+        store_z<H>(acc, c, Pt + Q.bphi, h1t, S.Zs, nullptr, nullptr, r0, B);
+        __syncthreads();
+        iqn_layer2_head<H>(acc, c, S, Pt, A.L, nullptr, r0, B);
+        for (int i = threadIdx.x; i < T::BM; i += T::NT) {
+            const int gr = r0 + i;
+            if (gr >= B) continue;
+            const size_t o = sb + gr;
+            Q.t[o * Q.n_p + j] = __fadd_rn(A.r_hat[o], __fmul_rn(A.disc_b[o], S.qs[i * 4 + S.as[i]]));
+            for (int a = 0; a < nA; ++a) S.qsum[i * 4 + a] = __fadd_rn(S.qsum[i * 4 + a], S.qs[i * 4 + a]);
+        }
+    }
+    for (int i = threadIdx.x; i < T::BM; i += T::NT) {
+        const int gr = r0 + i;
+        if (gr >= B) continue;
+        for (int a = 0; a < 4; ++a) A.tq_all[(sb + gr) * 4 + a] = a < nA ? __fdiv_rn(S.qsum[i * 4 + a], (float)Q.n_p) : 0.f;
+    }
+}
+
+// IQN K4a: at s, layer 1 (h1 -> workspace), the N sampled passes (c, phi, z, h2 -> scratch), the pair terms against T, the
+// row loss, priority and metric partials; then per fraction, the backward pass: dh2 (-> scratch over h2, with the W3 / b3 /
+// b2 partials), dz = dh2 W2^T, dphi = dz * h1 * relu'(phi) (-> scratch over phi, dbphi partial) and dh1 += dz * phi; last,
+// dh1 masked by relu'(h1) (-> workspace, db1 partial).  Partials of this row tile are summed over the fractions in order.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) iqn_online_kernel(const LearnArgs A, const IqnArgs Q) {
+    using T = Tile<H>;
+    extern __shared__ __align__(16) float smem[];
+    const int g = blockIdx.x / A.ws_tiles, rt = blockIdx.x % A.ws_tiles;
+    if (!A.active[g]) return;
+    const int B = A.d.batch, Dp = A.d.obs_stride, r0 = rt * T::BM, nA = A.d.n_actions, N = Q.n;
+    IqnSmem<H> S(smem, Dp, Q.ncp, N);
+    const Coord<H> c;
+    const int32_t* rows = A.rows + (size_t)g * B;
+    const float* P = A.nets.theta + (size_t)g * A.L.stride;
+    const size_t sb = (size_t)g * B;
+    const size_t pt = (size_t)g * A.ws_tiles + rt;
+    const uint64_t key = Q.key[g];
+    const uint32_t step = (uint32_t)(A.nets.learn_step[g] - 1);
+    const float* h1 = A.h1 + sb * H;
+    auto pass_rows = [&](float* buf, int i, int w) { return buf + ((size_t)g * N + i) * B * w; };   // [g][i][B][w]
+    gather_tile<H>(S.Cs, S.ldc, A.rp.obs, rows, r0, B, Dp);
+
+    float acc[8][8];
+    gemm_rowA<H, false>(acc, c, S.Cs, S.ldc, P + A.L.w1, H, Dp, S.Ws);
+    store_relu<H>(acc, c, P + A.L.b1, S.Zs, A.h1 + sb * H, r0, B);
+    for (int i = threadIdx.x; i < T::BM; i += T::NT) {
+        S.as[i] = r0 + i < B ? A.act_b[sb + r0 + i] : 0;
+        for (int a = 0; a < 4; ++a) S.qsum[i * 4 + a] = 0.f;
+    }
+    __syncthreads();
+
+#pragma unroll 1
+    for (int i = 0; i < N; ++i) {                   // forward passes
+        for (int r = threadIdx.x; r < T::BM; r += T::NT) {
+            const int gr = r0 + r;
+            float tau = 0.f;
+            if (gr < B) {
+                tau = iqn_tau(key, (uint32_t)(Q.row_base + gr), (uint32_t)i, step, 0);
+                Q.tau[(sb + gr) * N + i] = tau;
+            }
+            S.tv[r] = tau;
+        }
+        __syncthreads();
+        iqn_cos_tile<H>(S, Q, r0, B, pass_rows(Q.c, i, Q.n_cos));
+        gemm_phi<H>(acc, c, S.Cs, S.ldc, P + Q.wphi, Q.n_cos, S.Ws);
+        store_z<H>(acc, c, P + Q.bphi, h1, S.Zs, pass_rows(Q.phi, i, H), pass_rows(Q.z, i, H), r0, B);
+        __syncthreads();
+        iqn_layer2_head<H>(acc, c, S, P, A.L, pass_rows(Q.h2, i, H), r0, B);
+        for (int r = threadIdx.x; r < T::BM; r += T::NT) {
+            const int gr = r0 + r;
+            const float th = S.qs[r * 4 + S.as[r]];
+            S.th[r * N + i] = th;
+            if (gr < B) Q.theta[(sb + gr) * N + i] = th;
+            for (int a = 0; a < nA; ++a) S.qsum[r * 4 + a] = __fadd_rn(S.qsum[r * 4 + a], S.qs[r * 4 + a]);
+        }
+    }
+    __syncthreads();
+
+    const float k = Q.kappa, inv_lb = (float)A.loss_batch;
+    for (int f = threadIdx.x; f < T::BM * N; f += T::NT) {   // one thread per (row, fraction i): the pair terms over j
+        const int r = f / N, i = f % N, gr = r0 + r;
+        float gv = 0.f, l = 0.f;
+        if (gr < B) {
+            const float tau = Q.tau[(sb + gr) * N + i], omt = __fsub_rn(1.f, tau), th = S.th[f];
+            const float* t = Q.t + (sb + gr) * Q.n_p;
+            float gs = 0.f;
+            for (int j = 0; j < Q.n_p; ++j) {
+                float rho, dr;
+                quantile_pair(__fsub_rn(t[j], th), tau, omt, k, rho, dr);
+                l = __fadd_rn(l, rho);
+                gs = __fadd_rn(gs, dr);
+            }
+            const float wi = A.per ? A.is_w[sb + gr] : 1.f;
+            gv = __fdiv_rn(__fmul_rn(wi, __fdiv_rn(gs, (float)Q.n_p)), inv_lb);
+            Q.grad[(sb + gr) * N + i] = gv;
+        }
+        S.th[f] = gv;                                // theta_i is not needed again: the slot takes the gradient
+        S.lr[f] = l;
+    }
+    __syncthreads();
+    for (int r = threadIdx.x; r < T::BM; r += T::NT) {       // one thread per row: L_r, the loss term, the priority, q_all
+        const int gr = r0 + r;
+        float term = 0.f;
+        if (gr < B) {
+            float L = 0.f;
+            for (int i = 0; i < N; ++i) L = __fadd_rn(L, S.lr[r * N + i]);
+            L = __fdiv_rn(L, (float)Q.n_p);
+            if (A.per) {                             // a transition drawn twice: its last row stores (their fractions differ)
+                bool last = true;
+                for (int k = gr + 1; k < B && last; ++k) last = rows[k] != rows[gr];
+                if (last) per_store_priority(A, rows[gr], L);
+            }
+            term = __fmul_rn(A.per ? A.is_w[sb + gr] : 1.f, L);
+            for (int a = 0; a < 4; ++a) {
+                const float q = a < nA ? __fdiv_rn(S.qsum[r * 4 + a], (float)N) : 0.f;
+                S.qsum[r * 4 + a] = q;
+                A.q_all[(sb + gr) * 4 + a] = q;
+            }
+        }
+        S.terms[r] = term;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {                          // per-tile loss / metric partials, rows in order
+        float ls = 0.f, qsum = 0.f, qsq = 0.f, hist[4] = {0.f, 0.f, 0.f, 0.f};
+        for (int r = 0; r < T::BM && r0 + r < B; ++r) {
+            ls += S.terms[r];
+            for (int a = 0; a < nA; ++a) {
+                const float q = S.qsum[r * 4 + a];
+                qsum += q;
+                qsq = fmaf(q, q, qsq);
+            }
+            hist[S.as[r]] += 1.f;
+        }
+        float* pl = A.part_loss + pt * 8;
+        pl[0] = ls; pl[1] = qsum; pl[2] = qsq;
+        pl[3] = hist[0]; pl[4] = hist[1]; pl[5] = hist[2]; pl[6] = hist[3]; pl[7] = 0.f;
+    }
+
+#pragma unroll 1
+    for (int i = 0; i < N; ++i) {                   // backward passes
+        float* gh2 = pass_rows(Q.h2, i, H);
+        float* gphi = pass_rows(Q.phi, i, H);
+        for (int f = threadIdx.x; f < T::BM * (H / 4); f += T::NT) {
+            const int r = f / (H / 4), c4 = f % (H / 4);
+            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (r0 + r < B) v = *reinterpret_cast<const float4*>(gh2 + (size_t)(r0 + r) * H + c4 * 4);
+            *reinterpret_cast<float4*>(S.Zs + r * T::LDH + c4 * 4) = v;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {                      // db3 partial
+            float db3[4] = {0.f, 0.f, 0.f, 0.f};
+            for (int r = 0; r < T::BM; ++r) db3[S.as[r]] += S.th[r * N + i];
+            for (int a = 0; a < 4; ++a) A.part_b3[pt * 4 + a] = i ? A.part_b3[pt * 4 + a] + db3[a] : db3[a];
+        }
+        // dW3 partial, dh2 = (dZ W3^T) * relu'(h2) in place, db2 partial: one thread per column
+        for (int j = threadIdx.x; j < H; j += T::NT) {
+            const float4 w3 = __ldg(reinterpret_cast<const float4*>(P + A.L.w3) + j);
+            float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f, sb2 = 0.f;
+            for (int r = 0; r < T::BM; ++r) {
+                const float h = S.Zs[r * T::LDH + j];
+                const float gi = S.th[r * N + i];
+                const int ai = S.as[r];
+                const float t = h * gi;
+                d0 += ai == 0 ? t : 0.f; d1 += ai == 1 ? t : 0.f;
+                d2 += ai == 2 ? t : 0.f; d3 += ai == 3 ? t : 0.f;
+                const float w = ai == 0 ? w3.x : ai == 1 ? w3.y : ai == 2 ? w3.z : w3.w;
+                const float dh = h > 0.f ? gi * w : 0.f;
+                S.Zs[r * T::LDH + j] = dh;
+                sb2 += dh;
+            }
+            float4* pw = reinterpret_cast<float4*>(A.part_w3 + pt * H * 4) + j;
+            if (i) {
+                const float4 o = *pw;
+                d0 += o.x; d1 += o.y; d2 += o.z; d3 += o.w;
+                sb2 += A.part_b2[pt * H + j];
+            }
+            *pw = make_float4(d0, d1, d2, d3);
+            A.part_b2[pt * H + j] = sb2;
+        }
+        __syncthreads();
+        for (int f = threadIdx.x; f < T::BM * (H / 4); f += T::NT) {    // dh2 over h2 in the scratch
+            const int r = f / (H / 4), c4 = f % (H / 4);
+            if (r0 + r < B)
+                *reinterpret_cast<float4*>(gh2 + (size_t)(r0 + r) * H + c4 * 4) = *reinterpret_cast<const float4*>(S.Zs + r * T::LDH + c4 * 4);
+        }
+        // dz = dh2 W2^T; dphi = dz * h1 * relu'(phi) over phi and into Zs; dh1 += dz * phi
+        gemm_rowA<H, true>(acc, c, S.Zs, T::LDH, P + A.L.w2, H, H, S.Ws);
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+            const int col = c.col0(half);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                const int row = c.row(e);
+                float4 dp = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (r0 + row < B) {
+                    const size_t o = (size_t)(r0 + row) * H + col;
+                    const float4 p = *reinterpret_cast<const float4*>(gphi + o);
+                    const float4 h = *reinterpret_cast<const float4*>(h1 + o);
+                    const float dz[4] = {acc[e][half * 4], acc[e][half * 4 + 1], acc[e][half * 4 + 2], acc[e][half * 4 + 3]};
+                    dp.x = p.x > 0.f ? __fmul_rn(dz[0], h.x) : 0.f;
+                    dp.y = p.y > 0.f ? __fmul_rn(dz[1], h.y) : 0.f;
+                    dp.z = p.z > 0.f ? __fmul_rn(dz[2], h.z) : 0.f;
+                    dp.w = p.w > 0.f ? __fmul_rn(dz[3], h.w) : 0.f;
+                    *reinterpret_cast<float4*>(gphi + o) = dp;
+                    float4* d1p = reinterpret_cast<float4*>(A.dh1 + sb * H + o);
+                    float4 d1 = i ? *d1p : make_float4(0.f, 0.f, 0.f, 0.f);
+                    d1.x = __fadd_rn(d1.x, __fmul_rn(dz[0], p.x)); d1.y = __fadd_rn(d1.y, __fmul_rn(dz[1], p.y));
+                    d1.z = __fadd_rn(d1.z, __fmul_rn(dz[2], p.z)); d1.w = __fadd_rn(d1.w, __fmul_rn(dz[3], p.w));
+                    *d1p = d1;
+                }
+                *reinterpret_cast<float4*>(S.Zs + row * T::LDH + col) = dp;
+            }
+        }
+        __syncthreads();
+        for (int j = threadIdx.x; j < H; j += T::NT) {   // dbphi partial
+            float s = 0.f;
+            for (int r = 0; r < T::BM; ++r) s += S.Zs[r * T::LDH + j];
+            float* pb = Q.part_bphi + pt * H + j;
+            *pb = i ? *pb + s : s;
+        }
+        __syncthreads();
+    }
+    for (int f = threadIdx.x; f < T::BM * (H / 4); f += T::NT) {    // dh1 * relu'(h1)
+        const int r = f / (H / 4), c4 = f % (H / 4);
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (r0 + r < B) {
+            float4* dp = reinterpret_cast<float4*>(A.dh1 + (sb + r0 + r) * H + c4 * 4);
+            const float4 h = *reinterpret_cast<const float4*>(h1 + (size_t)(r0 + r) * H + c4 * 4);
+            v = *dp;
+            v.x = h.x > 0.f ? v.x : 0.f; v.y = h.y > 0.f ? v.y : 0.f;
+            v.z = h.z > 0.f ? v.z : 0.f; v.w = h.w > 0.f ? v.w : 0.f;
+            *dp = v;
+        }
+        *reinterpret_cast<float4*>(S.Zs + r * T::LDH + c4 * 4) = v;
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < H; j += T::NT) {   // db1 partial
+        float s = 0.f;
+        for (int r = 0; r < T::BM; ++r) s += S.Zs[r * T::LDH + j];
+        A.part_b1[pt * H + j] = s;
+    }
+}
+
+// IQN K4b, gradients only: dW2 = z^T dh2 and dWphi = c^T dphi over the network's N * B (row, fraction) rows, dW1 = s^T dh1
+// over its B rows, in wgrad_adam_kernel's tile form, and a misc tile for b1 / b2 / bphi (partials in tile order), W3 / b3
+// (the online kernel's partials in tile order) and the metrics.
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT) iqn_wgrad_kernel(const LearnArgs A, const IqnArgs Q) {
+    using T = Tile<H>;
+    constexpr int LDA = T::BM + 4;
+    extern __shared__ __align__(16) float smem[];
+    float (*As)[T::KC * LDA] = reinterpret_cast<float (*)[T::KC * LDA]>(smem);
+    float (*Bs)[T::KC * T::LDW] = reinterpret_cast<float (*)[T::KC * T::LDW]>(smem + 2 * T::KC * LDA);
+    const int B = A.d.batch, Dp = A.d.obs_stride, N = Q.n;
+    const int tiles_w2 = H / T::BM, tiles_w1 = (Dp + T::BM - 1) / T::BM, tiles_wp = (Q.n_cos + T::BM - 1) / T::BM;
+    const int per_net = tiles_w2 + tiles_w1 + tiles_wp + 1;
+    const int g = blockIdx.x / per_net, t = blockIdx.x % per_net;
+    const size_t sb = (size_t)g * B;
+    float* gout = A.grads + (size_t)g * A.L.stride;
+
+    if (t == per_net - 1) {
+        if (!A.active[g]) {
+            if (threadIdx.x < DMDQN_METRICS_STRIDE && A.metrics) A.metrics[g * DMDQN_METRICS_STRIDE + threadIdx.x] = 0.f;
+            return;
+        }
+        const size_t p0 = (size_t)g * A.ws_tiles;
+        for (int e = threadIdx.x; e < 4 * H + 1; e += T::NT) {
+            if (e < 3 * H) {                         // b1, b2, bphi
+                const int kind = e / H, j = e % H;
+                const float* part = kind == 0 ? A.part_b1 : kind == 1 ? A.part_b2 : Q.part_bphi;
+                float gsum = 0.f;
+                for (int r = 0; r < A.ws_tiles; ++r) gsum += part[(p0 + r) * H + j];
+                gout[(kind == 0 ? A.L.b1 : kind == 1 ? A.L.b2 : Q.bphi) + j] = gsum;
+                continue;
+            }
+            const int j = e - 3 * H;                 // one head row W3[j][0..3] (j < H) or b3 (j == H)
+            float4 w = make_float4(0.f, 0.f, 0.f, 0.f);
+            for (int r = 0; r < A.ws_tiles; ++r) {
+                const float4 pw = j < H ? *reinterpret_cast<const float4*>(A.part_w3 + ((p0 + r) * H + j) * 4)
+                                        : *reinterpret_cast<const float4*>(A.part_b3 + (p0 + r) * 4);
+                w.x += pw.x; w.y += pw.y; w.z += pw.z; w.w += pw.w;
+            }
+            *reinterpret_cast<float4*>(gout + (j < H ? A.L.w3 + (int64_t)j * 4 : A.L.b3)) = w;
+        }
+        if (threadIdx.x == 0 && A.metrics) finish_metrics(A, g, A.ws_tiles, [](const float* p) { return *p; });
+        return;
+    }
+    if (!A.active[g]) return;
+
+    // tile kinds: W2 (A = z, D = dh2, K = N B), W1 (A = gathered s, D = dh1, K = B), Wphi (A = c, D = dphi, K = N B)
+    const bool is_w2 = t < tiles_w2, is_w1 = !is_w2 && t < tiles_w2 + tiles_w1;
+    const int m0 = (is_w2 ? t : is_w1 ? t - tiles_w2 : t - tiles_w2 - tiles_w1) * T::BM;
+    const int m_valid = is_w2 ? H : is_w1 ? Dp : Q.n_cos;
+    const size_t prow = (size_t)g * N * B;           // first (row, fraction) row of network g
+    const float* Asrc = is_w2 ? Q.z + prow * H : is_w1 ? A.rp.obs : Q.c + prow * Q.n_cos;
+    const int lda_src = is_w2 ? H : is_w1 ? Dp : Q.n_cos;
+    const float* Dsrc = is_w2 ? Q.h2 + prow * H : is_w1 ? A.dh1 + sb * H : Q.phi + prow * H;
+    const int K = is_w1 ? B : N * B;
+    const int32_t* rows = A.rows + sb;
+    const Coord<H> c;
+
+    constexpr int A4 = T::KC * T::BM / 4;            // 16-byte pieces in an A chunk
+    constexpr int NA = (A4 + T::NT - 1) / T::NT;
+    auto issue = [&](int k0, int buf) {
+#pragma unroll
+        for (int r = 0; r < NA; ++r) {
+            const int f = threadIdx.x + r * T::NT;
+            if (f < A4) {
+                const int kk = f / (T::BM / 4), m4 = f % (T::BM / 4);
+                const int kr = k0 + kk, m = m0 + m4 * 4;
+                const bool ok = kr < K && m < m_valid;
+                const size_t src_row = ok ? (is_w1 ? (size_t)rows[kr] : (size_t)kr) : 0;
+                cp_async16(&As[buf][kk * LDA + m4 * 4], Asrc + src_row * lda_src + (ok ? m : 0), ok);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < T::KC * H / 4 / T::NT; ++r) {
+            const int f = threadIdx.x + r * T::NT;
+            const int kk = f / (H / 4), n4 = f % (H / 4);
+            const bool ok = k0 + kk < K;
+            cp_async16(&Bs[buf][kk * T::LDW + n4 * 4], Dsrc + (ok ? (size_t)(k0 + kk) * H + n4 * 4 : 0), ok);
+        }
+        cp_async_commit();
+    };
+
+    float acc[8][8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+    issue(0, 0);
+    cp_async_wait_all();
+    __syncthreads();
+    int buf = 0;
+    for (int k0 = 0; k0 < K; k0 += T::KC) {
+        const bool more = k0 + T::KC < K;
+        if (more) issue(k0 + T::KC, buf ^ 1);
+#pragma unroll
+        for (int kk = 0; kk < T::KC; ++kk) {
+            const float4 a0 = *reinterpret_cast<const float4*>(&As[buf][kk * LDA + c.wm * 32 + c.lm * 4]);
+            const float4 a1 = *reinterpret_cast<const float4*>(&As[buf][kk * LDA + c.wm * 32 + 16 + c.lm * 4]);
+            const float4 b0 = *reinterpret_cast<const float4*>(&Bs[buf][kk * T::LDW + c.col0(0)]);
+            const float4 b1 = *reinterpret_cast<const float4*>(&Bs[buf][kk * T::LDW + c.col0(1)]);
+            fma8(acc[0], a0.x, b0, b1); fma8(acc[1], a0.y, b0, b1);
+            fma8(acc[2], a0.z, b0, b1); fma8(acc[3], a0.w, b0, b1);
+            fma8(acc[4], a1.x, b0, b1); fma8(acc[5], a1.y, b0, b1);
+            fma8(acc[6], a1.z, b0, b1); fma8(acc[7], a1.w, b0, b1);
+        }
+        if (more) cp_async_wait_all();
+        __syncthreads();
+        buf ^= 1;
+    }
+
+    const int64_t wbase = is_w2 ? A.L.w2 : is_w1 ? A.L.w1 : Q.wphi;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const int m = m0 + c.row(i);
+        if (m >= m_valid) continue;
+#pragma unroll
+        for (int half = 0; half < 2; ++half)
+            *reinterpret_cast<float4*>(gout + wbase + (int64_t)m * H + c.col0(half)) =
+                make_float4(acc[i][half * 4], acc[i][half * 4 + 1], acc[i][half * 4 + 2], acc[i][half * 4 + 3]);
+    }
+}
+
+template <int H>
+int launch_learn_iqn_h(const LearnArgs& A, const IqnArgs& Q, cudaStream_t s) {
+    using T = Tile<H>;
+    const size_t smem_t = IqnSmem<H>::bytes(A.d.obs_stride, Q.ncp, 0), smem_o = IqnSmem<H>::bytes(A.d.obs_stride, Q.ncp, Q.n);
+    const size_t smem_w = sizeof(float) * 2 * T::KC * ((T::BM + 4) + T::LDW);
+    static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(iqn_target_kernel<H>), smem_t, cfg_t)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(iqn_online_kernel<H>), smem_o, cfg_o)) return rc;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(iqn_wgrad_kernel<H>), smem_w, cfg_w)) return rc;
+    const int grid = A.d.n_nets * A.ws_tiles;
+    iqn_target_kernel<H><<<grid, T::NT, smem_t, s>>>(A, Q);
+    DMDQN_CUDA(cudaGetLastError());
+    iqn_online_kernel<H><<<grid, T::NT, smem_o, s>>>(A, Q);
+    DMDQN_CUDA(cudaGetLastError());
+    const int per_net = H / T::BM + (A.d.obs_stride + T::BM - 1) / T::BM + (Q.n_cos + T::BM - 1) / T::BM + 1;
+    iqn_wgrad_kernel<H><<<A.d.n_nets * per_net, T::NT, smem_w, s>>>(A, Q);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
 // One dynamic shared-memory opt-in record for clip_adam_apply_kernel, whichever layout the launch carries (the attribute
 // belongs to the kernel: a smaller request after a larger one must not lower it below what the larger launch needs).
 size_t g_clip_smem_cfg[kMaxDevices] = {};
@@ -1607,6 +2193,46 @@ int launch_adam_apply_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const d
 int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_atoms, const uint8_t* mask, double tau,
                             cudaStream_t s) {
     const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(n_atoms));
+    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_learn_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
+                     const dmdqn_iqn& q, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch, cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    A.L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos).L;
+    const IqnArgs Q = make_iqn_args(d, q);
+    switch (d.hidden) {
+        case 64: return launch_learn_iqn_h<64>(A, Q, s);
+        case 128: return launch_learn_iqn_h<128>(A, Q, s);
+        case 256: return launch_learn_iqn_h<256>(A, Q, s);
+        case 512: return launch_learn_iqn_h<512>(A, Q, s);
+    }
+    set_error("unsupported hidden width %d", d.hidden);
+    return DMDQN_ERR_ARG;
+}
+
+// adam_apply_kernel (clipnorm == 0) or clip_adam_apply_kernel on the IQN layout: the same arithmetic over [0, end)
+int launch_adam_apply_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_cos, const float* grads,
+                          double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    A.L = make_layout_iqn(d.obs_stride, d.hidden, n_cos).L;
+    if (clipnorm == 0.0) {
+        adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
+        DMDQN_CUDA(cudaGetLastError());
+        return DMDQN_OK;
+    }
+    const int64_t per = clip_per_cta(A.L);
+    const size_t smem = (size_t)per * 16;
+    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
+    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_sync_target_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, int n_cos, const uint8_t* mask, double tau, cudaStream_t s) {
+    const Layout L = make_layout_iqn(d.obs_stride, d.hidden, n_cos).L;
     sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;

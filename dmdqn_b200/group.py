@@ -52,6 +52,11 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # quantile regression DQN (QR-DQN, Dabney et al. 2018): num_quantiles learned return quantiles per action at the
     # midpoints (2i + 1) / 2N, the quantile Huber loss with threshold quantile_kappa (0: the pure quantile loss)
     "quantile": False, "num_quantiles": 50, "quantile_kappa": 1.0,
+    # implicit quantile networks (IQN, Dabney et al. 2018): the quantile fraction is an input (cosine embedding of
+    # iqn_embedding_dim features multiplied into layer 1's output); iqn_num_tau / iqn_num_tau_prime fractions drawn per row
+    # for the online values and the targets, acting on the mean over iqn_num_policy_tau midpoints; the Huber threshold is
+    # quantile_kappa
+    "iqn": False, "iqn_num_tau": 8, "iqn_num_tau_prime": 8, "iqn_num_policy_tau": 32, "iqn_embedding_dim": 64,
 }
 
 
@@ -116,6 +121,42 @@ def quantile_config(cfg: dict) -> dict:
     return cfg
 
 
+def iqn_config(cfg: dict) -> dict:
+    """Validate the IQN keys of ``cfg`` and resolve its precision (in place; returns ``cfg``).  With ``iqn: true`` the learn
+    step runs the fp32 (FFMA) kernels only, so ``precision: auto`` becomes fp32 and an explicit tcgen05 precision, C51,
+    QR-DQN, dueling heads, noisy networks and the Huber loss key are refused."""
+    if not isinstance(cfg["iqn"], (bool, np.bool_)):
+        raise ValueError(f"iqn={cfg['iqn']!r}: must be true or false")
+    if not cfg["iqn"]:
+        return cfg
+    for key in ("iqn_num_tau", "iqn_num_tau_prime", "iqn_num_policy_tau"):
+        n = cfg[key]
+        if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n <= N.IQN_MAX_TAU:
+            raise ValueError(f"{key}={n!r}: must be an integer in [1, {N.IQN_MAX_TAU}]")
+    n = cfg["iqn_embedding_dim"]
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 4 <= n <= N.IQN_MAX_COS or n % 4:
+        raise ValueError(f"iqn_embedding_dim={n!r}: must be a multiple of 4 in [4, {N.IQN_MAX_COS}]")
+    k = cfg["quantile_kappa"]
+    if isinstance(k, bool) or not isinstance(k, numbers.Real) or not math.isfinite(k) or k < 0:
+        raise ValueError(f"quantile_kappa={k!r}: must be a finite number >= 0 (0 = the pure quantile loss)")
+    for other in ("distributional", "quantile"):
+        if cfg[other]:
+            raise ValueError(f"iqn=true cannot be combined with {other}=true: they are different distributional heads; "
+                             "choose one")
+    if cfg["precision"] not in ("auto", "fp32"):
+        raise ValueError(f"precision={cfg['precision']!r}: IQN networks run the fp32 (FFMA) learn path only; the tcgen05 IQN "
+                         "kernels are not built (use precision: auto or fp32)")
+    if cfg["dueling"]:
+        raise ValueError("iqn=true cannot be combined with dueling=true: dueling IQN heads are not implemented")
+    if cfg["noisy"]:
+        raise ValueError("iqn=true cannot be combined with noisy=true: noisy IQN networks are not implemented")
+    if cfg["loss"] != "mse":
+        raise ValueError(f"loss={cfg['loss']!r}: IQN networks minimise the quantile Huber loss, whose threshold is "
+                         "quantile_kappa; the loss key does not apply (leave it at mse)")
+    cfg["precision"] = "fp32"
+    return cfg
+
+
 def _ptr(t: torch.Tensor | None) -> int | None:
     return None if t is None else t.data_ptr()
 
@@ -132,10 +173,13 @@ def _on_device(method):
     return wrapper
 
 
-def keras_init(seed: int, state_size: int, hidden: int, action_size: int, dueling: bool = False) -> list[torch.Tensor]:
+def keras_init(seed: int, state_size: int, hidden: int, action_size: int, dueling: bool = False,
+               n_cos: int = 0) -> list[torch.Tensor]:
     """HeNormal hidden kernels, GlorotUniform head, zero biases (dqn_agent.py:166-181), as
     [W1,b1,W2,b2,W3,b3] in Keras ``get_weights()`` order, kernels ``[in,out]``.  ``dueling`` appends the value head
-    [Wv [H,1], bv [1]], Wv GlorotUniform drawn from the same generator after W3 (the other draws do not change)."""
+    [Wv [H,1], bv [1]], Wv GlorotUniform drawn from the same generator after W3 (the other draws do not change).
+    ``n_cos`` > 0 (IQN) appends the cosine embedding [Wphi [n_cos, H], bphi [H]], Wphi HeNormal (truncated, fan_in = n_cos)
+    drawn after every other weight."""
     gen = torch.Generator().manual_seed(int(seed))
     out = []
     dims = [state_size, hidden, hidden]
@@ -149,6 +193,11 @@ def keras_init(seed: int, state_size: int, hidden: int, action_size: int, duelin
     if dueling:
         limit = math.sqrt(6.0 / (hidden + 1))
         out += [(torch.rand(hidden, 1, generator=gen) * 2 - 1) * limit, torch.zeros(1)]
+    if n_cos:
+        std = math.sqrt(2.0 / n_cos) / 0.87962566103423978
+        w = torch.empty(n_cos, hidden)
+        torch.nn.init.trunc_normal_(w, 0.0, std, -2 * std, 2 * std, generator=gen)
+        out += [w, torch.zeros(hidden)]
     return out
 
 
@@ -201,6 +250,7 @@ class AgentGroup:
                              "sigma gradients is not implemented")
         dist_config(cfg)
         quantile_config(cfg)
+        iqn_config(cfg)
         self.distributional = bool(cfg["distributional"])     # C51
         self.num_atoms = int(cfg["num_atoms"]) if self.distributional else 0
         self.quantile = bool(cfg["quantile"])                 # QR-DQN
@@ -208,6 +258,9 @@ class AgentGroup:
         # either head uses the distributional layout W3[H][4 * Np] | b3[4 * Np] of N = head_atoms atoms or quantiles
         self.dist_layout = self.distributional or self.quantile
         self.head_atoms = self.num_atoms or self.num_quantiles
+        self.iqn = bool(cfg["iqn"])
+        self.n_cos = int(cfg["iqn_embedding_dim"]) if self.iqn else 0
+        self.iqn_row_base = 0        # global index of this group's first sampled row (SharedParameterStep: rank * B)
         self.n_nets = 1 if self.shared else self.n_agents
         self.state_size, self.action_size = int(state_size), int(action_size)
         self.obs_stride = (self.state_size + 15) // 16 * 16
@@ -226,6 +279,9 @@ class AgentGroup:
         if self.dueling:        # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
             self.layout = N.DuelingLayout()
             N.check(self.lib.dmdqn_param_layout_dueling(C.byref(self.dims), C.byref(self.layout)))
+        elif self.iqn:              # the plain block with Wphi[n_cos][H] | bphi[H] after b3
+            self.layout = N.IqnLayout()
+            N.check(self.lib.dmdqn_param_layout_iqn(C.byref(self.dims), self.n_cos, C.byref(self.layout)))
         elif self.dist_layout:      # the head W3[H][4 * Np] | b3[4 * Np]
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout_dist(C.byref(self.dims), self.head_atoms, C.byref(self.layout)))
@@ -268,8 +324,10 @@ class AgentGroup:
             # gradient clipping: the raw gradient blocks of a step and each network's norm before clipping (last step)
             self.grads = torch.zeros_like(self.theta) if self.global_clipnorm is not None else None
             self.grad_norms = torch.zeros((g,), dtype=torch.float32, device=dev) if self.global_clipnorm is not None else None
-            if self.dist_layout:        # the gradient block between the dist / quantile learn_grads and dmdqn_adam_apply_dist
+            if self.dist_layout or self.iqn:    # the gradient block between the two learn calls
                 self.grads = torch.zeros_like(self.theta)
+            if self.iqn:
+                self.key = torch.zeros((g,), dtype=torch.int64, device=dev)
             if self.noisy:      # sigma with its target and moments, the effective blocks, the gradient and the noise record
                 self.sigma, self.sigma_tgt = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
                 self.sigma_m, self.sigma_v = torch.zeros_like(self.theta), torch.zeros_like(self.theta)
@@ -295,6 +353,8 @@ class AgentGroup:
             if self.noisy:
                 for name in self._NOISY:
                     setattr(self, name, getattr(p, name)[j:j + 1])
+            if self.iqn:
+                self.key = p.key[j:j + 1]
             self.n_written_host = p.n_written_host[i:i + 1]
             self.learn_step_host = p.learn_step_host[j:j + 1]
         self.replay = N.Replay(_ptr(self.obs), _ptr(self.next_obs), _ptr(self.act_ring), _ptr(self.rew_ring),
@@ -312,6 +372,13 @@ class AgentGroup:
             else:
                 self.dist = N.Dist(self.num_atoms, float(cfg["v_min"]), float(cfg["v_max"]), _ptr(self.dist_scratch),
                                    nbytes.value)
+        self.iqn_scratch, self.iqn_args = None, None
+        if self.iqn:                # per group, like the workspace
+            q = self._iqn_struct(None, 0)
+            nbytes = C.c_size_t()
+            N.check(self.lib.dmdqn_iqn_scratch_bytes(C.byref(self.dims), C.byref(q), C.byref(nbytes)))
+            self.iqn_scratch = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
+            self.iqn_args = self._iqn_struct(_ptr(self.iqn_scratch), nbytes.value)
         nbytes = C.c_size_t()
         N.check(self.lib.dmdqn_workspace_bytes(C.byref(self.dims), C.byref(nbytes)))
         self.workspace = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
@@ -333,6 +400,11 @@ class AgentGroup:
     _NOISY = _NOISY_PTRS + ("grads",)
 
     # ------------------------------------------------------------------ helpers ---------
+    def _iqn_struct(self, scratch: int | None, nbytes: int) -> "N.Iqn":
+        c = self.config
+        return N.Iqn(int(c["iqn_num_tau"]), int(c["iqn_num_tau_prime"]), int(c["iqn_num_policy_tau"]), self.n_cos,
+                     float(c["quantile_kappa"]), int(self.iqn_row_base), _ptr(self.key), scratch, nbytes)
+
     @property
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
@@ -360,8 +432,9 @@ class AgentGroup:
         """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]; dueling: + [Wv [H,1], bv [1]]) -> one parameter block."""
         L, H, A = self.layout, self.hidden, self.action_size
         ws = [torch.as_tensor(np.asarray(w), dtype=torch.float32) for w in weights]
-        if len(ws) != (8 if self.dueling else 6):
-            raise ValueError(f"expected {8 if self.dueling else 6} weight tensors, got {len(ws)}")
+        want = 8 if self.dueling or getattr(self, "iqn", False) else 6
+        if len(ws) != want:
+            raise ValueError(f"expected {want} weight tensors, got {len(ws)}")
         w1, b1, w2, b2, w3, b3 = ws[:6]
         blk = torch.zeros((L.stride,), dtype=torch.float32)
         blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size] = w1
@@ -378,6 +451,9 @@ class AgentGroup:
         if self.dueling:
             blk[L.wv:L.wv + H] = ws[6].reshape(H)
             blk[L.bv:L.bv + 1] = ws[7].reshape(1)
+        if getattr(self, "iqn", False):
+            blk[L.wphi:L.wphi + self.n_cos * H] = ws[6].reshape(-1)
+            blk[L.bphi:L.bphi + H] = ws[7].reshape(H)
         return blk
 
     def unpack(self, blk: torch.Tensor) -> list[torch.Tensor]:
@@ -392,6 +468,8 @@ class AgentGroup:
         out += [blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(), blk[L.b3:L.b3 + A].clone()]
         if self.dueling:
             out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
+        if getattr(self, "iqn", False):
+            out += [blk[L.wphi:L.wphi + self.n_cos * H].view(self.n_cos, H).clone(), blk[L.bphi:L.bphi + H].clone()]
         return out
 
     def sigma_init(self) -> list[torch.Tensor]:
@@ -408,18 +486,19 @@ class AgentGroup:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
         (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
         head = self.action_size * self.head_atoms if self.dist_layout else self.action_size   # dist: W3 GlorotUniform over [H, A*N]
-        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, self.dueling))
+        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, self.dueling, self.n_cos))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
         self.adam_m.zero_(); self.adam_v.zero_(); self.learn_step.zero_()
         self.learn_step_host[:] = 0
+        if self.noisy or self.iqn:      # the Philox key of each network (noise, or the IQN fractions)
+            keys = [noise_key(seed + g) for g in range(self.n_nets)]
+            self.key.copy_(torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in keys], dtype=torch.int64))
         if self.noisy:
             sig = self.pack(self.sigma_init()).to(self.device)
             self.sigma.copy_(sig.expand_as(self.sigma)); self.sigma_tgt.copy_(self.sigma)
             self.sigma_m.zero_(); self.sigma_v.zero_()
-            keys = [noise_key(seed + g) for g in range(self.n_nets)]
-            self.key.copy_(torch.tensor([k - (1 << 64) if k >= 1 << 63 else k for k in keys], dtype=torch.int64))
 
     def _blocks(self, which: str) -> list[torch.Tensor]:
         t = {"online": (self.theta, self.sigma), "target": (self.theta_tgt, self.sigma_tgt), "m": (self.adam_m, self.sigma_m),
@@ -517,6 +596,8 @@ class AgentGroup:
             N.check(self.lib.dmdqn_act_dist(C.byref(self.dims), C.byref(nets), C.byref(self.dist), *args))
         elif self.quantile:
             N.check(self.lib.dmdqn_act_quantile(C.byref(self.dims), C.byref(nets), C.byref(self.qr), *args))
+        elif self.iqn:
+            N.check(self.lib.dmdqn_act_iqn(C.byref(self.dims), C.byref(nets), C.byref(self.iqn_args), *args))
         elif self.noisy and noisy is not False and not target:
             N.check(self.lib.dmdqn_act_noisy(C.byref(self.dims), C.byref(nets), C.byref(self.noisy_ptrs), int(self.dueling),
                                              *args))
@@ -618,11 +699,25 @@ class AgentGroup:
                                                     C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
                                                     _ptr(self.metrics), ws, nws, stream_ptr))
 
+    def _iqn_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
+        """``dmdqn_learn_grads_iqn`` into ``grads_ptr``, the loss mean over ``global_batch``, the fractions keyed from row
+        ``iqn_row_base``."""
+        self.iqn_args.row_base = int(self.iqn_row_base)
+        N.check(self.lib.dmdqn_learn_grads_iqn(C.byref(self.dims), C.byref(hp), C.byref(self.iqn_args), C.byref(self.replay),
+                                               C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
+                                               _ptr(self.metrics), _ptr(self.workspace), self.workspace.numel(), stream_ptr))
+
     def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
         """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
         (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
         ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
         ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.iqn:                # the IQN gradient, then Adam (clipped when global_clipnorm is set)
+            self._iqn_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
+            N.check(self.lib.dmdqn_adam_apply_iqn(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.n_cos,
+                                                  _ptr(self.grads), self.global_clipnorm or 0.0, _ptr(self.grad_norms), ws, nws,
+                                                  stream_ptr))
+            return
         if self.dist_layout:        # the C51 / QR-DQN gradient, then Adam (clipped when global_clipnorm is set)
             self._dist_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
             N.check(self.lib.dmdqn_adam_apply_dist(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.head_atoms,
@@ -714,7 +809,7 @@ class AgentGroup:
         """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
         one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy; the
         same with ``noisy`` set and the noisy learn calls."""
-        if self.global_clipnorm is None and not self.noisy and not self.dist_layout:
+        if self.global_clipnorm is None and not self.noisy and not self.dist_layout and not self.iqn:
             N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                              C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
                                              _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
@@ -807,6 +902,19 @@ class AgentGroup:
                                     ("dlogits", dv.dlogits, 4 * self.atom_stride)):
                 off = ptr - sbase
                 out[key] = self.dist_scratch[off:off + g * b * width * 4].view(torch.float32).view(g, b, width)
+        if self.iqn:             # fractions [network][row][N] / [N'], target samples, online values and their gradients, and
+                                 # the activation gradients of every (row, fraction)
+            iv = N.IqnViews()
+            N.check(self.lib.dmdqn_debug_iqn(C.byref(self.dims), C.byref(self.iqn_args), C.byref(iv)))
+            c, sbase = self.config, self.iqn_scratch.data_ptr()
+            n, n_p = int(c["iqn_num_tau"]), int(c["iqn_num_tau_prime"])
+            for key, ptr, width in (("tau", iv.tau, n), ("tau_prime", iv.tau_prime, n_p), ("target", iv.target, n_p),
+                                    ("theta", iv.theta, n), ("grad", iv.grad, n)):
+                off = ptr - sbase
+                out[key] = self.iqn_scratch[off:off + g * b * width * 4].view(torch.float32).view(g, b, width)
+            for key, ptr in (("dh2_pass", iv.dh2), ("dphi_pass", iv.dphi)):     # [network][fraction][row][H]
+                off = ptr - sbase
+                out[key] = self.iqn_scratch[off:off + g * n * b * self.hidden * 4].view(torch.float32).view(g, n, b, self.hidden)
         if self.dueling:         # the folded heads W3e[H][4] | b3e[4] of the last learn step, online (0) and target (1)
             dv = N.DuelingViews()
             N.check(self.lib.dmdqn_debug_dueling(C.byref(self.dims), _ptr(self.workspace), self.workspace.numel(), C.byref(dv)))
@@ -828,6 +936,10 @@ class AgentGroup:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
         tau = -1.0 if tau is None else float(tau)
+        if self.iqn:
+            N.check(self.lib.dmdqn_sync_target_iqn(C.byref(self.dims), C.byref(self.nets), self.n_cos, _ptr(mask_t), tau,
+                                                   self._stream))
+            return
         if self.dist_layout:
             N.check(self.lib.dmdqn_sync_target_dist(C.byref(self.dims), C.byref(self.nets), self.head_atoms, _ptr(mask_t), tau,
                                                     self._stream))

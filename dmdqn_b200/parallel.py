@@ -208,7 +208,8 @@ class SharedParameterStep:
         ``fused=True`` is refused there, because the peer-memory kernel does not know sigma.  A ``distributional`` group takes
         the NCCL path as well: ``dmdqn_learn_grads_dist``, the all-reduce of its gradient block, then ``dmdqn_adam_apply_dist``
         (clipped when ``global_clipnorm`` is set); ``fused=True`` is refused there.  A ``quantile`` (QR-DQN) group does the
-        same with ``dmdqn_learn_grads_quantile``."""
+        same with ``dmdqn_learn_grads_quantile``, and an ``iqn`` group with ``dmdqn_learn_grads_iqn`` (its fractions keyed from
+        row ``rank * batch``, so ranks draw different fractions) and ``dmdqn_adam_apply_iqn``."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
@@ -227,8 +228,13 @@ class SharedParameterStep:
         if grp.quantile and fused:
             raise ValueError("quantile=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the quantile "
                              "head's layout; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_dist path)")
+        if grp.iqn and fused:
+            raise ValueError("iqn=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the IQN layout; use "
+                             "fused=False (the NCCL all-reduce + dmdqn_adam_apply_iqn path)")
+        if grp.iqn:
+            grp.iqn_row_base = (dist.get_rank(group) if world > 1 else 0) * grp.batch_size
         if fused is None:
-            fused = clip is None and not grp.noisy and not grp.dist_layout and (world > 1 or exchange is not None)
+            fused = clip is None and not grp.noisy and not grp.dist_layout and not grp.iqn and (world > 1 or exchange is not None)
         if fused and exchange is None:
             rank = dist.get_rank(group) if world > 1 else 0
             exchange = PeerExchange(grp, rank, world).connect(group)
@@ -245,7 +251,9 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                if grp.dist_layout:             # C51 or QR-DQN
+                if grp.iqn:
+                    grp._iqn_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
+                elif grp.dist_layout:           # C51 or QR-DQN
                     grp._dist_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
                 elif grp.noisy:
                     N.check(grp.lib.dmdqn_learn_grads_noisy(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay),
@@ -277,6 +285,11 @@ class SharedParameterStep:
 
         def apply(g: torch.Tensor):
             with torch.cuda.device(grp.device):
+                if grp.iqn:                     # clipped (the norm of the all-reduced block) when global_clipnorm is set
+                    N.check(grp.lib.dmdqn_adam_apply_iqn(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.n_cos,
+                                                         _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),
+                                                         grp.workspace.numel(), grp._stream))
+                    return
                 if grp.dist_layout:             # clipped (the norm of the all-reduced block) when global_clipnorm is set
                     N.check(grp.lib.dmdqn_adam_apply_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.head_atoms,
                                                           _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),

@@ -43,6 +43,8 @@
  *   distributional networks (C51; dmdqn_param_layout_dist, see dmdqn_dist below) widen the head to 4 * Np columns:
  *     W1 | b1 | W2 | b2 | W3[H][4 * Np] | b3[4 * Np] | pad
  *   quantile networks (QR-DQN, see dmdqn_quantile below) use the same block with N quantiles in place of N atoms.
+ *   implicit quantile networks (IQN, see dmdqn_iqn below) append the cosine embedding after b3:
+ *     W1 | b1 | W2 | b2 | W3[H][4] | b3[4] | Wphi[n_cos][H] | bphi[H] | pad
  */
 #ifndef DMDQN_B200_H
 #define DMDQN_B200_H
@@ -654,6 +656,100 @@ int dmdqn_act_quantile(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmd
 /* The scratch's views after dmdqn_learn_grads_quantile: target_dist holds the target samples T [n_nets][B][Np]; h2 and
  * dlogits are as in dmdqn_debug_dist. */
 int dmdqn_debug_quantile(const dmdqn_dims* dims, const dmdqn_quantile* quantile, dmdqn_dist_views* out);
+
+/* Implicit quantile networks (IQN, Dabney, Ostrovski, Silver & Munos 2018), fp32 (FFMA) path only.  The network takes a
+ * quantile fraction tau as an input and returns the return quantile Z_tau(s, a).  Layer 1 is the state embedding and layer 2
+ * plus the head are the function of the product:
+ *   h1       = relu(s W1 + b1)                                     (once per row)
+ *   c_m(tau) = (float)cos(M_PI * m * (double)tau),  m = 0 .. n_cos - 1   (float64, then rounded)
+ *   phi(tau) = relu(c(tau) Wphi + bphi)
+ *   z        = h1 * phi(tau)                                       (one fp32 product per element)
+ *   h2       = relu(z W2 + b2)
+ *   Z_tau(s, a) = h2 . W3[:, a] + b3[a]                            (the plain 4-wide head; 0 for a >= A)
+ * Parameter block (dmdqn_param_layout_iqn):
+ *   W1 | b1 | W2 | b2 | W3[H][4] | b3[4] | Wphi[n_cos][H] | bphi[H] | pad
+ * with the plain offsets up to b3 and Wphi at b3 + 4 (16-byte aligned); Adam updates [0, end = bphi + H); the stride is
+ * rounded up to 32 floats.
+ * Fractions, drawn on the device: fraction i of sampled row r of network g, set 0 (tau_i, i < N) or 1 (tau'_j, j < N'), is
+ *   (x, -, -, -) = Philox4x32-10(key = {key[g] low word, high word}, counter = {row_base + r, i, t, 0x69716e00 | set})
+ *   tau = ((x >> 9) + 0.5) * 2^-23       (the top 23 bits, exact in fp32, strictly inside (0, 1))
+ * with t the network's learn_step before the sample kernel increments it (the noisy networks' rule) and row_base the global
+ * index of the caller's first row (0 in one process, rank * B when ranks split a shared batch).
+ * Policy: Q(s, a) = (sum_k Z_{tau~_k}(s, a), k order) / (float)K at the K midpoints tau~_k = (float)((2k + 1) / (2.0 K)).  (The
+ * paper draws K random fractions; the midpoint rule estimates the same integral and makes acting deterministic.)  a* is the
+ * argmax of the online (double_dqn = 1) or the target (double_dqn = 0) network's Q at s', ties to the lowest index.
+ * Target samples T_j = R + d * Z^tgt_{tau'_j}(s', a*) (product and sum rounded separately; R, d and the bootstrap row as
+ * dmdqn_sample forms them).  With theta_i = Z_{tau_i}(s, a_r), rho_ij and drho_ij are dmdqn_quantile's pair terms with w taken
+ * from the sampled tau_i, and
+ *   L_r = (sum_i (sum_j rho_ij, j order), i order) / (float)N',   g_i = (sum_j drho_ij, j order) / (float)N'
+ * (with N = N' and the midpoints as tau_i these are QR-DQN's formulas).  The loss term is w_r * L_r, the gradient of
+ * Z_{tau_i}(s, a_r) is (w_r * g_i) / loss_batch, and prioritized replay stores (float)pow(L_r + per_eps, per_alpha)
+ * (a transition drawn by several rows of the batch gets the priority of its last row: the rows' fractions differ).
+ * hp->loss is not read.  The backward pass runs through the head, layer 2 (dz = dh2 W2^T), the product (dphi = dz * h1 masked
+ * by relu'(phi); dh1 = (sum_i dz_i * phi_i, i order) masked by relu'(h1)) and both embeddings.
+ * Metrics row: [0] the weighted batch-mean loss, [1] / [2] the mean and std over a < A of the online Q at s taken as the
+ * SAMPLE mean over the N fractions tau_i (not the K-midpoint Q), the action histogram and the learned flag.  dmdqn_debug's
+ * q_all holds those sample means, q_next the K-midpoint Q of the network that picks a*, tq_all the mean of the N' sampled
+ * target values of every action; y is not written.
+ *   n_tau N, n_tau_prime N', n_policy K   each in [1, DMDQN_IQN_MAX_TAU]
+ *   n_cos      a multiple of 4 in [4, DMDQN_IQN_MAX_COS]
+ *   kappa      the Huber threshold: finite and >= 0
+ *   row_base   >= 0
+ *   key        device uint64 [n_nets]: each network's Philox key (read by the learn call only)
+ *   scratch    caller-owned device memory of at least dmdqn_iqn_scratch_bytes, 16-byte aligned (learn and debug only)
+ * Every call below refuses, before anything is launched: counts outside their range, a bad n_cos, kappa negative, NaN or
+ * infinite, row_base < 0, hp->precision other than DMDQN_PRECISION_FP32, hp->dueling != 0, NULL or misaligned pointers (a
+ * NULL key for learn) and a short scratch. */
+typedef struct dmdqn_iqn {
+    int32_t n_tau, n_tau_prime, n_policy, n_cos;
+    double kappa;
+    int64_t row_base;
+    const uint64_t* key;
+    void* scratch;
+    size_t scratch_bytes;
+} dmdqn_iqn;
+#define DMDQN_IQN_MAX_TAU 64
+#define DMDQN_IQN_MAX_COS 128
+
+typedef struct dmdqn_iqn_layout {
+    int64_t w1, b1, w2, b2, w3, b3, wphi, bphi, end, stride;
+} dmdqn_iqn_layout;
+int dmdqn_param_layout_iqn(const dmdqn_dims* dims, int32_t n_cos, dmdqn_iqn_layout* out);
+int dmdqn_iqn_scratch_bytes(const dmdqn_dims* dims, const dmdqn_iqn* iqn, size_t* out_bytes);
+
+/* One IQN learn step up to the gradient: the sample kernel of dmdqn_learn (learn_step, Adam scalars, n-step and prioritized
+ * rows), then iqn_target_kernel, iqn_online_kernel and iqn_wgrad_kernel.  grads_out[n_nets][stride] receives dL/dtheta for
+ * every float of [0, end) with the loss mean over global_batch (>= batch).  Finish with dmdqn_adam_apply_iqn. */
+int dmdqn_learn_grads_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_iqn* iqn, const dmdqn_replay* replay,
+                          const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
+                          float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Adam + target sync on IQN blocks, as dmdqn_adam_apply_dist: global_clipnorm == 0 is dmdqn_adam_apply's arithmetic,
+ * global_clipnorm > 0 (finite) dmdqn_clip_adam_apply's with the norm over [0, end) (Wphi and bphi included). */
+int dmdqn_adam_apply_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, int32_t n_cos,
+                         const float* grads, double global_clipnorm, float* norms_out, void* workspace, size_t workspace_bytes,
+                         void* stream);
+
+/* dmdqn_act on IQN blocks: q_out holds the K-midpoint Q (0 for a >= A), the action is its argmax under dmdqn_act's epsilon
+ * rule, and exploring agents skip the forward pass (their q_out rows are untouched).  iqn->key, kappa, row_base, n_tau,
+ * n_tau_prime and the scratch are not used. */
+int dmdqn_act_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_iqn* iqn, const float* obs, int32_t obs_in_stride,
+                  const double* eps, const uint32_t* w_explore, const uint32_t* w_action, int32_t* actions_out, float* q_out,
+                  void* stream);
+
+/* dmdqn_sync_target over the whole IQN stride. */
+int dmdqn_sync_target_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, int32_t n_cos, const uint8_t* mask, double tau,
+                          void* stream);
+
+/* The scratch's views after dmdqn_learn_grads_iqn: tau [n_nets][B][N], tau_prime [n_nets][B][N'], target (T) [n_nets][B][N'],
+ * theta [n_nets][B][N] (the online values of the taken action), grad [n_nets][B][N] ((w_r g_i) / loss_batch), and the
+ * activation gradients of every (row, fraction) at s, fraction-major: dh2 and dphi [n_nets][N][B][H] (dmdqn_debug's dh1
+ * holds dh1 [n_nets][B][H]). */
+typedef struct dmdqn_iqn_views {
+    const float* tau; const float* tau_prime; const float* target; const float* theta; const float* grad;
+    const float* dh2; const float* dphi;
+} dmdqn_iqn_views;
+int dmdqn_debug_iqn(const dmdqn_dims* dims, const dmdqn_iqn* iqn, dmdqn_iqn_views* out);
 
 #ifdef __cplusplus
 }
