@@ -113,6 +113,14 @@ class IqnViews(C.Structure):
 
 IQN_MAX_TAU, IQN_MAX_COS = 64, 128
 
+
+class RainbowLayout(C.Structure):
+    _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "w2", "b2", "w3", "b3", "wv", "bv", "end", "stride")]
+
+
+class RainbowViews(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("target_dist", "h2", "dlogits", "head")]
+
 MAX_PEERS, PEER_BLOCKS, PEER_TIMEOUT = 8, 128, 77
 
 
@@ -196,6 +204,19 @@ SIGNATURES = {
     "dmdqn_act_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Iqn), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "dmdqn_sync_target_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.c_int32, _P, C.c_double, _P]),
     "dmdqn_debug_iqn": (C.c_int, [C.POINTER(Dims), C.POINTER(Iqn), C.POINTER(IqnViews)]),
+    "dmdqn_param_layout_rainbow": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(RainbowLayout)]),
+    "dmdqn_noise_layout_rainbow": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(NoiseRecord)]),
+    "dmdqn_rainbow_scratch_bytes": (C.c_int, [C.POINTER(Dims), C.c_int32, C.POINTER(C.c_size_t)]),
+    "dmdqn_rainbow_fold": (C.c_int, [C.POINTER(Dims), C.POINTER(Dist), C.POINTER(Nets), C.POINTER(Noisy), _P]),
+    "dmdqn_learn_grads_rainbow": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Dist), C.POINTER(Replay),
+                                            C.POINTER(Nets), C.POINTER(Noisy), _P, _P, C.c_int32, _P, _P, _P, C.c_size_t, _P]),
+    "dmdqn_adam_apply_rainbow": (C.c_int, [C.POINTER(Dims), C.POINTER(HParams), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32,
+                                           _P, _P, C.c_size_t, _P]),
+    "dmdqn_act_rainbow": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.POINTER(Dist), _P, C.c_int32, _P,
+                                    _P, _P, _P, _P, _P]),
+    "dmdqn_sync_target_rainbow": (C.c_int, [C.POINTER(Dims), C.POINTER(Nets), C.POINTER(Noisy), C.c_int32, _P, C.c_double,
+                                            _P]),
+    "dmdqn_debug_rainbow": (C.c_int, [C.POINTER(Dims), C.POINTER(Dist), C.POINTER(RainbowViews)]),
 }
 
 _lib = None

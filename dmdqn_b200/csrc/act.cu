@@ -412,6 +412,103 @@ act_quantile_kernel(dmdqn_dims d, Layout L, int n_quantiles, const float* __rest
     }
 }
 
+// Rainbow heads (include/dmdqn_b200.h dmdqn_rainbow_layout): act_dist_kernel's scheme on the per-atom folded head, formed in
+// registers: thread (group, j) of CTA `rank` loads the four advantage weights of atom j in row k and Wv[k][j] (NOISY: each as
+// mu + sigma * eps with the online noise at the network's learn_step), folds them with head_fold and keeps column rank.
+// The trunk is gemv_slice_noisy (NOISY) or act_trunk (mu alone).  (act_dist_kernel keeps its own head: see
+// act_quantile_kernel.)
+template <int H, bool NOISY>
+__global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads, 4)
+act_rainbow_kernel(dmdqn_dims d, RainbowLayout RL, int n_atoms, double v_min, double dz64, const float* __restrict__ theta,
+                   const float* __restrict__ obs, int stride, const double* __restrict__ eps,
+                   const uint32_t* __restrict__ w_explore, const uint32_t* __restrict__ w_action, int32_t* __restrict__ actions,
+                   float* __restrict__ q_out, ActNoise nz) {
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int a = blockIdx.x / kActCluster, rank = (int)cluster.block_rank();
+    const bool explore = (double)w_explore[a] < eps[a] * 4294967296.0;
+    if (explore) {
+        if (threadIdx.x == 0 && rank == 0) actions[a] = (int32_t)__umulhi(w_action[a], (uint32_t)d.n_actions);
+        return;
+    }
+    const Layout& L = RL.L;
+    const int Dp = d.obs_stride;
+    float* xs = smem;                        // [Dp]
+    float* h1 = xs + Dp;                     // [H]
+    float* h2 = h1 + H;                      // [H]
+    float* part = h2 + H;                    // [1024]: trunk partials, then head partials [4][64] and rank 0's Q[4] at 512
+    float* lg = part + kActThreads * 4;      // [64] logits
+    float* zs = lg + kDistMaxAtoms;          // [64] support
+    float* rec = zs + kDistMaxAtoms;         // NOISY: the online noise record
+    const int net = d.n_nets == 1 ? 0 : a;
+    const float* P = theta + (size_t)net * L.stride;
+    const float* S = nullptr;
+    const int np = (n_atoms + 3) / 4 * 4, nh = 4 * np;
+    if constexpr (NOISY) {
+        S = nz.sigma + (size_t)net * L.stride;
+        noise_record_build_rainbow(rec, nz.R, d.obs_dim, d.n_actions, n_atoms, np, __ldg(nz.key + net),
+                                   (uint32_t)__ldg(nz.learn_step + net), 0);
+        for (int c = threadIdx.x; c < Dp; c += kActThreads) xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
+        __syncthreads();
+        gemv_slice_noisy(cluster, P + L.w1, S + L.w1, P + L.b1, S + L.b1, rec + nz.R.off[0], rec + nz.R.off[1], xs, h1, part,
+                         Dp, H, rank);
+        gemv_slice_noisy(cluster, P + L.w2, S + L.w2, P + L.b2, S + L.b2, rec + nz.R.off[2], rec + nz.R.off[3], h1, h2, part,
+                         H, H, rank);
+    } else {
+        act_trunk<H>(cluster, d, L, P, obs + (size_t)a * stride, xs, h1, h2, part, rank);
+    }
+
+    // the folded head weight of column rank * Np + j in row k (k == H: the bias), in act_dist_kernel's column
+    auto folded = [&](int k, int j) {
+        const float* w = P + (k < H ? L.w3 + (size_t)k * nh : L.b3) + j;
+        const int64_t vo = (k < H ? RL.wv + (int64_t)k * np : RL.bv) + j;
+        float x[4] = {__ldg(w), __ldg(w + np), __ldg(w + 2 * np), __ldg(w + 3 * np)};
+        float v = __ldg(P + vo);
+        if constexpr (NOISY) {
+            const float* s = S + (w - P);
+            const float fi = k < H ? rec[nz.R.off[4] + k] : 1.f, vi = k < H ? rec[nz.R.off[6] + k] : 1.f;
+            const float* fo = rec + nz.R.off[5] + j;
+#pragma unroll
+            for (int b = 0; b < 4; ++b) {
+                const float e = k < H ? __fmul_rn(fi, fo[b * np]) : fo[b * np];
+                x[b] = noisy_weight(x[b], __ldg(s + b * np), e);
+            }
+            const float fv = rec[nz.R.off[7] + j];
+            v = noisy_weight(v, __ldg(S + vo), k < H ? __fmul_rn(vi, fv) : fv);
+        }
+        head_fold(x, v, d.n_actions);
+        return rank == 0 ? x[0] : rank == 1 ? x[1] : rank == 2 ? x[2] : x[3];
+    };
+    const int j = threadIdx.x & 63, grp = threadIdx.x >> 6;
+    const bool mine = rank < d.n_actions;
+    if (mine && j < np) {
+        float s = 0.f;
+        for (int k = grp; k < H; k += 4) s = fmaf(h2[k], folded(k, j), s);
+        part[grp * 64 + j] = s;
+    }
+    if (threadIdx.x < n_atoms) zs[threadIdx.x] = dist_z(v_min, dz64, threadIdx.x);
+    __syncthreads();
+    if (mine && threadIdx.x < n_atoms) {
+        float x = folded(H, threadIdx.x);
+        for (int g = 0; g < 4; ++g) x += part[g * 64 + threadIdx.x];
+        lg[threadIdx.x] = x;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float mx, s;
+        cluster.map_shared_rank(part, 0)[512 + rank] = mine ? dist_expect(lg, n_atoms, zs, mx, s) : 0.f;
+    }
+    cluster.sync();
+    if (threadIdx.x == 0 && rank == 0) {
+        const float* q = part + 512;
+        int best = 0;                                   // ties -> lowest index
+        for (int k = 1; k < d.n_actions; ++k) if (q[k] > q[best]) best = k;
+        actions[a] = best;
+        if (q_out)
+            for (int k = 0; k < 4; ++k) q_out[(size_t)a * 4 + k] = q[k];
+    }
+}
+
 // Implicit quantile networks (include/dmdqn_b200.h dmdqn_iqn): layer 1 as a column-split GEMV (h1 in every CTA), then CTA
 // `rank` forms phi of its H/4 columns at the K midpoints and broadcasts z = h1 * phi [K][H] over DSMEM; layer 2 is a small
 // GEMM per CTA (its H/4 columns for all K rows: every W2 row is loaded once per CTA and used for the K rows, FFMA in k
@@ -556,6 +653,39 @@ int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dis
         case 128: run(act_dist_kernel<128>); break;
         case 256: run(act_dist_kernel<256>); break;
         case 512: run(act_dist_kernel<512>); break;
+        default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
+    }
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy* noisy, const dmdqn_dist& ds,
+                       const float* obs, int32_t stride, const double* eps, const uint32_t* w1, const uint32_t* w2,
+                       int32_t* actions, float* q_out, cudaStream_t s) {
+    const int np = dist_np(ds.n_atoms);
+    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
+    const double dz64 = (ds.v_max - ds.v_min) / (ds.n_atoms - 1);
+    ActNoise nz = {};
+    nz.R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
+    size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + 2 * kDistMaxAtoms) * sizeof(float);
+    if (noisy) {
+        nz.sigma = noisy->sigma; nz.key = noisy->key; nz.learn_step = nets.learn_step;
+        smem += (size_t)nz.R.stride * sizeof(float);
+    }
+    const dim3 grid(d.n_agents * kActCluster);
+    auto run = [&](auto kernel) {
+        kernel<<<grid, kActThreads, smem, s>>>(d, RL, ds.n_atoms, ds.v_min, dz64, nets.theta, obs, stride, eps, w1, w2, actions,
+                                               q_out, nz);
+    };
+    switch (d.hidden * 2 + (noisy ? 1 : 0)) {
+        case 128: run(act_rainbow_kernel<64, false>); break;
+        case 129: run(act_rainbow_kernel<64, true>); break;
+        case 256: run(act_rainbow_kernel<128, false>); break;
+        case 257: run(act_rainbow_kernel<128, true>); break;
+        case 512: run(act_rainbow_kernel<256, false>); break;
+        case 513: run(act_rainbow_kernel<256, true>); break;
+        case 1024: run(act_rainbow_kernel<512, false>); break;
+        case 1025: run(act_rainbow_kernel<512, true>); break;
         default: DMDQN_CHECK_ARG(false, "hidden=%d: the act kernel is built for 64, 128, 256, 512", d.hidden);
     }
     DMDQN_CUDA(cudaGetLastError());

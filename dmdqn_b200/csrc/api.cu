@@ -562,7 +562,9 @@ static int check_dist_hp(const dmdqn_hparams* hp) {
     DMDQN_CHECK_ARG(hp != nullptr, "dist: hp is NULL");
     DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32,
                     "precision=%d: distributional networks run the fp32 (FFMA) path only", hp->precision);
-    DMDQN_CHECK_ARG(hp->dueling == 0, "dueling=%d: dueling heads are not supported with distributional networks", hp->dueling);
+    DMDQN_CHECK_ARG(hp->dueling == 0,
+                    "dueling=%d: dueling heads are not supported with distributional networks (dueling noisy C51 heads: the "
+                    "dmdqn_*_rainbow calls)", hp->dueling);
     return DMDQN_OK;
 }
 
@@ -839,6 +841,140 @@ int dmdqn_debug_iqn(const dmdqn_dims* dims, const dmdqn_iqn* iqn, dmdqn_iqn_view
     const IqnArgs Q = make_iqn_args(*dims, *iqn);
     out->tau = Q.tau; out->tau_prime = Q.tau_p; out->target = Q.t; out->theta = Q.theta; out->grad = Q.grad;
     out->dh2 = Q.h2; out->dphi = Q.phi;
+    return DMDQN_OK;
+}
+
+// Rainbow calls (include/dmdqn_b200.h dmdqn_rainbow_layout): dmdqn_dist's atom and support checks, the Rainbow scratch,
+// dueling == 1 where hparams are taken, and dmdqn_noisy's pointer checks; every check runs before anything is launched.
+static int check_rainbow(const dmdqn_dims* dims, const dmdqn_dist* ds, bool scratch) {
+    if (int rc = check_dist(dims, ds, false)) return rc;
+    if (scratch) {
+        DMDQN_CHECK_ARG(ds->scratch && aligned16(ds->scratch), "rainbow: scratch is NULL or not 16-byte aligned");
+        const size_t need = make_rainbow_scratch(*dims, dist_np(ds->n_atoms)).total;
+        DMDQN_CHECK_ARG(ds->scratch_bytes >= need, "rainbow: scratch has %zu bytes, %zu needed", ds->scratch_bytes, need);
+    }
+    return DMDQN_OK;
+}
+
+static int check_rainbow_hp(const dmdqn_hparams* hp) {
+    DMDQN_CHECK_ARG(hp != nullptr, "rainbow: hp is NULL");
+    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32, "precision=%d: Rainbow networks run the fp32 (FFMA) path only",
+                    hp->precision);
+    DMDQN_CHECK_ARG(hp->dueling == 1, "dueling=%d: Rainbow blocks carry the value stream, so hp->dueling must be 1", hp->dueling);
+    return DMDQN_OK;
+}
+
+int dmdqn_param_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_rainbow_layout* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const RainbowLayout r = make_layout_rainbow(dims->obs_stride, dims->hidden, dist_np(n_atoms));
+    out->w1 = r.L.w1; out->b1 = r.L.b1; out->w2 = r.L.w2; out->b2 = r.L.b2; out->w3 = r.L.w3; out->b3 = r.L.b3;
+    out->wv = r.wv; out->bv = r.bv; out->end = r.L.end; out->stride = r.L.stride;
+    return DMDQN_OK;
+}
+
+int dmdqn_noise_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_noise_record* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const int np = dist_np(n_atoms);
+    const NoiseRec r = make_noise_rec(dims->obs_stride, dims->hidden, 4 * np, np);
+    int64_t* f[8] = {&out->w1_in, &out->w1_out, &out->w2_in, &out->w2_out, &out->w3_in, &out->w3_out, &out->v_in, &out->v_out};
+    for (int v = 0; v < 8; ++v) *f[v] = r.off[v];
+    out->stride = r.stride;
+    return DMDQN_OK;
+}
+
+int dmdqn_rainbow_scratch_bytes(const dmdqn_dims* dims, int32_t n_atoms, size_t* out_bytes) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    DMDQN_CHECK_ARG(out_bytes != nullptr, "out_bytes is NULL");
+    *out_bytes = make_rainbow_scratch(*dims, dist_np(n_atoms)).total;
+    return DMDQN_OK;
+}
+
+int dmdqn_rainbow_fold(const dmdqn_dims* dims, const dmdqn_dist* dist, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                       void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_rainbow(dims, dist, true))) return rc;
+    if ((rc = check_noisy(nets, noisy, false))) return rc;
+    return launch_rainbow_fold(*dims, *dist, *nets, *noisy, (cudaStream_t)stream);
+}
+
+int dmdqn_learn_grads_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_dist* dist,
+                              const dmdqn_replay* replay, const dmdqn_nets* nets, const dmdqn_noisy* noisy, const void* draws,
+                              const uint8_t* learn_mask, int32_t global_batch, float* grads_out, float* metrics_out,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    if ((rc = check_rainbow_hp(hp))) return rc;
+    if ((rc = check_rainbow(dims, dist, true))) return rc;
+    if ((rc = check_noisy(nets, noisy, true))) return rc;
+    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = launch_rainbow_fold(*dims, *dist, *nets, *noisy, s))) return rc;
+    dmdqn_nets eff = *nets;
+    eff.theta = noisy->eff;
+    eff.theta_tgt = noisy->eff_tgt;
+    if ((rc = launch_sample(*dims, *hp, *replay, eff, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
+    return launch_learn_rainbow(*dims, *hp, *replay, eff, *dist, metrics_out, (char*)workspace, w, grads_out, global_batch, s);
+}
+
+int dmdqn_adam_apply_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                             int32_t n_atoms, const float* grads, void* workspace, size_t workspace_bytes, void* stream) {
+    Workspace w;
+    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    if (rc) return rc;
+    if ((rc = check_rainbow_hp(hp))) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    if ((rc = check_noisy(nets, noisy, true))) return rc;
+    DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_rainbow: grads is NULL or not 16-byte aligned");
+    return launch_adam_apply_rainbow(*dims, *hp, *nets, *noisy, n_atoms, grads, (char*)workspace, w, (cudaStream_t)stream);
+}
+
+int dmdqn_act_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, const dmdqn_dist* dist,
+                      const float* obs, int32_t obs_in_stride, const double* eps, const uint32_t* w_explore,
+                      const uint32_t* w_action, int32_t* actions_out, float* q_out, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_rainbow(dims, dist, false))) return rc;
+    DMDQN_CHECK_ARG(nets && nets->theta && aligned16(nets->theta), "act_rainbow: theta is NULL or not 16-byte aligned");
+    if (noisy)
+        DMDQN_CHECK_ARG(noisy->sigma && aligned16(noisy->sigma) && noisy->key && nets->learn_step,
+                        "act_rainbow: sigma, key or learn_step is NULL, or sigma is not 16-byte aligned");
+    DMDQN_CHECK_ARG(obs && eps && w_explore && w_action && actions_out, "act_rainbow: NULL argument");
+    DMDQN_CHECK_ARG(obs_in_stride >= dims->obs_dim, "obs_in_stride=%d < obs_dim=%d", obs_in_stride, dims->obs_dim);
+    return launch_act_rainbow(*dims, *nets, noisy, *dist, obs, obs_in_stride, eps, w_explore, w_action, actions_out, q_out,
+                              (cudaStream_t)stream);
+}
+
+int dmdqn_sync_target_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t n_atoms,
+                              const uint8_t* mask, double tau, void* stream) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_atoms(n_atoms))) return rc;
+    if ((rc = check_noisy(nets, noisy, false))) return rc;
+    return launch_sync_target_rainbow(*dims, *nets, *noisy, n_atoms, mask, tau, (cudaStream_t)stream);
+}
+
+int dmdqn_debug_rainbow(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_rainbow_views* out) {
+    int rc = validate_dims(dims);
+    if (rc) return rc;
+    if ((rc = check_rainbow(dims, dist, true))) return rc;
+    DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
+    const DistArgs D = make_dist_args(*dims, *dist);
+    out->target_dist = D.m;
+    out->h2 = D.h2;
+    out->dlogits = D.dx;
+    out->head = reinterpret_cast<const float*>(static_cast<const char*>(dist->scratch) + make_rainbow_scratch(*dims, D.np).head);
     return DMDQN_OK;
 }
 

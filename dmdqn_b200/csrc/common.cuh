@@ -94,13 +94,14 @@ __host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 
 // Offsets (floats) of the eight factor vectors inside one network's noise record for one set (include/dmdqn_b200.h
 // dmdqn_noise_record): off[2 * layer + side], layer 0..3 = W1, W2, W3, value head, side 0 = inputs, 1 = outputs; off[8]
-// is the end of the last vector, `stride` the record's stride (a network's two sets are adjacent records).
+// is the end of the last vector, `stride` the record's stride (a network's two sets are adjacent records).  nh / nv: the
+// widths of the head's and the value head's output vectors (4 and 4 for plain and dueling blocks, 4 * Np and Np for Rainbow).
 struct NoiseRec {
     int32_t off[9];
     int32_t stride;
 };
-__host__ __device__ inline NoiseRec make_noise_rec(int dp, int h) {
-    const int32_t len[8] = {dp, h, h, h, h, 4, h, 4};
+__host__ __device__ inline NoiseRec make_noise_rec(int dp, int h, int nh = 4, int nv = 4) {
+    const int32_t len[8] = {dp, h, h, h, h, nh, h, nv};
     NoiseRec r;
     r.off[0] = 0;
     for (int v = 0; v < 8; ++v) r.off[v + 1] = r.off[v] + len[v];
@@ -225,6 +226,67 @@ __device__ __forceinline__ float dist_expect(const float* x, int n, const float*
     float q = 0.f;
     for (int j = 0; j < n; ++j) q = fmaf(__fdiv_rn(expf(__fsub_rn(x[j], mx)), s), z[j], q);
     return q;
+}
+
+// Rainbow networks (include/dmdqn_b200.h dmdqn_rainbow_layout): the C51 block with the value stream Wv[H][Np] | bv[Np] after
+// b3 (at the C51 end); Adam covers all of it.
+struct RainbowLayout {
+    Layout L;                         // L.end = bv + Np
+    int64_t wv, bv;
+};
+__host__ __device__ inline RainbowLayout make_layout_rainbow(int dp, int h, int np) {
+    RainbowLayout r;
+    r.L = make_layout_dist(dp, h, np);
+    r.wv = r.L.end;
+    r.bv = r.wv + (int64_t)h * np;
+    r.L.end = r.bv + np;
+    r.L.stride = (r.L.end + 31) / 32 * 32;
+    return r;
+}
+// The Rainbow scratch: the C51 regions, then the folded heads W3e[H][4 * Np] | b3e[4 * Np] of the online (0) and the target
+// (1) network, [2][n_nets][(H + 1) * 4 * Np] floats.
+struct RainbowScratch {
+    DistScratch dist;
+    size_t head, total;
+};
+inline RainbowScratch make_rainbow_scratch(const dmdqn_dims& d, int np) {
+    RainbowScratch s;
+    s.dist = make_dist_scratch(d, np);
+    s.head = s.dist.total;
+    s.total = s.head + (2 * (size_t)d.n_nets * (d.hidden + 1) * 4 * np * 4 + 255) / 256 * 256;
+    return s;
+}
+// The Rainbow noise record (dmdqn_noise_layout_rainbow): output factor i of W3 is column a * Np + j (0 unless a < A and
+// j < N), entry j of the value head's outputs is atom j (0 for j >= N).  Otherwise noise_record_build's rule.
+__device__ __forceinline__ void noise_record_build_rainbow(float* rec, const NoiseRec& R, int obs_dim, int n_actions, int n_atoms,
+                                                           int np, uint64_t key, uint32_t t, int set) {
+    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) {
+        int v = 0;
+        while (v < 8 && e >= R.off[v + 1]) ++v;
+        const int i = e - R.off[v];
+        const bool valid = v == 0 ? i < obs_dim : v == 5 ? i / np < n_actions && i % np < n_atoms : v == 7 ? i < n_atoms : v < 8;
+        rec[e] = valid ? noise_factor(key, (uint32_t)i, v, set, t) : 0.f;
+    }
+}
+// noise_eps4 on a Rainbow block: W3 / b3 take the head's output side at column (e - w3) % (4 * Np), Wv / bv the value head's
+// input side and output side at atom (e - wv) % Np.  A float4 never straddles two rows (Np is a multiple of 4).
+__device__ __forceinline__ float4 noise_eps4_rainbow(const float* rec, const NoiseRec& R, const RainbowLayout& RL, int H, int np,
+                                                     int64_t e) {
+    const Layout& L = RL.L;
+    const int nh = 4 * np;
+    auto outer = [&](float fi, const float* fo) {
+        return make_float4(__fmul_rn(fi, fo[0]), __fmul_rn(fi, fo[1]), __fmul_rn(fi, fo[2]), __fmul_rn(fi, fo[3]));
+    };
+    auto vec = [](const float* f) { return make_float4(f[0], f[1], f[2], f[3]); };
+    if (e < L.b1) return outer(rec[R.off[0] + e / H], rec + R.off[1] + e % H);
+    if (e < L.w2) return vec(rec + R.off[1] + (e - L.b1));
+    if (e < L.b2) return outer(rec[R.off[2] + (e - L.w2) / H], rec + R.off[3] + (e - L.w2) % H);
+    if (e < L.w3) return vec(rec + R.off[3] + (e - L.b2));
+    if (e < L.b3) return outer(rec[R.off[4] + (e - L.w3) / nh], rec + R.off[5] + (e - L.w3) % nh);
+    if (e < RL.wv) return vec(rec + R.off[5] + (e - L.b3));
+    if (e < RL.bv) return outer(rec[R.off[6] + (e - RL.wv) / np], rec + R.off[7] + (e - RL.wv) % np);
+    if (e < L.end) return vec(rec + R.off[7] + (e - RL.bv));
+    return make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
 // Quantile (QR-DQN) networks (include/dmdqn_b200.h dmdqn_quantile): the C51 head layout, scratch and Adam range for
@@ -587,5 +649,16 @@ int launch_adam_apply_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
 int launch_sync_target_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, int n_cos, const uint8_t* mask, double tau, cudaStream_t s);
 int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn& q, const float* obs, int32_t stride,
                    const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
+int launch_rainbow_fold(const dmdqn_dims& d, const dmdqn_dist& ds, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s);
+int launch_learn_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& eff,
+                         const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                         cudaStream_t s);
+int launch_adam_apply_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
+                              int n_atoms, const float* grads, char* ws, const Workspace& w, cudaStream_t s);
+int launch_sync_target_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy& nz, int n_atoms,
+                               const uint8_t* mask, double tau, cudaStream_t s);
+int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy* noisy, const dmdqn_dist& ds,
+                       const float* obs, int32_t stride, const double* eps, const uint32_t* w1, const uint32_t* w2,
+                       int32_t* actions, float* q_out, cudaStream_t s);
 
 }  // namespace dmdqn

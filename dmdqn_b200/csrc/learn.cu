@@ -680,6 +680,94 @@ noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, con
     }
 }
 
+// Rainbow (include/dmdqn_b200.h dmdqn_rainbow_layout).  Noise fold: noisy_fold_kernel with the Rainbow record and eps.
+__global__ void __launch_bounds__(kNoisyThreads)
+rainbow_noisy_fold_kernel(RainbowLayout RL, NoiseRec R, int H, int obs_dim, int n_actions, int n_atoms, int np,
+                          const dmdqn_nets nets, const dmdqn_noisy nz, int64_t per) {
+    extern __shared__ __align__(16) float rec[];
+    const int g = blockIdx.y, set = blockIdx.z;
+    noise_record_build_rainbow(rec, R, obs_dim, n_actions, n_atoms, np, __ldg(nz.key + g), (uint32_t)__ldg(nets.learn_step + g),
+                               set);
+    __syncthreads();
+    if (blockIdx.x == 0)
+        for (int e = threadIdx.x; e < R.stride; e += blockDim.x) nz.noise[((size_t)g * 2 + set) * R.stride + e] = rec[e];
+    const size_t base = (size_t)g * RL.L.stride;
+    const float4* mu = reinterpret_cast<const float4*>((set ? nets.theta_tgt : nets.theta) + base);
+    const float4* sg = reinterpret_cast<const float4*>((set ? nz.sigma_tgt : nz.sigma) + base);
+    float4* out = reinterpret_cast<float4*>((set ? nz.eff_tgt : nz.eff) + base);
+    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, RL.L.stride / 4);
+    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        const float4 m = __ldg(mu + i), s = __ldg(sg + i), e = noise_eps4_rainbow(rec, R, RL, H, np, i * 4);
+        out[i] = make_float4(noisy_weight(m.x, s.x, e.x), noisy_weight(m.y, s.y, e.y), noisy_weight(m.z, s.z, e.z),
+                             noisy_weight(m.w, s.w, e.w));
+    }
+}
+
+// Per-atom head fold: W3e | b3e of the effective online (blockIdx.z = 0) and target (1) block of network blockIdx.y into
+// head[z][y], one thread per (row k <= H, atom j < Np): head_fold of {W3[k][b * Np + j]}_b with Wv[k][j] (row H: b3 / bv).
+__global__ void __launch_bounds__(256) rainbow_head_fold_kernel(RainbowLayout RL, int H, int n_actions, int n_atoms, int np,
+                                                                const float* __restrict__ eff, const float* __restrict__ eff_tgt,
+                                                                float* __restrict__ head) {
+    const int g = blockIdx.y, nh = 4 * np;
+    const float* P = (blockIdx.z ? eff_tgt : eff) + (size_t)g * RL.L.stride;
+    float* out = head + ((size_t)blockIdx.z * gridDim.y + g) * (size_t)(H + 1) * nh;
+    const int total = (H + 1) * np;
+    for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < total; f += gridDim.x * blockDim.x) {
+        const int k = f / np, j = f % np;
+        const float* row = P + (k < H ? RL.L.w3 + (int64_t)k * nh : RL.L.b3);
+        float x[4] = {__ldg(row + j), __ldg(row + np + j), __ldg(row + 2 * np + j), __ldg(row + 3 * np + j)};
+        head_fold(x, __ldg(P + (k < H ? RL.wv + (int64_t)k * np : RL.bv) + j), n_actions);
+        float* o = out + (size_t)k * nh + j;
+#pragma unroll
+        for (int a = 0; a < 4; ++a) o[a * np] = j < n_atoms ? x[a] : 0.f;
+    }
+}
+
+// Projection of the folded head's gradient, in place over the W3 / b3 rows of grads, and Wv / bv from its sums: head_project
+// per (row k <= H, atom j < Np) of every network that learned this step; atoms j >= N get gradient 0.
+__global__ void __launch_bounds__(256) rainbow_project_kernel(RainbowLayout RL, int H, int n_actions, int n_atoms, int np,
+                                                              const int32_t* __restrict__ active, float* __restrict__ grads) {
+    const int g = blockIdx.y, nh = 4 * np;
+    if (!active[g]) return;
+    float* G = grads + (size_t)g * RL.L.stride;
+    const int total = (H + 1) * np;
+    for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < total; f += gridDim.x * blockDim.x) {
+        const int k = f / np, j = f % np;
+        float* row = G + (k < H ? RL.L.w3 + (int64_t)k * nh : RL.L.b3) + j;
+        float x[4] = {row[0], row[np], row[2 * np], row[3 * np]};
+        const float sv = head_project(x, n_actions);
+        const bool ok = j < n_atoms;
+#pragma unroll
+        for (int a = 0; a < 4; ++a) row[a * np] = ok ? x[a] : 0.f;
+        G[(k < H ? RL.wv + (int64_t)k * np : RL.bv) + j] = ok ? sv : 0.f;
+    }
+}
+
+// noisy_adam_apply_kernel over a Rainbow block: eps from the Rainbow record of set 0.
+__global__ void __launch_bounds__(kNoisyThreads)
+rainbow_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, RainbowLayout RL, NoiseRec R, int np,
+                          const float* __restrict__ grads, int64_t per) {
+    extern __shared__ __align__(16) float rec[];
+    const int g = blockIdx.y;
+    if (!A.active[g] || *reinterpret_cast<volatile int*>(A.error) != 0) return;
+    const float* src = nz.noise + (size_t)g * 2 * R.stride;
+    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) rec[e] = src[e];
+    __syncthreads();
+    const AdamStep k = adam_step(A, g);
+    const int H = A.d.hidden;
+    const size_t base = (size_t)g * RL.L.stride;
+    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, RL.L.end / 4);
+    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        const float4 g4 = *reinterpret_cast<const float4*>(grads + base + i * 4);
+        const float4 e = noise_eps4_rainbow(rec, R, RL, H, np, i * 4);
+        const float gm[4] = {g4.x, g4.y, g4.z, g4.w};
+        const float gs[4] = {__fmul_rn(g4.x, e.x), __fmul_rn(g4.y, e.y), __fmul_rn(g4.z, e.z), __fmul_rn(g4.w, e.w)};
+        const size_t o = base + i * 4;
+        adam_vec4(k, gm, A.nets.theta + o, A.nets.adam_m + o, A.nets.adam_v + o, A.nets.theta_tgt + o);
+        adam_vec4(k, gs, nz.sigma + o, nz.sigma_m + o, nz.sigma_v + o, nz.sigma_tgt + o);
+    }
+}
+
 // CTAs per network (fold: per network and set) of the two noisy kernels: enough for two waves over the SMs, each CTA
 // streaming at least 2048 float4s.
 inline int noisy_chunks(int n_sm, int64_t pairs, int64_t n4) {
@@ -971,9 +1059,18 @@ __device__ __forceinline__ void head_target(float* m, const float* x, const Dist
     for (int j = 0; j < D.np; ++j) m[j] = j < D.n_atoms ? __fadd_rn(R, __fmul_rn(d, x[j])) : 0.f;
 }
 
+// The block through whose offsets A.L.w3 / A.L.b3 the distributional kernels read the head of network g's set `tgt` (P: that
+// set's parameter block): P itself, or for DUELING (Rainbow) the folded W3e[H][nh] | b3e[nh] at A.head[tgt] + g * head_stride,
+// which keeps the block's b3 - w3 spacing (H * nh), so the head code is the same with another base.
+template <bool DUELING>
+__device__ __forceinline__ const float* dist_head_block(const LearnArgs& A, const float* P, int tgt, int g) {
+    if constexpr (DUELING) return A.head[tgt] + (size_t)g * A.head_stride - A.L.w3;
+    else return P;
+}
+
 // Distributional K3: online and target trunk + head on s', expected Q, a*, the head's target (C51: the projected
-// distribution, QR-DQN: the target samples) -> D.m.
-template <int H, class DA>
+// distribution, QR-DQN: the target samples) -> D.m.  DUELING: the head is the folded Rainbow head (dist_head_block).
+template <int H, bool DUELING = false, class DA>
 __device__ __forceinline__ void dist_target_body(const LearnArgs& A, const DA& D) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
@@ -993,7 +1090,7 @@ __device__ __forceinline__ void dist_target_body(const LearnArgs& A, const DA& D
         store_relu<H>(acc, c, P + A.L.b1, S.Hs1, nullptr, r0, B);
         gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
         store_relu<H>(acc, c, P + A.L.b2, S.Hs2, nullptr, r0, B);
-        dist_head<H>(acc, c, S, P, A.L, D.nh);
+        dist_head<H>(acc, c, S, dist_head_block<DUELING>(A, P, pass, g), A.L, D.nh);
         float* qs = pass == 0 ? S.qs0 : S.qs1;
         for (int f = threadIdx.x; f < T::BM * 4; f += T::NT) {   // one thread per (row, action)
             const int i = f >> 2, a = f & 3;
@@ -1033,6 +1130,11 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_target_kernel(const Learn
 template <int H>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) quantile_target_kernel(const LearnArgs A, const QuantArgs D) {
     dist_target_body<H>(A, D);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) rainbow_target_kernel(const LearnArgs A, const DistArgs D) {
+    dist_target_body<H, true>(A, D);
 }
 
 // head_loss: the per-row loss of the online kernel over the logits Ls of the tile.  It leaves every action's expected Q
@@ -1153,8 +1255,8 @@ __device__ __forceinline__ void head_loss(const LearnArgs& A, const QuantArgs& D
 
 // Distributional K4a: forward on s (h1 -> workspace, h2 -> scratch), every action's expected Q, the head's loss (C51:
 // the cross-entropy of a_i against m, QR-DQN: the quantile Huber loss against T), the logit gradient dX (-> scratch),
-// dh2 = (dX W3^T) * relu'(h2), dh1, and the per-tile partials.
-template <int H, class DA>
+// dh2 = (dX W3^T) * relu'(h2), dh1, and the per-tile partials.  DUELING: the head is the folded Rainbow head.
+template <int H, bool DUELING = false, class DA>
 __device__ __forceinline__ void dist_online_body(const LearnArgs& A, const DA& D) {
     using T = Tile<H>;
     extern __shared__ __align__(16) float smem[];
@@ -1174,7 +1276,7 @@ __device__ __forceinline__ void dist_online_body(const LearnArgs& A, const DA& D
     store_relu<H>(acc, c, P + A.L.b1, S.Hs1, A.h1 + sb * H, r0, B);
     gemm_rowA<H, false>(acc, c, S.Hs1, T::LDH, P + A.L.w2, H, H, S.Ws);
     store_relu<H>(acc, c, P + A.L.b2, S.Hs2, D.h2 + sb * H, r0, B);
-    dist_head<H>(acc, c, S, P, A.L, nh);
+    dist_head<H>(acc, c, S, dist_head_block<DUELING>(A, P, 0, g), A.L, nh);
     head_loss<H>(A, D, S, r0, sb, rows);
 
     const size_t pt = (size_t)g * A.ws_tiles + rt;   // partial slot of this (network, row tile)
@@ -1199,7 +1301,7 @@ __device__ __forceinline__ void dist_online_body(const LearnArgs& A, const DA& D
             reinterpret_cast<float4*>(D.dx + (sb + r0 + i) * nh)[c4] = *reinterpret_cast<const float4*>(S.Ls + i * S.ldl + c4 * 4);
     }
     // dh2 = (dX W3^T) * relu'(h2), in place over h2
-    gemm_rowA<H, true>(acc, c, S.Ls, S.ldl, P + A.L.w3, nh, nh, S.Ws);
+    gemm_rowA<H, true>(acc, c, S.Ls, S.ldl, dist_head_block<DUELING>(A, P, 0, g) + A.L.w3, nh, nh, S.Ws);
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
         const int col = c.col0(half);
@@ -1264,6 +1366,11 @@ __global__ void __launch_bounds__(Tile<H>::NT, 1) dist_online_kernel(const Learn
 template <int H>
 __global__ void __launch_bounds__(Tile<H>::NT, 1) quantile_online_kernel(const LearnArgs A, const QuantArgs D) {
     dist_online_body<H>(A, D);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Tile<H>::NT, 1) rainbow_online_kernel(const LearnArgs A, const DistArgs D) {
+    dist_online_body<H, true>(A, D);
 }
 
 // Distributional K4b, gradients only (A.grads): dW2 = h1^T dh2, dW1 = s^T dh1 and dW3 = h2^T dX (column slabs of H) tiles
@@ -1389,13 +1496,21 @@ __global__ void __launch_bounds__(Tile<H>::NT) dist_wgrad_kernel(const LearnArgs
 }
 
 // The target and online kernels of the head of DA (C51 or QR-DQN), then dist_wgrad_kernel on Dw, the same head width
-// and scratch as DistArgs.
-template <int H, class DA>
+// and scratch as DistArgs.  RAINBOW: the C51 kernels that read the folded head.
+template <int H, class DA, bool RAINBOW = false>
 int launch_learn_dist_h(const LearnArgs& A, const DA& D, const DistArgs& Dw, cudaStream_t s) {
     using T = Tile<H>;
     constexpr bool qr = std::is_same<DA, QuantArgs>::value;
-    const auto target = [] { if constexpr (qr) return quantile_target_kernel<H>; else return dist_target_kernel<H>; }();
-    const auto online = [] { if constexpr (qr) return quantile_online_kernel<H>; else return dist_online_kernel<H>; }();
+    const auto target = [] {
+        if constexpr (qr) return quantile_target_kernel<H>;
+        else if constexpr (RAINBOW) return rainbow_target_kernel<H>;
+        else return dist_target_kernel<H>;
+    }();
+    const auto online = [] {
+        if constexpr (qr) return quantile_online_kernel<H>;
+        else if constexpr (RAINBOW) return rainbow_online_kernel<H>;
+        else return dist_online_kernel<H>;
+    }();
     const size_t smem = DistSmem<H>::bytes(A.d.obs_stride, D.nh);
     const size_t smem_w = sizeof(float) * 2 * T::KC * ((T::BM + 4) + T::LDW);
     static size_t cfg_t[kMaxDevices] = {}, cfg_o[kMaxDevices] = {}, cfg_w[kMaxDevices] = {};
@@ -2278,6 +2393,81 @@ int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const 
     const int chunks = noisy_chunks(n_sm, d.n_nets, n4);
     const int64_t per = (n4 + chunks - 1) / chunks;
     noisy_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, R, grads, per);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+// Rainbow: the noise fold into eff / eff_tgt, then the per-atom head fold of both into the scratch's head region.
+int launch_rainbow_fold(const dmdqn_dims& d, const dmdqn_dist& ds, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s) {
+    const int np = dist_np(ds.n_atoms);
+    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
+    int n_sm = 0;
+    if (int rc = device_sm_count(&n_sm)) return rc;
+    const int64_t n4 = RL.L.stride / 4;
+    const int chunks = noisy_chunks(n_sm, 2 * (int64_t)d.n_nets, n4);
+    const int64_t per = (n4 + chunks - 1) / chunks;
+    rainbow_noisy_fold_kernel<<<dim3(chunks, d.n_nets, 2), kNoisyThreads, R.stride * sizeof(float), s>>>(
+        RL, R, d.hidden, d.obs_dim, d.n_actions, ds.n_atoms, np, nets, nz, per);
+    DMDQN_CUDA(cudaGetLastError());
+    float* head = reinterpret_cast<float*>(static_cast<char*>(ds.scratch) + make_rainbow_scratch(d, np).head);
+    const int blocks = ((d.hidden + 1) * np + 255) / 256;
+    rainbow_head_fold_kernel<<<dim3(blocks, d.n_nets, 2), 256, 0, s>>>(RL, d.hidden, d.n_actions, ds.n_atoms, np, nz.eff,
+                                                                        nz.eff_tgt, head);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+// Rainbow learn step after the sample kernel: the C51 target / online kernels on the folded heads with the effective trunks,
+// dist_wgrad_kernel, and the projection of the head gradient onto W3 / b3 / Wv / bv.
+int launch_learn_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& eff,
+                         const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
+                         cudaStream_t s) {
+    LearnArgs A = make_learn_args(d, hp, rp, eff, ws, w, metrics, grads, loss_batch);
+    const DistArgs D = make_dist_args(d, ds);
+    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, D.np);
+    A.L = RL.L;
+    A.head_stride = (int64_t)(d.hidden + 1) * D.nh;
+    A.head[0] = reinterpret_cast<const float*>(static_cast<char*>(ds.scratch) + make_rainbow_scratch(d, D.np).head);
+    A.head[1] = A.head[0] + (size_t)d.n_nets * A.head_stride;
+    int rc = DMDQN_ERR_ARG;
+    switch (d.hidden) {
+        case 64: rc = launch_learn_dist_h<64, DistArgs, true>(A, D, D, s); break;
+        case 128: rc = launch_learn_dist_h<128, DistArgs, true>(A, D, D, s); break;
+        case 256: rc = launch_learn_dist_h<256, DistArgs, true>(A, D, D, s); break;
+        case 512: rc = launch_learn_dist_h<512, DistArgs, true>(A, D, D, s); break;
+        default: set_error("unsupported hidden width %d", d.hidden);
+    }
+    if (rc) return rc;
+    const int blocks = ((d.hidden + 1) * D.np + 255) / 256;
+    rainbow_project_kernel<<<dim3(blocks, d.n_nets), 256, 0, s>>>(RL, d.hidden, d.n_actions, D.n_atoms, D.np, A.active, grads);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_adam_apply_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
+                              int n_atoms, const float* grads, char* ws, const Workspace& w, cudaStream_t s) {
+    const int np = dist_np(n_atoms);
+    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
+    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    A.L = RL.L;
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
+    int n_sm = 0;
+    if (int rc = device_sm_count(&n_sm)) return rc;
+    const int64_t n4 = RL.L.end / 4;
+    const int chunks = noisy_chunks(n_sm, d.n_nets, n4);
+    const int64_t per = (n4 + chunks - 1) / chunks;
+    rainbow_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, RL, R, np, grads, per);
+    DMDQN_CUDA(cudaGetLastError());
+    return DMDQN_OK;
+}
+
+int launch_sync_target_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy& nz, int n_atoms,
+                               const uint8_t* mask, double tau, cudaStream_t s) {
+    const int64_t stride = make_layout_rainbow(d.obs_stride, d.hidden, dist_np(n_atoms)).L.stride;
+    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(stride, nets.theta, nets.theta_tgt, mask, (float)tau);
+    DMDQN_CUDA(cudaGetLastError());
+    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(stride, nz.sigma, nz.sigma_tgt, mask, (float)tau);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

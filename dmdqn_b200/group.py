@@ -57,7 +57,20 @@ DEFAULTS = {  # DQNAgent defaults, dqn_agent.py:112-127
     # for the online values and the targets, acting on the mean over iqn_num_policy_tau midpoints; the Huber threshold is
     # quantile_kappa
     "iqn": False, "iqn_num_tau": 8, "iqn_num_tau_prime": 8, "iqn_num_policy_tau": 32, "iqn_embedding_dim": 64,
+    # Rainbow (Hessel et al. 2018): C51 heads (num_atoms, v_min, v_max) with dueling value / advantage streams and noisy
+    # layers everywhere (noisy_sigma0), on top of whatever replay, n_step, double_dqn and target sync the config sets
+    "rainbow": False,
 }
+
+
+def _check_atoms_and_support(cfg: dict) -> None:
+    """The C51 keys num_atoms, v_min and v_max (distributional and Rainbow heads)."""
+    n = cfg["num_atoms"]
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 2 <= n <= N.DIST_MAX_ATOMS:
+        raise ValueError(f"num_atoms={n!r}: must be an integer in [2, {N.DIST_MAX_ATOMS}]")
+    lo, hi = cfg["v_min"], cfg["v_max"]
+    if any(isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v) for v in (lo, hi)) or lo >= hi:
+        raise ValueError(f"v_min={lo!r}, v_max={hi!r}: the support needs finite numbers with v_min < v_max")
 
 
 def dist_config(cfg: dict) -> dict:
@@ -68,21 +81,16 @@ def dist_config(cfg: dict) -> dict:
         raise ValueError(f"distributional={cfg['distributional']!r}: must be true or false")
     if not cfg["distributional"]:
         return cfg
-    n = cfg["num_atoms"]
-    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 2 <= n <= N.DIST_MAX_ATOMS:
-        raise ValueError(f"num_atoms={n!r}: must be an integer in [2, {N.DIST_MAX_ATOMS}]")
-    lo, hi = cfg["v_min"], cfg["v_max"]
-    if any(isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v) for v in (lo, hi)) or lo >= hi:
-        raise ValueError(f"v_min={lo!r}, v_max={hi!r}: the support needs finite numbers with v_min < v_max")
+    _check_atoms_and_support(cfg)
     if cfg["precision"] not in ("auto", "fp32"):
         raise ValueError(f"precision={cfg['precision']!r}: distributional networks run the fp32 (FFMA) learn path only; the "
                          "tcgen05 distributional kernels are not built yet (use precision: auto or fp32)")
     if cfg["dueling"]:
         raise ValueError("distributional=true cannot be combined with dueling=true yet: the per-atom dueling fold is not "
-                         "implemented")
+                         "implemented for plain C51 groups (dueling noisy C51 heads: use rainbow: true)")
     if cfg["noisy"]:
         raise ValueError("distributional=true cannot be combined with noisy=true yet: noisy distributional heads are not "
-                         "implemented")
+                         "implemented for plain C51 groups (dueling noisy C51 heads: use rainbow: true)")
     if cfg["loss"] != "mse":
         raise ValueError(f"loss={cfg['loss']!r}: distributional networks minimise the cross-entropy of the projected target; "
                          "the loss key does not apply (leave it at mse)")
@@ -117,6 +125,32 @@ def quantile_config(cfg: dict) -> dict:
     if cfg["loss"] != "mse":
         raise ValueError(f"loss={cfg['loss']!r}: quantile networks minimise the quantile Huber loss, whose threshold is "
                          "quantile_kappa; the loss key does not apply (leave it at mse)")
+    cfg["precision"] = "fp32"
+    return cfg
+
+
+def rainbow_config(cfg: dict) -> dict:
+    """Validate the Rainbow key of ``cfg`` and resolve its precision (in place; returns ``cfg``).  ``rainbow: true`` implies
+    C51 heads, dueling streams and noisy layers, so setting distributional, quantile, iqn, dueling or noisy as well is
+    refused, as are an explicit tcgen05 precision (``auto`` becomes fp32), the Huber loss key and global_clipnorm."""
+    if not isinstance(cfg["rainbow"], (bool, np.bool_)):
+        raise ValueError(f"rainbow={cfg['rainbow']!r}: must be true or false")
+    if not cfg["rainbow"]:
+        return cfg
+    for other in ("distributional", "quantile", "iqn", "dueling", "noisy"):
+        if cfg[other]:
+            raise ValueError(f"rainbow=true cannot be combined with {other}=true: rainbow is C51 heads with dueling streams "
+                             "and noisy layers already (leave the other keys at false)")
+    _check_atoms_and_support(cfg)
+    if cfg["precision"] not in ("auto", "fp32"):
+        raise ValueError(f"precision={cfg['precision']!r}: Rainbow networks run the fp32 (FFMA) learn path only (use "
+                         "precision: auto or fp32)")
+    if cfg["loss"] != "mse":
+        raise ValueError(f"loss={cfg['loss']!r}: Rainbow networks minimise the cross-entropy of the projected target; the "
+                         "loss key does not apply (leave it at mse)")
+    if cfg["global_clipnorm"] is not None:
+        raise ValueError("rainbow=true cannot be combined with global_clipnorm: the global norm over the mean and the sigma "
+                         "gradients is not implemented")
     cfg["precision"] = "fp32"
     return cfg
 
@@ -174,10 +208,11 @@ def _on_device(method):
 
 
 def keras_init(seed: int, state_size: int, hidden: int, action_size: int, dueling: bool = False,
-               n_cos: int = 0) -> list[torch.Tensor]:
+               n_cos: int = 0, value_size: int = 1) -> list[torch.Tensor]:
     """HeNormal hidden kernels, GlorotUniform head, zero biases (dqn_agent.py:166-181), as
     [W1,b1,W2,b2,W3,b3] in Keras ``get_weights()`` order, kernels ``[in,out]``.  ``dueling`` appends the value head
-    [Wv [H,1], bv [1]], Wv GlorotUniform drawn from the same generator after W3 (the other draws do not change).
+    [Wv [H,1], bv [1]], Wv GlorotUniform drawn from the same generator after W3 (the other draws do not change); Rainbow's
+    per-atom value stream is ``value_size`` = N wide ([Wv [H,N], bv [N]]).
     ``n_cos`` > 0 (IQN) appends the cosine embedding [Wphi [n_cos, H], bphi [H]], Wphi HeNormal (truncated, fan_in = n_cos)
     drawn after every other weight."""
     gen = torch.Generator().manual_seed(int(seed))
@@ -191,8 +226,8 @@ def keras_init(seed: int, state_size: int, hidden: int, action_size: int, duelin
     limit = math.sqrt(6.0 / (hidden + action_size))
     out += [(torch.rand(hidden, action_size, generator=gen) * 2 - 1) * limit, torch.zeros(action_size)]
     if dueling:
-        limit = math.sqrt(6.0 / (hidden + 1))
-        out += [(torch.rand(hidden, 1, generator=gen) * 2 - 1) * limit, torch.zeros(1)]
+        limit = math.sqrt(6.0 / (hidden + value_size))
+        out += [(torch.rand(hidden, value_size, generator=gen) * 2 - 1) * limit, torch.zeros(value_size)]
     if n_cos:
         std = math.sqrt(2.0 / n_cos) / 0.87962566103423978
         w = torch.empty(n_cos, hidden)
@@ -248,16 +283,21 @@ class AgentGroup:
         if self.noisy and self.global_clipnorm is not None:
             raise ValueError("noisy=true cannot be combined with global_clipnorm yet: the global norm over the mean and the "
                              "sigma gradients is not implemented")
+        rainbow_config(cfg)
         dist_config(cfg)
         quantile_config(cfg)
         iqn_config(cfg)
+        # Rainbow: C51 heads with dueling streams on noisy layers.  The group is noisy (acting, sigma, the noise record and
+        # the effective blocks are the noisy ones); its layout, scratch and calls are the *_rainbow ones
+        self.rainbow = bool(cfg["rainbow"])
+        self.noisy = self.noisy or self.rainbow
         self.distributional = bool(cfg["distributional"])     # C51
-        self.num_atoms = int(cfg["num_atoms"]) if self.distributional else 0
+        self.num_atoms = int(cfg["num_atoms"]) if self.distributional or self.rainbow else 0
         self.quantile = bool(cfg["quantile"])                 # QR-DQN
         self.num_quantiles = int(cfg["num_quantiles"]) if self.quantile else 0
         # either head uses the distributional layout W3[H][4 * Np] | b3[4 * Np] of N = head_atoms atoms or quantiles
         self.dist_layout = self.distributional or self.quantile
-        self.head_atoms = self.num_atoms or self.num_quantiles
+        self.head_atoms = self.num_atoms or self.num_quantiles     # Rainbow: its C51 atoms
         self.iqn = bool(cfg["iqn"])
         self.n_cos = int(cfg["iqn_embedding_dim"]) if self.iqn else 0
         self.iqn_row_base = 0        # global index of this group's first sampled row (SharedParameterStep: rank * B)
@@ -276,7 +316,11 @@ class AgentGroup:
 
         self.dims = N.Dims(self.n_agents, self.n_nets, self.state_size, self.obs_stride, self.hidden,
                            self.action_size, self.batch_size, self.capacity)
-        if self.dueling:        # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
+        if self.rainbow:        # the C51 block with the value stream Wv[H][Np] | bv[Np] after b3
+            self.layout = N.RainbowLayout()
+            N.check(self.lib.dmdqn_param_layout_rainbow(C.byref(self.dims), self.num_atoms, C.byref(self.layout)))
+            self.atom_stride = (self.num_atoms + 3) // 4 * 4
+        elif self.dueling:      # W1 | b1 | W2 | b2 | W3 | b3 | wv | bv: the same offsets up to b3, a longer stride
             self.layout = N.DuelingLayout()
             N.check(self.lib.dmdqn_param_layout_dueling(C.byref(self.dims), C.byref(self.layout)))
         elif self.iqn:              # the plain block with Wphi[n_cos][H] | bphi[H] after b3
@@ -290,7 +334,10 @@ class AgentGroup:
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
         self.noise_record = N.NoiseRecord()
-        N.check(self.lib.dmdqn_noise_layout(C.byref(self.dims), C.byref(self.noise_record)))
+        if self.rainbow:
+            N.check(self.lib.dmdqn_noise_layout_rainbow(C.byref(self.dims), self.num_atoms, C.byref(self.noise_record)))
+        else:
+            N.check(self.lib.dmdqn_noise_layout(C.byref(self.dims), C.byref(self.noise_record)))
         if cfg["precision"] == "auto":   # fp32-class either way (same 1e-5 bar): tcgen05 3xTF32 where that path is built, FFMA elsewhere
             cfg["precision"] = "tf32x3" if (self.hidden == 256 and self.obs_stride in (32, 64, 96) and self.batch_size % 4 == 0
                                             and self.batch_size <= 4096) else "fp32"
@@ -301,7 +348,7 @@ class AgentGroup:
             int(cfg["target_update_frequency"]), N.LOSS[cfg["loss"]], int(bool(cfg["normalize_rewards"])),
             int(bool(cfg["double_dqn"])), N.ADAM[cfg["adam_form"]], N.SAMPLE[cfg["sample_mode"]],
             N.PRECISION[cfg["precision"]], float(cfg["per_alpha"]), float(cfg["per_beta"]), float(cfg["per_eps"]),
-            int(cfg["per_beta_steps"]), self.n_step, dueling=int(self.dueling))
+            int(cfg["per_beta_steps"]), self.n_step, dueling=int(self.dueling or self.rainbow))
 
         dev, n, c, dp, g = self.device, self.n_agents, self.capacity, self.obs_stride, self.n_nets
         for name in self._NOISY_PTRS:
@@ -363,6 +410,11 @@ class AgentGroup:
                            _ptr(self.learn_step))
         self.noisy_ptrs = N.Noisy(*(_ptr(getattr(self, k)) for k in self._NOISY_PTRS)) if self.noisy else None
         self.dist_scratch, self.dist, self.qr = None, None, None
+        if self.rainbow:            # per group, like the workspace: the C51 regions and the folded heads
+            nbytes = C.c_size_t()
+            N.check(self.lib.dmdqn_rainbow_scratch_bytes(C.byref(self.dims), self.num_atoms, C.byref(nbytes)))
+            self.dist_scratch = torch.zeros((nbytes.value,), dtype=torch.uint8, device=dev)
+            self.dist = N.Dist(self.num_atoms, float(cfg["v_min"]), float(cfg["v_max"]), _ptr(self.dist_scratch), nbytes.value)
         if self.dist_layout:        # per group, like the workspace: what the distributional kernels of one step pass on
             nbytes = C.c_size_t()
             N.check(self.lib.dmdqn_dist_scratch_bytes(C.byref(self.dims), self.head_atoms, C.byref(nbytes)))
@@ -432,7 +484,8 @@ class AgentGroup:
         """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]; dueling: + [Wv [H,1], bv [1]]) -> one parameter block."""
         L, H, A = self.layout, self.hidden, self.action_size
         ws = [torch.as_tensor(np.asarray(w), dtype=torch.float32) for w in weights]
-        want = 8 if self.dueling or getattr(self, "iqn", False) else 6
+        rainbow = getattr(self, "rainbow", False)
+        want = 8 if self.dueling or rainbow or getattr(self, "iqn", False) else 6
         if len(ws) != want:
             raise ValueError(f"expected {want} weight tensors, got {len(ws)}")
         w1, b1, w2, b2, w3, b3 = ws[:6]
@@ -441,10 +494,13 @@ class AgentGroup:
         blk[L.b1:L.b1 + H] = b1
         blk[L.w2:L.w2 + H * H] = w2.reshape(-1)
         blk[L.b2:L.b2 + H] = b2
-        if getattr(self, "dist_layout", False):     # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
+        if getattr(self, "dist_layout", False) or rainbow:  # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
             n, npad = self.head_atoms, self.atom_stride
             blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n] = w3.reshape(H, A, n)
             blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n] = b3.reshape(A, n)
+            if rainbow:                                     # Wv [H, N] / bv [N], atom j -> column j of Np
+                blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n] = ws[6].reshape(H, n)
+                blk[L.bv:L.bv + n] = ws[7].reshape(n)
             return blk
         blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A] = w3
         blk[L.b3:L.b3 + A] = b3
@@ -461,10 +517,13 @@ class AgentGroup:
         blk = blk.detach().cpu()
         out = [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
                blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(), blk[L.b2:L.b2 + H].clone()]
-        if getattr(self, "dist_layout", False):
+        if getattr(self, "dist_layout", False) or getattr(self, "rainbow", False):
             n, npad = self.head_atoms, self.atom_stride
-            return out + [blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
-                          blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
+            out += [blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
+                    blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
+            if getattr(self, "rainbow", False):
+                out += [blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n].clone(), blk[L.bv:L.bv + n].clone()]
+            return out
         out += [blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(), blk[L.b3:L.b3 + A].clone()]
         if self.dueling:
             out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
@@ -477,6 +536,10 @@ class AgentGroup:
         of a layer (Fortunato et al.'s factorized rule), fan_in = state_size for layer 1 and H after it."""
         d, h, a = self.state_size, self.hidden, self.action_size
         s1, s2 = np.float32(self.noisy_sigma0 / math.sqrt(d)), np.float32(self.noisy_sigma0 / math.sqrt(h))
+        if getattr(self, "rainbow", False):     # the C51 head [H, A*N] and the value stream [H, N]
+            a, n = a * self.num_atoms, self.num_atoms
+            shapes = [((d, h), s1), ((h,), s1), ((h, h), s2), ((h,), s2), ((h, a), s2), ((a,), s2), ((h, n), s2), ((n,), s2)]
+            return [torch.full(shape, float(v), dtype=torch.float32) for shape, v in shapes]
         shapes = [((d, h), s1), ((h,), s1), ((h, h), s2), ((h,), s2), ((h, a), s2), ((a,), s2)]
         if self.dueling:
             shapes += [((h, 1), s2), ((1,), s2)]
@@ -485,8 +548,10 @@ class AgentGroup:
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
         (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
-        head = self.action_size * self.head_atoms if self.dist_layout else self.action_size   # dist: W3 GlorotUniform over [H, A*N]
-        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, self.dueling, self.n_cos))
+        head = self.action_size * self.head_atoms if self.dist_layout or self.rainbow else self.action_size   # dist: W3 over [H, A*N]
+        # Rainbow: W1..b3 drawn as a C51 group's, then Wv GlorotUniform over [H, N]
+        value = dict(dueling=True, value_size=self.num_atoms) if self.rainbow else dict(dueling=self.dueling)
+        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, n_cos=self.n_cos, **value))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
@@ -518,7 +583,8 @@ class AgentGroup:
                 tg[net].copy_(t[net])
 
     def get_weights(self, net: int, which: str = "online") -> list[torch.Tensor]:
-        """[W1, b1, W2, b2, W3, b3] (+ [Wv, bv] with dueling heads); noisy networks: the mu list, then the sigma list."""
+        """[W1, b1, W2, b2, W3, b3] (+ [Wv, bv] with dueling heads; Rainbow: W3 [H, A*N], b3 [A*N], Wv [H, N], bv [N]); noisy
+        networks: the mu list, then the sigma list."""
         return [w for t in self._blocks(which) for w in self.unpack(t[net])]
 
     # ------------------------------------------------------------------ K0 --------------
@@ -592,7 +658,10 @@ class AgentGroup:
         nets = self.nets if not target else N.Nets(_ptr(self.theta_tgt), _ptr(self.theta_tgt), _ptr(self.adam_m),
                                                    _ptr(self.adam_v), _ptr(self.learn_step))
         args = (_ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream)
-        if self.distributional:
+        if self.rainbow:            # set 0's noise at the current learn_step, or mu alone (noisy=False, the target network)
+            nz = C.byref(self.noisy_ptrs) if noisy is not False and not target else None
+            N.check(self.lib.dmdqn_act_rainbow(C.byref(self.dims), C.byref(nets), nz, C.byref(self.dist), *args))
+        elif self.distributional:
             N.check(self.lib.dmdqn_act_dist(C.byref(self.dims), C.byref(nets), C.byref(self.dist), *args))
         elif self.quantile:
             N.check(self.lib.dmdqn_act_quantile(C.byref(self.dims), C.byref(nets), C.byref(self.qr), *args))
@@ -707,11 +776,28 @@ class AgentGroup:
                                                C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
                                                _ptr(self.metrics), _ptr(self.workspace), self.workspace.numel(), stream_ptr))
 
+    def _rainbow_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
+        """``dmdqn_learn_grads_rainbow`` into ``grads_ptr`` (dL/d eff), the loss mean over ``global_batch``."""
+        N.check(self.lib.dmdqn_learn_grads_rainbow(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
+                                                   C.byref(self.nets), C.byref(self.noisy_ptrs), draws_ptr, mask_ptr,
+                                                   int(global_batch), grads_ptr, _ptr(self.metrics), _ptr(self.workspace),
+                                                   self.workspace.numel(), stream_ptr))
+
+    def _rainbow_adam_call(self, hp, grads_ptr, stream_ptr) -> None:
+        """``dmdqn_adam_apply_rainbow``: Adam on mu and sigma from the gradient block, and their target sync."""
+        N.check(self.lib.dmdqn_adam_apply_rainbow(C.byref(self.dims), C.byref(hp), C.byref(self.nets), C.byref(self.noisy_ptrs),
+                                                  self.num_atoms, grads_ptr, _ptr(self.workspace), self.workspace.numel(),
+                                                  stream_ptr))
+
     def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
         """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
         (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
         ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
         ws, nws = _ptr(self.workspace), self.workspace.numel()
+        if self.rainbow:            # the gradient of the effective weights, then Adam on mu and sigma
+            self._rainbow_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
+            self._rainbow_adam_call(hp, _ptr(self.grads), stream_ptr)
+            return
         if self.iqn:                # the IQN gradient, then Adam (clipped when global_clipnorm is set)
             self._iqn_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
             N.check(self.lib.dmdqn_adam_apply_iqn(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.n_cos,
@@ -891,6 +977,15 @@ class AgentGroup:
                "next_rows": view(nv.next_rows, torch.int32, (g, b)), "discount": view(nv.discount, torch.float32, (g, b))}
         if self.noisy:           # factor vectors [network][set][record] and effective blocks of the last fold
             out["noise"], out["eff"], out["eff_tgt"] = self.noise, self.eff, self.eff_tgt
+        if self.rainbow:         # the C51 views and the folded heads [set][network][(H + 1) * 4 * Np] of the last fold
+            rv = N.RainbowViews()
+            N.check(self.lib.dmdqn_debug_rainbow(C.byref(self.dims), C.byref(self.dist), C.byref(rv)))
+            sbase = self.dist_scratch.data_ptr()
+            hw = (self.hidden + 1) * 4 * self.atom_stride
+            for key, ptr, shape in (("target_dist", rv.target_dist, (g, b, self.atom_stride)), ("h2", rv.h2, (g, b, self.hidden)),
+                                    ("dlogits", rv.dlogits, (g, b, 4 * self.atom_stride)), ("head", rv.head, (2, g, hw))):
+                off = ptr - sbase
+                out[key] = self.dist_scratch[off:off + int(np.prod(shape)) * 4].view(torch.float32).view(*shape)
         if self.dist_layout:     # the targets [network][row][Np] of the last learn step: C51's projected m, QR-DQN's T
             dv = N.DistViews()
             if self.quantile:
@@ -936,6 +1031,10 @@ class AgentGroup:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
         tau = -1.0 if tau is None else float(tau)
+        if self.rainbow:         # mu and sigma over the Rainbow stride
+            N.check(self.lib.dmdqn_sync_target_rainbow(C.byref(self.dims), C.byref(self.nets), C.byref(self.noisy_ptrs),
+                                                       self.num_atoms, _ptr(mask_t), tau, self._stream))
+            return
         if self.iqn:
             N.check(self.lib.dmdqn_sync_target_iqn(C.byref(self.dims), C.byref(self.nets), self.n_cos, _ptr(mask_t), tau,
                                                    self._stream))

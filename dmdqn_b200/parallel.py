@@ -209,7 +209,9 @@ class SharedParameterStep:
         the NCCL path as well: ``dmdqn_learn_grads_dist``, the all-reduce of its gradient block, then ``dmdqn_adam_apply_dist``
         (clipped when ``global_clipnorm`` is set); ``fused=True`` is refused there.  A ``quantile`` (QR-DQN) group does the
         same with ``dmdqn_learn_grads_quantile``, and an ``iqn`` group with ``dmdqn_learn_grads_iqn`` (its fractions keyed from
-        row ``rank * batch``, so ranks draw different fractions) and ``dmdqn_adam_apply_iqn``."""
+        row ``rank * batch``, so ranks draw different fractions) and ``dmdqn_adam_apply_iqn``.  A ``rainbow`` group takes the
+        NCCL path with ``dmdqn_learn_grads_rainbow`` (every rank folds the same noise) and ``dmdqn_adam_apply_rainbow``;
+        ``fused=True`` is refused there."""
         from . import _native as N
         from .group import _ptr
         if not grp.shared:
@@ -219,6 +221,10 @@ class SharedParameterStep:
         if clip is not None and fused:
             raise ValueError("global_clipnorm is set: the fused peer-memory kernel (dmdqn_allreduce_adam) does not clip; "
                              "use fused=False (the NCCL all-reduce + dmdqn_clip_adam_apply path)")
+        rainbow = getattr(grp, "rainbow", False)
+        if rainbow and fused:
+            raise ValueError("rainbow=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the Rainbow layout "
+                             "or sigma; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_rainbow path)")
         if grp.noisy and fused:
             raise ValueError("noisy=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not update sigma; use "
                              "fused=False (the NCCL all-reduce + dmdqn_noisy_adam_apply path)")
@@ -251,7 +257,9 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                if grp.iqn:
+                if rainbow:
+                    grp._rainbow_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
+                elif grp.iqn:
                     grp._iqn_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
                 elif grp.dist_layout:           # C51 or QR-DQN
                     grp._dist_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
@@ -285,6 +293,9 @@ class SharedParameterStep:
 
         def apply(g: torch.Tensor):
             with torch.cuda.device(grp.device):
+                if rainbow:
+                    grp._rainbow_adam_call(grp.hp, _ptr(g), grp._stream)
+                    return
                 if grp.iqn:                     # clipped (the norm of the all-reduced block) when global_clipnorm is set
                     N.check(grp.lib.dmdqn_adam_apply_iqn(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.n_cos,
                                                          _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),

@@ -45,6 +45,9 @@
  *   quantile networks (QR-DQN, see dmdqn_quantile below) use the same block with N quantiles in place of N atoms.
  *   implicit quantile networks (IQN, see dmdqn_iqn below) append the cosine embedding after b3:
  *     W1 | b1 | W2 | b2 | W3[H][4] | b3[4] | Wphi[n_cos][H] | bphi[H] | pad
+ *   Rainbow networks (dueling noisy C51; dmdqn_param_layout_rainbow, see dmdqn_rainbow_layout below) append the per-atom
+ *   value stream to the C51 block:
+ *     W1 | b1 | W2 | b2 | W3[H][4 * Np] | b3[4 * Np] | Wv[H][Np] | bv[Np] | pad
  */
 #ifndef DMDQN_B200_H
 #define DMDQN_B200_H
@@ -750,6 +753,77 @@ typedef struct dmdqn_iqn_views {
     const float* dh2; const float* dphi;
 } dmdqn_iqn_views;
 int dmdqn_debug_iqn(const dmdqn_dims* dims, const dmdqn_iqn* iqn, dmdqn_iqn_views* out);
+
+/* Rainbow (Hessel et al. 2018): C51 heads (dmdqn_dist) with dueling value / advantage streams and noisy layers everywhere
+ * (dmdqn_noisy), fp32 (FFMA) path only.  Prioritized replay, n-step returns and double DQN apply as for every learn step.
+ * Parameter block (dmdqn_param_layout_rainbow):
+ *   W1 | b1 | W2 | b2 | W3[H][4 * Np] | b3[4 * Np] | Wv[H][Np] | bv[Np] | pad
+ * with the C51 offsets up to b3, wv at the C51 end (b3 + 4 * Np, 16-byte aligned), bv = wv + H * Np, end = bv + Np (Adam
+ * updates [0, end)) and the stride rounded up to 32 floats.  Value columns j >= N are 0 and keep gradient 0, as do the C51
+ * pad columns.  The logits x_{a,j} = V_j + Adv_{a,j} - (1/A) sum_{b<A} Adv_{b,j} are linear in h2, so the head folds per atom:
+ * for every row k < H, and the bias row (b3 / bv), and every j < N
+ *   W3e[k][a * Np + j] = head_fold({W3[k][b * Np + j]}_{b<4}, Wv[k][j], A)[a]      (dmdqn_hparams.dueling's fold, per atom)
+ * and columns j >= N or a >= A of W3e | b3e are 0.  After the fold the step is dmdqn_dist's on W3e | b3e: softmax, expected Q,
+ * projection, cross-entropy, priority and metrics row.  With G the gradient with respect to W3e | b3e, the head update is
+ * head_project per (k, j): the advantage gradient {dW3[k][a * Np + j]}_a = G[k][a * Np + j] - (1/A) sum_{b<A} G[k][b * Np + j]
+ * (0 for a >= A) and dWv[k][j] = sum_{b<A} G[k][b * Np + j] (likewise b3 / bv; 0 for j >= N).
+ * Noise: dmdqn_noisy's rule with the Rainbow record (dmdqn_noise_layout_rainbow; the same struct)
+ *   w1_in[obs_stride] | w1_out[H] | w2_in[H] | w2_out[H] | w3_in[H] | w3_out[4 * Np] | v_in[H] | v_out[Np]
+ * (stride a multiple of 32): output factor i of w3_out is column a * Np + j, 0 unless a < A and j < N; v_out[j] is 0 for
+ * j >= N.  The Philox counters, Box-Muller, eps = fin[k] * fout[col] for a weight and fout[col] for a bias, and
+ * eff = mu + sigma * eps are dmdqn_noisy's.
+ * A learn step runs, in order: 1. the noise fold (sets 0 and 1 at the learn_step t before the increment, into eff / eff_tgt);
+ * 2. the head fold of eff (online) and eff_tgt (target) into the scratch; 3. the sample kernel; 4. the C51 target and online
+ * kernels on the folded heads with the eff trunks; 5. the C51 weight-gradient kernel; 6. the projection, which leaves dL/d eff
+ * in the Rainbow layout in grads_out; then dmdqn_adam_apply_rainbow: 7. Adam on mu (g) and sigma (g * eps of set 0) and the
+ * target sync of both.  Acting uses set 0 at the current learn_step (the noisy rule); greedy evaluation uses mu alone.
+ *   dist       dmdqn_dist (n_atoms, support); its scratch holds at least dmdqn_rainbow_scratch_bytes, 16-byte aligned: the C51
+ *              regions, then the folded heads float [2][n_nets][(H + 1) * 4 * Np] (W3e | b3e, online then target).
+ *   noisy      dmdqn_noisy over Rainbow blocks; noise is [n_nets][2][record stride] of the Rainbow record.
+ * Every call below refuses, before anything is launched: n_atoms outside [2, 64], a bad support, hp->precision other than
+ * DMDQN_PRECISION_FP32, hp->dueling != 1 (calls that take hparams: Rainbow blocks always carry the value stream), NULL or
+ * misaligned pointers (every dmdqn_noisy field for learn, Adam and the target sync) and a short scratch. */
+typedef struct dmdqn_rainbow_layout {
+    int64_t w1, b1, w2, b2, w3, b3, wv, bv, end, stride;
+} dmdqn_rainbow_layout;
+int dmdqn_param_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_rainbow_layout* out);
+int dmdqn_noise_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_noise_record* out);
+int dmdqn_rainbow_scratch_bytes(const dmdqn_dims* dims, int32_t n_atoms, size_t* out_bytes);
+
+/* Steps 1 and 2 at every network's current learn_step: the factor vectors into noisy->noise, eff / eff_tgt, and the folded
+ * heads into dist->scratch. */
+int dmdqn_rainbow_fold(const dmdqn_dims* dims, const dmdqn_dist* dist, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                       void* stream);
+
+/* Steps 1 to 6: grads_out[n_nets][stride] receives dL/d eff for every float of [0, end) with the loss mean over global_batch
+ * (>= batch); learn_step advances as in dmdqn_learn_grads.  Finish the step with dmdqn_adam_apply_rainbow. */
+int dmdqn_learn_grads_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_dist* dist,
+                              const dmdqn_replay* replay, const dmdqn_nets* nets, const dmdqn_noisy* noisy, const void* draws,
+                              const uint8_t* learn_mask, int32_t global_batch, float* grads_out, float* metrics_out,
+                              void* workspace, size_t workspace_bytes, void* stream);
+
+/* Step 7, as dmdqn_noisy_adam_apply over [0, end) of Rainbow blocks. */
+int dmdqn_adam_apply_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_noisy* noisy,
+                             int32_t n_atoms, const float* grads, void* workspace, size_t workspace_bytes, void* stream);
+
+/* dmdqn_act_dist on Rainbow blocks, the head folded per atom in registers.  noisy set: mu + sigma * eps with set 0's noise at
+ * the current learn_step, so q_out and the actions equal dmdqn_act_dist's on the C51 block that holds eff's trunk and its
+ * folded head after a dmdqn_rainbow_fold at the same learn_step, bit for bit.  noisy NULL: mu alone (greedy evaluation).
+ * dist->scratch is not used and may be NULL. */
+int dmdqn_act_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, const dmdqn_dist* dist,
+                      const float* obs, int32_t obs_in_stride, const double* eps, const uint32_t* w_explore,
+                      const uint32_t* w_action, int32_t* actions_out, float* q_out, void* stream);
+
+/* dmdqn_sync_target over the whole Rainbow stride, of mu (theta -> theta_tgt) and of sigma (sigma -> sigma_tgt). */
+int dmdqn_sync_target_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t n_atoms,
+                              const uint8_t* mask, double tau, void* stream);
+
+/* The scratch's views after dmdqn_learn_grads_rainbow (or dmdqn_rainbow_fold, for head): dmdqn_dist_views, and head float
+ * [2][n_nets][(H + 1) * 4 * Np], the folded W3e | b3e of the online (0) and the target (1) network. */
+typedef struct dmdqn_rainbow_views {
+    const float* target_dist; const float* h2; const float* dlogits; const float* head;
+} dmdqn_rainbow_views;
+int dmdqn_debug_rainbow(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_rainbow_views* out);
 
 #ifdef __cplusplus
 }
