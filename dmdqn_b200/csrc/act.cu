@@ -223,7 +223,7 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
     float* rec = part + kActThreads * 4;                 // NOISY: the online noise record
     if constexpr (NOISY) {
         S = nz.sigma + (size_t)net * L.stride;
-        noise_record_build(rec, nz.R, d.obs_dim, d.n_actions, __ldg(nz.key + net), (uint32_t)__ldg(nz.learn_step + net), 0);
+        noise_record_build(rec, nz.R, d.obs_dim, d.n_actions, 1, 1, __ldg(nz.key + net), (uint32_t)__ldg(nz.learn_step + net), 0);
         for (int c = threadIdx.x; c < Dp; c += kActThreads)
             xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
         __syncthreads();
@@ -243,14 +243,14 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
         const int j = rank * Hs + threadIdx.x;
         float4 w = __ldg(reinterpret_cast<const float4*>(P + L.w3) + j);
         float v = 0.f;
-        if constexpr (DUELING) v = __ldg(P + layout_wv(L) + j);
+        if constexpr (DUELING) v = __ldg(P + L.wv + j);
         if constexpr (NOISY) {
             const float4 s = __ldg(reinterpret_cast<const float4*>(S + L.w3) + j);
             const float fi = rec[nz.R.off[4] + j], *fo = rec + nz.R.off[5];
             w = make_float4(noisy_weight(w.x, s.x, __fmul_rn(fi, fo[0])), noisy_weight(w.y, s.y, __fmul_rn(fi, fo[1])),
                             noisy_weight(w.z, s.z, __fmul_rn(fi, fo[2])), noisy_weight(w.w, s.w, __fmul_rn(fi, fo[3])));
             if constexpr (DUELING)
-                v = noisy_weight(v, __ldg(S + layout_wv(L) + j), __fmul_rn(rec[nz.R.off[6] + j], rec[nz.R.off[7]]));
+                v = noisy_weight(v, __ldg(S + L.wv + j), __fmul_rn(rec[nz.R.off[6] + j], rec[nz.R.off[7]]));
         }
         if constexpr (DUELING) {
             float x[4] = {w.x, w.y, w.z, w.w};
@@ -279,11 +279,11 @@ act_kernel(dmdqn_dims d, Layout L, const float* __restrict__ theta, const float*
     if (threadIdx.x == 0 && rank == 0) {
         float q[4] = {P[L.b3 + 0], P[L.b3 + 1], P[L.b3 + 2], P[L.b3 + 3]};
         float bv = 0.f;
-        if constexpr (DUELING) bv = P[layout_bv(L, H)];
+        if constexpr (DUELING) bv = P[L.bv];
         if constexpr (NOISY) {
             const float* fo = rec + nz.R.off[5];
             for (int k = 0; k < 4; ++k) q[k] = noisy_weight(q[k], S[L.b3 + k], fo[k]);
-            if constexpr (DUELING) bv = noisy_weight(bv, S[layout_bv(L, H)], rec[nz.R.off[7]]);
+            if constexpr (DUELING) bv = noisy_weight(bv, S[L.bv], rec[nz.R.off[7]]);
         }
         if constexpr (DUELING) head_fold(q, bv, d.n_actions);
         for (int r = 0; r < kActCluster; ++r) {
@@ -419,7 +419,7 @@ act_quantile_kernel(dmdqn_dims d, Layout L, int n_quantiles, const float* __rest
 // act_quantile_kernel.)
 template <int H, bool NOISY>
 __global__ void __cluster_dims__(kActCluster, 1, 1) __launch_bounds__(kActThreads, 4)
-act_rainbow_kernel(dmdqn_dims d, RainbowLayout RL, int n_atoms, double v_min, double dz64, const float* __restrict__ theta,
+act_rainbow_kernel(dmdqn_dims d, Layout L, int n_atoms, double v_min, double dz64, const float* __restrict__ theta,
                    const float* __restrict__ obs, int stride, const double* __restrict__ eps,
                    const uint32_t* __restrict__ w_explore, const uint32_t* __restrict__ w_action, int32_t* __restrict__ actions,
                    float* __restrict__ q_out, ActNoise nz) {
@@ -431,7 +431,6 @@ act_rainbow_kernel(dmdqn_dims d, RainbowLayout RL, int n_atoms, double v_min, do
         if (threadIdx.x == 0 && rank == 0) actions[a] = (int32_t)__umulhi(w_action[a], (uint32_t)d.n_actions);
         return;
     }
-    const Layout& L = RL.L;
     const int Dp = d.obs_stride;
     float* xs = smem;                        // [Dp]
     float* h1 = xs + Dp;                     // [H]
@@ -446,8 +445,8 @@ act_rainbow_kernel(dmdqn_dims d, RainbowLayout RL, int n_atoms, double v_min, do
     const int np = (n_atoms + 3) / 4 * 4, nh = 4 * np;
     if constexpr (NOISY) {
         S = nz.sigma + (size_t)net * L.stride;
-        noise_record_build_rainbow(rec, nz.R, d.obs_dim, d.n_actions, n_atoms, np, __ldg(nz.key + net),
-                                   (uint32_t)__ldg(nz.learn_step + net), 0);
+        noise_record_build(rec, nz.R, d.obs_dim, d.n_actions, n_atoms, np, __ldg(nz.key + net), (uint32_t)__ldg(nz.learn_step + net),
+                           0);
         for (int c = threadIdx.x; c < Dp; c += kActThreads) xs[c] = c < d.obs_dim ? obs[(size_t)a * stride + c] : 0.f;
         __syncthreads();
         gemv_slice_noisy(cluster, P + L.w1, S + L.w1, P + L.b1, S + L.b1, rec + nz.R.off[0], rec + nz.R.off[1], xs, h1, part,
@@ -461,7 +460,7 @@ act_rainbow_kernel(dmdqn_dims d, RainbowLayout RL, int n_atoms, double v_min, do
     // the folded head weight of column rank * Np + j in row k (k == H: the bias), in act_dist_kernel's column
     auto folded = [&](int k, int j) {
         const float* w = P + (k < H ? L.w3 + (size_t)k * nh : L.b3) + j;
-        const int64_t vo = (k < H ? RL.wv + (int64_t)k * np : RL.bv) + j;
+        const int64_t vo = (k < H ? L.wv + (int64_t)k * np : L.bv) + j;
         float x[4] = {__ldg(w), __ldg(w + np), __ldg(w + 2 * np), __ldg(w + 3 * np)};
         float v = __ldg(P + vo);
         if constexpr (NOISY) {
@@ -613,7 +612,7 @@ act_iqn_kernel(dmdqn_dims d, Layout L, int64_t wphi, int64_t bphi, int K, int n_
 
 int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn& q, const float* obs, int32_t stride,
                    const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s) {
-    const IqnLayout L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos);
+    const Layout L = make_layout(d.obs_stride, d.hidden, {1, 1, false, q.n_cos});
     const int K = q.n_policy, tw = std::max(q.n_cos, d.hidden / kActCluster);
     const size_t smem = ((size_t)d.obs_stride + d.hidden + kActThreads * 4 + (size_t)K * d.hidden + (size_t)K * tw +
                          (size_t)kActCluster * K * 4) * sizeof(float);
@@ -621,7 +620,7 @@ int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn&
     static size_t cfg[4][kMaxDevices] = {};
     auto run = [&](auto kernel, size_t (&c)[kMaxDevices]) {
         if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kernel), smem, c)) return rc;
-        kernel<<<grid, kActThreads, smem, s>>>(d, L.L, L.wphi, L.bphi, K, q.n_cos, nets.theta, obs, stride, eps, w1, w2, actions,
+        kernel<<<grid, kActThreads, smem, s>>>(d, L, L.wphi, L.bphi, K, q.n_cos, nets.theta, obs, stride, eps, w1, w2, actions,
                                                q_out);
         return 0;
     };
@@ -640,7 +639,7 @@ int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn&
 
 int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
                     const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s) {
-    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(ds.n_atoms));
+    const Layout L = make_layout(d.obs_stride, d.hidden, atom_shape(ds.n_atoms, false));
     const double dz64 = (ds.v_max - ds.v_min) / (ds.n_atoms - 1);
     const size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + 2 * kDistMaxAtoms) * sizeof(float);
     const dim3 grid(d.n_agents * kActCluster);
@@ -662,11 +661,11 @@ int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dis
 int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy* noisy, const dmdqn_dist& ds,
                        const float* obs, int32_t stride, const double* eps, const uint32_t* w1, const uint32_t* w2,
                        int32_t* actions, float* q_out, cudaStream_t s) {
-    const int np = dist_np(ds.n_atoms);
-    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
+    const HeadShape hs = atom_shape(ds.n_atoms, true);
+    const Layout L = make_layout(d.obs_stride, d.hidden, hs);
     const double dz64 = (ds.v_max - ds.v_min) / (ds.n_atoms - 1);
     ActNoise nz = {};
-    nz.R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
+    nz.R = make_noise_rec(d.obs_stride, d.hidden, hs);
     size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + 2 * kDistMaxAtoms) * sizeof(float);
     if (noisy) {
         nz.sigma = noisy->sigma; nz.key = noisy->key; nz.learn_step = nets.learn_step;
@@ -674,7 +673,7 @@ int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_
     }
     const dim3 grid(d.n_agents * kActCluster);
     auto run = [&](auto kernel) {
-        kernel<<<grid, kActThreads, smem, s>>>(d, RL, ds.n_atoms, ds.v_min, dz64, nets.theta, obs, stride, eps, w1, w2, actions,
+        kernel<<<grid, kActThreads, smem, s>>>(d, L, ds.n_atoms, ds.v_min, dz64, nets.theta, obs, stride, eps, w1, w2, actions,
                                                q_out, nz);
     };
     switch (d.hidden * 2 + (noisy ? 1 : 0)) {
@@ -695,7 +694,7 @@ int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_
 int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_quantile& qs, const float* obs, int32_t stride,
                         const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out,
                         cudaStream_t s) {
-    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(qs.n_quantiles));
+    const Layout L = make_layout(d.obs_stride, d.hidden, atom_shape(qs.n_quantiles, false));
     const size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4 + kDistMaxAtoms) * sizeof(float);
     const dim3 grid(d.n_agents * kActCluster);
     auto run = [&](auto kernel) {
@@ -715,7 +714,7 @@ int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
                const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,
                cudaStream_t s, const dmdqn_noisy* noisy) {
-    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
+    const Layout L = make_layout(d.obs_stride, d.hidden, {1, 1, dueling, 0});
     ActNoise nz = {};
     nz.R = make_noise_rec(d.obs_stride, d.hidden);
     size_t smem = (size_t)(d.obs_stride + 2 * d.hidden + kActThreads * 4) * sizeof(float);

@@ -78,6 +78,34 @@ static int check_workspace(const dmdqn_dims* dims, void* ws, size_t bytes, Works
 
 using namespace dmdqn;
 
+// The offsets every public layout struct shares
+template <class T>
+static void copy_trunk(const Layout& l, T* out) {
+    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
+    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
+}
+
+static void copy_noise_rec(const NoiseRec& r, dmdqn_noise_record* out) {
+    int64_t* f[8] = {&out->w1_in, &out->w1_out, &out->w2_in, &out->w2_out, &out->w3_in, &out->w3_out, &out->v_in, &out->v_out};
+    for (int v = 0; v < 8; ++v) *f[v] = r.off[v];
+    out->stride = r.stride;
+}
+
+// Adam over the block of head shape hs, after global-norm clipping when clipnorm > 0
+static int run_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, HeadShape hs, const dmdqn_nets& nets, const float* grads,
+                    double clipnorm, float* norms_out, void* workspace, const Workspace& w, void* stream) {
+    const LearnArgs A = make_learn_args(d, hp, hs, {}, nets, (char*)workspace, w, nullptr, nullptr, 0);
+    return launch_adam(A, grads, clipnorm, norms_out, (cudaStream_t)stream);
+}
+
+// The target sync of a noisy block: mu, then sigma
+static int sync_noisy(const dmdqn_dims& d, HeadShape hs, const dmdqn_nets& nets, const dmdqn_noisy& nz, const uint8_t* mask,
+                      double tau, void* stream) {
+    const int64_t stride = make_layout(d.obs_stride, d.hidden, hs).stride;
+    if (int rc = launch_sync_target(d, stride, nets.theta, nets.theta_tgt, mask, tau, (cudaStream_t)stream)) return rc;
+    return launch_sync_target(d, stride, nz.sigma, nz.sigma_tgt, mask, tau, (cudaStream_t)stream);
+}
+
 extern "C" {
 
 const char* dmdqn_last_error(void) { return g_error; }
@@ -87,9 +115,7 @@ int dmdqn_param_layout(const dmdqn_dims* dims, dmdqn_layout* out) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const Layout l = make_layout(dims->obs_stride, dims->hidden);
-    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
-    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
+    copy_trunk(make_layout(dims->obs_stride, dims->hidden), out);
     return DMDQN_OK;
 }
 
@@ -97,10 +123,9 @@ int dmdqn_param_layout_dueling(const dmdqn_dims* dims, dmdqn_dueling_layout* out
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const Layout l = make_layout(dims->obs_stride, dims->hidden, true);
-    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
-    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
-    out->wv = layout_wv(l); out->bv = layout_bv(l, dims->hidden);
+    const Layout l = make_layout(dims->obs_stride, dims->hidden, {1, 1, true, 0});
+    copy_trunk(l, out);
+    out->wv = l.wv; out->bv = l.bv;
     return DMDQN_OK;
 }
 
@@ -225,7 +250,8 @@ static int run_learn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     if (grads) DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     if (stages & DMDQN_STAGE_SAMPLE) {
         if (hp->dueling) {            // W3e | b3e of this step's weights, complete before the sample -> K3 -> K4a -> K4b chain
-            rc = launch_fold(*dims, *nets, (char*)workspace, w, (cudaStream_t)stream);
+            rc = launch_head_fold(*dims, {1, 1, true, 0}, nets->theta, nets->theta_tgt,
+                                  reinterpret_cast<float*>((char*)workspace + w.head), (cudaStream_t)stream);
             if (rc) return rc;
         }
         rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, (cudaStream_t)stream);
@@ -316,7 +342,7 @@ int dmdqn_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
                     "adam_apply: NULL argument");
     rc = check_dueling(hp);
     if (rc) return rc;
-    return launch_adam_apply(*dims, *hp, *nets, grads, (char*)workspace, w, (cudaStream_t)stream);
+    return run_adam(*dims, *hp, {1, 1, hp->dueling == 1, 0}, *nets, grads, 0.0, nullptr, workspace, w, stream);
 }
 
 int dmdqn_clip_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const float* grads,
@@ -330,8 +356,7 @@ int dmdqn_clip_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, const
     if (rc) return rc;
     DMDQN_CHECK_ARG(global_clipnorm > 0.0 && isfinite(global_clipnorm),
                     "global_clipnorm=%g must be a positive finite number", global_clipnorm);
-    return launch_clip_adam_apply(*dims, *hp, *nets, grads, global_clipnorm, norms_out, (char*)workspace, w,
-                                  (cudaStream_t)stream);
+    return run_adam(*dims, *hp, {1, 1, hp->dueling == 1, 0}, *nets, grads, global_clipnorm, norms_out, workspace, w, stream);
 }
 
 int dmdqn_allreduce_adam(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_nets* nets, const dmdqn_peers* peers,
@@ -444,10 +469,22 @@ int dmdqn_noise_layout(const dmdqn_dims* dims, dmdqn_noise_record* out) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const NoiseRec r = make_noise_rec(dims->obs_stride, dims->hidden);
-    int64_t* f[8] = {&out->w1_in, &out->w1_out, &out->w2_in, &out->w2_out, &out->w3_in, &out->w3_out, &out->v_in, &out->v_out};
-    for (int v = 0; v < 8; ++v) *f[v] = r.off[v];
-    out->stride = r.stride;
+    copy_noise_rec(make_noise_rec(dims->obs_stride, dims->hidden), out);
+    return DMDQN_OK;
+}
+
+static bool aligned16(const void* p) { return (uintptr_t)p % 16 == 0; }
+
+// What every dmdqn_learn_grads_* call checks before it launches, besides the checks of its own arguments: the workspace,
+// the learn arguments, the gradient block and global_batch.
+static int check_learn_grads(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay, const dmdqn_nets* nets,
+                             const void* draws, int32_t global_batch, const float* grads_out, void* workspace,
+                             size_t workspace_bytes, Workspace* w) {
+    int rc = check_workspace(dims, workspace, workspace_bytes, w);
+    if (rc) return rc;
+    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
+    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
+    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     return DMDQN_OK;
 }
 
@@ -469,7 +506,7 @@ int dmdqn_noisy_fold(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdq
     DMDQN_CHECK_ARG(hp != nullptr, "noisy_fold: hp is NULL");
     if ((rc = check_dueling(hp))) return rc;
     if ((rc = check_noisy(nets, noisy, false))) return rc;
-    return launch_noisy_fold(*dims, hp->dueling == 1, *nets, *noisy, (cudaStream_t)stream);
+    return launch_noisy_fold(*dims, {1, 1, hp->dueling == 1, 0}, *nets, *noisy, (cudaStream_t)stream);
 }
 
 int dmdqn_learn_grads_noisy(const dmdqn_dims* dims, const dmdqn_hparams* hp, const dmdqn_replay* replay,
@@ -477,16 +514,13 @@ int dmdqn_learn_grads_noisy(const dmdqn_dims* dims, const dmdqn_hparams* hp, con
                             int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
                             size_t workspace_bytes, void* stream) {
     Workspace w;                      // everything run_learn checks, before the fold is launched
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    int rc = check_learn_grads(dims, hp, replay, nets, draws, global_batch, grads_out, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
     if ((rc = check_noisy(nets, noisy, true))) return rc;
-    DMDQN_CHECK_ARG(grads_out != nullptr, "grads_out is NULL");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32 || tc_supported(*dims),
                     "precision=%d (tcgen05) needs hidden=256 and obs_stride in {32,64,96}; got hidden=%d obs_stride=%d",
                     hp->precision, dims->hidden, dims->obs_stride);
-    if ((rc = launch_noisy_fold(*dims, hp->dueling == 1, *nets, *noisy, (cudaStream_t)stream))) return rc;
+    if ((rc = launch_noisy_fold(*dims, {1, 1, hp->dueling == 1, 0}, *nets, *noisy, (cudaStream_t)stream))) return rc;
     dmdqn_nets eff = *nets;
     eff.theta = noisy->eff;
     eff.theta_tgt = noisy->eff_tgt;
@@ -503,7 +537,8 @@ int dmdqn_noisy_adam_apply(const dmdqn_dims* dims, const dmdqn_hparams* hp, cons
     if ((rc = check_dueling(hp))) return rc;
     if ((rc = check_noisy(nets, noisy, true))) return rc;
     DMDQN_CHECK_ARG((uintptr_t)grads % 16 == 0, "noisy_adam_apply: grads is not 16-byte aligned");
-    return launch_noisy_adam_apply(*dims, *hp, *nets, *noisy, grads, (char*)workspace, w, (cudaStream_t)stream);
+    return launch_noisy_adam_apply(*dims, *hp, {1, 1, hp->dueling == 1, 0}, *nets, *noisy, grads, (char*)workspace, w,
+                                   (cudaStream_t)stream);
 }
 
 int dmdqn_act_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, int32_t dueling,
@@ -528,11 +563,7 @@ int dmdqn_sync_target_noisy(const dmdqn_dims* dims, const dmdqn_nets* nets, cons
     DMDQN_CHECK_ARG(dueling == 0 || dueling == 1, "dueling=%d must be 0 or 1", dueling);
     DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt && noisy && noisy->sigma && noisy->sigma_tgt,
                     "sync_target_noisy: NULL network pointer");
-    dmdqn_nets sigma = *nets;
-    sigma.theta = noisy->sigma;
-    sigma.theta_tgt = noisy->sigma_tgt;
-    if ((rc = launch_sync_target(*dims, *nets, mask, tau, dueling == 1, (cudaStream_t)stream))) return rc;
-    return launch_sync_target(*dims, sigma, mask, tau, dueling == 1, (cudaStream_t)stream);
+    return sync_noisy(*dims, {1, 1, dueling == 1, 0}, *nets, *noisy, mask, tau, stream);
 }
 
 // Distributional calls (include/dmdqn_b200.h dmdqn_dist): the atom count, the support and, where the call reads it, the
@@ -542,8 +573,6 @@ static int check_atoms(int32_t n_atoms) {
                     DMDQN_DIST_MAX_ATOMS);
     return DMDQN_OK;
 }
-
-static bool aligned16(const void* p) { return (uintptr_t)p % 16 == 0; }
 
 static int check_dist(const dmdqn_dims* dims, const dmdqn_dist* ds, bool scratch) {
     DMDQN_CHECK_ARG(ds != nullptr, "dist is NULL");
@@ -558,15 +587,24 @@ static int check_dist(const dmdqn_dims* dims, const dmdqn_dist* ds, bool scratch
     return DMDQN_OK;
 }
 
-static int check_dist_hp(const dmdqn_hparams* hp) {
-    DMDQN_CHECK_ARG(hp != nullptr, "dist: hp is NULL");
-    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32,
-                    "precision=%d: distributional networks run the fp32 (FFMA) path only", hp->precision);
-    DMDQN_CHECK_ARG(hp->dueling == 0,
-                    "dueling=%d: dueling heads are not supported with distributional networks (dueling noisy C51 heads: the "
-                    "dmdqn_*_rainbow calls)", hp->dueling);
+// The hparams of the fp32-only kinds: `tag` names the call family, `kind` the networks; `dueling` is the hp->dueling the
+// block needs (1: it carries a value stream), `note` trails the refusal of a dueling head where none is supported.
+static int check_kind_hp(const dmdqn_hparams* hp, const char* tag, const char* kind, int32_t dueling, const char* note = "") {
+    DMDQN_CHECK_ARG(hp != nullptr, "%s: hp is NULL", tag);
+    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32, "precision=%d: %s networks run the fp32 (FFMA) path only",
+                    hp->precision, kind);
+    if (dueling)
+        DMDQN_CHECK_ARG(hp->dueling == 1, "dueling=%d: %s blocks carry the value stream, so hp->dueling must be 1", hp->dueling,
+                        kind);
+    else
+        DMDQN_CHECK_ARG(hp->dueling == 0, "dueling=%d: dueling heads are not supported with %s networks%s", hp->dueling, kind,
+                        note);
     return DMDQN_OK;
 }
+static int check_dist_hp(const dmdqn_hparams* hp) {
+    return check_kind_hp(hp, "dist", "distributional", 0, " (dueling noisy C51 heads: the dmdqn_*_rainbow calls)");
+}
+
 
 static int check_dist_nets(const dmdqn_nets* nets, bool adam) {
     DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt, "dist: NULL network pointer");
@@ -581,9 +619,7 @@ int dmdqn_param_layout_dist(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_layou
     if (rc) return rc;
     if ((rc = check_atoms(n_atoms))) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const Layout l = make_layout_dist(dims->obs_stride, dims->hidden, dist_np(n_atoms));
-    out->w1 = l.w1; out->b1 = l.b1; out->w2 = l.w2; out->b2 = l.b2;
-    out->w3 = l.w3; out->b3 = l.b3; out->stride = l.stride;
+    copy_trunk(make_layout(dims->obs_stride, dims->hidden, atom_shape(n_atoms, false)), out);
     return DMDQN_OK;
 }
 
@@ -600,14 +636,11 @@ int dmdqn_learn_grads_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, cons
                            const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
                            float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream) {
     Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    int rc = check_learn_grads(dims, hp, replay, nets, draws, global_batch, grads_out, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
     if ((rc = check_dist_hp(hp))) return rc;
     if ((rc = check_dist(dims, dist, true))) return rc;
     if ((rc = check_dist_nets(nets, true))) return rc;
-    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     cudaStream_t s = (cudaStream_t)stream;
     if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
     return launch_learn_dist(*dims, *hp, *replay, *nets, *dist, metrics_out, (char*)workspace, w, grads_out, global_batch, s);
@@ -625,8 +658,7 @@ int dmdqn_adam_apply_dist(const dmdqn_dims* dims, const dmdqn_hparams* hp, const
     DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_dist: grads is NULL or not 16-byte aligned");
     DMDQN_CHECK_ARG(global_clipnorm >= 0.0 && isfinite(global_clipnorm),
                     "global_clipnorm=%g must be 0 (no clipping) or a positive finite number", global_clipnorm);
-    return launch_adam_apply_dist(*dims, *hp, *nets, n_atoms, grads, global_clipnorm, norms_out, (char*)workspace, w,
-                                  (cudaStream_t)stream);
+    return run_adam(*dims, *hp, atom_shape(n_atoms, false), *nets, grads, global_clipnorm, norms_out, workspace, w, stream);
 }
 
 int dmdqn_act_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_dist* dist, const float* obs,
@@ -648,7 +680,8 @@ int dmdqn_sync_target_dist(const dmdqn_dims* dims, const dmdqn_nets* nets, int32
     if (rc) return rc;
     if ((rc = check_atoms(n_atoms))) return rc;
     if ((rc = check_dist_nets(nets, false))) return rc;
-    return launch_sync_target_dist(*dims, *nets, n_atoms, mask, tau, (cudaStream_t)stream);
+    return launch_sync_target(*dims, make_layout(dims->obs_stride, dims->hidden, atom_shape(n_atoms, false)).stride, nets->theta,
+                              nets->theta_tgt, mask, tau, (cudaStream_t)stream);
 }
 
 int dmdqn_debug_dist(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_dist_views* out) {
@@ -683,14 +716,11 @@ int dmdqn_learn_grads_quantile(const dmdqn_dims* dims, const dmdqn_hparams* hp, 
                                int32_t global_batch, float* grads_out, float* metrics_out, void* workspace,
                                size_t workspace_bytes, void* stream) {
     Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    int rc = check_learn_grads(dims, hp, replay, nets, draws, global_batch, grads_out, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
     if ((rc = check_dist_hp(hp))) return rc;
     if ((rc = check_quantile(dims, quantile, true))) return rc;
     if ((rc = check_dist_nets(nets, true))) return rc;
-    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     cudaStream_t s = (cudaStream_t)stream;
     if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
     return launch_learn_quantile(*dims, *hp, *replay, *nets, *quantile, metrics_out, (char*)workspace, w, grads_out,
@@ -749,22 +779,16 @@ static int check_iqn(const dmdqn_dims* dims, const dmdqn_iqn* q, bool learn) {
     return DMDQN_OK;
 }
 
-static int check_iqn_hp(const dmdqn_hparams* hp) {
-    DMDQN_CHECK_ARG(hp != nullptr, "iqn: hp is NULL");
-    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32, "precision=%d: IQN networks run the fp32 (FFMA) path only",
-                    hp->precision);
-    DMDQN_CHECK_ARG(hp->dueling == 0, "dueling=%d: dueling heads are not supported with IQN networks", hp->dueling);
-    return DMDQN_OK;
-}
+static int check_iqn_hp(const dmdqn_hparams* hp) { return check_kind_hp(hp, "iqn", "IQN", 0); }
 
 int dmdqn_param_layout_iqn(const dmdqn_dims* dims, int32_t n_cos, dmdqn_iqn_layout* out) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     if ((rc = check_n_cos(n_cos))) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const IqnLayout q = make_layout_iqn(dims->obs_stride, dims->hidden, n_cos);
-    out->w1 = q.L.w1; out->b1 = q.L.b1; out->w2 = q.L.w2; out->b2 = q.L.b2; out->w3 = q.L.w3; out->b3 = q.L.b3;
-    out->wphi = q.wphi; out->bphi = q.bphi; out->end = q.L.end; out->stride = q.L.stride;
+    const Layout l = make_layout(dims->obs_stride, dims->hidden, {1, 1, false, n_cos});
+    copy_trunk(l, out);
+    out->wphi = l.wphi; out->bphi = l.bphi; out->end = l.end;
     return DMDQN_OK;
 }
 
@@ -781,14 +805,11 @@ int dmdqn_learn_grads_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const
                           const dmdqn_nets* nets, const void* draws, const uint8_t* learn_mask, int32_t global_batch,
                           float* grads_out, float* metrics_out, void* workspace, size_t workspace_bytes, void* stream) {
     Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    int rc = check_learn_grads(dims, hp, replay, nets, draws, global_batch, grads_out, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
     if ((rc = check_iqn_hp(hp))) return rc;
     if ((rc = check_iqn(dims, iqn, true))) return rc;
     if ((rc = check_dist_nets(nets, true))) return rc;
-    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     cudaStream_t s = (cudaStream_t)stream;
     if ((rc = launch_sample(*dims, *hp, *replay, *nets, draws, learn_mask, 1, (char*)workspace, w, s))) return rc;
     return launch_learn_iqn(*dims, *hp, *replay, *nets, *iqn, metrics_out, (char*)workspace, w, grads_out, global_batch, s);
@@ -806,8 +827,7 @@ int dmdqn_adam_apply_iqn(const dmdqn_dims* dims, const dmdqn_hparams* hp, const 
     DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_iqn: grads is NULL or not 16-byte aligned");
     DMDQN_CHECK_ARG(global_clipnorm >= 0.0 && isfinite(global_clipnorm),
                     "global_clipnorm=%g must be 0 (no clipping) or a positive finite number", global_clipnorm);
-    return launch_adam_apply_iqn(*dims, *hp, *nets, n_cos, grads, global_clipnorm, norms_out, (char*)workspace, w,
-                                 (cudaStream_t)stream);
+    return run_adam(*dims, *hp, {1, 1, false, n_cos}, *nets, grads, global_clipnorm, norms_out, workspace, w, stream);
 }
 
 int dmdqn_act_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_iqn* iqn, const float* obs, int32_t obs_in_stride,
@@ -829,7 +849,8 @@ int dmdqn_sync_target_iqn(const dmdqn_dims* dims, const dmdqn_nets* nets, int32_
     if (rc) return rc;
     if ((rc = check_n_cos(n_cos))) return rc;
     if ((rc = check_dist_nets(nets, false))) return rc;
-    return launch_sync_target_iqn(*dims, *nets, n_cos, mask, tau, (cudaStream_t)stream);
+    return launch_sync_target(*dims, make_layout(dims->obs_stride, dims->hidden, {1, 1, false, n_cos}).stride, nets->theta,
+                              nets->theta_tgt, mask, tau, (cudaStream_t)stream);
 }
 
 int dmdqn_debug_iqn(const dmdqn_dims* dims, const dmdqn_iqn* iqn, dmdqn_iqn_views* out) {
@@ -856,22 +877,16 @@ static int check_rainbow(const dmdqn_dims* dims, const dmdqn_dist* ds, bool scra
     return DMDQN_OK;
 }
 
-static int check_rainbow_hp(const dmdqn_hparams* hp) {
-    DMDQN_CHECK_ARG(hp != nullptr, "rainbow: hp is NULL");
-    DMDQN_CHECK_ARG(hp->precision == DMDQN_PRECISION_FP32, "precision=%d: Rainbow networks run the fp32 (FFMA) path only",
-                    hp->precision);
-    DMDQN_CHECK_ARG(hp->dueling == 1, "dueling=%d: Rainbow blocks carry the value stream, so hp->dueling must be 1", hp->dueling);
-    return DMDQN_OK;
-}
+static int check_rainbow_hp(const dmdqn_hparams* hp) { return check_kind_hp(hp, "rainbow", "Rainbow", 1); }
 
 int dmdqn_param_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_rainbow_layout* out) {
     int rc = validate_dims(dims);
     if (rc) return rc;
     if ((rc = check_atoms(n_atoms))) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const RainbowLayout r = make_layout_rainbow(dims->obs_stride, dims->hidden, dist_np(n_atoms));
-    out->w1 = r.L.w1; out->b1 = r.L.b1; out->w2 = r.L.w2; out->b2 = r.L.b2; out->w3 = r.L.w3; out->b3 = r.L.b3;
-    out->wv = r.wv; out->bv = r.bv; out->end = r.L.end; out->stride = r.L.stride;
+    const Layout l = make_layout(dims->obs_stride, dims->hidden, atom_shape(n_atoms, true));
+    copy_trunk(l, out);
+    out->wv = l.wv; out->bv = l.bv; out->end = l.end;
     return DMDQN_OK;
 }
 
@@ -880,11 +895,7 @@ int dmdqn_noise_layout_rainbow(const dmdqn_dims* dims, int32_t n_atoms, dmdqn_no
     if (rc) return rc;
     if ((rc = check_atoms(n_atoms))) return rc;
     DMDQN_CHECK_ARG(out != nullptr, "out is NULL");
-    const int np = dist_np(n_atoms);
-    const NoiseRec r = make_noise_rec(dims->obs_stride, dims->hidden, 4 * np, np);
-    int64_t* f[8] = {&out->w1_in, &out->w1_out, &out->w2_in, &out->w2_out, &out->w3_in, &out->w3_out, &out->v_in, &out->v_out};
-    for (int v = 0; v < 8; ++v) *f[v] = r.off[v];
-    out->stride = r.stride;
+    copy_noise_rec(make_noise_rec(dims->obs_stride, dims->hidden, atom_shape(n_atoms, true)), out);
     return DMDQN_OK;
 }
 
@@ -911,14 +922,11 @@ int dmdqn_learn_grads_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, c
                               const uint8_t* learn_mask, int32_t global_batch, float* grads_out, float* metrics_out,
                               void* workspace, size_t workspace_bytes, void* stream) {
     Workspace w;
-    int rc = check_workspace(dims, workspace, workspace_bytes, &w);
+    int rc = check_learn_grads(dims, hp, replay, nets, draws, global_batch, grads_out, workspace, workspace_bytes, &w);
     if (rc) return rc;
-    if ((rc = check_learn_args(dims, hp, replay, nets, draws))) return rc;
     if ((rc = check_rainbow_hp(hp))) return rc;
     if ((rc = check_rainbow(dims, dist, true))) return rc;
     if ((rc = check_noisy(nets, noisy, true))) return rc;
-    DMDQN_CHECK_ARG(grads_out && aligned16(grads_out), "grads_out is NULL or not 16-byte aligned");
-    DMDQN_CHECK_ARG(global_batch >= dims->batch, "global_batch=%d < batch=%d", global_batch, dims->batch);
     cudaStream_t s = (cudaStream_t)stream;
     if ((rc = launch_rainbow_fold(*dims, *dist, *nets, *noisy, s))) return rc;
     dmdqn_nets eff = *nets;
@@ -937,7 +945,8 @@ int dmdqn_adam_apply_rainbow(const dmdqn_dims* dims, const dmdqn_hparams* hp, co
     if ((rc = check_atoms(n_atoms))) return rc;
     if ((rc = check_noisy(nets, noisy, true))) return rc;
     DMDQN_CHECK_ARG(grads && aligned16(grads), "adam_apply_rainbow: grads is NULL or not 16-byte aligned");
-    return launch_adam_apply_rainbow(*dims, *hp, *nets, *noisy, n_atoms, grads, (char*)workspace, w, (cudaStream_t)stream);
+    return launch_noisy_adam_apply(*dims, *hp, atom_shape(n_atoms, true), *nets, *noisy, grads, (char*)workspace, w,
+                                   (cudaStream_t)stream);
 }
 
 int dmdqn_act_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, const dmdqn_noisy* noisy, const dmdqn_dist* dist,
@@ -962,7 +971,7 @@ int dmdqn_sync_target_rainbow(const dmdqn_dims* dims, const dmdqn_nets* nets, co
     if (rc) return rc;
     if ((rc = check_atoms(n_atoms))) return rc;
     if ((rc = check_noisy(nets, noisy, false))) return rc;
-    return launch_sync_target_rainbow(*dims, *nets, *noisy, n_atoms, mask, tau, (cudaStream_t)stream);
+    return sync_noisy(*dims, atom_shape(n_atoms, true), *nets, *noisy, mask, tau, stream);
 }
 
 int dmdqn_debug_rainbow(const dmdqn_dims* dims, const dmdqn_dist* dist, dmdqn_rainbow_views* out) {
@@ -983,7 +992,8 @@ static int run_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const
     int rc = validate_dims(dims);
     if (rc) return rc;
     DMDQN_CHECK_ARG(nets && nets->theta && nets->theta_tgt, "sync_target: NULL network pointer");
-    return launch_sync_target(*dims, *nets, mask, tau, dueling, (cudaStream_t)stream);
+    return launch_sync_target(*dims, make_layout(dims->obs_stride, dims->hidden, {1, 1, dueling, 0}).stride, nets->theta,
+                              nets->theta_tgt, mask, tau, (cudaStream_t)stream);
 }
 
 int dmdqn_sync_target(const dmdqn_dims* dims, const dmdqn_nets* nets, const uint8_t* mask, double tau,

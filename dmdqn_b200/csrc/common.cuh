@@ -26,27 +26,45 @@ void set_error(const char* fmt, ...);
         }                                                                             \
     } while (0)
 
-// Float offsets of W1|b1|W2|b2|W3|b3 inside one parameter block (include/dmdqn_b200.h).  `end` closes the range the
-// Adam kernels update: b3 + 4, or with the dueling value head wv[H] | bv | pad[3] after b3, b3 + 8 + H.
+// Every parameter block (include/dmdqn_b200.h) is W1|b1|W2|b2|W3|b3, then an optional value stream or cosine embedding.
+// The head shape decides the offsets: n atoms per action (1: a scalar head), np the column stride per action (1, or n
+// rounded up to a multiple of 4), value: Wv[H][np] | bv[round4(np)] after b3 (dueling and Rainbow), n_cos > 0: Wphi[n_cos][H]
+// | bphi[H] after b3 (IQN).  The plain, dueling, C51 / QR-DQN, IQN and Rainbow blocks are (1, 1, -, 0), (1, 1, value, 0),
+// (N, Np, -, 0), (1, 1, -, n_cos) and (N, Np, value, 0).
+struct HeadShape {
+    int n = 1, np = 1;
+    bool value = false;
+    int n_cos = 0;
+};
+inline int dist_np(int n_atoms) { return (n_atoms + 3) / 4 * 4; }
+inline HeadShape atom_shape(int n_atoms, bool value) { return {n_atoms, dist_np(n_atoms), value, 0}; }
+// Float offsets inside one block.  `end` closes the range the Adam kernels update; wv / bv and wphi / bphi equal the end
+// of the head (b3 + 4 * np) when the block has no value stream or embedding.
 struct Layout {
     int64_t w1, b1, w2, b2, w3, b3, stride;
     int64_t end;
+    int64_t wv, bv, wphi, bphi;
 };
-__host__ __device__ inline Layout make_layout(int dp, int h, bool dueling = false) {
+__host__ __device__ inline Layout make_layout(int dp, int h, HeadShape hs = {}) {
     Layout l;
     l.w1 = 0;
     l.b1 = (int64_t)dp * h;
     l.w2 = l.b1 + h;
     l.b2 = l.w2 + (int64_t)h * h;
     l.w3 = l.b2 + h;
-    l.b3 = l.w3 + (int64_t)h * 4;
-    l.end = l.b3 + 4 + (dueling ? h + 4 : 0);
+    l.b3 = l.w3 + (int64_t)h * 4 * hs.np;
+    l.end = l.b3 + 4 * hs.np;
+    l.wv = l.bv = l.wphi = l.bphi = l.end;
+    if (hs.value) {
+        l.bv = l.wv + (int64_t)h * hs.np;
+        l.end = l.bv + (hs.np + 3) / 4 * 4;
+    } else if (hs.n_cos) {
+        l.bphi = l.wphi + (int64_t)hs.n_cos * h;
+        l.end = l.bphi + h;
+    }
     l.stride = (l.end + 31) / 32 * 32;  // blocks start on 128-byte lines
     return l;
 }
-// Dueling value head: wv[H] right after b3 (16-byte aligned), bv after it.
-__host__ __device__ inline int64_t layout_wv(const Layout& l) { return l.b3 + 4; }
-__host__ __device__ inline int64_t layout_bv(const Layout& l, int h) { return l.b3 + 4 + h; }
 
 // The dueling fold (include/dmdqn_b200.h): the mean over the first A of four values, summed left to right in fp32 and
 // divided by A, and the effective head value (x - mean) + v.  Shared by the fold kernel, act and both head updates.
@@ -94,14 +112,14 @@ __host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 
 // Offsets (floats) of the eight factor vectors inside one network's noise record for one set (include/dmdqn_b200.h
 // dmdqn_noise_record): off[2 * layer + side], layer 0..3 = W1, W2, W3, value head, side 0 = inputs, 1 = outputs; off[8]
-// is the end of the last vector, `stride` the record's stride (a network's two sets are adjacent records).  nh / nv: the
-// widths of the head's and the value head's output vectors (4 and 4 for plain and dueling blocks, 4 * Np and Np for Rainbow).
+// is the end of the last vector, `stride` the record's stride (a network's two sets are adjacent records).  The head's
+// output vector has 4 * np entries (column a * np + j), the value head's round4(np) (entry j = atom j).
 struct NoiseRec {
     int32_t off[9];
     int32_t stride;
 };
-__host__ __device__ inline NoiseRec make_noise_rec(int dp, int h, int nh = 4, int nv = 4) {
-    const int32_t len[8] = {dp, h, h, h, h, nh, h, nv};
+__host__ __device__ inline NoiseRec make_noise_rec(int dp, int h, HeadShape hs = {}) {
+    const int32_t len[8] = {dp, h, h, h, h, 4 * hs.np, h, (hs.np + 3) / 4 * 4};
     NoiseRec r;
     r.off[0] = 0;
     for (int v = 0; v < 8; ++v) r.off[v + 1] = r.off[v] + len[v];
@@ -120,22 +138,26 @@ __device__ __forceinline__ float noise_factor(uint64_t key, uint32_t i, int vec,
 }
 
 // The whole record of one network and set into `rec` (shared memory), every thread of the block taking part; entries for
-// padding (W1 input rows >= obs_dim, W3 output columns >= A, the value head's outputs >= 1, the tail up to the stride) are 0.
-__device__ __forceinline__ void noise_record_build(float* rec, const NoiseRec& R, int obs_dim, int n_actions, uint64_t key,
-                                                   uint32_t t, int set) {
+// padding are 0: W1 input rows >= obs_dim, head output columns a * np + j with a >= A or j >= n_atoms, value head outputs
+// >= n_atoms, and the tail up to the stride.  Scalar heads pass n_atoms = np = 1.
+__device__ __forceinline__ void noise_record_build(float* rec, const NoiseRec& R, int obs_dim, int n_actions, int n_atoms, int np,
+                                                   uint64_t key, uint32_t t, int set) {
     for (int e = threadIdx.x; e < R.stride; e += blockDim.x) {
         int v = 0;
         while (v < 8 && e >= R.off[v + 1]) ++v;
         const int i = e - R.off[v];
-        const int valid = v == 0 ? obs_dim : v == 5 ? n_actions : v == 7 ? 1 : R.off[v + 1] - R.off[v];
-        rec[e] = v < 8 && i < valid ? noise_factor(key, (uint32_t)i, v, set, t) : 0.f;
+        const bool valid = v == 0 ? i < obs_dim : v == 5 ? i / np < n_actions && i % np < n_atoms : v == 7 ? i < n_atoms : v < 8;
+        rec[e] = valid ? noise_factor(key, (uint32_t)i, v, set, t) : 0.f;
     }
 }
 
 // The weight noise of the four floats at offset e (a multiple of 4) of a parameter block: f_in[i] * f_out[j] for a weight,
-// f_out[j] for a bias, 0 on padding.  rec: the record of the set (include/dmdqn_b200.h: wv is the value head's input side
-// and column 0 of its output side, bv with its three pad floats takes the output side's four entries).
-__device__ __forceinline__ float4 noise_eps4(const float* rec, const NoiseRec& R, const Layout& L, int H, bool dueling, int64_t e) {
+// f_out[j] for a bias, 0 on padding.  rec: the record of the set.  W3 / b3 take the head's output side at column
+// (e - w3) % (4 * np); Wv / bv the value head's input side at row (e - wv) / np and its output side at atom (e - wv) % np.
+// With np a multiple of 4 a float4 never straddles two rows; with np == 1 (the dueling value head wv[H] | bv | pad[3]) one
+// float4 of wv spans four rows, so that case takes one input factor per element.
+__device__ __forceinline__ float4 noise_eps4(const float* rec, const NoiseRec& R, const Layout& L, int H, int np, int64_t e) {
+    const int nh = 4 * np;
     auto outer = [&](float fi, const float* fo) {
         return make_float4(__fmul_rn(fi, fo[0]), __fmul_rn(fi, fo[1]), __fmul_rn(fi, fo[2]), __fmul_rn(fi, fo[3]));
     };
@@ -144,14 +166,17 @@ __device__ __forceinline__ float4 noise_eps4(const float* rec, const NoiseRec& R
     if (e < L.w2) return vec(rec + R.off[1] + (e - L.b1));
     if (e < L.b2) return outer(rec[R.off[2] + (e - L.w2) / H], rec + R.off[3] + (e - L.w2) % H);
     if (e < L.w3) return vec(rec + R.off[3] + (e - L.b2));
-    if (e < L.b3) return outer(rec[R.off[4] + (e - L.w3) / 4], rec + R.off[5]);
-    if (e < L.b3 + 4) return vec(rec + R.off[5]);
-    if (dueling && e < layout_bv(L, H)) {
-        const float fo = rec[R.off[7]];
-        const float* fi = rec + R.off[6] + (e - layout_wv(L));
-        return make_float4(__fmul_rn(fi[0], fo), __fmul_rn(fi[1], fo), __fmul_rn(fi[2], fo), __fmul_rn(fi[3], fo));
+    if (e < L.b3) return outer(rec[R.off[4] + (e - L.w3) / nh], rec + R.off[5] + (e - L.w3) % nh);
+    if (e < L.wv) return vec(rec + R.off[5] + (e - L.b3));
+    if (e < L.bv) {
+        if (np == 1) {
+            const float fo = rec[R.off[7]];
+            const float* fi = rec + R.off[6] + (e - L.wv);
+            return make_float4(__fmul_rn(fi[0], fo), __fmul_rn(fi[1], fo), __fmul_rn(fi[2], fo), __fmul_rn(fi[3], fo));
+        }
+        return outer(rec[R.off[6] + (e - L.wv) / np], rec + R.off[7] + (e - L.wv) % np);
     }
-    if (dueling && e == layout_bv(L, H)) return vec(rec + R.off[7]);
+    if (e < L.end) return vec(rec + R.off[7] + (e - L.bv));
     return make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
@@ -161,14 +186,6 @@ __device__ __forceinline__ float noisy_weight(float mu, float sigma, float eps) 
 // Distributional (C51) networks (include/dmdqn_b200.h dmdqn_dist).  The head is W3[H][4 * Np] | b3[4 * Np], Np = N rounded
 // up to a multiple of 4, column a * Np + j = atom j of action a; the Adam range ends after b3.
 constexpr int kDistMaxAtoms = 64;
-inline int dist_np(int n_atoms) { return (n_atoms + 3) / 4 * 4; }
-__host__ __device__ inline Layout make_layout_dist(int dp, int h, int np) {
-    Layout l = make_layout(dp, h);
-    l.b3 = l.w3 + (int64_t)h * 4 * np;
-    l.end = l.b3 + 4 * np;
-    l.stride = (l.end + 31) / 32 * 32;
-    return l;
-}
 // The caller-owned scratch of the distributional learn kernels, byte offsets (256-aligned): the projected target
 // distribution m [n_nets][B][Np], h2 [n_nets][B][H] and the logit gradient dX [n_nets][B][4 * Np].
 struct DistScratch {
@@ -228,21 +245,6 @@ __device__ __forceinline__ float dist_expect(const float* x, int n, const float*
     return q;
 }
 
-// Rainbow networks (include/dmdqn_b200.h dmdqn_rainbow_layout): the C51 block with the value stream Wv[H][Np] | bv[Np] after
-// b3 (at the C51 end); Adam covers all of it.
-struct RainbowLayout {
-    Layout L;                         // L.end = bv + Np
-    int64_t wv, bv;
-};
-__host__ __device__ inline RainbowLayout make_layout_rainbow(int dp, int h, int np) {
-    RainbowLayout r;
-    r.L = make_layout_dist(dp, h, np);
-    r.wv = r.L.end;
-    r.bv = r.wv + (int64_t)h * np;
-    r.L.end = r.bv + np;
-    r.L.stride = (r.L.end + 31) / 32 * 32;
-    return r;
-}
 // The Rainbow scratch: the C51 regions, then the folded heads W3e[H][4 * Np] | b3e[4 * Np] of the online (0) and the target
 // (1) network, [2][n_nets][(H + 1) * 4 * Np] floats.
 struct RainbowScratch {
@@ -256,39 +258,6 @@ inline RainbowScratch make_rainbow_scratch(const dmdqn_dims& d, int np) {
     s.total = s.head + (2 * (size_t)d.n_nets * (d.hidden + 1) * 4 * np * 4 + 255) / 256 * 256;
     return s;
 }
-// The Rainbow noise record (dmdqn_noise_layout_rainbow): output factor i of W3 is column a * Np + j (0 unless a < A and
-// j < N), entry j of the value head's outputs is atom j (0 for j >= N).  Otherwise noise_record_build's rule.
-__device__ __forceinline__ void noise_record_build_rainbow(float* rec, const NoiseRec& R, int obs_dim, int n_actions, int n_atoms,
-                                                           int np, uint64_t key, uint32_t t, int set) {
-    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) {
-        int v = 0;
-        while (v < 8 && e >= R.off[v + 1]) ++v;
-        const int i = e - R.off[v];
-        const bool valid = v == 0 ? i < obs_dim : v == 5 ? i / np < n_actions && i % np < n_atoms : v == 7 ? i < n_atoms : v < 8;
-        rec[e] = valid ? noise_factor(key, (uint32_t)i, v, set, t) : 0.f;
-    }
-}
-// noise_eps4 on a Rainbow block: W3 / b3 take the head's output side at column (e - w3) % (4 * Np), Wv / bv the value head's
-// input side and output side at atom (e - wv) % Np.  A float4 never straddles two rows (Np is a multiple of 4).
-__device__ __forceinline__ float4 noise_eps4_rainbow(const float* rec, const NoiseRec& R, const RainbowLayout& RL, int H, int np,
-                                                     int64_t e) {
-    const Layout& L = RL.L;
-    const int nh = 4 * np;
-    auto outer = [&](float fi, const float* fo) {
-        return make_float4(__fmul_rn(fi, fo[0]), __fmul_rn(fi, fo[1]), __fmul_rn(fi, fo[2]), __fmul_rn(fi, fo[3]));
-    };
-    auto vec = [](const float* f) { return make_float4(f[0], f[1], f[2], f[3]); };
-    if (e < L.b1) return outer(rec[R.off[0] + e / H], rec + R.off[1] + e % H);
-    if (e < L.w2) return vec(rec + R.off[1] + (e - L.b1));
-    if (e < L.b2) return outer(rec[R.off[2] + (e - L.w2) / H], rec + R.off[3] + (e - L.w2) % H);
-    if (e < L.w3) return vec(rec + R.off[3] + (e - L.b2));
-    if (e < L.b3) return outer(rec[R.off[4] + (e - L.w3) / nh], rec + R.off[5] + (e - L.w3) % nh);
-    if (e < RL.wv) return vec(rec + R.off[5] + (e - L.b3));
-    if (e < RL.bv) return outer(rec[R.off[6] + (e - RL.wv) / np], rec + R.off[7] + (e - RL.wv) % np);
-    if (e < L.end) return vec(rec + R.off[7] + (e - RL.bv));
-    return make_float4(0.f, 0.f, 0.f, 0.f);
-}
-
 // Quantile (QR-DQN) networks (include/dmdqn_b200.h dmdqn_quantile): the C51 head layout, scratch and Adam range for
 // N = n_quantiles atoms; the scratch's m region holds the target samples T.  What the kernels take beyond LearnArgs:
 struct QuantArgs {
@@ -316,21 +285,6 @@ __device__ __forceinline__ float quantile_mean(const float* x, int n) {
     return __fdiv_rn(s, (float)n);
 }
 
-// Implicit quantile networks (include/dmdqn_b200.h dmdqn_iqn).  The block is the plain one with the cosine embedding
-// Wphi[n_cos][H] | bphi[H] after b3; Adam covers all of it.
-struct IqnLayout {
-    Layout L;                         // L.end = bphi + H
-    int64_t wphi, bphi;
-};
-__host__ __device__ inline IqnLayout make_layout_iqn(int dp, int h, int n_cos) {
-    IqnLayout q;
-    q.L = make_layout(dp, h);
-    q.wphi = q.L.b3 + 4;
-    q.bphi = q.wphi + (int64_t)n_cos * h;
-    q.L.end = q.bphi + h;
-    q.L.stride = (q.L.end + 31) / 32 * 32;
-    return q;
-}
 // Fraction i of sampled row `row` (row_base + r), set 0 (tau) or 1 (tau') at step t: the top 23 bits of the first Philox
 // word, ((x >> 9) + 0.5) * 2^-23, exact in fp32 and strictly inside (0, 1).
 __host__ __device__ __forceinline__ float iqn_tau(uint64_t key, uint32_t row, uint32_t i, uint32_t t, int set) {
@@ -483,7 +437,7 @@ inline IqnArgs make_iqn_args(const dmdqn_dims& d, const dmdqn_iqn& q) {
     Q.kappa = (float)q.kappa;
     Q.row_base = q.row_base;
     Q.key = q.key;
-    const IqnLayout L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos);
+    const Layout L = make_layout(d.obs_stride, d.hidden, {1, 1, false, q.n_cos});
     Q.wphi = L.wphi; Q.bphi = L.bphi;
     const IqnScratch s = make_iqn_scratch(d, q.n_tau, q.n_tau_prime, q.n_cos);
     char* p = static_cast<char*>(q.scratch);
@@ -537,8 +491,8 @@ struct LearnArgs {
     int64_t head_stride;
     int dueling;                      // K4b projects the head gradient onto W3 / b3 / wv / bv
 };
-LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                          char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch);
+LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, HeadShape hs, const dmdqn_replay& rp,
+                          const dmdqn_nets& nets, char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch);
 
 // Prioritized replay, K4a of both paths: the priority of the transition behind row `row` (agent * C + slot) from its TD
 // error, (float)pow(|delta| + eps, alpha) in float64, and the agent's running maximum (positive floats order like their
@@ -602,9 +556,9 @@ int launch_featurize_alt(int32_t n, const int32_t* halting, const int32_t* phase
 int launch_act(const dmdqn_dims& d, const dmdqn_nets& nets, const float* obs, int32_t stride,
                const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, bool dueling,
                cudaStream_t s, const dmdqn_noisy* noisy = nullptr);
-int launch_noisy_fold(const dmdqn_dims& d, bool dueling, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s);
-int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
-                            const float* grads, char* ws, const Workspace& w, cudaStream_t s);
+int launch_noisy_fold(const dmdqn_dims& d, HeadShape hs, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s);
+int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, HeadShape hs, const dmdqn_nets& nets,
+                            const dmdqn_noisy& nz, const float* grads, char* ws, const Workspace& w, cudaStream_t s);
 int launch_push(const dmdqn_dims& d, const dmdqn_replay& rp, const float* obs, const int32_t* act,
                 const double* rew, const float* next_obs, const uint8_t* done, int32_t in_stride,
                 const uint8_t* mask, cudaStream_t s);
@@ -618,22 +572,17 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
                  float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch, cudaStream_t s);
 bool tc_supported(const dmdqn_dims& d);
 int launch_learn_tc(const LearnArgs& A, int precision, int stages, cudaStream_t s);
-int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads, char* ws,
-                      const Workspace& w, cudaStream_t s);
-int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads,
-                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
-int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau, bool dueling,
+// Adam over [0, A.L.end) of every active block: plain (clipnorm == 0) or after global-norm clipping
+int launch_adam(const LearnArgs& A, const float* grads, double clipnorm, float* norms_out, cudaStream_t s);
+int launch_sync_target(const dmdqn_dims& d, int64_t stride, float* theta, float* theta_tgt, const uint8_t* mask, double tau,
                        cudaStream_t s);
-int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Workspace& w, cudaStream_t s);
+// W3e | b3e of the online and the target block of every network into head[2][n_nets][(H + 1) * 4 * np] (hs.value blocks)
+int launch_head_fold(const dmdqn_dims& d, HeadShape hs, const float* theta, const float* theta_tgt, float* head, cudaStream_t s);
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,
                      const float* my_loss_src, float* loss_out, char* ws, const Workspace& w, cudaStream_t s);
 int launch_learn_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                       const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
                       cudaStream_t s);
-int launch_adam_apply_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_atoms, const float* grads,
-                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
-int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_atoms, const uint8_t* mask, double tau,
-                            cudaStream_t s);
 int launch_act_dist(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_dist& ds, const float* obs, int32_t stride,
                     const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
 int launch_learn_quantile(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
@@ -644,19 +593,12 @@ int launch_act_quantile(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn
                         cudaStream_t s);
 int launch_learn_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                      const dmdqn_iqn& q, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch, cudaStream_t s);
-int launch_adam_apply_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_cos, const float* grads,
-                          double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s);
-int launch_sync_target_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, int n_cos, const uint8_t* mask, double tau, cudaStream_t s);
 int launch_act_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_iqn& q, const float* obs, int32_t stride,
                    const double* eps, const uint32_t* w1, const uint32_t* w2, int32_t* actions, float* q_out, cudaStream_t s);
 int launch_rainbow_fold(const dmdqn_dims& d, const dmdqn_dist& ds, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s);
 int launch_learn_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& eff,
                          const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
                          cudaStream_t s);
-int launch_adam_apply_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
-                              int n_atoms, const float* grads, char* ws, const Workspace& w, cudaStream_t s);
-int launch_sync_target_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy& nz, int n_atoms,
-                               const uint8_t* mask, double tau, cudaStream_t s);
 int launch_act_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy* noisy, const dmdqn_dist& ds,
                        const float* obs, int32_t stride, const double* eps, const uint32_t* w1, const uint32_t* w2,
                        int32_t* actions, float* q_out, cudaStream_t s);

@@ -12,6 +12,7 @@
 // 16-byte shared-memory access of a quarter-warp is conflict-free).  All sums run in a
 // fixed order: results are deterministic run to run.
 #include <algorithm>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -486,9 +487,9 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
                 w[0] += pw.x; w[1] += pw.y; w[2] += pw.z; w[3] += pw.w;
             }
             if (A.dueling) {
-                upd(j < H ? layout_wv(A.L) + j : layout_bv(A.L, H), head_project(w, A.d.n_actions));
+                upd(j < H ? A.L.wv + j : A.L.bv, head_project(w, A.d.n_actions));
                 if (j == H && A.grads)                     // the pad after bv is inside the Adam range: its gradient is 0
-                    for (int p = 1; p < 4; ++p) A.grads[(size_t)g * A.L.stride + layout_bv(A.L, H) + p] = 0.f;
+                    for (int p = 1; p < 4; ++p) A.grads[(size_t)g * A.L.stride + A.L.bv + p] = 0.f;
             }
             const int64_t off = j < H ? A.L.w3 + (int64_t)j * 4 : A.L.b3;
             for (int a = 0; a < 4; ++a) upd(off + a, w[a]);
@@ -578,21 +579,6 @@ __global__ void __launch_bounds__(Tile<H>::NT) wgrad_adam_kernel(const LearnArgs
     }
 }
 
-// Dueling fold (include/dmdqn_b200.h): W3e | b3e of network blockIdx.x's online (blockIdx.y = 0) or target (1) block into
-// head[blockIdx.y][blockIdx.x], one thread per W3 row and one more for the bias.
-__global__ void __launch_bounds__(256) fold_kernel(Layout L, int H, int n_actions, const float* __restrict__ theta,
-                                                   const float* __restrict__ theta_tgt, float* __restrict__ head) {
-    const int g = blockIdx.x, n_nets = gridDim.x;
-    const float* P = (blockIdx.y ? theta_tgt : theta) + (size_t)g * L.stride;
-    float* out = head + ((size_t)blockIdx.y * n_nets + g) * (4 * H + 4);
-    for (int j = threadIdx.x; j <= H; j += blockDim.x) {
-        const float4 w = __ldg(reinterpret_cast<const float4*>(P + (j < H ? L.w3 + 4 * j : L.b3)));
-        float x[4] = {w.x, w.y, w.z, w.w};
-        head_fold(x, __ldg(P + (j < H ? layout_wv(L) + j : layout_bv(L, H))), n_actions);
-        reinterpret_cast<float4*>(out)[j] = make_float4(x[0], x[1], x[2], x[3]);
-    }
-}
-
 // theta_tgt <- theta (tau < 0) or Polyak (tau >= 0) for the masked networks.
 __global__ void sync_target_kernel(int64_t stride, const float* __restrict__ theta, float* __restrict__ tgt,
                                    const uint8_t* __restrict__ mask, float tau) {
@@ -635,11 +621,11 @@ __global__ void adam_apply_kernel(const LearnArgs A, const float* __restrict__ g
 constexpr int kNoisyThreads = 256;
 
 __global__ void __launch_bounds__(kNoisyThreads)
-noisy_fold_kernel(Layout L, NoiseRec R, int H, int obs_dim, int n_actions, int dueling, const dmdqn_nets nets,
+noisy_fold_kernel(Layout L, NoiseRec R, int H, int obs_dim, int n_actions, int n_atoms, int np, const dmdqn_nets nets,
                   const dmdqn_noisy nz, int64_t per) {
     extern __shared__ __align__(16) float rec[];
     const int g = blockIdx.y, set = blockIdx.z;
-    noise_record_build(rec, R, obs_dim, n_actions, __ldg(nz.key + g), (uint32_t)__ldg(nets.learn_step + g), set);
+    noise_record_build(rec, R, obs_dim, n_actions, n_atoms, np, __ldg(nz.key + g), (uint32_t)__ldg(nets.learn_step + g), set);
     __syncthreads();
     if (blockIdx.x == 0)
         for (int e = threadIdx.x; e < R.stride; e += blockDim.x) nz.noise[((size_t)g * 2 + set) * R.stride + e] = rec[e];
@@ -649,7 +635,7 @@ noisy_fold_kernel(Layout L, NoiseRec R, int H, int obs_dim, int n_actions, int d
     float4* out = reinterpret_cast<float4*>((set ? nz.eff_tgt : nz.eff) + base);
     const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, L.stride / 4);
     for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
-        const float4 m = __ldg(mu + i), s = __ldg(sg + i), e = noise_eps4(rec, R, L, H, dueling, i * 4);
+        const float4 m = __ldg(mu + i), s = __ldg(sg + i), e = noise_eps4(rec, R, L, H, np, i * 4);
         out[i] = make_float4(noisy_weight(m.x, s.x, e.x), noisy_weight(m.y, s.y, e.y), noisy_weight(m.z, s.z, e.z),
                              noisy_weight(m.w, s.w, e.w));
     }
@@ -658,7 +644,7 @@ noisy_fold_kernel(Layout L, NoiseRec R, int H, int obs_dim, int n_actions, int d
 // Adam on mu and sigma from the effective-weight gradient g: g_mu = g, g_sigma = g * eps with set 0's record, each through
 // adam_vec4 as adam_apply_kernel applies it.  HBM bound: g once, and theta / m / v (+ target) of mu and of sigma.
 __global__ void __launch_bounds__(kNoisyThreads)
-noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, const float* __restrict__ grads, int64_t per) {
+noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, int np, const float* __restrict__ grads, int64_t per) {
     extern __shared__ __align__(16) float rec[];
     const int g = blockIdx.y;
     if (!A.active[g] || *reinterpret_cast<volatile int*>(A.error) != 0) return;
@@ -671,7 +657,7 @@ noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, con
     const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, A.L.end / 4);
     for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
         const float4 g4 = *reinterpret_cast<const float4*>(grads + base + i * 4);
-        const float4 e = noise_eps4(rec, R, A.L, H, A.dueling, i * 4);
+        const float4 e = noise_eps4(rec, R, A.L, H, np, i * 4);
         const float gm[4] = {g4.x, g4.y, g4.z, g4.w};
         const float gs[4] = {__fmul_rn(g4.x, e.x), __fmul_rn(g4.y, e.y), __fmul_rn(g4.z, e.z), __fmul_rn(g4.w, e.w)};
         const size_t o = base + i * 4;
@@ -680,91 +666,53 @@ noisy_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, NoiseRec R, con
     }
 }
 
-// Rainbow (include/dmdqn_b200.h dmdqn_rainbow_layout).  Noise fold: noisy_fold_kernel with the Rainbow record and eps.
-__global__ void __launch_bounds__(kNoisyThreads)
-rainbow_noisy_fold_kernel(RainbowLayout RL, NoiseRec R, int H, int obs_dim, int n_actions, int n_atoms, int np,
-                          const dmdqn_nets nets, const dmdqn_noisy nz, int64_t per) {
-    extern __shared__ __align__(16) float rec[];
-    const int g = blockIdx.y, set = blockIdx.z;
-    noise_record_build_rainbow(rec, R, obs_dim, n_actions, n_atoms, np, __ldg(nz.key + g), (uint32_t)__ldg(nets.learn_step + g),
-                               set);
-    __syncthreads();
-    if (blockIdx.x == 0)
-        for (int e = threadIdx.x; e < R.stride; e += blockDim.x) nz.noise[((size_t)g * 2 + set) * R.stride + e] = rec[e];
-    const size_t base = (size_t)g * RL.L.stride;
-    const float4* mu = reinterpret_cast<const float4*>((set ? nets.theta_tgt : nets.theta) + base);
-    const float4* sg = reinterpret_cast<const float4*>((set ? nz.sigma_tgt : nz.sigma) + base);
-    float4* out = reinterpret_cast<float4*>((set ? nz.eff_tgt : nz.eff) + base);
-    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, RL.L.stride / 4);
-    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
-        const float4 m = __ldg(mu + i), s = __ldg(sg + i), e = noise_eps4_rainbow(rec, R, RL, H, np, i * 4);
-        out[i] = make_float4(noisy_weight(m.x, s.x, e.x), noisy_weight(m.y, s.y, e.y), noisy_weight(m.z, s.z, e.z),
-                             noisy_weight(m.w, s.w, e.w));
-    }
-}
-
-// Per-atom head fold: W3e | b3e of the effective online (blockIdx.z = 0) and target (1) block of network blockIdx.y into
-// head[z][y], one thread per (row k <= H, atom j < Np): head_fold of {W3[k][b * Np + j]}_b with Wv[k][j] (row H: b3 / bv).
-__global__ void __launch_bounds__(256) rainbow_head_fold_kernel(RainbowLayout RL, int H, int n_actions, int n_atoms, int np,
-                                                                const float* __restrict__ eff, const float* __restrict__ eff_tgt,
-                                                                float* __restrict__ head) {
-    const int g = blockIdx.y, nh = 4 * np;
-    const float* P = (blockIdx.z ? eff_tgt : eff) + (size_t)g * RL.L.stride;
+// Head fold of a block with a value stream (include/dmdqn_b200.h, dueling and Rainbow): W3e | b3e of network blockIdx.y's
+// online (blockIdx.z = 0) or target (1) block into head[z][y], one thread per (row k <= H, atom j < np): head_fold of
+// {W3[k][a * np + j]}_a with Wv[k][j] (row H: b3 / bv).  Dueling blocks are the n_atoms = np = 1 case (ONE_ATOM), whose
+// four values are one float4.
+template <bool ONE_ATOM>
+__global__ void __launch_bounds__(256) head_fold_kernel(Layout L, int H, int n_actions, int n_atoms, int np_,
+                                                        const float* __restrict__ theta, const float* __restrict__ theta_tgt,
+                                                        float* __restrict__ head) {
+    const int np = ONE_ATOM ? 1 : np_, g = blockIdx.y, nh = 4 * np;
+    const float* P = (blockIdx.z ? theta_tgt : theta) + (size_t)g * L.stride;
     float* out = head + ((size_t)blockIdx.z * gridDim.y + g) * (size_t)(H + 1) * nh;
     const int total = (H + 1) * np;
     for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < total; f += gridDim.x * blockDim.x) {
         const int k = f / np, j = f % np;
-        const float* row = P + (k < H ? RL.L.w3 + (int64_t)k * nh : RL.L.b3);
-        float x[4] = {__ldg(row + j), __ldg(row + np + j), __ldg(row + 2 * np + j), __ldg(row + 3 * np + j)};
-        head_fold(x, __ldg(P + (k < H ? RL.wv + (int64_t)k * np : RL.bv) + j), n_actions);
-        float* o = out + (size_t)k * nh + j;
+        const float* row = P + (k < H ? L.w3 + (int64_t)k * nh : L.b3);
+        if constexpr (ONE_ATOM) {
+            const float4 w = __ldg(reinterpret_cast<const float4*>(row));
+            float x[4] = {w.x, w.y, w.z, w.w};
+            head_fold(x, __ldg(P + (k < H ? L.wv + k : L.bv)), n_actions);
+            reinterpret_cast<float4*>(out)[k] = make_float4(x[0], x[1], x[2], x[3]);
+        } else {
+            float x[4] = {__ldg(row + j), __ldg(row + np + j), __ldg(row + 2 * np + j), __ldg(row + 3 * np + j)};
+            head_fold(x, __ldg(P + (k < H ? L.wv + (int64_t)k * np : L.bv) + j), n_actions);
+            float* o = out + (size_t)k * nh + j;
 #pragma unroll
-        for (int a = 0; a < 4; ++a) o[a * np] = j < n_atoms ? x[a] : 0.f;
+            for (int a = 0; a < 4; ++a) o[a * np] = j < n_atoms ? x[a] : 0.f;
+        }
     }
 }
 
 // Projection of the folded head's gradient, in place over the W3 / b3 rows of grads, and Wv / bv from its sums: head_project
 // per (row k <= H, atom j < Np) of every network that learned this step; atoms j >= N get gradient 0.
-__global__ void __launch_bounds__(256) rainbow_project_kernel(RainbowLayout RL, int H, int n_actions, int n_atoms, int np,
+__global__ void __launch_bounds__(256) rainbow_project_kernel(Layout L, int H, int n_actions, int n_atoms, int np,
                                                               const int32_t* __restrict__ active, float* __restrict__ grads) {
     const int g = blockIdx.y, nh = 4 * np;
     if (!active[g]) return;
-    float* G = grads + (size_t)g * RL.L.stride;
+    float* G = grads + (size_t)g * L.stride;
     const int total = (H + 1) * np;
     for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < total; f += gridDim.x * blockDim.x) {
         const int k = f / np, j = f % np;
-        float* row = G + (k < H ? RL.L.w3 + (int64_t)k * nh : RL.L.b3) + j;
+        float* row = G + (k < H ? L.w3 + (int64_t)k * nh : L.b3) + j;
         float x[4] = {row[0], row[np], row[2 * np], row[3 * np]};
         const float sv = head_project(x, n_actions);
         const bool ok = j < n_atoms;
 #pragma unroll
         for (int a = 0; a < 4; ++a) row[a * np] = ok ? x[a] : 0.f;
-        G[(k < H ? RL.wv + (int64_t)k * np : RL.bv) + j] = ok ? sv : 0.f;
-    }
-}
-
-// noisy_adam_apply_kernel over a Rainbow block: eps from the Rainbow record of set 0.
-__global__ void __launch_bounds__(kNoisyThreads)
-rainbow_adam_apply_kernel(const LearnArgs A, const dmdqn_noisy nz, RainbowLayout RL, NoiseRec R, int np,
-                          const float* __restrict__ grads, int64_t per) {
-    extern __shared__ __align__(16) float rec[];
-    const int g = blockIdx.y;
-    if (!A.active[g] || *reinterpret_cast<volatile int*>(A.error) != 0) return;
-    const float* src = nz.noise + (size_t)g * 2 * R.stride;
-    for (int e = threadIdx.x; e < R.stride; e += blockDim.x) rec[e] = src[e];
-    __syncthreads();
-    const AdamStep k = adam_step(A, g);
-    const int H = A.d.hidden;
-    const size_t base = (size_t)g * RL.L.stride;
-    const int64_t i0 = blockIdx.x * per, i1 = min(i0 + per, RL.L.end / 4);
-    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
-        const float4 g4 = *reinterpret_cast<const float4*>(grads + base + i * 4);
-        const float4 e = noise_eps4_rainbow(rec, R, RL, H, np, i * 4);
-        const float gm[4] = {g4.x, g4.y, g4.z, g4.w};
-        const float gs[4] = {__fmul_rn(g4.x, e.x), __fmul_rn(g4.y, e.y), __fmul_rn(g4.z, e.z), __fmul_rn(g4.w, e.w)};
-        const size_t o = base + i * 4;
-        adam_vec4(k, gm, A.nets.theta + o, A.nets.adam_m + o, A.nets.adam_v + o, A.nets.theta_tgt + o);
-        adam_vec4(k, gs, nz.sigma + o, nz.sigma_m + o, nz.sigma_v + o, nz.sigma_tgt + o);
+        G[(k < H ? L.wv + (int64_t)k * np : L.bv) + j] = ok ? sv : 0.f;
     }
 }
 
@@ -2153,13 +2101,26 @@ int launch_learn_h(const LearnArgs& A, int stages, cudaStream_t s) {
     return DMDQN_OK;
 }
 
+// f(std::integral_constant<int, H>) for the hidden width d.hidden: the one place a width picks a kernel instantiation
+template <class F>
+int with_hidden(int hidden, F&& f) {
+    switch (hidden) {
+        case 64: return f(std::integral_constant<int, 64>{});
+        case 128: return f(std::integral_constant<int, 128>{});
+        case 256: return f(std::integral_constant<int, 256>{});
+        case 512: return f(std::integral_constant<int, 512>{});
+    }
+    set_error("unsupported hidden width %d", hidden);
+    return DMDQN_ERR_ARG;
+}
+
 }  // namespace
 
-LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
-                          char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch) {
+LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, HeadShape hs, const dmdqn_replay& rp,
+                          const dmdqn_nets& nets, char* ws, const Workspace& w, float* metrics, float* grads, int loss_batch) {
     LearnArgs A = {};
     A.d = d;
-    A.L = make_layout(d.obs_stride, d.hidden, hp.dueling == 1);
+    A.L = make_layout(d.obs_stride, d.hidden, hs);
     A.rp = rp;
     A.nets = nets;
     A.loss = hp.loss;
@@ -2214,7 +2175,7 @@ LearnArgs make_learn_args(const dmdqn_dims& d, const dmdqn_hparams& hp, const dm
 
 int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                  float* metrics, char* ws, const Workspace& w, int stages, float* grads, int loss_batch, cudaStream_t s) {
-    const LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    const LearnArgs A = make_learn_args(d, hp, {1, 1, hp.dueling == 1, 0}, rp, nets, ws, w, metrics, grads, loss_batch);
     if (hp.precision != DMDQN_PRECISION_FP32) {
         if (!tc_supported(d)) {
             set_error("precision=%d (tcgen05) needs hidden=256 and obs_stride in {32,64,96}; got hidden=%d obs_stride=%d",
@@ -2223,31 +2184,22 @@ int launch_learn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_repla
         }
         return launch_learn_tc(A, hp.precision, stages, s);
     }
-    switch (d.hidden) {
-        case 64: return A.dueling ? launch_learn_h<64, true>(A, stages, s) : launch_learn_h<64, false>(A, stages, s);
-        case 128: return A.dueling ? launch_learn_h<128, true>(A, stages, s) : launch_learn_h<128, false>(A, stages, s);
-        case 256: return A.dueling ? launch_learn_h<256, true>(A, stages, s) : launch_learn_h<256, false>(A, stages, s);
-        case 512: return A.dueling ? launch_learn_h<512, true>(A, stages, s) : launch_learn_h<512, false>(A, stages, s);
+    return with_hidden(d.hidden, [&](auto h) {
+        return A.dueling ? launch_learn_h<h.value, true>(A, stages, s) : launch_learn_h<h.value, false>(A, stages, s);
+    });
+}
+
+// adam_apply_kernel (clipnorm == 0) or clip_adam_apply_kernel over [0, A.L.end) of every block
+int launch_adam(const LearnArgs& A, const float* grads, double clipnorm, float* norms_out, cudaStream_t s) {
+    if (clipnorm == 0.0) {
+        adam_apply_kernel<<<dim3(64, A.d.n_nets), 256, 0, s>>>(A, grads);
+        DMDQN_CUDA(cudaGetLastError());
+        return DMDQN_OK;
     }
-    set_error("unsupported hidden width %d", d.hidden);
-    return DMDQN_ERR_ARG;
-}
-
-int launch_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads, char* ws,
-                      const Workspace& w, cudaStream_t s) {
-    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
-    adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
-}
-
-int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const float* grads,
-                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
-    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
     const int64_t per = clip_per_cta(A.L);
     const size_t smem = (size_t)per * 16;
     if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
-    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
+    clip_adam_apply_kernel<<<dim3(kClipCtas, A.d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
@@ -2255,167 +2207,80 @@ int launch_clip_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const d
 int launch_learn_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                       const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
                       cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    const LearnArgs A = make_learn_args(d, hp, atom_shape(ds.n_atoms, false), rp, nets, ws, w, metrics, grads, loss_batch);
     const DistArgs D = make_dist_args(d, ds);
-    A.L = make_layout_dist(d.obs_stride, d.hidden, D.np);
-    switch (d.hidden) {
-        case 64: return launch_learn_dist_h<64>(A, D, D, s);
-        case 128: return launch_learn_dist_h<128>(A, D, D, s);
-        case 256: return launch_learn_dist_h<256>(A, D, D, s);
-        case 512: return launch_learn_dist_h<512>(A, D, D, s);
-    }
-    set_error("unsupported hidden width %d", d.hidden);
-    return DMDQN_ERR_ARG;
+    return with_hidden(d.hidden, [&](auto h) { return launch_learn_dist_h<h.value>(A, D, D, s); });
 }
 
 int launch_learn_quantile(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                           const dmdqn_quantile& qs, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
                           cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
+    const LearnArgs A = make_learn_args(d, hp, atom_shape(qs.n_quantiles, false), rp, nets, ws, w, metrics, grads, loss_batch);
     const QuantArgs Q = make_quantile_args(d, qs);
-    A.L = make_layout_dist(d.obs_stride, d.hidden, Q.np);
     DistArgs D = {};                                 // what dist_wgrad_kernel reads: the head width and the scratch
     D.n_atoms = Q.n_atoms; D.np = Q.np; D.nh = Q.nh;
     D.m = Q.m; D.h2 = Q.h2; D.dx = Q.dx;
-    switch (d.hidden) {
-        case 64: return launch_learn_dist_h<64>(A, Q, D, s);
-        case 128: return launch_learn_dist_h<128>(A, Q, D, s);
-        case 256: return launch_learn_dist_h<256>(A, Q, D, s);
-        case 512: return launch_learn_dist_h<512>(A, Q, D, s);
-    }
-    set_error("unsupported hidden width %d", d.hidden);
-    return DMDQN_ERR_ARG;
-}
-
-// adam_apply_kernel (clipnorm == 0) or clip_adam_apply_kernel on the distributional layout: the same arithmetic over [0, end)
-int launch_adam_apply_dist(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_atoms, const float* grads,
-                           double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
-    A.L = make_layout_dist(d.obs_stride, d.hidden, dist_np(n_atoms));
-    if (clipnorm == 0.0) {
-        adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
-        DMDQN_CUDA(cudaGetLastError());
-        return DMDQN_OK;
-    }
-    const int64_t per = clip_per_cta(A.L);
-    const size_t smem = (size_t)per * 16;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
-    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
-}
-
-int launch_sync_target_dist(const dmdqn_dims& d, const dmdqn_nets& nets, int n_atoms, const uint8_t* mask, double tau,
-                            cudaStream_t s) {
-    const Layout L = make_layout_dist(d.obs_stride, d.hidden, dist_np(n_atoms));
-    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
+    return with_hidden(d.hidden, [&](auto h) { return launch_learn_dist_h<h.value>(A, Q, D, s); });
 }
 
 int launch_learn_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& nets,
                      const dmdqn_iqn& q, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch, cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, rp, nets, ws, w, metrics, grads, loss_batch);
-    A.L = make_layout_iqn(d.obs_stride, d.hidden, q.n_cos).L;
+    const LearnArgs A = make_learn_args(d, hp, {1, 1, false, q.n_cos}, rp, nets, ws, w, metrics, grads, loss_batch);
     const IqnArgs Q = make_iqn_args(d, q);
-    switch (d.hidden) {
-        case 64: return launch_learn_iqn_h<64>(A, Q, s);
-        case 128: return launch_learn_iqn_h<128>(A, Q, s);
-        case 256: return launch_learn_iqn_h<256>(A, Q, s);
-        case 512: return launch_learn_iqn_h<512>(A, Q, s);
-    }
-    set_error("unsupported hidden width %d", d.hidden);
-    return DMDQN_ERR_ARG;
-}
-
-// adam_apply_kernel (clipnorm == 0) or clip_adam_apply_kernel on the IQN layout: the same arithmetic over [0, end)
-int launch_adam_apply_iqn(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, int n_cos, const float* grads,
-                          double clipnorm, float* norms_out, char* ws, const Workspace& w, cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
-    A.L = make_layout_iqn(d.obs_stride, d.hidden, n_cos).L;
-    if (clipnorm == 0.0) {
-        adam_apply_kernel<<<dim3(64, d.n_nets), 256, 0, s>>>(A, grads);
-        DMDQN_CUDA(cudaGetLastError());
-        return DMDQN_OK;
-    }
-    const int64_t per = clip_per_cta(A.L);
-    const size_t smem = (size_t)per * 16;
-    if (int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(clip_adam_apply_kernel), smem, g_clip_smem_cfg)) return rc;
-    clip_adam_apply_kernel<<<dim3(kClipCtas, d.n_nets), kClipThreads, smem, s>>>(A, grads, per, clipnorm, norms_out);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
-}
-
-int launch_sync_target_iqn(const dmdqn_dims& d, const dmdqn_nets& nets, int n_cos, const uint8_t* mask, double tau, cudaStream_t s) {
-    const Layout L = make_layout_iqn(d.obs_stride, d.hidden, n_cos).L;
-    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
+    return with_hidden(d.hidden, [&](auto h) { return launch_learn_iqn_h<h.value>(A, Q, s); });
 }
 
 int launch_peer_adam(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_peers& peers,
                      const float* my_loss_src, float* loss_out, char* ws, const Workspace& w, cudaStream_t s) {
-    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
+    const LearnArgs A = make_learn_args(d, hp, {1, 1, hp.dueling == 1, 0}, {}, nets, ws, w, nullptr, nullptr, 0);
     peer_reduce_adam_kernel<<<DMDQN_PEER_BLOCKS, 256, 0, s>>>(A, peers, my_loss_src, loss_out);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
 
-int launch_fold(const dmdqn_dims& d, const dmdqn_nets& nets, char* ws, const Workspace& w, cudaStream_t s) {
-    const Layout L = make_layout(d.obs_stride, d.hidden, true);
-    fold_kernel<<<dim3(d.n_nets, 2), 256, 0, s>>>(L, d.hidden, d.n_actions, nets.theta, nets.theta_tgt,
-                                                  reinterpret_cast<float*>(ws + w.head));
+int launch_head_fold(const dmdqn_dims& d, HeadShape hs, const float* theta, const float* theta_tgt, float* head, cudaStream_t s) {
+    const Layout L = make_layout(d.obs_stride, d.hidden, hs);
+    const int blocks = hs.np == 1 ? 1 : ((d.hidden + 1) * hs.np + 255) / 256;    // a dueling head: one CTA per block and set
+    auto kernel = hs.np == 1 ? head_fold_kernel<true> : head_fold_kernel<false>;
+    kernel<<<dim3(blocks, d.n_nets, 2), 256, 0, s>>>(L, d.hidden, d.n_actions, hs.n, hs.np, theta, theta_tgt, head);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
 
-int launch_noisy_fold(const dmdqn_dims& d, bool dueling, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s) {
-    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
-    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden);
+int launch_noisy_fold(const dmdqn_dims& d, HeadShape hs, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s) {
+    const Layout L = make_layout(d.obs_stride, d.hidden, hs);
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, hs);
     int n_sm = 0;
     if (int rc = device_sm_count(&n_sm)) return rc;
     const int64_t n4 = L.stride / 4;
     const int chunks = noisy_chunks(n_sm, 2 * (int64_t)d.n_nets, n4);
     const int64_t per = (n4 + chunks - 1) / chunks;
     noisy_fold_kernel<<<dim3(chunks, d.n_nets, 2), kNoisyThreads, R.stride * sizeof(float), s>>>(
-        L, R, d.hidden, d.obs_dim, d.n_actions, dueling ? 1 : 0, nets, nz, per);
+        L, R, d.hidden, d.obs_dim, d.n_actions, hs.n, hs.np, nets, nz, per);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
 
-int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
-                            const float* grads, char* ws, const Workspace& w, cudaStream_t s) {
-    const LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
-    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden);
+int launch_noisy_adam_apply(const dmdqn_dims& d, const dmdqn_hparams& hp, HeadShape hs, const dmdqn_nets& nets,
+                            const dmdqn_noisy& nz, const float* grads, char* ws, const Workspace& w, cudaStream_t s) {
+    const LearnArgs A = make_learn_args(d, hp, hs, {}, nets, ws, w, nullptr, nullptr, 0);
+    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, hs);
     int n_sm = 0;
     if (int rc = device_sm_count(&n_sm)) return rc;
     const int64_t n4 = A.L.end / 4;
     const int chunks = noisy_chunks(n_sm, d.n_nets, n4);
     const int64_t per = (n4 + chunks - 1) / chunks;
-    noisy_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, R, grads, per);
+    noisy_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, R, hs.np, grads, per);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
 
 // Rainbow: the noise fold into eff / eff_tgt, then the per-atom head fold of both into the scratch's head region.
 int launch_rainbow_fold(const dmdqn_dims& d, const dmdqn_dist& ds, const dmdqn_nets& nets, const dmdqn_noisy& nz, cudaStream_t s) {
-    const int np = dist_np(ds.n_atoms);
-    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
-    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
-    int n_sm = 0;
-    if (int rc = device_sm_count(&n_sm)) return rc;
-    const int64_t n4 = RL.L.stride / 4;
-    const int chunks = noisy_chunks(n_sm, 2 * (int64_t)d.n_nets, n4);
-    const int64_t per = (n4 + chunks - 1) / chunks;
-    rainbow_noisy_fold_kernel<<<dim3(chunks, d.n_nets, 2), kNoisyThreads, R.stride * sizeof(float), s>>>(
-        RL, R, d.hidden, d.obs_dim, d.n_actions, ds.n_atoms, np, nets, nz, per);
-    DMDQN_CUDA(cudaGetLastError());
-    float* head = reinterpret_cast<float*>(static_cast<char*>(ds.scratch) + make_rainbow_scratch(d, np).head);
-    const int blocks = ((d.hidden + 1) * np + 255) / 256;
-    rainbow_head_fold_kernel<<<dim3(blocks, d.n_nets, 2), 256, 0, s>>>(RL, d.hidden, d.n_actions, ds.n_atoms, np, nz.eff,
-                                                                        nz.eff_tgt, head);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
+    const HeadShape hs = atom_shape(ds.n_atoms, true);
+    if (int rc = launch_noisy_fold(d, hs, nets, nz, s)) return rc;
+    float* head = reinterpret_cast<float*>(static_cast<char*>(ds.scratch) + make_rainbow_scratch(d, hs.np).head);
+    return launch_head_fold(d, hs, nz.eff, nz.eff_tgt, head, s);
 }
 
 // Rainbow learn step after the sample kernel: the C51 target / online kernels on the folded heads with the effective trunks,
@@ -2423,60 +2288,22 @@ int launch_rainbow_fold(const dmdqn_dims& d, const dmdqn_dist& ds, const dmdqn_n
 int launch_learn_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_replay& rp, const dmdqn_nets& eff,
                          const dmdqn_dist& ds, float* metrics, char* ws, const Workspace& w, float* grads, int loss_batch,
                          cudaStream_t s) {
-    LearnArgs A = make_learn_args(d, hp, rp, eff, ws, w, metrics, grads, loss_batch);
+    LearnArgs A = make_learn_args(d, hp, atom_shape(ds.n_atoms, true), rp, eff, ws, w, metrics, grads, loss_batch);
     const DistArgs D = make_dist_args(d, ds);
-    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, D.np);
-    A.L = RL.L;
     A.head_stride = (int64_t)(d.hidden + 1) * D.nh;
     A.head[0] = reinterpret_cast<const float*>(static_cast<char*>(ds.scratch) + make_rainbow_scratch(d, D.np).head);
     A.head[1] = A.head[0] + (size_t)d.n_nets * A.head_stride;
-    int rc = DMDQN_ERR_ARG;
-    switch (d.hidden) {
-        case 64: rc = launch_learn_dist_h<64, DistArgs, true>(A, D, D, s); break;
-        case 128: rc = launch_learn_dist_h<128, DistArgs, true>(A, D, D, s); break;
-        case 256: rc = launch_learn_dist_h<256, DistArgs, true>(A, D, D, s); break;
-        case 512: rc = launch_learn_dist_h<512, DistArgs, true>(A, D, D, s); break;
-        default: set_error("unsupported hidden width %d", d.hidden);
-    }
-    if (rc) return rc;
+    if (int rc = with_hidden(d.hidden, [&](auto h) { return launch_learn_dist_h<h.value, DistArgs, true>(A, D, D, s); }))
+        return rc;
     const int blocks = ((d.hidden + 1) * D.np + 255) / 256;
-    rainbow_project_kernel<<<dim3(blocks, d.n_nets), 256, 0, s>>>(RL, d.hidden, d.n_actions, D.n_atoms, D.np, A.active, grads);
+    rainbow_project_kernel<<<dim3(blocks, d.n_nets), 256, 0, s>>>(A.L, d.hidden, d.n_actions, D.n_atoms, D.np, A.active, grads);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }
 
-int launch_adam_apply_rainbow(const dmdqn_dims& d, const dmdqn_hparams& hp, const dmdqn_nets& nets, const dmdqn_noisy& nz,
-                              int n_atoms, const float* grads, char* ws, const Workspace& w, cudaStream_t s) {
-    const int np = dist_np(n_atoms);
-    const RainbowLayout RL = make_layout_rainbow(d.obs_stride, d.hidden, np);
-    LearnArgs A = make_learn_args(d, hp, {}, nets, ws, w, nullptr, nullptr, 0);
-    A.L = RL.L;
-    const NoiseRec R = make_noise_rec(d.obs_stride, d.hidden, 4 * np, np);
-    int n_sm = 0;
-    if (int rc = device_sm_count(&n_sm)) return rc;
-    const int64_t n4 = RL.L.end / 4;
-    const int chunks = noisy_chunks(n_sm, d.n_nets, n4);
-    const int64_t per = (n4 + chunks - 1) / chunks;
-    rainbow_adam_apply_kernel<<<dim3(chunks, d.n_nets), kNoisyThreads, R.stride * sizeof(float), s>>>(A, nz, RL, R, np, grads, per);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
-}
-
-int launch_sync_target_rainbow(const dmdqn_dims& d, const dmdqn_nets& nets, const dmdqn_noisy& nz, int n_atoms,
-                               const uint8_t* mask, double tau, cudaStream_t s) {
-    const int64_t stride = make_layout_rainbow(d.obs_stride, d.hidden, dist_np(n_atoms)).L.stride;
-    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(stride, nets.theta, nets.theta_tgt, mask, (float)tau);
-    DMDQN_CUDA(cudaGetLastError());
-    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(stride, nz.sigma, nz.sigma_tgt, mask, (float)tau);
-    DMDQN_CUDA(cudaGetLastError());
-    return DMDQN_OK;
-}
-
-int launch_sync_target(const dmdqn_dims& d, const dmdqn_nets& nets, const uint8_t* mask, double tau, bool dueling,
+int launch_sync_target(const dmdqn_dims& d, int64_t stride, float* theta, float* theta_tgt, const uint8_t* mask, double tau,
                        cudaStream_t s) {
-    const Layout L = make_layout(d.obs_stride, d.hidden, dueling);
-    dim3 grid(32, d.n_nets);
-    sync_target_kernel<<<grid, 256, 0, s>>>(L.stride, nets.theta, nets.theta_tgt, mask, (float)tau);
+    sync_target_kernel<<<dim3(32, d.n_nets), 256, 0, s>>>(stride, theta, theta_tgt, mask, (float)tau);
     DMDQN_CUDA(cudaGetLastError());
     return DMDQN_OK;
 }

@@ -1510,15 +1510,15 @@ __global__ void __launch_bounds__(Wg::NTW, 1) tc_wgrad_kernel(const LearnArgs A,
                 }
                 upd(A.L.b2 + et, s2);
                 if (A.dueling) {          // the folded head's gradient projected onto W3[et][.] | wv[et], and b3 | bv by one thread
-                    upd(layout_wv(A.L) + et, head_project(w, A.d.n_actions));
+                    upd(A.L.wv + et, head_project(w, A.d.n_actions));
                     if (et == 0) {
                         float b[4] = {0.f, 0.f, 0.f, 0.f};
                         for (int r = 0; r < A.tc_tiles; ++r)
                             for (int a = 0; a < 4; ++a) b[a] += ldcg_f(A.part_b3 + (p0 + r) * 4 + a);
-                        upd(layout_bv(A.L, H), head_project(b, A.d.n_actions));
+                        upd(A.L.bv, head_project(b, A.d.n_actions));
                         for (int a = 0; a < 4; ++a) upd(A.L.b3 + a, b[a]);
                         if (A.grads)              // the pad after bv is inside the Adam range: its gradient is 0
-                            for (int p = 1; p < 4; ++p) A.grads[pb + layout_bv(A.L, H) + p] = 0.f;
+                            for (int p = 1; p < 4; ++p) A.grads[pb + A.L.bv + p] = 0.f;
                     }
                 }
                 for (int a = 0; a < 4; ++a) upd(A.L.w3 + (int64_t)et * 4 + a, w[a]);

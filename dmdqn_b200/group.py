@@ -191,6 +191,12 @@ def iqn_config(cfg: dict) -> dict:
     return cfg
 
 
+def _head_shape(grp) -> tuple:
+    """``AgentGroup.head_shape``; an object that stands in for a group without it (a namespace with the layout and the
+    flags) has a scalar head, dueling or not."""
+    return getattr(grp, "head_shape", None) or (1, 1, grp.dueling, 0)
+
+
 def _ptr(t: torch.Tensor | None) -> int | None:
     return None if t is None else t.data_ptr()
 
@@ -333,6 +339,10 @@ class AgentGroup:
         else:
             self.layout = N.Layout()
             N.check(self.lib.dmdqn_param_layout(C.byref(self.dims), C.byref(self.layout)))
+        # the block's head shape (n atoms per action, their column stride, a value stream, the cosine embedding width): what
+        # pack, unpack and the initial weights lay out (common.cuh HeadShape)
+        n = self.head_atoms or 1
+        self.head_shape = (n, (n + 3) // 4 * 4 if n > 1 else 1, self.dueling or self.rainbow, self.n_cos)
         self.noise_record = N.NoiseRecord()
         if self.rainbow:
             N.check(self.lib.dmdqn_noise_layout_rainbow(C.byref(self.dims), self.num_atoms, C.byref(self.noise_record)))
@@ -444,6 +454,7 @@ class AgentGroup:
         self._gen = torch.Generator(device=dev)
         self._gen.manual_seed(int(seed) + 0x5EED)
         self._views: dict[int, AgentGroup] = {}
+        self._resolve_calls()
         if _parent is None:
             self.init_weights(seed)
 
@@ -481,11 +492,13 @@ class AgentGroup:
 
     # ------------------------------------------------------------------ weights ---------
     def pack(self, weights) -> torch.Tensor:
-        """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]; dueling: + [Wv [H,1], bv [1]]) -> one parameter block."""
+        """[W1,b1,W2,b2,W3,b3] (Keras order, kernels [in,out]) and, with a value stream, [Wv [H,N], bv [N]] (dueling: N = 1)
+        or, with a cosine embedding, [Wphi [n_cos,H], bphi [H]] -> one parameter block.  W3 [H, A*N] / b3 [A*N]: column
+        a*N + j goes to a*Np + j."""
         L, H, A = self.layout, self.hidden, self.action_size
+        n, npad, value, n_cos = _head_shape(self)
         ws = [torch.as_tensor(np.asarray(w), dtype=torch.float32) for w in weights]
-        rainbow = getattr(self, "rainbow", False)
-        want = 8 if self.dueling or rainbow or getattr(self, "iqn", False) else 6
+        want = 8 if value or n_cos else 6
         if len(ws) != want:
             raise ValueError(f"expected {want} weight tensors, got {len(ws)}")
         w1, b1, w2, b2, w3, b3 = ws[:6]
@@ -494,64 +507,49 @@ class AgentGroup:
         blk[L.b1:L.b1 + H] = b1
         blk[L.w2:L.w2 + H * H] = w2.reshape(-1)
         blk[L.b2:L.b2 + H] = b2
-        if getattr(self, "dist_layout", False) or rainbow:  # W3 [H, A*N] / b3 [A*N], column a*N + j -> a*Np + j
-            n, npad = self.head_atoms, self.atom_stride
-            blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n] = w3.reshape(H, A, n)
-            blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n] = b3.reshape(A, n)
-            if rainbow:                                     # Wv [H, N] / bv [N], atom j -> column j of Np
-                blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n] = ws[6].reshape(H, n)
-                blk[L.bv:L.bv + n] = ws[7].reshape(n)
-            return blk
-        blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A] = w3
-        blk[L.b3:L.b3 + A] = b3
-        if self.dueling:
-            blk[L.wv:L.wv + H] = ws[6].reshape(H)
-            blk[L.bv:L.bv + 1] = ws[7].reshape(1)
-        if getattr(self, "iqn", False):
-            blk[L.wphi:L.wphi + self.n_cos * H] = ws[6].reshape(-1)
+        blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n] = w3.reshape(H, A, n)
+        blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n] = b3.reshape(A, n)
+        if value:
+            blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n] = ws[6].reshape(H, n)
+            blk[L.bv:L.bv + n] = ws[7].reshape(n)
+        if n_cos:
+            blk[L.wphi:L.wphi + n_cos * H] = ws[6].reshape(-1)
             blk[L.bphi:L.bphi + H] = ws[7].reshape(H)
         return blk
 
     def unpack(self, blk: torch.Tensor) -> list[torch.Tensor]:
         L, H, A = self.layout, self.hidden, self.action_size
+        n, npad, value, n_cos = _head_shape(self)
         blk = blk.detach().cpu()
         out = [blk[L.w1:L.w1 + self.obs_stride * H].view(self.obs_stride, H)[: self.state_size].clone(),
-               blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(), blk[L.b2:L.b2 + H].clone()]
-        if getattr(self, "dist_layout", False) or getattr(self, "rainbow", False):
-            n, npad = self.head_atoms, self.atom_stride
-            out += [blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
-                    blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
-            if getattr(self, "rainbow", False):
-                out += [blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n].clone(), blk[L.bv:L.bv + n].clone()]
-            return out
-        out += [blk[L.w3:L.w3 + H * 4].view(H, 4)[:, :A].clone(), blk[L.b3:L.b3 + A].clone()]
-        if self.dueling:
-            out += [blk[L.wv:L.wv + H].view(H, 1).clone(), blk[L.bv:L.bv + 1].clone()]
-        if getattr(self, "iqn", False):
-            out += [blk[L.wphi:L.wphi + self.n_cos * H].view(self.n_cos, H).clone(), blk[L.bphi:L.bphi + H].clone()]
+               blk[L.b1:L.b1 + H].clone(), blk[L.w2:L.w2 + H * H].view(H, H).clone(), blk[L.b2:L.b2 + H].clone(),
+               blk[L.w3:L.w3 + H * 4 * npad].view(H, 4, npad)[:, :A, :n].reshape(H, A * n).clone(),
+               blk[L.b3:L.b3 + 4 * npad].view(4, npad)[:A, :n].reshape(A * n).clone()]
+        if value:
+            out += [blk[L.wv:L.wv + H * npad].view(H, npad)[:, :n].clone(), blk[L.bv:L.bv + n].clone()]
+        if n_cos:
+            out += [blk[L.wphi:L.wphi + n_cos * H].view(n_cos, H).clone(), blk[L.bphi:L.bphi + H].clone()]
         return out
 
     def sigma_init(self) -> list[torch.Tensor]:
         """Initial sigma of a noisy network in ``keras_init``'s order: noisy_sigma0 / sqrt(fan_in) for every weight and bias
         of a layer (Fortunato et al.'s factorized rule), fan_in = state_size for layer 1 and H after it."""
-        d, h, a = self.state_size, self.hidden, self.action_size
+        d, h = self.state_size, self.hidden
+        n, _, value, _ = _head_shape(self)
+        a = self.action_size * n
         s1, s2 = np.float32(self.noisy_sigma0 / math.sqrt(d)), np.float32(self.noisy_sigma0 / math.sqrt(h))
-        if getattr(self, "rainbow", False):     # the C51 head [H, A*N] and the value stream [H, N]
-            a, n = a * self.num_atoms, self.num_atoms
-            shapes = [((d, h), s1), ((h,), s1), ((h, h), s2), ((h,), s2), ((h, a), s2), ((a,), s2), ((h, n), s2), ((n,), s2)]
-            return [torch.full(shape, float(v), dtype=torch.float32) for shape, v in shapes]
         shapes = [((d, h), s1), ((h,), s1), ((h, h), s2), ((h,), s2), ((h, a), s2), ((a,), s2)]
-        if self.dueling:
-            shapes += [((h, 1), s2), ((1,), s2)]
+        if value:
+            shapes += [((h, n), s2), ((n,), s2)]
         return [torch.full(shape, float(v), dtype=torch.float32) for shape, v in shapes]
 
     def init_weights(self, seed: int = 0) -> None:
         """Per-network Keras-style init (seed + g), target = online, Adam state zero
-        (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``."""
-        head = self.action_size * self.head_atoms if self.dist_layout or self.rainbow else self.action_size   # dist: W3 over [H, A*N]
-        # Rainbow: W1..b3 drawn as a C51 group's, then Wv GlorotUniform over [H, N]
-        value = dict(dueling=True, value_size=self.num_atoms) if self.rainbow else dict(dueling=self.dueling)
-        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, head, n_cos=self.n_cos, **value))
+        (dqn_agent.py:129-137).  Noisy networks: sigma from ``sigma_init``, the Philox key ``noise_key(seed + g)``.
+        The head is drawn over [H, A*N] and the value stream over [H, N] (Rainbow: W1..b3 drawn as a C51 group's)."""
+        n, _, value, n_cos = self.head_shape
+        blocks = torch.stack([self.pack(keras_init(seed + g, self.state_size, self.hidden, self.action_size * n, dueling=value,
+                                                   n_cos=n_cos, value_size=n))
                               for g in range(self.n_nets)])
         self.theta.copy_(blocks)
         self.theta_tgt.copy_(blocks)
@@ -657,22 +655,9 @@ class AgentGroup:
         q = torch.full((n, 4), float("nan"), dtype=torch.float32, device=self.device) if return_q else None
         nets = self.nets if not target else N.Nets(_ptr(self.theta_tgt), _ptr(self.theta_tgt), _ptr(self.adam_m),
                                                    _ptr(self.adam_v), _ptr(self.learn_step))
-        args = (_ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2), _ptr(actions), _ptr(q), self._stream)
-        if self.rainbow:            # set 0's noise at the current learn_step, or mu alone (noisy=False, the target network)
-            nz = C.byref(self.noisy_ptrs) if noisy is not False and not target else None
-            N.check(self.lib.dmdqn_act_rainbow(C.byref(self.dims), C.byref(nets), nz, C.byref(self.dist), *args))
-        elif self.distributional:
-            N.check(self.lib.dmdqn_act_dist(C.byref(self.dims), C.byref(nets), C.byref(self.dist), *args))
-        elif self.quantile:
-            N.check(self.lib.dmdqn_act_quantile(C.byref(self.dims), C.byref(nets), C.byref(self.qr), *args))
-        elif self.iqn:
-            N.check(self.lib.dmdqn_act_iqn(C.byref(self.dims), C.byref(nets), C.byref(self.iqn_args), *args))
-        elif self.noisy and noisy is not False and not target:
-            N.check(self.lib.dmdqn_act_noisy(C.byref(self.dims), C.byref(nets), C.byref(self.noisy_ptrs), int(self.dueling),
-                                             *args))
-        else:
-            act = self.lib.dmdqn_act_dueling if self.dueling else self.lib.dmdqn_act
-            N.check(act(C.byref(self.dims), C.byref(nets), *args))
+        fn, mid = self._act_noisy if noisy is not False and not target else self._act
+        N.check(fn(C.byref(self.dims), C.byref(nets), *mid, _ptr(obs), obs.shape[1], _ptr(eps_t), _ptr(w1), _ptr(w2),
+                   _ptr(actions), _ptr(q), self._stream))
         return (actions, q) if return_q else actions
 
     def draw_words(self, shape) -> torch.Tensor:
@@ -755,77 +740,77 @@ class AgentGroup:
         return states, actions, rewards, next_states, dones, active
 
     # ------------------------------------------------------------------ K1b+K3+K4 -------
-    def _dist_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
-        """The gradient half of a distributional-layout learn step: ``dmdqn_learn_grads_dist`` (C51) or
-        ``dmdqn_learn_grads_quantile`` (QR-DQN) into ``grads_ptr``, the loss mean over ``global_batch``."""
-        ws, nws = _ptr(self.workspace), self.workspace.numel()
-        if self.quantile:
-            N.check(self.lib.dmdqn_learn_grads_quantile(C.byref(self.dims), C.byref(hp), C.byref(self.qr), C.byref(self.replay),
-                                                        C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
-                                                        _ptr(self.metrics), ws, nws, stream_ptr))
-        else:
-            N.check(self.lib.dmdqn_learn_grads_dist(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
-                                                    C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
-                                                    _ptr(self.metrics), ws, nws, stream_ptr))
+    def _resolve_calls(self) -> None:
+        """The native calls of this group's kind, resolved once: ``_grads`` = (learn_grads call, the arguments between hp and
+        the replay, those between the networks and the draws), ``_adam`` = (Adam call, the arguments between the networks
+        and the gradient, whether it takes global_clipnorm and the norms after it; None for a plain block, whose call
+        global_clipnorm selects when it runs), ``_sync`` = (sync call, the arguments between the networks and the mask),
+        ``_act`` / ``_act_noisy`` = (act call, the arguments between the networks and the observations) on mu alone / with
+        the online noise (noisy and Rainbow networks; the same call for every other kind)."""
+        lib, by = self.lib, C.byref
+        if self.rainbow:            # acting: set 0's noise at the current learn_step, or mu alone
+            nz = by(self.noisy_ptrs)
+            self._act = (lib.dmdqn_act_rainbow, [None, by(self.dist)])
+            self._act_noisy = (lib.dmdqn_act_rainbow, [nz, by(self.dist)])
+            self._grads = (lib.dmdqn_learn_grads_rainbow, [by(self.dist)], [nz])
+            self._adam = (lib.dmdqn_adam_apply_rainbow, [nz, self.num_atoms], False)
+            self._sync = (lib.dmdqn_sync_target_rainbow, [nz, self.num_atoms])
+        elif self.iqn:
+            self._act = self._act_noisy = (lib.dmdqn_act_iqn, [by(self.iqn_args)])
+            self._grads = (lib.dmdqn_learn_grads_iqn, [by(self.iqn_args)], [])
+            self._adam = (lib.dmdqn_adam_apply_iqn, [self.n_cos], True)
+            self._sync = (lib.dmdqn_sync_target_iqn, [self.n_cos])
+        elif self.dist_layout:      # C51 or QR-DQN
+            head = by(self.qr) if self.quantile else by(self.dist)
+            self._act = self._act_noisy = (lib.dmdqn_act_quantile if self.quantile else lib.dmdqn_act_dist, [head])
+            self._grads = (lib.dmdqn_learn_grads_quantile if self.quantile else lib.dmdqn_learn_grads_dist, [head], [])
+            self._adam = (lib.dmdqn_adam_apply_dist, [self.head_atoms], True)
+            self._sync = (lib.dmdqn_sync_target_dist, [self.head_atoms])
+        else:                       # plain or dueling, noisy or not
+            self._act = self._act_noisy = (lib.dmdqn_act_dueling if self.dueling else lib.dmdqn_act, [])
+            self._grads = (lib.dmdqn_learn_grads, [], [])
+            self._adam = (None, [], None)
+            self._sync = (lib.dmdqn_sync_target_dueling if self.dueling else lib.dmdqn_sync_target, [])
+            if self.noisy:          # mu + sigma * eps, and mu and sigma
+                nz = by(self.noisy_ptrs)
+                self._act_noisy = (lib.dmdqn_act_noisy, [nz, int(self.dueling)])
+                self._grads = (lib.dmdqn_learn_grads_noisy, [], [nz])
+                self._adam = (lib.dmdqn_noisy_adam_apply, [nz], False)
+                self._sync = (lib.dmdqn_sync_target_noisy, [nz, int(self.dueling)])
 
-    def _iqn_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
-        """``dmdqn_learn_grads_iqn`` into ``grads_ptr``, the loss mean over ``global_batch``, the fractions keyed from row
-        ``iqn_row_base``."""
-        self.iqn_args.row_base = int(self.iqn_row_base)
-        N.check(self.lib.dmdqn_learn_grads_iqn(C.byref(self.dims), C.byref(hp), C.byref(self.iqn_args), C.byref(self.replay),
-                                               C.byref(self.nets), draws_ptr, mask_ptr, int(global_batch), grads_ptr,
-                                               _ptr(self.metrics), _ptr(self.workspace), self.workspace.numel(), stream_ptr))
+    def _fused_learn(self) -> bool:
+        """Whether the learn step is the one ``dmdqn_learn`` / ``dmdqn_step_host`` call (a plain block, unclipped)."""
+        return self._adam[0] is None and self.global_clipnorm is None
 
-    def _rainbow_grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
-        """``dmdqn_learn_grads_rainbow`` into ``grads_ptr`` (dL/d eff), the loss mean over ``global_batch``."""
-        N.check(self.lib.dmdqn_learn_grads_rainbow(C.byref(self.dims), C.byref(hp), C.byref(self.dist), C.byref(self.replay),
-                                                   C.byref(self.nets), C.byref(self.noisy_ptrs), draws_ptr, mask_ptr,
-                                                   int(global_batch), grads_ptr, _ptr(self.metrics), _ptr(self.workspace),
-                                                   self.workspace.numel(), stream_ptr))
+    def _grads_call(self, hp, draws_ptr, mask_ptr, global_batch, grads_ptr, stream_ptr) -> None:
+        """The gradient half of a learn step (``dmdqn_learn_grads`` or the kind's ``dmdqn_learn_grads_*``) into
+        ``grads_ptr``, the loss mean over ``global_batch``; IQN fractions are keyed from row ``iqn_row_base``."""
+        if self.iqn:
+            self.iqn_args.row_base = int(self.iqn_row_base)
+        fn, head, noisy = self._grads
+        N.check(fn(C.byref(self.dims), C.byref(hp), *head, C.byref(self.replay), C.byref(self.nets), *noisy, draws_ptr, mask_ptr,
+                   int(global_batch), grads_ptr, _ptr(self.metrics), _ptr(self.workspace), self.workspace.numel(), stream_ptr))
 
-    def _rainbow_adam_call(self, hp, grads_ptr, stream_ptr) -> None:
-        """``dmdqn_adam_apply_rainbow``: Adam on mu and sigma from the gradient block, and their target sync."""
-        N.check(self.lib.dmdqn_adam_apply_rainbow(C.byref(self.dims), C.byref(hp), C.byref(self.nets), C.byref(self.noisy_ptrs),
-                                                  self.num_atoms, grads_ptr, _ptr(self.workspace), self.workspace.numel(),
-                                                  stream_ptr))
+    def _adam_call(self, hp, grads_ptr, stream_ptr) -> None:
+        """Adam (and the target sync) from the gradient block: clipped when ``global_clipnorm`` is set (norms ->
+        ``grad_norms``), on mu and sigma for noisy and Rainbow networks."""
+        fn, mid, clipped = self._adam
+        clip = self.global_clipnorm
+        if fn is None:
+            fn, clipped = (self.lib.dmdqn_adam_apply, False) if clip is None else (self.lib.dmdqn_clip_adam_apply, True)
+        tail = [clip or 0.0, _ptr(self.grad_norms)] if clipped else []
+        N.check(fn(C.byref(self.dims), C.byref(hp), C.byref(self.nets), *mid, grads_ptr, *tail, _ptr(self.workspace),
+                   self.workspace.numel(), stream_ptr))
 
     def _learn_call(self, hp, draws_ptr, mask_ptr, stream_ptr) -> None:
-        """The learn step's native calls: ``dmdqn_learn``, or with ``global_clipnorm`` set the raw gradients
-        (``dmdqn_learn_grads``) followed by the clipped Adam step (``dmdqn_clip_adam_apply``, norms -> ``grad_norms``), or with
-        ``noisy`` set ``dmdqn_learn_grads_noisy`` followed by ``dmdqn_noisy_adam_apply``."""
-        ws, nws = _ptr(self.workspace), self.workspace.numel()
-        if self.rainbow:            # the gradient of the effective weights, then Adam on mu and sigma
-            self._rainbow_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
-            self._rainbow_adam_call(hp, _ptr(self.grads), stream_ptr)
-            return
-        if self.iqn:                # the IQN gradient, then Adam (clipped when global_clipnorm is set)
-            self._iqn_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
-            N.check(self.lib.dmdqn_adam_apply_iqn(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.n_cos,
-                                                  _ptr(self.grads), self.global_clipnorm or 0.0, _ptr(self.grad_norms), ws, nws,
-                                                  stream_ptr))
-            return
-        if self.dist_layout:        # the C51 / QR-DQN gradient, then Adam (clipped when global_clipnorm is set)
-            self._dist_grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
-            N.check(self.lib.dmdqn_adam_apply_dist(C.byref(self.dims), C.byref(hp), C.byref(self.nets), self.head_atoms,
-                                                   _ptr(self.grads), self.global_clipnorm or 0.0, _ptr(self.grad_norms), ws, nws,
-                                                   stream_ptr))
-            return
-        if self.noisy:          # gradient of the effective weights, then Adam on mu and sigma
-            N.check(self.lib.dmdqn_learn_grads_noisy(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                                     C.byref(self.noisy_ptrs), draws_ptr, mask_ptr, self.batch_size,
-                                                     _ptr(self.grads), _ptr(self.metrics), ws, nws, stream_ptr))
-            N.check(self.lib.dmdqn_noisy_adam_apply(C.byref(self.dims), C.byref(hp), C.byref(self.nets), C.byref(self.noisy_ptrs),
-                                                    _ptr(self.grads), ws, nws, stream_ptr))
-            return
-        if self.global_clipnorm is None:
+        """The learn step's native calls: ``dmdqn_learn``, or the gradient block (``_grads_call``) followed by ``_adam_call``."""
+        if self._fused_learn():
             N.check(self.lib.dmdqn_learn(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                         draws_ptr, mask_ptr, _ptr(self.metrics), ws, nws, stream_ptr))
+                                         draws_ptr, mask_ptr, _ptr(self.metrics), _ptr(self.workspace), self.workspace.numel(),
+                                         stream_ptr))
             return
-        N.check(self.lib.dmdqn_learn_grads(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
-                                           draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), _ptr(self.metrics), ws, nws,
-                                           stream_ptr))
-        N.check(self.lib.dmdqn_clip_adam_apply(C.byref(self.dims), C.byref(hp), C.byref(self.nets), _ptr(self.grads),
-                                               self.global_clipnorm, _ptr(self.grad_norms), ws, nws, stream_ptr))
+        self._grads_call(hp, draws_ptr, mask_ptr, self.batch_size, _ptr(self.grads), stream_ptr)
+        self._adam_call(hp, _ptr(self.grads), stream_ptr)
 
     @_on_device
     def learn(self, draws=None, mask=None, sample_mode: str | None = None) -> torch.Tensor:
@@ -892,10 +877,10 @@ class AgentGroup:
                 "metrics_host": torch.zeros((g, N.METRICS_STRIDE), dtype=torch.float32).pin_memory()}
 
     def _step_host_call(self, hp, sb, stream_ptr) -> None:
-        """``dmdqn_step_host``; with ``global_clipnorm`` set the same step from its parts on the same stream (the current
-        one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the clipped learn calls and the metrics D2H copy; the
-        same with ``noisy`` set and the noisy learn calls."""
-        if self.global_clipnorm is None and not self.noisy and not self.dist_layout and not self.iqn:
+        """``dmdqn_step_host``; where the learn step is two calls (``_learn_call``) the same step from its parts on the same
+        stream (the current one, ``stream_ptr``): the H2D copy of the block, ``dmdqn_push``, the learn calls and the metrics
+        D2H copy."""
+        if self._fused_learn():
             N.check(self.lib.dmdqn_step_host(C.byref(self.dims), C.byref(hp), C.byref(self.replay), C.byref(self.nets),
                                              C.byref(sb["desc"]), sb["host_block"].data_ptr(), sb["dev_block"].data_ptr(),
                                              _ptr(self.metrics), sb["metrics_host"].data_ptr(), _ptr(self.workspace),
@@ -1031,21 +1016,5 @@ class AgentGroup:
         """update_target_network (tau None, dqn_agent.py:382-384) / soft update (:389-399)."""
         mask_t = None if mask is None else self._dev(mask, torch.uint8)
         tau = -1.0 if tau is None else float(tau)
-        if self.rainbow:         # mu and sigma over the Rainbow stride
-            N.check(self.lib.dmdqn_sync_target_rainbow(C.byref(self.dims), C.byref(self.nets), C.byref(self.noisy_ptrs),
-                                                       self.num_atoms, _ptr(mask_t), tau, self._stream))
-            return
-        if self.iqn:
-            N.check(self.lib.dmdqn_sync_target_iqn(C.byref(self.dims), C.byref(self.nets), self.n_cos, _ptr(mask_t), tau,
-                                                   self._stream))
-            return
-        if self.dist_layout:
-            N.check(self.lib.dmdqn_sync_target_dist(C.byref(self.dims), C.byref(self.nets), self.head_atoms, _ptr(mask_t), tau,
-                                                    self._stream))
-            return
-        if self.noisy:           # mu and sigma
-            N.check(self.lib.dmdqn_sync_target_noisy(C.byref(self.dims), C.byref(self.nets), C.byref(self.noisy_ptrs),
-                                                     int(self.dueling), _ptr(mask_t), tau, self._stream))
-            return
-        sync = self.lib.dmdqn_sync_target_dueling if self.dueling else self.lib.dmdqn_sync_target
-        N.check(sync(C.byref(self.dims), C.byref(self.nets), _ptr(mask_t), tau, self._stream))
+        fn, mid = self._sync            # noisy and Rainbow networks: mu and sigma
+        N.check(fn(C.byref(self.dims), C.byref(self.nets), *mid, _ptr(mask_t), tau, self._stream))

@@ -221,8 +221,7 @@ class SharedParameterStep:
         if clip is not None and fused:
             raise ValueError("global_clipnorm is set: the fused peer-memory kernel (dmdqn_allreduce_adam) does not clip; "
                              "use fused=False (the NCCL all-reduce + dmdqn_clip_adam_apply path)")
-        rainbow = getattr(grp, "rainbow", False)
-        if rainbow and fused:
+        if getattr(grp, "rainbow", False) and fused:
             raise ValueError("rainbow=true: the fused peer-memory kernel (dmdqn_allreduce_adam) does not know the Rainbow layout "
                              "or sigma; use fused=False (the NCCL all-reduce + dmdqn_adam_apply_rainbow path)")
         if grp.noisy and fused:
@@ -257,21 +256,7 @@ class SharedParameterStep:
                 return out, grp.metrics
             d = grp.draw_words((1, grp.batch_size))
             with torch.cuda.device(grp.device):
-                if rainbow:
-                    grp._rainbow_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
-                elif grp.iqn:
-                    grp._iqn_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
-                elif grp.dist_layout:           # C51 or QR-DQN
-                    grp._dist_grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
-                elif grp.noisy:
-                    N.check(grp.lib.dmdqn_learn_grads_noisy(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay),
-                                                            C.byref(grp.nets), C.byref(grp.noisy_ptrs), _ptr(d), None,
-                                                            int(global_batch), _ptr(out), _ptr(grp.metrics), _ptr(grp.workspace),
-                                                            grp.workspace.numel(), grp._stream))
-                else:
-                    N.check(grp.lib.dmdqn_learn_grads(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.replay), C.byref(grp.nets),
-                                                      _ptr(d), None, int(global_batch), _ptr(out), _ptr(grp.metrics),
-                                                      _ptr(grp.workspace), grp.workspace.numel(), grp._stream))
+                grp._grads_call(grp.hp, _ptr(d), None, global_batch, _ptr(out), grp._stream)
             grp.learn_step_host += 1
             return out, grp.metrics
 
@@ -291,33 +276,9 @@ class SharedParameterStep:
             fused_begin(global_batch)
             return fused_finish()
 
-        def apply(g: torch.Tensor):
+        def apply(g: torch.Tensor):             # clipped (the norm of the all-reduced block) when global_clipnorm is set
             with torch.cuda.device(grp.device):
-                if rainbow:
-                    grp._rainbow_adam_call(grp.hp, _ptr(g), grp._stream)
-                    return
-                if grp.iqn:                     # clipped (the norm of the all-reduced block) when global_clipnorm is set
-                    N.check(grp.lib.dmdqn_adam_apply_iqn(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.n_cos,
-                                                         _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),
-                                                         grp.workspace.numel(), grp._stream))
-                    return
-                if grp.dist_layout:             # clipped (the norm of the all-reduced block) when global_clipnorm is set
-                    N.check(grp.lib.dmdqn_adam_apply_dist(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), grp.head_atoms,
-                                                          _ptr(g), clip or 0.0, _ptr(grp.grad_norms), _ptr(grp.workspace),
-                                                          grp.workspace.numel(), grp._stream))
-                    return
-                if clip is not None:            # the norm of the all-reduced block: the same scale on every replica
-                    N.check(grp.lib.dmdqn_clip_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g), clip,
-                                                          _ptr(grp.grad_norms), _ptr(grp.workspace), grp.workspace.numel(),
-                                                          grp._stream))
-                    return
-                if grp.noisy:
-                    N.check(grp.lib.dmdqn_noisy_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets),
-                                                           C.byref(grp.noisy_ptrs), _ptr(g), _ptr(grp.workspace),
-                                                           grp.workspace.numel(), grp._stream))
-                    return
-                N.check(grp.lib.dmdqn_adam_apply(C.byref(grp.dims), C.byref(grp.hp), C.byref(grp.nets), _ptr(g),
-                                                 _ptr(grp.workspace), grp.workspace.numel(), grp._stream))
+                grp._adam_call(grp.hp, _ptr(g), grp._stream)
         step = cls(local_grads, apply, grp.batch_size, group, local_ready=local_ready, flag_device=grp.device,
                    fused_apply=fused_apply if fused else None,
                    world=exchange.world if (exchange is not None and world == 1 and exchange.world > 1) else None)

@@ -387,12 +387,12 @@ def test_shared_parameters_nccl_path_and_two_simulated_ranks():
     for g in [one] + ranks:
         fill(g, 100, seed=31)
     idx = draw_words(np.random.default_rng(32), 1, 128)
-    one._iqn_grads_call(one.hp, idx.data_ptr(), None, 128, one.grads.data_ptr(), one._stream)
+    one._grads_call(one.hp, idx.data_ptr(), None, 128, one.grads.data_ptr(), one._stream)
     total = torch.zeros_like(one.grads)
     for r, g in enumerate(ranks):
         g.iqn_row_base = 64 * r
         part = idx[:, 64 * r:64 * r + 64].contiguous()
-        g._iqn_grads_call(g.hp, part.data_ptr(), None, 128, g.grads.data_ptr(), g._stream)
+        g._grads_call(g.hp, part.data_ptr(), None, 128, g.grads.data_ptr(), g._stream)
         total += g.grads
     torch.cuda.synchronize()
     for k, (x, y) in enumerate(zip(one.unpack(total[0]), one.unpack(one.grads[0]))):

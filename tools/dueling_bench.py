@@ -96,16 +96,16 @@ def stage_times(grp, draws, start):
     return {k: v / (draws.shape[0] - start) for k, v in tot.items()}
 
 
-def fold_kernel_us(grp, draws, start):
-    """Mean device time of fold_kernel over the learn sweeps, from torch.profiler (a pass of its own)."""
+def head_fold_kernel_us(grp, draws, start):
+    """Mean device time of head_fold_kernel over the learn sweeps, from torch.profiler (a pass of its own)."""
     from torch.profiler import ProfilerActivity, profile
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         for i in range(start, draws.shape[0]):
             grp.learn(draws[i])
         torch.cuda.synchronize()
-    times = [e.device_time for e in prof.events() if "fold_kernel" in e.name]          # us per launch
+    times = [e.device_time for e in prof.events() if "head_fold_kernel" in e.name]          # us per launch
     if not times:
-        raise RuntimeError("torch.profiler recorded no fold_kernel launch")
+        raise RuntimeError("torch.profiler recorded no head_fold_kernel launch")
     return {"median": statistics.median(times), "launches": len(times)}
 
 
@@ -140,7 +140,7 @@ def main():
         for k, g in g3.items():
             per_stage[k].append(stage_times(g, draws, args.warmup))
     per_stage = {k: {s: statistics.median(r[s] for r in v) for s in STAGES} for k, v in per_stage.items()}
-    fold = fold_kernel_us(g3["dueling"], draws, args.warmup)
+    fold = head_fold_kernel_us(g3["dueling"], draws, args.warmup)
     for g in g3.values():
         g.check_errors()
     precision = list(N.PRECISION)[g3["plain"].hp.precision]
@@ -180,7 +180,7 @@ def main():
         "stage_method": "each stage of dmdqn_learn_stages as its own call, CUDA events between the calls (no chaining, so "
                         "the stages add up to more than the chained sweep); median over the rounds of the mean per sweep",
         "fold_kernel_us_cfg3": fold,
-        "fold_method": "torch.profiler device time of fold_kernel in dueling learn sweeps (a pass of its own)",
+        "fold_method": "torch.profiler device time of head_fold_kernel in dueling learn sweeps (a pass of its own)",
         "fold_bytes_cfg3": 2 * 256 * (5 * 256 + 5 + 4 * 256 + 4) * 4,
         "cfg2_graph_sweep_us": cfg2,
         "cfg2_sweep_extra_us": cfg2["dueling"]["median"] - cfg2["plain"]["median"],

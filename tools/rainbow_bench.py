@@ -33,8 +33,8 @@ from tools.sample_bench import card  # noqa: E402
 D, A, ATOMS = 89, 4, 51
 CFG3 = dict(agents=256, batch=256, hidden=256, capacity=30000)
 CFG2 = dict(agents=16, batch=64, hidden=256, capacity=30000)
-RAINBOW_KERNELS = ("rainbow_noisy_fold_kernel", "rainbow_head_fold_kernel", "rainbow_target_kernel", "rainbow_online_kernel",
-                   "dist_wgrad_kernel", "rainbow_project_kernel", "rainbow_adam_apply_kernel")
+RAINBOW_KERNELS = ("noisy_fold_kernel", "head_fold_kernel", "rainbow_target_kernel", "rainbow_online_kernel",
+                   "dist_wgrad_kernel", "rainbow_project_kernel", "noisy_adam_apply_kernel")
 DIST_KERNELS = ("dist_target_kernel", "dist_online_kernel", "dist_wgrad_kernel", "adam_apply_kernel")
 
 
@@ -44,10 +44,10 @@ def hbm_bytes(grp):
     npad = grp.atom_stride
     rows, nh = h + 1, 4 * npad
     return {
-        "rainbow_noisy_fold_kernel": 2 * n * L.stride * 12,                       # per set: mu + sigma read, eff written
-        "rainbow_head_fold_kernel": 2 * n * rows * (nh + npad + nh) * 4,          # per set: W3 | b3 and Wv | bv read, W3e written
+        "noisy_fold_kernel": 2 * n * L.stride * 12,                               # per set: mu + sigma read, eff written
+        "head_fold_kernel": 2 * n * rows * (nh + npad + nh) * 4,                  # per set: W3 | b3 and Wv | bv read, W3e written
         "rainbow_project_kernel": n * rows * (2 * nh + npad) * 4,                 # W3 | b3 read and written, Wv | bv written
-        "rainbow_adam_apply_kernel": n * L.end * 52,                               # g; mu, m, v and sigma, m, v read and written
+        "noisy_adam_apply_kernel": n * L.end * 52,                                 # g; mu, m, v and sigma, m, v read and written
     }
 
 
